@@ -22,6 +22,10 @@ One JSON line on stdout (rank 0).  `value` = device-resident whole-job shapes/s;
 host-buffer C-ABI entry point (pinned host buffers, H2D + kernels + D2H every step); `roofline` = the pool+fuse
 kernel's algorithmic bytes / its CUDA-event duration vs the measured HBM peak; `cpu_baseline` = the reference's op
 sequence restated in torch-CPU, timed on this box's cores.
+
+--dump-outputs DIR (CUDA arm) writes what the last timed headline step returned on rank 0 as DIR/<name>.npy:
+S [B, D], x [B, V], xsum [V], scores [V] (float32) and bins [V] (float64).  The inputs come from fixed seeds, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -43,6 +47,7 @@ METRIC = "grouping+fusion shapes/s (12-view, D=2048)"
 UNIT = "shapes/s"
 CFG = dict(B=4096, V=12, D=2048, G=8, C_raw=1024, pool="max", empty_fill=1.0, score_reduce="batch")
 NSETS = 3                                                            # rotating input AND output sets (SURVEY.md 8d)
+DUMP_LIMIT = 64 << 20                                                # bytes written by one --dump-outputs, all arrays
 
 
 def bench_config(world, scaling):
@@ -66,6 +71,20 @@ def algorithmic_bytes(B, V, D, C, s):
     pool = B * (V * D * s + D * s)
     bwd = B * (D * s + V * D * s)
     return {"score": score, "pool_fwd": pool, "fwd": score + pool, "bwd": bwd, "fwd_bwd": score + pool + bwd}
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each array of {name: ndarray} as dirname/<name>.npy: floating arrays as float32 (float64 kept),
+    integer arrays as float64, which holds every int32 exactly.  Refuses more than DUMP_LIMIT bytes in all."""
+    import numpy as np
+    out = {name: a.astype(np.float64 if a.dtype == np.float64 or a.dtype.kind in "iub" else np.float32)
+           for name, a in arrays.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes (limit %d)" % (total, DUMP_LIMIT))
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -521,6 +540,12 @@ def run_cuda_arm(args):
     if sampler:
         sampler.start()
     ms_fwd = timed(k_fwd_batch, K, graph_fwd)
+    if args.dump_outputs and rank == 0:
+        # step i writes output set i % NSETS, in a graph replay or eagerly; later regions overwrite the sets
+        o = outs[(K - 1) % NSETS]
+        dump_outputs(args.dump_outputs, {"S": o["S"].cpu().numpy(), "x": o["x"].cpu().numpy(),
+                                         "xsum": o["xsum"].cpu().numpy(), "scores": o["sc1"].cpu().numpy(),
+                                         "bins": o["bins1"].cpu().numpy()})
     # view_score, fused (column sums + exchange + mean/score/bin), pool+fuse; the NCCL route is 5 launches + NCCL's
     fwd_launches = 3 if (world == 1 or comm is not None) else 4
 
@@ -884,9 +909,13 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: 4096 shapes per GPU (default, the contract's line); strong: 4096 shapes in total")
     ap.add_argument("--no-graph", action="store_true", help="time plain stream launches instead of a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed forward step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
     if args.steps < 1:
         raise SystemExit("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "cuda":
+        raise SystemExit("--dump-outputs applies to the CUDA arm only")
     if args.impl == "reference":
         return run_reference_arm(args)
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -113,7 +113,10 @@ def _worker(rank, world, port, tmp):
         dist.destroy_process_group()
 
 
-def test_world_size_2_gloo(tmp_path):
+def test_world_size_2_gloo(tmp_path, monkeypatch):
+    # the workers check the no-GPU behaviour: hide any device, or on a GPU box both ranks would share one and P2PComm
+    # would come up
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     port = _free_port()
     mp.spawn(_worker, args=(2, port, str(tmp_path)), nprocs=2, join=True)
     assert os.path.exists(tmp_path / "ok_0") and os.path.exists(tmp_path / "ok_1")
