@@ -18,6 +18,7 @@ Reference map (all in /root/reference):
 """
 from __future__ import annotations
 
+import collections
 import ctypes
 import math
 from typing import Optional, Sequence
@@ -184,14 +185,58 @@ class _Views:
         if self.V > C.MAX_VIEWS:
             raise ValueError("%s: at most %d views are supported, got %d" % (name, C.MAX_VIEWS, self.V))
 
+    @classmethod
+    def of(cls, tensors, lay, name):
+        """From what _view_args returns."""
+        return cls(tensors if lay == "list" else tensors[0], lay, name)
+
     def empty_like(self):
         """Fresh storage of the same layout (for dF)."""
-        if self.kind == "list":
-            out = [torch.empty_like(t) for t in self.keep]
-            v = _Views(out, None, "dF")
-            return out, v
-        out = torch.empty_like(self.tensor)
+        out = [torch.empty_like(t) for t in self.keep] if self.kind == "list" else torch.empty_like(self.tensor)
         return out, _Views(out, self.kind, "dF")
+
+
+def _view_args(x, layout):
+    """A view argument - the reference's list of V tensors, or one stacked tensor in `layout` - as (tensors, lay):
+    the tensors as a tuple (how they travel through autograd.Function.apply) and 'list', 'bvd' or 'vbd'."""
+    if isinstance(x, (list, tuple)):
+        return tuple(x), "list"
+    return (x,), (layout or "bvd")
+
+
+def _tie_mask(fv, pool, want):
+    """Storage for max pooling's tie mask (one bit per view and element: which views the backward routes to)."""
+    if not (want and pool == "max"):
+        return None
+    return torch.empty(((fv.V + 7) // 8, fv.B, fv.D), dtype=torch.uint8, device=fv.device)
+
+
+def _bin_rows(bins, fv):
+    """bins as the pooling kernels read them: int32 [1, V] or [B, V], and the row stride (0: one row for the batch)."""
+    if bins.dtype != torch.int32 or not bins.is_contiguous():
+        bins = bins.to(torch.int32).contiguous()
+    if bins.dim() == 1:
+        bins = bins[None]
+    return bins, (fv.V if (bins.shape[0] == fv.B and fv.B > 1) else 0)
+
+
+def _check_score_fc(W, b):
+    """The V Dense(1) score layers' kernel and bias."""
+    _require_cuda(W, "W"), _require_cuda(b, "b")
+    if W.dtype != torch.float32 or b.dtype != torch.float32:
+        raise TypeError("W and b must be float32")
+
+
+def _exchange_forms(exchange):
+    """A gvcnn_exchange_fn given as (fn, user) - fn a ctypes function (P2PComm.exchange, an EXCHANGE_FN callback)
+    or its address as an int or c_void_p (P2PComm.exchange_c) - as (address, callable, user): the address for the
+    C entry points, the callable for score_bin's staged path.  None (no exchange) gives three Nones."""
+    if exchange is None:
+        return None, None, None
+    fn, user = exchange
+    if isinstance(fn, (int, ctypes.c_void_p)):
+        return fn, C.EXCHANGE_FN(fn if isinstance(fn, int) else fn.value), user
+    return ctypes.cast(fn, ctypes.c_void_p), fn, user
 
 
 def raise_for_status(status: torch.Tensor, num_group: int):
@@ -283,9 +328,7 @@ def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulp
        with raise_for_status instead of synchronising every step); with check=False and no status given
        nothing is recorded.
     """
-    _require_cuda(W, "W"), _require_cuda(b, "b")
-    if W.dtype != torch.float32 or b.dtype != torch.float32:
-        raise TypeError("W and b must be float32")
+    _check_score_fc(W, b)
     Wc, bc = W.contiguous(), b.contiguous()
     rv, HW = _raw_views(R, layout, int(Wc.shape[-1]) if Wc.dim() == 2 else -1)
     Craw = rv.D // HW
@@ -328,18 +371,15 @@ def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulp
             buf = torch.empty((4, 1, rv.V), dtype=torch.int32, device=dev)
             x, scores = buf[0].view(torch.float32), buf[1].view(torch.float32)
             bins, flags = buf[2], buf[3]
+            ex_ptr, ex_fn, ex_user = _exchange_forms(exchange)
             if not want_bound and process_group is None:
                 # no order-sensitivity report asked for: column sums + [exchange] + mean / score / bin in ONE call
                 denom = rv.B if global_count is None else int(global_count)
                 if denom <= 0:
                     raise ValueError("score_reduce='batch' over an empty (global) batch")
-                fn, user = (None, None)
-                if exchange is not None:
-                    fn, user = exchange
-                    fn = ctypes.cast(fn, ctypes.c_void_p) if not isinstance(fn, (int, ctypes.c_void_p)) else fn
                 C.check(L.gvcnn_batch_mean_bin(_ptr(xb[0]), _ptr(sums[0]), _ptr(x), _ptr(scores), _ptr(bins), _ptr(flags),
                                                _ptr(status), rv.B, rv.V, num_group, int(multiplier or 0), edge_ulps,
-                                               int(clamp), denom, fn, user, _stream()), "gvcnn_batch_mean_bin")
+                                               int(clamp), denom, ex_ptr, ex_user, _stream()), "gvcnn_batch_mean_bin")
                 res = ScoreResult(x, scores, bins, flags, status, num_group)
                 if check:
                     res.check()
@@ -352,8 +392,7 @@ def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulp
                 sums.zero_()
             denom = rv.B if global_count is None else int(global_count)
             if exchange is not None:                                 # a gvcnn_exchange_fn (e.g. parallel.P2PComm)
-                fn, user = exchange
-                C.check(fn(user, _ptr(sums), nsum * rv.V, _stream()), "exchange")
+                C.check(ex_fn(ex_user, _ptr(sums), nsum * rv.V, _stream()), "exchange")
             elif process_group is not None:
                 import torch.distributed as dist
                 dist.all_reduce(sums[:nsum], group=process_group)
@@ -568,20 +607,22 @@ def group_weight(g_schemes):
 # --------------------------------------------------------------------------
 # pooling + fusion                                      nets/model.py:44-102
 # --------------------------------------------------------------------------
+# What a forward launch ending in pooling + fusion returns: S [B, D], the tie mask, the G pooled groups [G, B, D] (if
+# asked for), the status words, and the bins and group weights as the kernel read them, with their row strides (None, 0:
+# the kernel computes 1 + n_g) - everything the pooling backward needs.
+_Pooled = collections.namedtuple("_Pooled", "S mask P status bins bin_stride weights w_stride")
+
+
 def _pool_fuse_fwd(fv: _Views, bins: torch.Tensor, G: int, pool: str, empty_fill: float,
                    weights: Optional[torch.Tensor], want_mask: bool, want_groups: bool, want_status: bool = True,
-                   variant: int = 0):
+                   variant: int = 0) -> _Pooled:
     dev = fv.device
     dt = _dtype_code(fv.dtype)
-    if bins.dtype != torch.int32 or not bins.is_contiguous():
-        bins = bins.to(torch.int32).contiguous()
-    if bins.dim() == 1:
-        bins = bins[None]
+    bins, bin_stride = _bin_rows(bins, fv)
     if bins.shape[-1] != fv.V or bins.shape[0] not in (1, fv.B):
         raise ValueError("bins must be [V], [1, V] or [B, V] with V=%d, B=%d; got %s"
                          % (fv.V, fv.B, tuple(bins.shape)))
-    bin_stride = fv.V if (bins.shape[0] == fv.B and fv.B > 1) else 0
-    w_ptr, w_stride = None, 0
+    w_stride = 0
     if weights is not None:
         _require_cuda(weights, "group_weight")
         weights = weights.to(torch.float32).contiguous()
@@ -589,19 +630,17 @@ def _pool_fuse_fwd(fv: _Views, bins: torch.Tensor, G: int, pool: str, empty_fill
             weights = weights[None]
         if weights.shape[-1] != G or weights.shape[0] not in (1, fv.B):
             raise ValueError("group_weight must be [G] or [B, G]")
-        w_ptr, w_stride = _ptr(weights), (G if (weights.shape[0] == fv.B and fv.B > 1) else 0)
+        w_stride = G if (weights.shape[0] == fv.B and fv.B > 1) else 0
     S = torch.empty((fv.B, fv.D), dtype=fv.dtype, device=dev)
-    mask = None
-    if want_mask and pool == "max":
-        mask = torch.empty(((fv.V + 7) // 8, fv.B, fv.D), dtype=torch.uint8, device=dev)
+    mask = _tie_mask(fv, pool, want_mask)
     P = torch.empty((G, fv.B, fv.D), dtype=fv.dtype, device=dev) if want_groups else None
     status = _new_status(dev) if want_status else None
     with _on(dev):
-        C.check(C.lib().gvcnn_pool_fuse_fwd(fv.arg, _ptr(bins), bin_stride, w_ptr, w_stride, _ptr(S), _ptr(P),
+        C.check(C.lib().gvcnn_pool_fuse_fwd(fv.arg, _ptr(bins), bin_stride, _ptr(weights), w_stride, _ptr(S), _ptr(P),
                                             _ptr(mask), _ptr(status), fv.B, fv.V, fv.D, G, _pool_code(pool, variant),
                                             ctypes.c_float(empty_fill), fv.layout, dt, _stream()),
                 "gvcnn_pool_fuse_fwd")
-    return S, mask, P, status, bins, bin_stride, weights, w_stride
+    return _Pooled(S, mask, P, status, bins, bin_stride, weights, w_stride)
 
 
 def _pool_fuse_bwd(dS: torch.Tensor, fv_like: _Views, bins, bin_stride, weights, w_stride, mask, G, pool, variant=0):
@@ -616,49 +655,46 @@ def _pool_fuse_bwd(dS: torch.Tensor, fv_like: _Views, bins, bin_stride, weights,
 
 
 class _PoolFuseFn(torch.autograd.Function):
-    """S = fused view_pooling + group_fusion; backward = TF autodiff of
-    nets/model.py:62-100 (dF only: no gradient reaches scores / weights,
-    train.py:127-128, utils/train_utils.py:203-206)."""
+    """S from `launch(fv, want_mask)` -> (_Pooled, extra outputs): pooling + fusion, on its own or after score + bin
+    in the same call into the library; backward = TF autodiff of nets/model.py:62-100 (dF only: no gradient reaches
+    scores / weights, train.py:127-128, utils/train_utils.py:203-206).  The extra outputs are non-differentiable."""
 
     @staticmethod
-    def forward(ctx, bins, weights, G, pool, empty_fill, layout, want_status, variant, *views):
-        is_list = layout == "list"
-        fv = _Views(list(views) if is_list else views[0], None if is_list else layout, "F")
-        need_grad = any(v.requires_grad for v in views)
-        S, mask, _, status, bins_c, bstride, w_c, wstride = _pool_fuse_fwd(
-            fv, bins, G, pool, empty_fill, weights, want_mask=need_grad, want_groups=False,
-            want_status=want_status, variant=variant)
+    def forward(ctx, launch, G, pool, variant, f_lay, *f_t):
+        fv = _Views.of(f_t, f_lay, "F")
+        out, extras = launch(fv, True)
         ctx.fv, ctx.G, ctx.pool, ctx.variant = fv, G, pool, variant
-        ctx.bstride, ctx.wstride = bstride, wstride
-        ctx.save_for_backward(bins_c, mask if mask is not None else torch.empty(0, device=S.device),
-                              w_c if w_c is not None else torch.empty(0, device=S.device))
-        if status is None:
-            status = torch.empty(0, dtype=torch.int32, device=S.device)
-        ctx.mark_non_differentiable(status)
-        return S.reshape(fv.view_shape), status
+        ctx.bin_stride, ctx.w_stride = out.bin_stride, out.w_stride
+        ctx.save_for_backward(out.bins, out.weights, out.mask)
+        ctx.mark_non_differentiable(*[t for t in extras if t is not None])
+        return (out.S.reshape(fv.view_shape),) + extras
 
     @staticmethod
-    def backward(ctx, dS, _dstatus):
-        bins_c, mask, w_c = ctx.saved_tensors
-        mask = mask if mask.numel() else None
-        w_c = w_c if w_c.numel() else None
+    def backward(ctx, dS, *_unused):
+        bins, weights, mask = ctx.saved_tensors
         fv = ctx.fv
-        out = _pool_fuse_bwd(dS.reshape(fv.B, fv.D), fv, bins_c, ctx.bstride, w_c, ctx.wstride, mask,
+        # bins may hold the raw out-of-range value (clamp=False); the backward kernel clamps like the forward did
+        out = _pool_fuse_bwd(dS.reshape(fv.B, fv.D), fv, bins, ctx.bin_stride, weights, ctx.w_stride, mask,
                              ctx.G, ctx.pool, ctx.variant)
-        grads = tuple(out) if isinstance(out, list) else (out,)
-        return (None,) * 8 + grads
+        return (None,) * 5 + (tuple(out) if isinstance(out, list) else (out,))
 
 
-def _run_pool_fuse(views, lay, bins, weights, G, pool, empty_fill, want_status, variant=0):
-    """Forward through autograd only when a gradient can be asked for; otherwise straight into the library
-    (saves the autograd.Function bookkeeping on the inference path)."""
-    if torch.is_grad_enabled() and any(v.requires_grad for v in views):
-        S, status = _PoolFuseFn.apply(bins, weights, G, pool, empty_fill, lay, want_status, variant, *views)
-        return S, (status if status.numel() else None)
-    fv = _Views(list(views) if lay == "list" else views[0], None if lay == "list" else lay, "F")
-    S, _, _, status, _, _, _, _ = _pool_fuse_fwd(fv, bins, G, pool, empty_fill, weights, want_mask=False,
-                                                 want_groups=False, want_status=want_status, variant=variant)
-    return S.reshape(fv.view_shape), status
+def _run_launch(launch, f_t, f_lay, G, pool, variant):
+    """(S in the shape of one view,) + the launch's extra outputs.  Through autograd only when a gradient can be asked for;
+    otherwise straight into the library (saves the autograd.Function bookkeeping on the inference path)."""
+    if torch.is_grad_enabled() and any(t.requires_grad for t in f_t):
+        return _PoolFuseFn.apply(launch, G, pool, variant, f_lay, *f_t)
+    fv = _Views.of(f_t, f_lay, "F")
+    out, extras = launch(fv, False)
+    return (out.S.reshape(fv.view_shape),) + extras
+
+
+def _run_pool_fuse(f_t, f_lay, bins, weights, G, pool, empty_fill, want_status, variant=0):
+    """Pooling + fusion from a bin map: (S, status)."""
+    def launch(fv, want_mask):
+        out = _pool_fuse_fwd(fv, bins, G, pool, empty_fill, weights, want_mask, False, want_status, variant)
+        return out, (out.status,)
+    return _run_launch(launch, f_t, f_lay, G, pool, variant)
 
 
 def pool_fuse(final_view_descriptors, bins, num_group, pool="max", empty_fill=1.0, layout=None,
@@ -671,10 +707,7 @@ def pool_fuse(final_view_descriptors, bins, num_group, pool="max", empty_fill=1.
     Returns the shape descriptor with the shape of one view, differentiable
     w.r.t. the view descriptors.
     """
-    if isinstance(final_view_descriptors, (list, tuple)):
-        views, lay = tuple(final_view_descriptors), "list"
-    else:
-        views, lay = (final_view_descriptors,), (layout or "bvd")
+    views, lay = _view_args(final_view_descriptors, layout)
     _require_cuda(bins, "bins")
     S, status = _run_pool_fuse(views, lay, bins, group_weight, num_group, pool, empty_fill, check, _variant)
     if check:
@@ -687,22 +720,15 @@ class _PoolFuseGapFn(torch.autograd.Function):
     writing the fused map: [B, C] out; backward takes the [B, C] gradient."""
 
     @staticmethod
-    def forward(ctx, bins, G, pool, empty_fill, layout, HW, Cch, n_views, *views):
+    def forward(ctx, bins, G, pool, empty_fill, layout, HW, Cch, *views):
         L = C.lib()
-        is_list = layout == "list"
-        fv = _Views(list(views) if is_list else views[0], None if is_list else layout, "F")
+        fv = _Views.of(views, layout, "F")
         dev = fv.device
         dt = _dtype_code(fv.dtype)
-        bins_c = bins.to(torch.int32).contiguous()
-        if bins_c.dim() == 1:
-            bins_c = bins_c[None]
-        bstride = fv.V if (bins_c.shape[0] == fv.B and fv.B > 1) else 0
-        need_grad = any(v.requires_grad for v in views)
+        bins_c, bstride = _bin_rows(bins, fv)
         out = torch.empty((fv.B, Cch), dtype=fv.dtype, device=dev)
-        mask = None
-        if need_grad and pool == "max":
-            mask = torch.empty(((fv.V + 7) // 8, fv.B, fv.D), dtype=torch.uint8, device=dev)
-        status = torch.zeros(C.STATUS_WORDS, dtype=torch.int32, device=dev)
+        mask = _tie_mask(fv, pool, any(v.requires_grad for v in views))
+        status = _new_status(dev)
         ws_bytes = L.gvcnn_pool_fuse_gap_workspace_bytes(fv.B, Cch, HW, dt)
         ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
         with _on(dev):
@@ -711,25 +737,24 @@ class _PoolFuseGapFn(torch.autograd.Function):
                                               ctypes.c_float(empty_fill), fv.layout, dt, _stream()),
                     "gvcnn_pool_fuse_gap_fwd")
         ctx.fv, ctx.G, ctx.pool, ctx.HW, ctx.Cch, ctx.bstride = fv, G, pool, HW, Cch, bstride
-        ctx.save_for_backward(bins_c, mask if mask is not None else torch.empty(0, device=dev))
+        ctx.save_for_backward(bins_c, mask)
         ctx.mark_non_differentiable(status)
         return out, status
 
     @staticmethod
     def backward(ctx, dOut, _dstatus):
         bins_c, mask = ctx.saved_tensors
-        mask = mask if mask.numel() else None
         fv = ctx.fv
         dOut = dOut.contiguous()
         out, gv = fv.empty_like()
-        status = torch.zeros(C.STATUS_WORDS, dtype=torch.int32, device=dOut.device)
+        status = _new_status(dOut.device)
         with _on(dOut.device):
             C.check(C.lib().gvcnn_pool_fuse_gap_bwd(_ptr(dOut), _ptr(bins_c), ctx.bstride, _ptr(mask), gv.arg,
                                                     _ptr(status), gv.B, gv.V, ctx.HW, ctx.Cch, ctx.G, _POOL[ctx.pool],
                                                     gv.layout, _dtype_code(gv.dtype), _stream()),
                     "gvcnn_pool_fuse_gap_bwd")
         grads = tuple(out) if isinstance(out, list) else (out,)
-        return (None,) * 8 + grads
+        return (None,) * 7 + grads
 
 
 def pool_fuse_gap(final_view_descriptors, bins, num_group, pool="max", empty_fill=1.0, layout=None):
@@ -738,21 +763,16 @@ def pool_fuse_gap(final_view_descriptors, bins, num_group, pool="max", empty_fil
     the pooled shape descriptor [N, C].  The fused map is never written.  Shapes the specialised kernel does
     not cover (see gvcnn_pool_fuse_gap_fwd) run pool_fuse and average afterwards - same result up to the
     float32 rounding of the mean."""
-    if isinstance(final_view_descriptors, (list, tuple)):
-        views, lay = tuple(final_view_descriptors), "list"
-        shp = tuple(views[0].shape)
-        spatial = shp[1:-1]
-    else:
-        views, lay = (final_view_descriptors,), (layout or "bvd")
-        shp = tuple(final_view_descriptors.shape)
-        spatial = shp[2:-1]
+    views, lay = _view_args(final_view_descriptors, layout)
+    shp = tuple(views[0].shape)
+    spatial = shp[1:-1] if lay == "list" else shp[2:-1]
     if len(shp) < 3:
         raise ValueError("pool_fuse_gap expects channel-last maps, e.g. [N, h, w, C] per view")
     Cch = shp[-1]
     HW = int(math.prod(spatial)) if len(spatial) else 1
     _require_cuda(bins, "bins")
     try:
-        out, _ = _PoolFuseGapFn.apply(bins, num_group, pool, empty_fill, lay, HW, Cch, len(views), *views)
+        out, _ = _PoolFuseGapFn.apply(bins, num_group, pool, empty_fill, lay, HW, Cch, *views)
         return out
     except C.GvcnnError as e:
         if e.code != C.E_UNSUPPORTED:
@@ -780,10 +800,9 @@ class GroupDescriptors(dict):
     def _materialise(self):
         if self._done:
             return
-        fv = _Views(list(self._views) if self._layout == "list" else self._views[0],
-                    None if self._layout == "list" else self._layout, "F")
-        _, _, P, _, _, _, _, _ = _pool_fuse_fwd(fv, self._bins, self._G, self._pool, self._fill, None,
-                                                want_mask=False, want_groups=True, want_status=False)
+        fv = _Views.of(self._views, self._layout, "F")
+        P = _pool_fuse_fwd(fv, self._bins, self._G, self._pool, self._fill, None, want_mask=False, want_groups=True,
+                           want_status=False).P
         for g in range(self._G):
             dict.__setitem__(self, g, P[g].reshape(fv.view_shape))
         self._done = True
@@ -852,10 +871,7 @@ def view_pooling(final_view_descriptors, group_scheme, pool="max", empty_fill=1.
     model.py behaviour (:63,:72); pool='mean', empty_fill=0.0 is unit_test.py's.
     Returns a GroupDescriptors dict {g: pooled descriptor}.
     """
-    if isinstance(final_view_descriptors, (list, tuple)):
-        views, lay = tuple(final_view_descriptors), "list"
-    else:
-        views, lay = (final_view_descriptors,), (layout or "bvd")
+    views, lay = _view_args(final_view_descriptors, layout)
     if len(views) == 0:
         raise ValueError("final_view_descriptors: empty view list")
     _require_cuda(views[0], "final_view_descriptors")
@@ -924,26 +940,44 @@ def basic_pool(final_view_descriptors, layout=None):
                      group_weight=w)
 
 
-def _fused_fwd(W, b, G, pool, empty_fill, rv, fv, edge_ulps, clamp, want_mask, status, variant):
-    """gvcnn_grouping_fusion_fwd: score + bin, then pool + fuse, chained on the device."""
+def _grouping_fusion_fwd(rv, fv, want_mask, W, b, G, pool, empty_fill, edge_ulps, clamp, status, variant, literal):
+    """Score + bin, then pool + fuse, chained on the device in one call into the library (PDL, no host hop):
+    gvcnn_grouping_fusion_fwd per shape, or - `literal` = (multiplier, global_count, exchange address, user) -
+    gvcnn_grouping_fusion_batch_fwd (x -> column sums -> [exchange] -> mean -> one bin row -> pool + fuse).
+    Extra outputs: (x, scores, bins, flags); x is the batch-mean row in the literal mode."""
     L = C.lib()
     if (rv.B, rv.V) != (fv.B, fv.V) or rv.dtype != fv.dtype:
         raise ValueError("raw and final view descriptors must agree in batch, views and dtype")
     dev = fv.device
     Wc, bc = W.contiguous(), b.contiguous()
-    buf = torch.empty((4, fv.B, fv.V), dtype=torch.int32, device=dev)      # x, scores, bins, flags: one allocation
-    x, scores, bins, flags = buf[0].view(torch.float32), buf[1].view(torch.float32), buf[2], buf[3]
+    if literal is None:
+        buf = torch.empty((4, fv.B, fv.V), dtype=torch.int32, device=dev)      # x, scores, bins, flags: one allocation
+        x, scores, bins, flags = buf[0].view(torch.float32), buf[1].view(torch.float32), buf[2], buf[3]
+    else:
+        xb = torch.empty((max(fv.B, 1), fv.V), dtype=torch.float32, device=dev)
+        buf = torch.empty((5, 1, fv.V), dtype=torch.int32, device=dev)           # xsum, x_mean, scores, bins, flags
+        xsum, x, scores = (buf[i].view(torch.float32) for i in range(3))
+        bins, flags = buf[3], buf[4]
     S = torch.empty((fv.B, fv.D), dtype=fv.dtype, device=dev)
-    mask = None
-    if want_mask and pool == "max":
-        mask = torch.empty(((fv.V + 7) // 8, fv.B, fv.D), dtype=torch.uint8, device=dev)
+    mask = _tie_mask(fv, pool, want_mask)
     with _on(dev):
-        C.check(L.gvcnn_grouping_fusion_fwd(rv.arg, _ptr(Wc), _ptr(bc), fv.arg, _ptr(x), _ptr(scores), _ptr(bins),
-                                            _ptr(flags), _ptr(S), _ptr(mask), _ptr(status), fv.B, fv.V, rv.D, fv.D,
-                                            G, _pool_code(pool, variant), ctypes.c_float(empty_fill), rv.layout,
-                                            fv.layout, _dtype_code(fv.dtype), edge_ulps, int(clamp), _stream()),
-                "gvcnn_grouping_fusion_fwd")
-    return S, x, scores, bins, flags, mask
+        if literal is None:
+            C.check(L.gvcnn_grouping_fusion_fwd(rv.arg, _ptr(Wc), _ptr(bc), fv.arg, _ptr(x), _ptr(scores), _ptr(bins),
+                                                _ptr(flags), _ptr(S), _ptr(mask), _ptr(status), fv.B, fv.V, rv.D, fv.D,
+                                                G, _pool_code(pool, variant), ctypes.c_float(empty_fill), rv.layout,
+                                                fv.layout, _dtype_code(fv.dtype), edge_ulps, int(clamp), _stream()),
+                    "gvcnn_grouping_fusion_fwd")
+        else:
+            multiplier, global_count, ex_ptr, ex_user = literal
+            C.check(L.gvcnn_grouping_fusion_batch_fwd(rv.arg, _ptr(Wc), _ptr(bc), fv.arg, _ptr(xb), _ptr(xsum), _ptr(x),
+                                                      _ptr(scores), _ptr(bins), _ptr(flags), _ptr(S), _ptr(mask),
+                                                      _ptr(status), fv.B, fv.V, rv.D, fv.D, G, int(multiplier or 0),
+                                                      _pool_code(pool, variant), ctypes.c_float(empty_fill), rv.layout,
+                                                      fv.layout, _dtype_code(fv.dtype), edge_ulps, int(clamp),
+                                                      int(global_count), ex_ptr, ex_user, _stream()),
+                    "gvcnn_grouping_fusion_batch_fwd")
+    bin_stride = fv.V if (literal is None and fv.B > 1) else 0
+    return _Pooled(S, mask, None, status, bins, bin_stride, None, 0), (x, scores, bins, flags)
 
 
 def _is_raw_maps(raw, W, layout):
@@ -957,56 +991,19 @@ def _is_raw_maps(raw, W, layout):
     return t.dim() > lead + 1 and t.shape[-1] == W.shape[1]
 
 
-_EXCHANGE_PROTO = ctypes.CFUNCTYPE(ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p)
-
-
-def _callable_exchange(exchange):
-    """(function pointer, user) as the C entry points take it -> (callable, user) as score_bin calls it."""
-    fn, user = exchange
-    if isinstance(fn, ctypes.c_void_p):
-        fn = _EXCHANGE_PROTO(fn.value)
-    return fn, user
-
-
-class _FusedFwdFn(torch.autograd.Function):
-    """Per-shape scores + bins + pooling + fusion through gvcnn_grouping_fusion_fwd (two launches chained
-    with programmatic dependent launch, no host hop); backward = the pooling/fusion backward (dF only, as
-    in the reference)."""
-
-    @staticmethod
-    def forward(ctx, W, b, G, pool, empty_fill, f_layout, r_layout, n_r, edge_ulps, clamp, status, variant, *tensors):
-        r_t, f_t = tensors[:n_r], tensors[n_r:]
-        rv = _Views(list(r_t) if r_layout == "list" else r_t[0], None if r_layout == "list" else r_layout, "R")
-        fv = _Views(list(f_t) if f_layout == "list" else f_t[0], None if f_layout == "list" else f_layout, "F")
-        need_grad = any(t.requires_grad for t in f_t)
-        S, x, scores, bins, flags, mask = _fused_fwd(W, b, G, pool, empty_fill, rv, fv, edge_ulps, clamp, need_grad,
-                                                     status, variant)
-        ctx.fv, ctx.G, ctx.pool, ctx.n_r, ctx.variant = fv, G, pool, n_r, variant
-        ctx.save_for_backward(bins, mask if mask is not None else torch.empty(0, device=S.device))
-        ctx.mark_non_differentiable(x, scores, bins, flags)
-        return S.reshape(fv.view_shape), x, scores, bins, flags
-
-    @staticmethod
-    def backward(ctx, dS, *_unused):
-        bins, mask = ctx.saved_tensors
-        mask = mask if mask.numel() else None
-        fv = ctx.fv
-        # bins may hold the raw out-of-range value (clamp=False); the backward kernel clamps like the forward did
-        out = _pool_fuse_bwd(dS.reshape(fv.B, fv.D), fv, bins, fv.V if fv.B > 1 else 0, None, 0, mask, ctx.G, ctx.pool,
-                             ctx.variant)
-        gf = tuple(out) if isinstance(out, list) else (out,)
-        return (None,) * 12 + (None,) * ctx.n_r + gf
-
-
 def grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_group, pool="max",
                     empty_fill=1.0, score_reduce="shape", layout=None, clamp=False, check=False,
                     process_group=None, edge_ulps=4, status=None, multiplier=None, exchange=None,
                     global_count=None, _variant=0):
     """The whole hot path with no host hop (replaces the partial_run split of
-    train.py:264-288): per-shape mode is one call into the library (score + bin,
-    then pool + fuse, chained on the device); the literal batch-mean mode needs
-    the cross-shape mean first and runs the stages separately.
+    train.py:264-288), one call into the library in either mode: per shape, score + bin
+    then pool + fuse, chained on the device; in the literal batch-mean mode, x -> column
+    sums -> [exchange] -> mean -> one bin row -> pool + fuse.
     Returns (shape_descriptor, ScoreResult).
+
+    exchange: a gvcnn_exchange_fn (fn, user) - P2PComm.exchange or .exchange_c - carrying the V column sums across
+    the ranks; without it, a ``process_group``'s torch.distributed does (called back from inside the library, in
+    stream order).
 
     check=True turns out-of-range / NaN scores into the reference's IndexError / ValueError right away (one
     16-byte device->host read per call, i.e. a synchronisation); the default records nothing.  For a training
@@ -1020,143 +1017,43 @@ def grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_grou
         # (gvcnn_gap_score_bin_fwd); pooling + fusion follow on the stream, chained with programmatic dependent launch
         sr = score_bin(raw_view_descriptors, W, b, num_group, score_reduce=score_reduce, layout=layout,
                        edge_ulps=edge_ulps, clamp=clamp, check=check, process_group=process_group, status=status,
-                       multiplier=multiplier, exchange=(None if exchange is None else _callable_exchange(exchange)),
-                       global_count=global_count)
+                       multiplier=multiplier, exchange=exchange, global_count=global_count)
         S = pool_fuse(final_view_descriptors, sr.bins, num_group, pool=pool, empty_fill=empty_fill, layout=layout,
                       _variant=_variant)
         return S, sr
     if score_reduce == "shape":
         if multiplier not in (None, num_group):
             raise ValueError("multiplier is only selectable with score_reduce='batch' or through group_scheme")
-        if isinstance(raw_view_descriptors, (list, tuple)):
-            r_t, r_lay = tuple(raw_view_descriptors), "list"
-        else:
-            r_t, r_lay = (raw_view_descriptors,), (layout or "bvd")
-        if isinstance(final_view_descriptors, (list, tuple)):
-            f_t, f_lay = tuple(final_view_descriptors), "list"
-        else:
-            f_t, f_lay = (final_view_descriptors,), (layout or "bvd")
-        _require_cuda(W, "W"), _require_cuda(b, "b")
-        if W.dtype != torch.float32 or b.dtype != torch.float32:
-            raise TypeError("W and b must be float32")
-        if torch.is_grad_enabled() and any(t.requires_grad for t in f_t):
-            S, x, scores, bins, flags = _FusedFwdFn.apply(W, b, num_group, pool, empty_fill, f_lay, r_lay, len(r_t),
-                                                          edge_ulps, clamp, status, _variant, *r_t, *f_t)
-        else:
-            rv = _Views(list(r_t) if r_lay == "list" else r_t[0], None if r_lay == "list" else r_lay, "R")
-            fv = _Views(list(f_t) if f_lay == "list" else f_t[0], None if f_lay == "list" else f_lay, "F")
-            S, x, scores, bins, flags, _ = _fused_fwd(W, b, num_group, pool, empty_fill, rv, fv, edge_ulps, clamp,
-                                                      False, status, _variant)
-            S = S.reshape(fv.view_shape)
-        sr = ScoreResult(x, scores, bins, flags, status, num_group)
-        if check:
-            sr.check()
-        return S, sr
-    if score_reduce != "batch":
+    elif score_reduce != "batch":
         raise ValueError("score_reduce must be 'shape' or 'batch'")
-    return _grouping_fusion_batch(raw_view_descriptors, W, b, final_view_descriptors, num_group, pool, empty_fill,
-                                  layout, clamp, check, process_group, edge_ulps, status, multiplier, exchange,
-                                  global_count, _variant)
+    r_t, r_lay = _view_args(raw_view_descriptors, layout)
+    f_t, f_lay = _view_args(final_view_descriptors, layout)
+    _check_score_fc(W, b)
+    literal, keep = None, None
+    if score_reduce == "batch":
+        B_local = r_t[0].shape[0] if r_lay in ("list", "bvd") else r_t[0].shape[1]
+        if exchange is None and process_group is not None:
+            cb, keep = make_exchange(process_group)
+            exchange = (cb, None)
+        ex_ptr, _, ex_user = _exchange_forms(exchange)
+        if global_count is None:
+            global_count = B_local
+            if process_group is not None:
+                import torch.distributed as dist
+                cnt = torch.tensor([B_local], dtype=torch.int64, device=W.device)
+                dist.all_reduce(cnt, group=process_group)
+                global_count = int(cnt.item())
+        if global_count <= 0:
+            raise ValueError("score_reduce='batch' over an empty (global) batch")
+        literal = (multiplier, global_count, ex_ptr, ex_user)
+    rv = _Views.of(r_t, r_lay, "R")
 
-
-class _BatchFwdFn(torch.autograd.Function):
-    """Reference-literal forward (one scheme per batch) through gvcnn_grouping_fusion_batch_fwd; backward = the
-    pooling/fusion backward with the shared bin row."""
-
-    @staticmethod
-    def forward(ctx, W, b, G, pool, empty_fill, f_layout, r_layout, n_r, edge_ulps, clamp, status, variant, multiplier,
-                global_count, exchange_c, *tensors):
-        r_t, f_t = tensors[:n_r], tensors[n_r:]
-        rv = _Views(list(r_t) if r_layout == "list" else r_t[0], None if r_layout == "list" else r_layout, "R")
-        fv = _Views(list(f_t) if f_layout == "list" else f_t[0], None if f_layout == "list" else f_layout, "F")
-        need_grad = any(t.requires_grad for t in f_t)
-        S, xm, scores, bins, flags, mask = _batch_fwd(W, b, G, pool, empty_fill, rv, fv, edge_ulps, clamp, need_grad,
-                                                      status, variant, multiplier, global_count, exchange_c)
-        ctx.fv, ctx.G, ctx.pool, ctx.n_r, ctx.variant = fv, G, pool, n_r, variant
-        ctx.save_for_backward(bins, mask if mask is not None else torch.empty(0, device=S.device))
-        ctx.mark_non_differentiable(xm, scores, bins, flags)
-        return S.reshape(fv.view_shape), xm, scores, bins, flags
-
-    @staticmethod
-    def backward(ctx, dS, *_unused):
-        bins, mask = ctx.saved_tensors
-        mask = mask if mask.numel() else None
-        fv = ctx.fv
-        out = _pool_fuse_bwd(dS.reshape(fv.B, fv.D), fv, bins, 0, None, 0, mask, ctx.G, ctx.pool, ctx.variant)
-        gf = tuple(out) if isinstance(out, list) else (out,)
-        return (None,) * 15 + (None,) * ctx.n_r + gf
-
-
-def _batch_fwd(W, b, G, pool, empty_fill, rv, fv, edge_ulps, clamp, want_mask, status, variant, multiplier,
-               global_count, exchange_c):
-    L = C.lib()
-    if (rv.B, rv.V) != (fv.B, fv.V) or rv.dtype != fv.dtype:
-        raise ValueError("raw and final view descriptors must agree in batch, views and dtype")
-    dev = fv.device
-    Wc, bc = W.contiguous(), b.contiguous()
-    xb = torch.empty((max(fv.B, 1), fv.V), dtype=torch.float32, device=dev)
-    buf = torch.empty((5, 1, fv.V), dtype=torch.int32, device=dev)           # xsum, x_mean, scores, bins, flags
-    xsum, xm, scores = (buf[i].view(torch.float32) for i in range(3))
-    bins, flags = buf[3], buf[4]
-    S = torch.empty((fv.B, fv.D), dtype=fv.dtype, device=dev)
-    mask = None
-    if want_mask and pool == "max":
-        mask = torch.empty(((fv.V + 7) // 8, fv.B, fv.D), dtype=torch.uint8, device=dev)
-    fn, user = exchange_c if exchange_c is not None else (None, None)
-    with _on(dev):
-        C.check(L.gvcnn_grouping_fusion_batch_fwd(rv.arg, _ptr(Wc), _ptr(bc), fv.arg, _ptr(xb), _ptr(xsum), _ptr(xm),
-                                                  _ptr(scores), _ptr(bins), _ptr(flags), _ptr(S), _ptr(mask),
-                                                  _ptr(status), fv.B, fv.V, rv.D, fv.D, G, int(multiplier or 0),
-                                                  _pool_code(pool, variant), ctypes.c_float(empty_fill), rv.layout,
-                                                  fv.layout, _dtype_code(fv.dtype), edge_ulps, int(clamp),
-                                                  int(global_count), fn, user, _stream()),
-                "gvcnn_grouping_fusion_batch_fwd")
-    return S, xm, scores, bins, flags, mask
-
-
-def _grouping_fusion_batch(raw_view_descriptors, W, b, final_view_descriptors, num_group, pool, empty_fill, layout,
-                           clamp, check, process_group, edge_ulps, status, multiplier, exchange, global_count, variant):
-    """score_reduce='batch': ONE call into the library (x -> column sums -> [exchange] -> mean -> one bin row ->
-    pool + fuse, PDL-chained).  `exchange`: a P2PComm.exchange_c pair, or None with `process_group` given, in which
-    case torch.distributed carries the V sums (called back from inside the library, in stream order)."""
-    if isinstance(raw_view_descriptors, (list, tuple)):
-        r_t, r_lay = tuple(raw_view_descriptors), "list"
-    else:
-        r_t, r_lay = (raw_view_descriptors,), (layout or "bvd")
-    if isinstance(final_view_descriptors, (list, tuple)):
-        f_t, f_lay = tuple(final_view_descriptors), "list"
-    else:
-        f_t, f_lay = (final_view_descriptors,), (layout or "bvd")
-    _require_cuda(W, "W"), _require_cuda(b, "b")
-    if W.dtype != torch.float32 or b.dtype != torch.float32:
-        raise TypeError("W and b must be float32")
-    B_local = r_t[0].shape[0] if r_lay in ("list", "bvd") else r_t[0].shape[1]
-    keep = None
-    exchange_c = exchange
-    if exchange_c is None and process_group is not None:
-        cb, keep = make_exchange(process_group)
-        exchange_c = (ctypes.cast(cb, ctypes.c_void_p), None)
-    if global_count is None:
-        global_count = B_local
-        if process_group is not None:
-            import torch.distributed as dist
-            cnt = torch.tensor([B_local], dtype=torch.int64, device=W.device)
-            dist.all_reduce(cnt, group=process_group)
-            global_count = int(cnt.item())
-    if global_count <= 0:
-        raise ValueError("score_reduce='batch' over an empty (global) batch")
-    if torch.is_grad_enabled() and any(t.requires_grad for t in f_t):
-        S, xm, scores, bins, flags = _BatchFwdFn.apply(W, b, num_group, pool, empty_fill, f_lay, r_lay, len(r_t),
-                                                       edge_ulps, clamp, status, variant, multiplier, global_count,
-                                                       exchange_c, *r_t, *f_t)
-    else:
-        rv = _Views(list(r_t) if r_lay == "list" else r_t[0], None if r_lay == "list" else r_lay, "R")
-        fv = _Views(list(f_t) if f_lay == "list" else f_t[0], None if f_lay == "list" else f_lay, "F")
-        S, xm, scores, bins, flags, _ = _batch_fwd(W, b, num_group, pool, empty_fill, rv, fv, edge_ulps, clamp, False,
-                                                   status, variant, multiplier, global_count, exchange_c)
-        S = S.reshape(fv.view_shape)
+    def launch(fv, want_mask):
+        return _grouping_fusion_fwd(rv, fv, want_mask, W, b, num_group, pool, empty_fill, edge_ulps, clamp, status,
+                                    _variant, literal)
+    S, x, scores, bins, flags = _run_launch(launch, f_t, f_lay, num_group, pool, _variant)
     del keep
-    sr = ScoreResult(xm, scores, bins, flags, status, num_group)
+    sr = ScoreResult(x, scores, bins, flags, status, num_group)
     if check:
         sr.check()
     return S, sr
@@ -1175,35 +1072,30 @@ class _PaperModeFn(torch.autograd.Function):
     def forward(ctx, W, b, G, pool, f_layout, r_layout, n_r, status, *tensors):
         L = C.lib()
         r_t, f_t = tensors[:n_r], tensors[n_r:]
-        rv = _Views(list(r_t) if r_layout == "list" else r_t[0], None if r_layout == "list" else r_layout, "R")
-        fv = _Views(list(f_t) if f_layout == "list" else f_t[0], None if f_layout == "list" else f_layout, "F")
+        rv = _Views.of(r_t, r_layout, "R")
+        fv = _Views.of(f_t, f_layout, "F")
         # no synchronisation in the training step: out-of-range / NaN scores are clamped for pooling and counted
         # into the caller's persistent `status` tensor (checked every N steps), as in grouping_fusion
-        sr = score_bin(list(r_t) if r_layout == "list" else r_t[0], W, b, G, score_reduce="shape",
-                       layout=None if r_layout == "list" else r_layout, edge_ulps=1, clamp=True, check=False,
-                       status=status)
+        sr = score_bin(r_t if r_layout == "list" else r_t[0], W, b, G, score_reduce="shape", layout=r_layout,
+                       edge_ulps=1, clamp=True, check=False, status=status)
         dev = fv.device
         weights = torch.empty((rv.B, G), dtype=torch.float32, device=dev)
         with _on(dev):
             C.check(L.gvcnn_group_weight_from_scores(_ptr(sr.scores), _ptr(sr.bins), _ptr(weights), rv.B, rv.V, G,
                                                      _stream()), "gvcnn_group_weight_from_scores")
-        S, mask, _, _, bins_c, bstride, w_c, wstride = _pool_fuse_fwd(fv, sr.bins, G, pool, 0.0, weights,
-                                                                      want_mask=True, want_groups=False,
-                                                                      want_status=False)
+        out = _pool_fuse_fwd(fv, sr.bins, G, pool, 0.0, weights, want_mask=True, want_groups=False, want_status=False)
         ctx.rv, ctx.fv, ctx.G, ctx.pool = rv, fv, G, pool
-        ctx.bstride, ctx.wstride = bstride, wstride
+        ctx.bstride, ctx.wstride = out.bin_stride, out.w_stride
         ctx.need_dr = any(t.requires_grad for t in r_t)
         ctx.n_r = n_r
-        ctx.save_for_backward(W.contiguous(), sr.x, bins_c, w_c, S,
-                              mask if mask is not None else torch.empty(0, device=dev))
+        ctx.save_for_backward(W.contiguous(), sr.x, out.bins, out.weights, out.S, out.mask)
         ctx.mark_non_differentiable(sr.scores, sr.bins, weights)
-        return S.reshape(fv.view_shape), sr.scores, sr.bins, weights
+        return out.S.reshape(fv.view_shape), sr.scores, sr.bins, weights
 
     @staticmethod
     def backward(ctx, dS, _ds, _db, _dw):
         L = C.lib()
         W, x, bins_c, w_c, S, mask = ctx.saved_tensors
-        mask = mask if mask.numel() else None
         rv, fv, G, pool = ctx.rv, ctx.fv, ctx.G, ctx.pool
         dS2 = dS.reshape(fv.B, fv.D).contiguous()
         dev = dS2.device
@@ -1241,15 +1133,9 @@ def grouping_fusion_paper(raw_view_descriptors, W, b, final_view_descriptors, nu
     """Paper-mode grouping + fusion: group weight = mean discrimination score of the group's views, empty
     groups vanish; differentiable w.r.t. the view descriptors AND the score FC (W, b, optionally the raw
     descriptors).  Returns (shape_descriptor, scores, bins, weights).  Per-shape scores/bins."""
-    if isinstance(raw_view_descriptors, (list, tuple)):
-        r_t, r_lay = tuple(raw_view_descriptors), "list"
-    else:
-        r_t, r_lay = (raw_view_descriptors,), (layout or "bvd")
-    if isinstance(final_view_descriptors, (list, tuple)):
-        f_t, f_lay = tuple(final_view_descriptors), "list"
-    else:
-        f_t, f_lay = (final_view_descriptors,), (layout or "bvd")
-    _require_cuda(W, "W"), _require_cuda(b, "b")
+    r_t, r_lay = _view_args(raw_view_descriptors, layout)
+    f_t, f_lay = _view_args(final_view_descriptors, layout)
+    _check_score_fc(W, b)
     return _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, *r_t, *f_t)
 
 
