@@ -59,11 +59,19 @@ SIGNATURES = {
     "gvcnn_pool_fuse_gap_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "gvcnn_pool_fuse_gap_fwd": (_i, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, _sz, _i, _i, _i, _i, _i, _i, _f, _i, _i, _vp]),
     "gvcnn_pool_fuse_gap_bwd": (_i, [_vp, _vp, _i64, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
+    "gvcnn_pool_fuse_gap_weighted_fwd": (_i, [_vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _sz, _i, _i, _i, _i, _i, _i,
+                                              _f, _i, _i, _vp]),
+    "gvcnn_pool_fuse_gap_weighted_bwd": (_i, [_vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i,
+                                              _vp]),
     "gvcnn_group_weight_from_scores": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp]),
     "gvcnn_pool_fuse_bwd_weights": (_i, [_vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _i, _i, _i64, _i, _i, _i, _i, _vp]),
     "gvcnn_score_weight_bwd": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     "gvcnn_view_score_bwd_workspace_bytes": (_sz, [_i, _i]),
     "gvcnn_view_score_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _i, _i, _i, _i, _i, _vp]),
+    "gvcnn_pool_fuse_gap_bwd_weights_workspace_bytes": (_sz, [_i, _i, _i, _i, _i]),
+    "gvcnn_pool_fuse_gap_bwd_weights": (_i, [_vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _sz, _i, _i, _i, _i, _i, _i,
+                                             _i, _i, _vp]),
+    "gvcnn_gap_score_bwd": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "gvcnn_comm_create": (_i, [ctypes.POINTER(_vp), _i, _i, _vp]),
     "gvcnn_comm_connect": (_i, [_vp, _vp]),
     "gvcnn_comm_allreduce_f32": (_i, [_vp, _vp, _i, _vp]),

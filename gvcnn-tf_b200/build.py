@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libgvcnn_sm100.so")
-SOURCES = ["capi.cu", "host_pipeline.cu", "comm.cu", "score.cu", "gap_score.cu", "scheme.cu", "pool_fwd.cu", "pool_fwd_ring.cu", "pool_fwd_direct.cu", "pool_gap_ring.cu", "pool_bwd.cu", "pool_bwd_fast.cu", "paper_mode.cu"]
+SOURCES = ["capi.cu", "host_pipeline.cu", "comm.cu", "score.cu", "gap_score.cu", "scheme.cu", "pool_fwd.cu", "pool_fwd_ring.cu", "pool_fwd_direct.cu", "pool_gap_ring.cu", "pool_bwd.cu", "pool_bwd_fast.cu", "paper_mode.cu", "paper_gap.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "ring_common.cuh"), os.path.join(ROOT, "include", "gvcnn_b200.h")]
 
 

@@ -417,9 +417,10 @@ size_t gvcnn_pool_fuse_gap_workspace_bytes(int B, int C, int HW, int dtype)
     return gap_workspace_bytes(B, C, HW, dtype);
 }
 
-int gvcnn_pool_fuse_gap_fwd(const void *F, const int32_t *bins, int64_t bin_stride_b, void *S_gap, uint8_t *tie_mask,
-                            int32_t *status, void *workspace, size_t workspace_bytes, int B, int V, int HW, int C,
-                            int G, int pool, float empty_fill, int f_layout, int dtype, void *stream)
+static int pool_fuse_gap_fwd_impl(const void *F, const int32_t *bins, int64_t bin_stride_b, const float *weights,
+                                  int64_t weight_stride_b, void *S_gap, uint8_t *tie_mask, int32_t *status,
+                                  void *workspace, size_t workspace_bytes, int B, int V, int HW, int C, int G, int pool,
+                                  float empty_fill, int f_layout, int dtype, void *stream)
 {
     if (HW <= 0 || C <= 0) return GVCNN_E_BAD_ARG;
     const int64_t D = (int64_t)HW * C;
@@ -427,6 +428,7 @@ int gvcnn_pool_fuse_gap_fwd(const void *F, const int32_t *bins, int64_t bin_stri
     if (rc) return rc == kEmptyBatch ? 0 : rc;
     if (!bins || !S_gap || !workspace || bin_stride_b < 0) return GVCNN_E_BAD_ARG;
     if (pool != GVCNN_POOL_MAX && pool != GVCNN_POOL_MEAN) return GVCNN_E_BAD_MODE;
+    if (weights && (!is_aligned(weights, 4) || weight_stride_b < 0)) return GVCNN_E_BAD_ARG;
     ViewPtrs fp;
     int64_t sb;
     bool al;
@@ -436,14 +438,32 @@ int gvcnn_pool_fuse_gap_fwd(const void *F, const int32_t *bins, int64_t bin_stri
     if (!al || need == 0 || V > 32 || (tie_mask && !is_aligned(tie_mask, 8)) || !is_aligned(workspace, 16))
         return GVCNN_E_UNSUPPORTED;
     if (workspace_bytes < need) return GVCNN_E_WORKSPACE;
-    rc = launch_pool_fuse_gap_fwd(fp, sb, bins, bin_stride_b, S_gap, tie_mask, status, static_cast<float *>(workspace),
-                                  B, V, HW, C, G, pool, empty_fill, dtype, static_cast<cudaStream_t>(stream));
+    rc = launch_pool_fuse_gap_fwd(fp, sb, bins, bin_stride_b, weights, weight_stride_b, S_gap, tie_mask, status,
+                                  static_cast<float *>(workspace), B, V, HW, C, G, pool, empty_fill, dtype,
+                                  static_cast<cudaStream_t>(stream));
     return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
 }
 
-int gvcnn_pool_fuse_gap_bwd(const void *dS_gap, const int32_t *bins, int64_t bin_stride_b, const uint8_t *tie_mask,
-                            void *dF, int32_t *status, int B, int V, int HW, int C, int G, int pool, int g_layout,
-                            int dtype, void *stream)
+int gvcnn_pool_fuse_gap_fwd(const void *F, const int32_t *bins, int64_t bin_stride_b, void *S_gap, uint8_t *tie_mask,
+                            int32_t *status, void *workspace, size_t workspace_bytes, int B, int V, int HW, int C,
+                            int G, int pool, float empty_fill, int f_layout, int dtype, void *stream)
+{
+    return pool_fuse_gap_fwd_impl(F, bins, bin_stride_b, nullptr, 0, S_gap, tie_mask, status, workspace, workspace_bytes,
+                                  B, V, HW, C, G, pool, empty_fill, f_layout, dtype, stream);
+}
+
+int gvcnn_pool_fuse_gap_weighted_fwd(const void *F, const int32_t *bins, int64_t bin_stride_b, const float *weights,
+                                     int64_t weight_stride_b, void *S_gap, uint8_t *tie_mask, int32_t *status,
+                                     void *workspace, size_t workspace_bytes, int B, int V, int HW, int C, int G,
+                                     int pool, float empty_fill, int f_layout, int dtype, void *stream)
+{
+    return pool_fuse_gap_fwd_impl(F, bins, bin_stride_b, weights, weight_stride_b, S_gap, tie_mask, status, workspace,
+                                  workspace_bytes, B, V, HW, C, G, pool, empty_fill, f_layout, dtype, stream);
+}
+
+static int pool_fuse_gap_bwd_impl(const void *dS_gap, const int32_t *bins, int64_t bin_stride_b, const float *weights,
+                                  int64_t weight_stride_b, const uint8_t *tie_mask, void *dF, int32_t *status, int B,
+                                  int V, int HW, int C, int G, int pool, int g_layout, int dtype, void *stream)
 {
     if (HW <= 0 || C <= 0) return GVCNN_E_BAD_ARG;
     const int64_t D = (int64_t)HW * C;
@@ -452,15 +472,33 @@ int gvcnn_pool_fuse_gap_bwd(const void *dS_gap, const int32_t *bins, int64_t bin
     if (!dS_gap || !bins || bin_stride_b < 0) return GVCNN_E_BAD_ARG;
     if (pool != GVCNN_POOL_MAX && pool != GVCNN_POOL_MEAN) return GVCNN_E_BAD_MODE;
     if (pool == GVCNN_POOL_MAX && !tie_mask) return GVCNN_E_BAD_ARG;
+    if (weights && (!is_aligned(weights, 4) || weight_stride_b < 0)) return GVCNN_E_BAD_ARG;
     ViewPtrs gp;
     int64_t sb;
     bool al;
     rc = make_view_ptrs(dF, g_layout, dtype, B, V, D, gp, sb, al);
     if (rc) return rc;
     if (!al || !is_aligned(dS_gap, 16) || (tie_mask && !is_aligned(tie_mask, 8))) return GVCNN_E_UNSUPPORTED;
-    rc = launch_pool_fuse_gap_bwd(dS_gap, bins, bin_stride_b, tie_mask, gp, sb, status, B, V, HW, C, G, pool, dtype,
-                                  static_cast<cudaStream_t>(stream));
+    rc = launch_pool_fuse_gap_bwd(dS_gap, bins, bin_stride_b, weights, weight_stride_b, tie_mask, gp, sb, status, B, V,
+                                  HW, C, G, pool, dtype, static_cast<cudaStream_t>(stream));
     return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
+}
+
+int gvcnn_pool_fuse_gap_bwd(const void *dS_gap, const int32_t *bins, int64_t bin_stride_b, const uint8_t *tie_mask,
+                            void *dF, int32_t *status, int B, int V, int HW, int C, int G, int pool, int g_layout,
+                            int dtype, void *stream)
+{
+    return pool_fuse_gap_bwd_impl(dS_gap, bins, bin_stride_b, nullptr, 0, tie_mask, dF, status, B, V, HW, C, G, pool,
+                                  g_layout, dtype, stream);
+}
+
+int gvcnn_pool_fuse_gap_weighted_bwd(const void *dS_gap, const int32_t *bins, int64_t bin_stride_b,
+                                     const float *weights, int64_t weight_stride_b, const uint8_t *tie_mask, void *dF,
+                                     int32_t *status, int B, int V, int HW, int C, int G, int pool, int g_layout,
+                                     int dtype, void *stream)
+{
+    return pool_fuse_gap_bwd_impl(dS_gap, bins, bin_stride_b, weights, weight_stride_b, tie_mask, dF, status, B, V, HW,
+                                  C, G, pool, g_layout, dtype, stream);
 }
 
 // ---------------------------------------------------------------------------
@@ -524,6 +562,65 @@ int gvcnn_view_score_bwd(const void *R, const float *dx, const float *W, float *
     return launch_view_score_bwd(rp, sb, dx, W, dW, dbias, drp, dsb, dR ? 1 : 0, static_cast<float *>(workspace),
                                  GVCNN_SCORE_BWD_SLICES, B, V, C, dtype, al && al2,
                                  static_cast<cudaStream_t>(stream));
+}
+
+// ---------------------------------------------------------------------------
+// paper mode on spatial maps: the GAP-folded weight gradient and the gradient of the score FC's GAP (paper_gap.cu)
+// ---------------------------------------------------------------------------
+static bool gap_view_count(int V) { return V == 4 || V == 6 || V == 8 || V == 12 || V == 16 || V == 20; }
+
+size_t gvcnn_pool_fuse_gap_bwd_weights_workspace_bytes(int B, int V, int HW, int C, int dtype)
+{
+    if (B <= 0 || V <= 0 || HW <= 0 || C <= 0) return 0;
+    return gap_bwd_weights_workspace_bytes(B, V, HW, C, dtype);
+}
+
+int gvcnn_pool_fuse_gap_bwd_weights(const void *F, const void *dS_gap, const void *S_gap, const int32_t *bins,
+                                    int64_t bin_stride_b, const float *weights, int64_t weight_stride_b,
+                                    float *dweights, void *workspace, size_t workspace_bytes, int B, int V, int HW,
+                                    int C, int G, int pool, int f_layout, int dtype, void *stream)
+{
+    if (HW <= 0 || C <= 0) return GVCNN_E_BAD_ARG;
+    const int64_t D = (int64_t)HW * C;
+    int rc = check_dims(B, V, D, G, dtype);
+    if (rc) return rc == kEmptyBatch ? 0 : rc;
+    if (!dS_gap || !S_gap || !bins || !weights || !dweights || !workspace || bin_stride_b < 0 || weight_stride_b < 0)
+        return GVCNN_E_BAD_ARG;
+    if (pool != GVCNN_POOL_MAX && pool != GVCNN_POOL_MEAN) return GVCNN_E_BAD_MODE;
+    ViewPtrs fp;
+    int64_t sb;
+    bool al;
+    rc = make_view_ptrs(F, f_layout, dtype, B, V, D, fp, sb, al);
+    if (rc) return rc;
+    const size_t need = gap_bwd_weights_workspace_bytes(B, V, HW, C, dtype);
+    if (!al || need == 0 || !gap_view_count(V) || G > 255) return GVCNN_E_UNSUPPORTED;
+    if (!is_aligned(dS_gap, 16) || !is_aligned(S_gap, 16) || !is_aligned(bins, 4) || !is_aligned(weights, 4) ||
+        !is_aligned(dweights, 4) || !is_aligned(workspace, 16))
+        return GVCNN_E_MISALIGNED;
+    if (workspace_bytes < need) return GVCNN_E_WORKSPACE;
+    rc = launch_gap_bwd_weights(fp, sb, dS_gap, S_gap, bins, bin_stride_b, weights, weight_stride_b, dweights,
+                                static_cast<float *>(workspace), B, V, HW, C, G, pool, dtype,
+                                static_cast<cudaStream_t>(stream));
+    return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
+}
+
+int gvcnn_gap_score_bwd(const float *dx, const float *W, void *dmaps, int B, int V, int HW, int C, int m_layout,
+                        int dtype, void *stream)
+{
+    if (HW <= 0 || C <= 0) return GVCNN_E_BAD_ARG;
+    const int64_t D = (int64_t)HW * C;
+    int rc = check_dims(B, V, D, 1, dtype);
+    if (rc) return rc == kEmptyBatch ? 0 : rc;
+    if (!dx || !W) return GVCNN_E_BAD_ARG;
+    ViewPtrs dp;
+    int64_t sb;
+    bool al;
+    rc = make_view_ptrs(dmaps, m_layout, dtype, B, V, D, dp, sb, al);
+    if (rc) return rc;
+    if (!is_aligned(dx, 4) || !is_aligned(W, 16)) return GVCNN_E_MISALIGNED;
+    if (!al) return GVCNN_E_UNSUPPORTED;
+    rc = launch_gap_score_bwd(dx, W, dp, sb, B, V, HW, C, dtype, static_cast<cudaStream_t>(stream));
+    return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
 }
 
 }  // extern "C"

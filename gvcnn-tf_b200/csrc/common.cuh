@@ -403,6 +403,20 @@ __device__ __forceinline__ void vec_add(float (&a)[E], const float (&b)[E])  // 
     }
 }
 
+// block-wide sum with a fixed tree: xor butterfly inside each warp, then warp sums added in warp order
+__device__ __forceinline__ float block_sum_256(float v, float *scratch /* [8] */)
+{
+#pragma unroll
+    for (int off = 16; off >= 1; off >>= 1) v = __fadd_rn(v, __shfl_xor_sync(0xffffffffu, v, off));
+    __syncthreads();
+    if ((threadIdx.x & 31) == 0) scratch[threadIdx.x >> 5] = v;
+    __syncthreads();
+    float t = scratch[0];
+#pragma unroll
+    for (int i = 1; i < 8; ++i) t = __fadd_rn(t, scratch[i]);
+    return t;
+}
+
 // ---- element packing ---------------------------------------------------------
 template <typename T> struct Elem;
 template <> struct Elem<float> {
@@ -579,12 +593,20 @@ int launch_pool_fuse_fwd_direct(const ViewPtrs &fp, int64_t f_sb, const int32_t 
                                 uint8_t *mask, int32_t *status, int B, int V, int64_t D, int G, int pool, float fill,
                                 int dtype, bool forced, bool f_ready, cudaStream_t st);
 size_t gap_workspace_bytes(int B, int C, int HW, int dtype);
-int launch_pool_fuse_gap_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb, void *out,
-                             uint8_t *mask, int32_t *status, float *partial, int B, int V, int HW, int C, int G,
-                             int pool, float fill, int dtype, cudaStream_t st);
-int launch_pool_fuse_gap_bwd(const void *dOut, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
-                             const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int HW, int C, int G,
-                             int pool, int dtype, cudaStream_t st);
+int launch_pool_fuse_gap_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb,
+                             const float *weights, int64_t w_sb, void *out, uint8_t *mask, int32_t *status,
+                             float *partial, int B, int V, int HW, int C, int G, int pool, float fill, int dtype,
+                             cudaStream_t st);
+int launch_pool_fuse_gap_bwd(const void *dOut, const int32_t *bins, int64_t bin_sb, const float *weights, int64_t w_sb,
+                             const uint8_t *mask, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V,
+                             int HW, int C, int G, int pool, int dtype, cudaStream_t st);
+void gap_split(int B, int CB, int HW, int &nsplit, int &pps);
+size_t gap_bwd_weights_workspace_bytes(int B, int V, int HW, int C, int dtype);
+int launch_gap_bwd_weights(const ViewPtrs &fp, int64_t f_sb, const void *dS_gap, const void *S_gap,
+                           const int32_t *bins, int64_t bin_sb, const float *weights, int64_t w_sb, float *dweights,
+                           float *partial, int B, int V, int HW, int C, int G, int pool, int dtype, cudaStream_t st);
+int launch_gap_score_bwd(const float *dx, const float *W, const ViewPtrs &dp, int64_t d_sb, int B, int V, int HW, int C,
+                         int dtype, cudaStream_t st);
 int launch_pool_fuse_bwd_fast(const void *dS, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
                               const float *weights, int64_t w_sb, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
                               int pool, int dtype, cudaStream_t st);

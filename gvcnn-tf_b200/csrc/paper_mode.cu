@@ -35,20 +35,6 @@ __global__ void __launch_bounds__(256) group_weight_from_scores_kernel(const flo
     weights[i] = n ? __fdiv_rn(sum, (float)n) : 0.0f;
 }
 
-// block-wide sum with a fixed tree: xor butterfly inside each warp, then warp sums added in warp order
-__device__ __forceinline__ float block_sum_256(float v, float *scratch /* [8] */)
-{
-#pragma unroll
-    for (int off = 16; off >= 1; off >>= 1) v = __fadd_rn(v, __shfl_xor_sync(0xffffffffu, v, off));
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) scratch[threadIdx.x >> 5] = v;
-    __syncthreads();
-    float t = scratch[0];
-#pragma unroll
-    for (int i = 1; i < 8; ++i) t = __fadd_rn(t, scratch[i]);
-    return t;
-}
-
 // One CTA per shape.  For every non-empty group, one streaming pass over its members' rows:
 // A_g = <dS, P_g>; then C = <dS, S>;  dw_g = (A_g - C) / sum_w.  Every view row is read once in total.
 // VEC: 16-byte loads (rows 16-byte aligned, D a multiple of the vector width).

@@ -288,8 +288,8 @@ static int launch_bwd_fast_v(const void *dS, const int32_t *bins, int64_t bin_sb
         else GVCNN_LAUNCH_BF(GVCNN_POOL_MEAN, GAP_, WTS_, upc);                                               \
     } while (0)
     if (gapC > 0) {
-        if (weights) return GVCNN_E_UNSUPPORTED;  // the GAP-folded backward always uses the reference's weights
-        GVCNN_LAUNCH_BF_P(true, false);
+        if (weights) GVCNN_LAUNCH_BF_P(true, true);  // paper mode: caller-supplied weights
+        else GVCNN_LAUNCH_BF_P(true, false);
     } else if (weights) {
         GVCNN_LAUNCH_BF_P(false, true);
     } else {
@@ -333,22 +333,23 @@ static int launch_bwd_fast_t(const void *dS, const int32_t *bins, int64_t bin_sb
     }
 }
 
-// GAP-folded backward: dOut [B, C] -> dF; same applicability as the forward GAP kernel plus the fast-kernel V set
-int launch_pool_fuse_gap_bwd(const void *dOut, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
-                             const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int HW, int C, int G,
-                             int pool, int dtype, cudaStream_t st)
+// GAP-folded backward: dOut [B, C] -> dF; same applicability as the forward GAP kernel plus the fast-kernel V set.
+// weights (nullable): caller-supplied group weights, as in the forward
+int launch_pool_fuse_gap_bwd(const void *dOut, const int32_t *bins, int64_t bin_sb, const float *weights, int64_t w_sb,
+                             const uint8_t *mask, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V,
+                             int HW, int C, int G, int pool, int dtype, cudaStream_t st)
 {
     const int64_t D = (int64_t)HW * C;
     const int td = 256 * (dtype == GVCNN_F32 ? 4 : 8);
     if (C % td != 0) return -1000;
 #define GVCNN_GAPB_CASE(T_)                                                                                   \
     switch (V) {                                                                                              \
-    case 4: return launch_bwd_fast_v<T_, 4>(dOut, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, D, G, pool, st, C, HW);   \
-    case 6: return launch_bwd_fast_v<T_, 6>(dOut, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, D, G, pool, st, C, HW);   \
-    case 8: return launch_bwd_fast_v<T_, 8>(dOut, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, D, G, pool, st, C, HW);   \
-    case 12: return launch_bwd_fast_v<T_, 12>(dOut, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, D, G, pool, st, C, HW); \
-    case 16: return launch_bwd_fast_v<T_, 16>(dOut, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, D, G, pool, st, C, HW); \
-    case 20: return launch_bwd_fast_v<T_, 20>(dOut, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, D, G, pool, st, C, HW); \
+    case 4: return launch_bwd_fast_v<T_, 4>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW);   \
+    case 6: return launch_bwd_fast_v<T_, 6>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW);   \
+    case 8: return launch_bwd_fast_v<T_, 8>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW);   \
+    case 12: return launch_bwd_fast_v<T_, 12>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW); \
+    case 16: return launch_bwd_fast_v<T_, 16>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW); \
+    case 20: return launch_bwd_fast_v<T_, 20>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW); \
     default: return -1000;                                                                                    \
     }
     if (dtype == GVCNN_F32) { GVCNN_GAPB_CASE(float) }

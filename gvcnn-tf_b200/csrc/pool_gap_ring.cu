@@ -13,12 +13,16 @@
 
 namespace gvcnn {
 
-template <typename T, int POOL, bool MASK, int V, int NCONS, int MINB>
+// WTS = caller-supplied group weights (paper mode: the mean score of the group's views): the producer publishes the
+// weights of the unit's shape like pool_fwd_ring.cu does, the consumers divide by their sum.  The trailing template flag
+// and the trailing parameters leave the reference-weights instantiations as they were.
+template <typename T, int POOL, bool MASK, int V, int NCONS, int MINB, bool WTS>
 __global__ void __launch_bounds__(NCONS + kRingProducerThreads, MINB)
 pool_fuse_gap_fwd_kernel(const ViewPtrs fp, const int64_t f_sb, const int32_t *__restrict__ bins,
                          const int64_t bin_sb, float *__restrict__ partial, uint8_t *__restrict__ mask,
                          int32_t *status, const int B, const int C, const int HW, const int G, const float fill,
-                         const int CB, const int NSPLIT, const int PPS, const int num_units, const int stages)
+                         const int CB, const int NSPLIT, const int PPS, const int num_units, const int stages,
+                         const float *__restrict__ weights, const int64_t w_sb)
 {
     constexpr int E = Elem<T>::kVec;
     constexpr int kMaxStages = 8;
@@ -30,6 +34,11 @@ pool_fuse_gap_fwd_kernel(const ViewPtrs fp, const int64_t f_sb, const int32_t *_
     __shared__ int32_t sorted_bin[32];
     __shared__ __align__(8) uint64_t full_bar[kMaxStages];
     __shared__ __align__(8) uint64_t empty_bar[kMaxStages];
+    RingWts *wts_s = nullptr;  // whole weight rows, one per slot: only with WTS
+    if constexpr (WTS) {
+        __shared__ RingWts wts_buf[kMaxStages];
+        wts_s = wts_buf;
+    }
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < stages; ++s) {
@@ -76,6 +85,17 @@ pool_fuse_gap_fwd_kernel(const ViewPtrs fp, const int64_t f_sb, const int32_t *_
             __syncwarp();
             const int prev = (lane < V && k > 0) ? sorted_bin[k - 1] : -1;
             const int last_bin = sorted_bin[V - 1];
+            float gw = 0.0f, sw = 0.0f, wlo = 0.0f, whi = 0.0f;  // WTS: this shape's weights, read once per unit
+            if constexpr (WTS) {
+                const float *wrow = weights + (int64_t)b * w_sb;
+                if (lane < V) gw = __ldg(wrow + bin);
+                if (lane == 0)
+                    for (int g = 0; g < G; ++g) sw = __fadd_rn(sw, __ldg(wrow + g));  // left to right, as the ring
+                // the whole row (G <= kRingMaxWtsGroups, checked by the launcher): ring_consume_tile reads the weight
+                // of every empty group it passes (w_g * fill), also when fill == 0
+                if (lane < G) wlo = __ldg(wrow + lane);
+                if (lane + 32 < G) whi = __ldg(wrow + lane + 32);
+            }
             const int p1 = min(HW, (ps + 1) * PPS);
             for (int p = ps * PPS; p < p1; ++p) {
                 const int64_t d0 = (int64_t)p * C + (int64_t)cb * TD;
@@ -85,6 +105,12 @@ pool_fuse_gap_fwd_kernel(const ViewPtrs fp, const int64_t f_sb, const int32_t *_
                 if (lane == 0) {
                     plans[s].first_mask = fm;
                     plans[s].tail_skip = (uint32_t)(G - 1 - last_bin);
+                }
+                if constexpr (WTS) {
+                    if (lane < V) plans[s].gw[k] = gw;
+                    if (lane == 0) plans[s].sumw = sw;
+                    if (lane < G) wts_s[s].wall[lane] = wlo;
+                    if (lane + 32 < G) wts_s[s].wall[lane + 32] = whi;
                 }
                 __syncwarp();
                 if (lane == 0) mbar_expect_tx(&full_bar[s], kRowStride * (uint32_t)V);
@@ -115,10 +141,23 @@ pool_fuse_gap_fwd_kernel(const ViewPtrs fp, const int64_t f_sb, const int32_t *_
             const unsigned char *col = smem_raw + (size_t)s * kStageBytes + (size_t)threadIdx.x * 16;
             mbar_wait(&full_bar[s], ph);
             float acc[E];
-            ring_consume_tile<T, POOL, MASK, V, kRowStride>(col, plans[s], fill, true, mask, B, D, out_off, acc);
+            float sw_given = 0.0f;
+            if constexpr (WTS) {
+                ring_consume_tile<T, POOL, MASK, V, kRowStride>(col, plans[s], fill, true, mask, B, D, out_off, acc, true,
+                                                                wts_s[s].wall);
+                sw_given = plans[s].sumw;
+            } else {
+                ring_consume_tile<T, POOL, MASK, V, kRowStride>(col, plans[s], fill, true, mask, B, D, out_off, acc);
+            }
             __syncwarp();
             if ((threadIdx.x & 31) == 0) mbar_arrive(&empty_bar[s]);
-            div_vec_by_rcp(acc, sumw, rcp_sumw);  // S at this position, then the running sum over positions
+            // S at this position (pool_fwd_ring.cu's division), then the running sum over positions
+            if constexpr (WTS) {
+#pragma unroll
+                for (int e = 0; e < E; ++e) acc[e] = __fdiv_rn(acc[e], sw_given);
+            } else {
+                div_vec_by_rcp(acc, sumw, rcp_sumw);
+            }
 #pragma unroll
             for (int e = 0; e < E; ++e) gacc[e] = __fadd_rn(gacc[e], acc[e]);
             if (++s == stages) { s = 0; ph ^= 1u; }
@@ -172,16 +211,17 @@ void gap_split(int B, int CB, int HW, int &nsplit, int &pps)
 }
 
 template <typename T, int V, int MINB>
-static int launch_gap_v(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb, void *out,
-                        uint8_t *mask, int32_t *status, float *partial, int B, int HW, int C, int G, int pool,
-                        float fill, cudaStream_t st)
+static int launch_gap_v(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb, const float *weights,
+                        int64_t w_sb, void *out, uint8_t *mask, int32_t *status, float *partial, int B, int HW, int C,
+                        int G, int pool, float fill, cudaStream_t st)
 {
     constexpr int NCONS = 256;
     constexpr int E = Elem<T>::kVec;
     constexpr int TD = NCONS * E;
     constexpr size_t stage_bytes = (size_t)V * NCONS * 16;
     if (C % TD != 0) return -1000;
-    int stages = (int)(((226 * 1024) / MINB - 3 * 1024) / stage_bytes);
+    // static shared memory per CTA: ~1.3 KB, plus 2 KB of weight rows with caller-supplied weights
+    int stages = (int)(((226 * 1024) / MINB - (weights ? 5 : 3) * 1024) / stage_bytes);
     if (stages > 8) stages = 8;
     if (stages < 2) return -1000;
     const int CB = C / TD;
@@ -194,19 +234,25 @@ static int launch_gap_v(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, i
     const int grid = (int)(units < max_grid ? units : max_grid);
     const bool want_mask = (mask != nullptr) && pool == GVCNN_POOL_MAX;
     cudaError_t err = cudaSuccess;
-#define GVCNN_LAUNCH_GAP(POOL_, MASK_)                                                                        \
+#define GVCNN_LAUNCH_GAP(POOL_, MASK_, WTS_)                                                                  \
     do {                                                                                                      \
-        auto kern = pool_fuse_gap_fwd_kernel<T, POOL_, MASK_, V, NCONS, MINB>;                                \
-        err = ensure_dyn_smem<pool_fuse_gap_fwd_kernel<T, POOL_, MASK_, V, NCONS, MINB>>((int)smem);          \
+        auto kern = pool_fuse_gap_fwd_kernel<T, POOL_, MASK_, V, NCONS, MINB, WTS_>;                          \
+        err = ensure_dyn_smem<pool_fuse_gap_fwd_kernel<T, POOL_, MASK_, V, NCONS, MINB, WTS_>>((int)smem);    \
         if (err == cudaSuccess)                                                                               \
             err = launch_pdl(kern, dim3(grid), dim3(NCONS + kRingProducerThreads), smem, st, fp, f_sb, bins,  \
                              bin_sb, partial, mask, status, B, C, HW, G, fill, CB, nsplit, pps, (int)units,   \
-                             stages);                                                                         \
+                             stages, weights, w_sb);                                                          \
     } while (0)
-    if (pool == GVCNN_POOL_MAX) {
-        if (want_mask) GVCNN_LAUNCH_GAP(GVCNN_POOL_MAX, true); else GVCNN_LAUNCH_GAP(GVCNN_POOL_MAX, false);
+    if (weights) {
+        if (pool == GVCNN_POOL_MAX) {
+            if (want_mask) GVCNN_LAUNCH_GAP(GVCNN_POOL_MAX, true, true); else GVCNN_LAUNCH_GAP(GVCNN_POOL_MAX, false, true);
+        } else {
+            GVCNN_LAUNCH_GAP(GVCNN_POOL_MEAN, false, true);
+        }
+    } else if (pool == GVCNN_POOL_MAX) {
+        if (want_mask) GVCNN_LAUNCH_GAP(GVCNN_POOL_MAX, true, false); else GVCNN_LAUNCH_GAP(GVCNN_POOL_MAX, false, false);
     } else {
-        GVCNN_LAUNCH_GAP(GVCNN_POOL_MEAN, false);
+        GVCNN_LAUNCH_GAP(GVCNN_POOL_MEAN, false, false);
     }
 #undef GVCNN_LAUNCH_GAP
     if (err != cudaSuccess) return (int)err;
@@ -225,20 +271,23 @@ size_t gap_workspace_bytes(int B, int C, int HW, int dtype)
     return (size_t)B * nsplit * C * sizeof(float);
 }
 
-// returns -1000 when the shapes are not supported (V not instantiated, C not a multiple of the tile, G > 255)
-int launch_pool_fuse_gap_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb, void *out,
-                             uint8_t *mask, int32_t *status, float *partial, int B, int V, int HW, int C, int G,
-                             int pool, float fill, int dtype, cudaStream_t st)
+// returns -1000 when the shapes are not supported (V not instantiated, C not a multiple of the tile, G > 255, or
+// caller-supplied weights and more groups than a slot's weight row holds)
+int launch_pool_fuse_gap_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb,
+                             const float *weights, int64_t w_sb, void *out, uint8_t *mask, int32_t *status,
+                             float *partial, int B, int V, int HW, int C, int G, int pool, float fill, int dtype,
+                             cudaStream_t st)
 {
     if (G > 255) return -1000;
+    if (weights && G > kRingMaxWtsGroups) return -1000;
 #define GVCNN_GAP_CASE(T_)                                                                                    \
     switch (V) {                                                                                              \
-    case 4: return launch_gap_v<T_, 4, 2>(fp, f_sb, bins, bin_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
-    case 6: return launch_gap_v<T_, 6, 2>(fp, f_sb, bins, bin_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
-    case 8: return launch_gap_v<T_, 8, 2>(fp, f_sb, bins, bin_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
-    case 12: return launch_gap_v<T_, 12, 2>(fp, f_sb, bins, bin_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
-    case 16: return launch_gap_v<T_, 16, 1>(fp, f_sb, bins, bin_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
-    case 20: return launch_gap_v<T_, 20, 1>(fp, f_sb, bins, bin_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
+    case 4: return launch_gap_v<T_, 4, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
+    case 6: return launch_gap_v<T_, 6, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
+    case 8: return launch_gap_v<T_, 8, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
+    case 12: return launch_gap_v<T_, 12, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
+    case 16: return launch_gap_v<T_, 16, 1>(fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
+    case 20: return launch_gap_v<T_, 20, 1>(fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
     default: return -1000;                                                                                    \
     }
     if (dtype == GVCNN_F32) { GVCNN_GAP_CASE(float) }

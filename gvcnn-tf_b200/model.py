@@ -613,6 +613,20 @@ def group_weight(g_schemes):
 _Pooled = collections.namedtuple("_Pooled", "S mask P status bins bin_stride weights w_stride")
 
 
+def _weight_rows(weights, G, fv):
+    """Caller-supplied group weights as the pooling kernels read them: float32 [1, G] or [B, G], and the row stride
+    (0: one row for the batch).  None stays None (the kernels compute 1 + n_g)."""
+    if weights is None:
+        return None, 0
+    _require_cuda(weights, "group_weight")
+    weights = weights.to(torch.float32).contiguous()
+    if weights.dim() == 1:
+        weights = weights[None]
+    if weights.shape[-1] != G or weights.shape[0] not in (1, fv.B):
+        raise ValueError("group_weight must be [G] or [B, G]")
+    return weights, (G if (weights.shape[0] == fv.B and fv.B > 1) else 0)
+
+
 def _pool_fuse_fwd(fv: _Views, bins: torch.Tensor, G: int, pool: str, empty_fill: float,
                    weights: Optional[torch.Tensor], want_mask: bool, want_groups: bool, want_status: bool = True,
                    variant: int = 0) -> _Pooled:
@@ -622,15 +636,7 @@ def _pool_fuse_fwd(fv: _Views, bins: torch.Tensor, G: int, pool: str, empty_fill
     if bins.shape[-1] != fv.V or bins.shape[0] not in (1, fv.B):
         raise ValueError("bins must be [V], [1, V] or [B, V] with V=%d, B=%d; got %s"
                          % (fv.V, fv.B, tuple(bins.shape)))
-    w_stride = 0
-    if weights is not None:
-        _require_cuda(weights, "group_weight")
-        weights = weights.to(torch.float32).contiguous()
-        if weights.dim() == 1:
-            weights = weights[None]
-        if weights.shape[-1] != G or weights.shape[0] not in (1, fv.B):
-            raise ValueError("group_weight must be [G] or [B, G]")
-        w_stride = G if (weights.shape[0] == fv.B and fv.B > 1) else 0
+    weights, w_stride = _weight_rows(weights, G, fv)
     S = torch.empty((fv.B, fv.D), dtype=fv.dtype, device=dev)
     mask = _tie_mask(fv, pool, want_mask)
     P = torch.empty((G, fv.B, fv.D), dtype=fv.dtype, device=dev) if want_groups else None
@@ -717,52 +723,70 @@ def pool_fuse(final_view_descriptors, bins, num_group, pool="max", empty_fill=1.
 
 class _PoolFuseGapFn(torch.autograd.Function):
     """Pooling + fusion + the global average pooling that follows it (nets/model.py:154-163) without ever
-    writing the fused map: [B, C] out; backward takes the [B, C] gradient."""
+    writing the fused map: [B, C] out; backward takes the [B, C] gradient.  `weights`: caller-supplied group
+    weights ([G] or [B, G]), None for the reference's 1 + n_g."""
 
     @staticmethod
-    def forward(ctx, bins, G, pool, empty_fill, layout, HW, Cch, *views):
+    def forward(ctx, bins, G, pool, empty_fill, layout, HW, Cch, weights, *views):
         L = C.lib()
         fv = _Views.of(views, layout, "F")
         dev = fv.device
         dt = _dtype_code(fv.dtype)
         bins_c, bstride = _bin_rows(bins, fv)
+        w_c, wstride = _weight_rows(weights, G, fv)
         out = torch.empty((fv.B, Cch), dtype=fv.dtype, device=dev)
         mask = _tie_mask(fv, pool, any(v.requires_grad for v in views))
         status = _new_status(dev)
         ws_bytes = L.gvcnn_pool_fuse_gap_workspace_bytes(fv.B, Cch, HW, dt)
         ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
         with _on(dev):
-            C.check(L.gvcnn_pool_fuse_gap_fwd(fv.arg, _ptr(bins_c), bstride, _ptr(out), _ptr(mask), _ptr(status),
-                                              _ptr(ws), ws_bytes, fv.B, fv.V, HW, Cch, G, _POOL[pool],
-                                              ctypes.c_float(empty_fill), fv.layout, dt, _stream()),
-                    "gvcnn_pool_fuse_gap_fwd")
-        ctx.fv, ctx.G, ctx.pool, ctx.HW, ctx.Cch, ctx.bstride = fv, G, pool, HW, Cch, bstride
-        ctx.save_for_backward(bins_c, mask)
+            if w_c is None:
+                C.check(L.gvcnn_pool_fuse_gap_fwd(fv.arg, _ptr(bins_c), bstride, _ptr(out), _ptr(mask), _ptr(status),
+                                                  _ptr(ws), ws_bytes, fv.B, fv.V, HW, Cch, G, _POOL[pool],
+                                                  ctypes.c_float(empty_fill), fv.layout, dt, _stream()),
+                        "gvcnn_pool_fuse_gap_fwd")
+            else:
+                C.check(L.gvcnn_pool_fuse_gap_weighted_fwd(fv.arg, _ptr(bins_c), bstride, _ptr(w_c), wstride, _ptr(out),
+                                                           _ptr(mask), _ptr(status), _ptr(ws), ws_bytes, fv.B, fv.V, HW,
+                                                           Cch, G, _POOL[pool], ctypes.c_float(empty_fill), fv.layout,
+                                                           dt, _stream()),
+                        "gvcnn_pool_fuse_gap_weighted_fwd")
+        ctx.fv, ctx.G, ctx.pool, ctx.HW, ctx.Cch, ctx.bstride, ctx.wstride = fv, G, pool, HW, Cch, bstride, wstride
+        ctx.save_for_backward(bins_c, w_c, mask)
         ctx.mark_non_differentiable(status)
         return out, status
 
     @staticmethod
     def backward(ctx, dOut, _dstatus):
-        bins_c, mask = ctx.saved_tensors
+        bins_c, w_c, mask = ctx.saved_tensors
         fv = ctx.fv
         dOut = dOut.contiguous()
         out, gv = fv.empty_like()
         status = _new_status(dOut.device)
+        L = C.lib()
         with _on(dOut.device):
-            C.check(C.lib().gvcnn_pool_fuse_gap_bwd(_ptr(dOut), _ptr(bins_c), ctx.bstride, _ptr(mask), gv.arg,
-                                                    _ptr(status), gv.B, gv.V, ctx.HW, ctx.Cch, ctx.G, _POOL[ctx.pool],
-                                                    gv.layout, _dtype_code(gv.dtype), _stream()),
-                    "gvcnn_pool_fuse_gap_bwd")
+            if w_c is None:
+                C.check(L.gvcnn_pool_fuse_gap_bwd(_ptr(dOut), _ptr(bins_c), ctx.bstride, _ptr(mask), gv.arg,
+                                                  _ptr(status), gv.B, gv.V, ctx.HW, ctx.Cch, ctx.G, _POOL[ctx.pool],
+                                                  gv.layout, _dtype_code(gv.dtype), _stream()),
+                        "gvcnn_pool_fuse_gap_bwd")
+            else:
+                C.check(L.gvcnn_pool_fuse_gap_weighted_bwd(_ptr(dOut), _ptr(bins_c), ctx.bstride, _ptr(w_c), ctx.wstride,
+                                                           _ptr(mask), gv.arg, _ptr(status), gv.B, gv.V, ctx.HW,
+                                                           ctx.Cch, ctx.G, _POOL[ctx.pool], gv.layout,
+                                                           _dtype_code(gv.dtype), _stream()),
+                        "gvcnn_pool_fuse_gap_weighted_bwd")
         grads = tuple(out) if isinstance(out, list) else (out,)
-        return (None,) * 7 + grads
+        return (None,) * 8 + grads
 
 
-def pool_fuse_gap(final_view_descriptors, bins, num_group, pool="max", empty_fill=1.0, layout=None):
+def pool_fuse_gap(final_view_descriptors, bins, num_group, pool="max", empty_fill=1.0, layout=None, group_weight=None):
     """view_pooling + group_fusion + GlobalAveragePooling2D (nets/model.py:154-163) in one pass: the
     descriptors are channel-last maps ([N, h, w, C] per view, or [B, V, h, w, C] / [V, B, h, w, C]); returns
-    the pooled shape descriptor [N, C].  The fused map is never written.  Shapes the specialised kernel does
-    not cover (see gvcnn_pool_fuse_gap_fwd) run pool_fuse and average afterwards - same result up to the
-    float32 rounding of the mean."""
+    the pooled shape descriptor [N, C].  The fused map is never written.  group_weight: caller-supplied group
+    weights ([G] or [B, G] float32, e.g. paper mode's mean scores) instead of the reference's 1 + n_g.  Shapes
+    the specialised kernel does not cover (see gvcnn_pool_fuse_gap_fwd) run pool_fuse and average afterwards -
+    same result up to the float32 rounding of the mean."""
     views, lay = _view_args(final_view_descriptors, layout)
     shp = tuple(views[0].shape)
     spatial = shp[1:-1] if lay == "list" else shp[2:-1]
@@ -772,12 +796,13 @@ def pool_fuse_gap(final_view_descriptors, bins, num_group, pool="max", empty_fil
     HW = int(math.prod(spatial)) if len(spatial) else 1
     _require_cuda(bins, "bins")
     try:
-        out, _ = _PoolFuseGapFn.apply(bins, num_group, pool, empty_fill, lay, HW, Cch, *views)
+        out, _ = _PoolFuseGapFn.apply(bins, num_group, pool, empty_fill, lay, HW, Cch, group_weight, *views)
         return out
     except C.GvcnnError as e:
         if e.code != C.E_UNSUPPORTED:
             raise
-    S = pool_fuse(final_view_descriptors, bins, num_group, pool=pool, empty_fill=empty_fill, layout=layout)
+    S = pool_fuse(final_view_descriptors, bins, num_group, pool=pool, empty_fill=empty_fill, layout=layout,
+                  group_weight=group_weight)
     return S.reshape(S.shape[0], -1, Cch).mean(dim=1)
 
 
@@ -1062,45 +1087,80 @@ def grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_grou
 # --------------------------------------------------------------------------
 # paper mode: score-derived, differentiable group weights (SURVEY.md 8f n2)
 # --------------------------------------------------------------------------
+class _GapScoreUnsupported(Exception):
+    """gvcnn_gap_score_bin_fwd does not cover these block3 maps (raised before anything was launched)."""
+
+
 class _PaperModeFn(torch.autograd.Function):
     """S = sum_g w_g P_g / sum_g w_g with w_g = mean score of the group's views (0 for an empty group).
     Unlike the reference (weights fed through placeholders, train.py:127-128), the gradient reaches the
     V Dense(1) score layers: dL/dW, dL/db (and dL/dR if the raw descriptors require grad) besides dL/dF.
-    No reference counterpart - checked against float64 autograd of the same formulas."""
+    No reference counterpart - checked against float64 autograd of the same formulas.
+    maps: R holds the block3 maps (HW_r > 1 positions); their GlobalAveragePooling2D runs inside the score kernel,
+    which also writes the pooled float32 R the score FC's gradient needs.  fold: the GlobalAveragePooling2D after
+    the fusion is folded into the pooling (S_gap [B, C] out, the [B, C] gradient in); where the folded kernels do not
+    cover the shapes the fused map is returned instead (the caller's _spatial_mean then averages it)."""
 
     @staticmethod
-    def forward(ctx, W, b, G, pool, f_layout, r_layout, n_r, status, *tensors):
+    def forward(ctx, W, b, G, pool, f_layout, r_layout, n_r, status, HW_r, fold, *tensors):
         L = C.lib()
         r_t, f_t = tensors[:n_r], tensors[n_r:]
         rv = _Views.of(r_t, r_layout, "R")
         fv = _Views.of(f_t, f_layout, "F")
+        dev = fv.device
+        R_out = None
         # no synchronisation in the training step: out-of-range / NaN scores are clamped for pooling and counted
         # into the caller's persistent `status` tensor (checked every N steps), as in grouping_fusion
-        sr = score_bin(r_t if r_layout == "list" else r_t[0], W, b, G, score_reduce="shape", layout=r_layout,
-                       edge_ulps=1, clamp=True, check=False, status=status)
-        dev = fv.device
+        if HW_r > 1:
+            Craw = rv.D // HW_r
+            Wc, bc = W.contiguous(), b.contiguous()
+            if tuple(Wc.shape) != (rv.V, Craw) or tuple(bc.shape) != (rv.V,):
+                raise ValueError("W must be [V, C] = %s and b [V], got %s and %s"
+                                 % ((rv.V, Craw), tuple(Wc.shape), tuple(bc.shape)))
+            buf = torch.empty((3, rv.B, rv.V), dtype=torch.int32, device=dev)     # x, scores, bins: one allocation
+            x, scores, bins = buf[0].view(torch.float32), buf[1].view(torch.float32), buf[2]
+            R_out = torch.empty((rv.B, rv.V, Craw), dtype=torch.float32, device=dev)
+            with _on(dev):
+                rc = L.gvcnn_gap_score_bin_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(R_out), _ptr(x), _ptr(scores),
+                                               _ptr(bins), None, _ptr(status), rv.B, rv.V, HW_r, Craw, G, rv.layout,
+                                               _dtype_code(rv.dtype), 1, 1, 1, _stream())
+            if rc == C.E_UNSUPPORTED:
+                raise _GapScoreUnsupported()
+            C.check(rc, "gvcnn_gap_score_bin_fwd")
+        else:
+            sr = score_bin(r_t if r_layout == "list" else r_t[0], W, b, G, score_reduce="shape", layout=r_layout,
+                           edge_ulps=1, clamp=True, check=False, status=status)
+            x, scores, bins = sr.x, sr.scores, sr.bins
         weights = torch.empty((rv.B, G), dtype=torch.float32, device=dev)
         with _on(dev):
-            C.check(L.gvcnn_group_weight_from_scores(_ptr(sr.scores), _ptr(sr.bins), _ptr(weights), rv.B, rv.V, G,
+            C.check(L.gvcnn_group_weight_from_scores(_ptr(scores), _ptr(bins), _ptr(weights), rv.B, rv.V, G,
                                                      _stream()), "gvcnn_group_weight_from_scores")
-        out = _pool_fuse_fwd(fv, sr.bins, G, pool, 0.0, weights, want_mask=True, want_groups=False, want_status=False)
-        ctx.rv, ctx.fv, ctx.G, ctx.pool = rv, fv, G, pool
+        out = _paper_gap_fwd(fv, bins, weights, G, pool) if fold else None
+        ctx.fold = out is not None
+        if out is None:
+            out = _pool_fuse_fwd(fv, bins, G, pool, 0.0, weights, want_mask=True, want_groups=False, want_status=False)
+        ctx.rv, ctx.fv, ctx.G, ctx.pool, ctx.HW_r = rv, fv, G, pool, HW_r
         ctx.bstride, ctx.wstride = out.bin_stride, out.w_stride
         ctx.need_dr = any(t.requires_grad for t in r_t)
         ctx.n_r = n_r
-        ctx.save_for_backward(W.contiguous(), sr.x, out.bins, out.weights, out.S, out.mask)
-        ctx.mark_non_differentiable(sr.scores, sr.bins, weights)
-        return out.S.reshape(fv.view_shape), sr.scores, sr.bins, weights
+        ctx.save_for_backward(W.contiguous(), x, out.bins, out.weights, out.S, out.mask, R_out)
+        ctx.mark_non_differentiable(scores, bins, weights)
+        S = out.S if ctx.fold else out.S.reshape(fv.view_shape)
+        return S, scores, bins, weights
 
     @staticmethod
     def backward(ctx, dS, _ds, _db, _dw):
         L = C.lib()
-        W, x, bins_c, w_c, S, mask = ctx.saved_tensors
+        W, x, bins_c, w_c, S, mask, R_out = ctx.saved_tensors
         rv, fv, G, pool = ctx.rv, ctx.fv, ctx.G, ctx.pool
-        dS2 = dS.reshape(fv.B, fv.D).contiguous()
+        dS2 = dS.contiguous() if ctx.fold else dS.reshape(fv.B, fv.D).contiguous()
         dev = dS2.device
-        dF = _pool_fuse_bwd(dS2, fv, bins_c, ctx.bstride, w_c, ctx.wstride, mask, G, pool)
-        ws_bytes = L.gvcnn_view_score_bwd_workspace_bytes(rv.V, rv.D)
+        Cr = rv.D // ctx.HW_r
+        if ctx.fold:
+            dF = _paper_gap_bwd_f(dS2, fv, bins_c, ctx.bstride, w_c, ctx.wstride, mask, G, pool)
+        else:
+            dF = _pool_fuse_bwd(dS2, fv, bins_c, ctx.bstride, w_c, ctx.wstride, mask, G, pool)
+        ws_bytes = L.gvcnn_view_score_bwd_workspace_bytes(rv.V, Cr)
         n_dw, n_dx, n_W = fv.B * G, fv.B * fv.V, W.numel()
         scratch = torch.empty(n_dw + n_dx + n_W + rv.V + (ws_bytes + 3) // 4, dtype=torch.float32, device=dev)  # one allocation
         dweights = scratch[:n_dw].view(fv.B, G)
@@ -1110,33 +1170,132 @@ class _PaperModeFn(torch.autograd.Function):
         ws = scratch[n_dw + n_dx + n_W + rv.V:]
         dR_out, dR_views = (rv.empty_like() if ctx.need_dr else (None, None))
         with _on(dev):
-            C.check(L.gvcnn_pool_fuse_bwd_weights(fv.arg, _ptr(dS2), _ptr(S), _ptr(bins_c), ctx.bstride, _ptr(w_c),
-                                                  ctx.wstride, _ptr(dweights), fv.B, fv.V, fv.D, G, _POOL[pool],
-                                                  fv.layout, _dtype_code(fv.dtype), _stream()),
-                    "gvcnn_pool_fuse_bwd_weights")
+            if ctx.fold:
+                _paper_gap_bwd_weights(fv, dS2, S, bins_c, ctx.bstride, w_c, ctx.wstride, dweights, G, pool)
+            else:
+                C.check(L.gvcnn_pool_fuse_bwd_weights(fv.arg, _ptr(dS2), _ptr(S), _ptr(bins_c), ctx.bstride, _ptr(w_c),
+                                                      ctx.wstride, _ptr(dweights), fv.B, fv.V, fv.D, G, _POOL[pool],
+                                                      fv.layout, _dtype_code(fv.dtype), _stream()),
+                        "gvcnn_pool_fuse_bwd_weights")
             C.check(L.gvcnn_score_weight_bwd(_ptr(dweights), _ptr(bins_c), _ptr(x), _ptr(dx), fv.B, fv.V, G, _stream()),
                     "gvcnn_score_weight_bwd")
-            C.check(L.gvcnn_view_score_bwd(rv.arg, _ptr(dx), _ptr(W), _ptr(dW), _ptr(dbias),
-                                           dR_views.arg if dR_views is not None else None, _ptr(ws), ws_bytes,
-                                           rv.B, rv.V, rv.D, rv.layout, _dtype_code(rv.dtype), _stream()),
-                    "gvcnn_view_score_bwd")
+            if R_out is None:
+                C.check(L.gvcnn_view_score_bwd(rv.arg, _ptr(dx), _ptr(W), _ptr(dW), _ptr(dbias),
+                                               dR_views.arg if dR_views is not None else None, _ptr(ws), ws_bytes,
+                                               rv.B, rv.V, rv.D, rv.layout, _dtype_code(rv.dtype), _stream()),
+                        "gvcnn_view_score_bwd")
+            else:
+                # block3 maps: dW, db from the pooled R the score kernel wrote; dmaps = dx W / HW, only if asked for
+                C.check(L.gvcnn_view_score_bwd(_ptr(R_out), _ptr(dx), _ptr(W), _ptr(dW), _ptr(dbias), None, _ptr(ws),
+                                               ws_bytes, rv.B, rv.V, Cr, C.LAYOUT_BVD, C.F32, _stream()),
+                        "gvcnn_view_score_bwd")
+                if dR_views is not None:
+                    C.check(L.gvcnn_gap_score_bwd(_ptr(dx), _ptr(W), dR_views.arg, rv.B, rv.V, ctx.HW_r, Cr,
+                                                  rv.layout, _dtype_code(rv.dtype), _stream()), "gvcnn_gap_score_bwd")
         if dR_out is None:
             gr = (None,) * ctx.n_r
         else:
             gr = tuple(dR_out) if isinstance(dR_out, list) else (dR_out,)
         gf = tuple(dF) if isinstance(dF, list) else (dF,)
-        return (dW, dbias, None, None, None, None, None, None) + gr + gf
+        return (dW, dbias, None, None, None, None, None, None, None, None) + gr + gf
+
+
+def _fold_geometry(fv):
+    """(HW, C) of channel-last per-view maps, or None when the views have no spatial axes."""
+    if len(fv.view_shape) < 3:
+        return None
+    Cch = int(fv.view_shape[-1])
+    return fv.D // Cch, Cch
+
+
+def _paper_gap_fwd(fv, bins, weights, G, pool):
+    """Paper-mode pooling + fusion + GlobalAveragePooling2D in one pass (S_gap [B, C] in `S`), or None when
+    gvcnn_pool_fuse_gap_weighted_fwd does not cover the shapes."""
+    geo = _fold_geometry(fv)
+    if geo is None:
+        return None
+    HW, Cch = geo
+    L = C.lib()
+    dt = _dtype_code(fv.dtype)
+    bins_c, bstride = _bin_rows(bins, fv)
+    w_c, wstride = _weight_rows(weights, G, fv)
+    S_gap = torch.empty((fv.B, Cch), dtype=fv.dtype, device=fv.device)
+    mask = _tie_mask(fv, pool, True)
+    ws_bytes = L.gvcnn_pool_fuse_gap_workspace_bytes(fv.B, Cch, HW, dt)
+    ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=fv.device)
+    with _on(fv.device):
+        rc = L.gvcnn_pool_fuse_gap_weighted_fwd(fv.arg, _ptr(bins_c), bstride, _ptr(w_c), wstride, _ptr(S_gap),
+                                                _ptr(mask), None, _ptr(ws), ws_bytes, fv.B, fv.V, HW, Cch, G,
+                                                _POOL[pool], ctypes.c_float(0.0), fv.layout, dt, _stream())
+    if rc == C.E_UNSUPPORTED:
+        return None
+    C.check(rc, "gvcnn_pool_fuse_gap_weighted_fwd")
+    return _Pooled(S_gap, mask, None, None, bins_c, bstride, w_c, wstride)
+
+
+def _paper_gap_bwd_f(dS_gap, fv, bins, bin_stride, weights, w_stride, mask, G, pool):
+    """dF from the [B, C] gradient of S_gap (gvcnn_pool_fuse_gap_weighted_bwd)."""
+    HW, Cch = _fold_geometry(fv)
+    out, gv = fv.empty_like()
+    with _on(dS_gap.device):
+        C.check(C.lib().gvcnn_pool_fuse_gap_weighted_bwd(_ptr(dS_gap), _ptr(bins), bin_stride, _ptr(weights), w_stride,
+                                                         _ptr(mask), gv.arg, None, gv.B, gv.V, HW, Cch, G, _POOL[pool],
+                                                         gv.layout, _dtype_code(gv.dtype), _stream()),
+                "gvcnn_pool_fuse_gap_weighted_bwd")
+    return out
+
+
+def _paper_gap_bwd_weights(fv, dS_gap, S_gap, bins, bin_stride, weights, w_stride, dweights, G, pool):
+    """dL/dw_g from the [B, C] gradient of S_gap (gvcnn_pool_fuse_gap_bwd_weights), into `dweights` [B, G]."""
+    HW, Cch = _fold_geometry(fv)
+    L = C.lib()
+    dt = _dtype_code(fv.dtype)
+    ws_bytes = L.gvcnn_pool_fuse_gap_bwd_weights_workspace_bytes(fv.B, fv.V, HW, Cch, dt)
+    ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=fv.device)
+    C.check(L.gvcnn_pool_fuse_gap_bwd_weights(fv.arg, _ptr(dS_gap), _ptr(S_gap), _ptr(bins), bin_stride, _ptr(weights),
+                                              w_stride, _ptr(dweights), _ptr(ws), ws_bytes, fv.B, fv.V, HW, Cch, G,
+                                              _POOL[pool], fv.layout, dt, _stream()),
+            "gvcnn_pool_fuse_gap_bwd_weights")
+
+
+def _spatial_mean_views(t, lay):
+    """GlobalAveragePooling2D of block3 maps in a view argument (list of [N, h, w, C], or stacked): the pooled raw
+    descriptors, through torch so that autograd carries their gradient back to the maps."""
+    if lay == "list":
+        return [v.reshape(v.shape[0], -1, v.shape[-1]).mean(dim=1) for v in t]
+    x = t[0]
+    return x.reshape(x.shape[0], x.shape[1], -1, x.shape[-1]).mean(dim=2)
 
 
 def grouping_fusion_paper(raw_view_descriptors, W, b, final_view_descriptors, num_group, pool="max", layout=None,
-                          status=None):
+                          status=None, fold_gap=False):
     """Paper-mode grouping + fusion: group weight = mean discrimination score of the group's views, empty
     groups vanish; differentiable w.r.t. the view descriptors AND the score FC (W, b, optionally the raw
-    descriptors).  Returns (shape_descriptor, scores, bins, weights).  Per-shape scores/bins."""
+    descriptors).  Returns (shape_descriptor, scores, bins, weights).  Per-shape scores/bins.
+    raw_view_descriptors may be the pooled [.., C_raw] descriptors or the block3 maps themselves ([.., h, w, C_raw],
+    told apart by the trailing dimension as in score_bin): the GlobalAveragePooling2D in front of the score FC then
+    runs inside the score kernel, forward and backward.
+    fold_gap=True also folds the GlobalAveragePooling2D after the fusion (nets/model.py:163) into the pooling: the
+    shape descriptor returned is the pooled [N, C] one and the fused map is never written.  Shapes the folded kernels
+    do not cover run the unfolded path and average the map afterwards."""
     r_t, r_lay = _view_args(raw_view_descriptors, layout)
     f_t, f_lay = _view_args(final_view_descriptors, layout)
     _check_score_fc(W, b)
-    return _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, *r_t, *f_t)
+    HW_r = 1
+    if _is_raw_maps(raw_view_descriptors, W, layout):
+        HW_r = _raw_views(raw_view_descriptors, layout, int(W.shape[1]))[1]
+    if HW_r == 1 and not fold_gap:
+        return _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, 1, False, *r_t, *f_t)
+    try:
+        S, scores, bins, w = _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, HW_r, fold_gap,
+                                                *r_t, *f_t)
+    except _GapScoreUnsupported:
+        # block3 maps the GAP-folded score kernel does not cover: pool them here, autograd carries dR to the maps
+        pooled = _spatial_mean_views(r_t, r_lay)
+        r_t = tuple(pooled) if r_lay == "list" else (pooled,)
+        S, scores, bins, w = _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, 1, fold_gap,
+                                                *r_t, *f_t)
+    return (_spatial_mean(S) if fold_gap else S), scores, bins, w
 
 
 def _spatial_mean(S):
@@ -1171,11 +1330,11 @@ class GVCNNHead(torch.nn.Module):
 
     def forward(self, raw_view_descriptors, final_view_descriptors, process_group=None, check=False, fold_gap=False,
                 status=None, global_count=None):
-        """raw: post-GAP block3 features [N, V, C_raw] (or list of V [N, C_raw]);
-        final: list of V [N, h, w, C] maps or [N, V, h, w, C].  Returns
+        """raw: post-GAP block3 features [N, V, C_raw] (or list of V [N, C_raw]), or the block3 maps
+        [N, V, h, w, C_raw] themselves; final: list of V [N, h, w, C] maps or [N, V, h, w, C].  Returns
         (view_discrimination_scores, shape_descriptor, logits) like
-        nets/model.py:166.  fold_gap=True (reference-literal weights only) folds the
-        GlobalAveragePooling2D of nets/model.py:163 into the pooling kernel: the fused
+        nets/model.py:166.  fold_gap=True folds the GlobalAveragePooling2D of nets/model.py:163 into the
+        pooling kernels, in both weight modes (paper mode: grouping_fusion_paper(fold_gap=True)): the fused
         map is never written and the second return value is the pooled [N, C] descriptor."""
         if fold_gap and self.weight_mode == "count":
             sr = score_bin(raw_view_descriptors, self.score_kernel.detach(), self.score_bias.detach(),
@@ -1187,7 +1346,7 @@ class GVCNNHead(torch.nn.Module):
         if self.weight_mode == "score":
             S, scores, _, _ = grouping_fusion_paper(raw_view_descriptors, self.score_kernel, self.score_bias,
                                                     final_view_descriptors, self.num_group, pool=self.pool,
-                                                    status=status)
+                                                    status=status, fold_gap=fold_gap)
         else:
             S, sr = grouping_fusion(raw_view_descriptors, self.score_kernel.detach(), self.score_bias.detach(),
                                     final_view_descriptors, self.num_group, pool=self.pool,

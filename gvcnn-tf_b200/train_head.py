@@ -60,6 +60,7 @@ def build_flags():
     p.add_argument("--val_size", type=int, default=32)
     p.add_argument("--weight_mode", default="count", choices=["count", "score"])
     p.add_argument("--score_reduce", default="batch", choices=["batch", "shape"])
+    p.add_argument("--fold_gap", action="store_true")              # GAP after the fusion folded into the pooling
     p.add_argument("--seed", type=int, default=0)
     return p
 
@@ -232,7 +233,7 @@ def main(argv=None):
             if len(y) > 0 or (world > 1 and flags.score_reduce == "batch"):
                 # literal mode on a sharded batch: every rank bins the same GLOBAL batch mean (SURVEY.md 8e (2))
                 _, _, logits = head(raw, final, process_group=pg if flags.score_reduce == "batch" else None,
-                                    status=status,
+                                    status=status, fold_gap=flags.fold_gap,
                                     global_count=parallel.global_batch_size(flags.train_size, world, flags.batch_size, _step))
             if len(y) > 0:
                 loss = torch.nn.functional.cross_entropy(logits, y)
@@ -252,7 +253,7 @@ def main(argv=None):
         correct, cm = 0, torch.zeros((num_classes, num_classes), dtype=torch.int64)
         with torch.no_grad():
             for raw, final, y in val.batches(flags.val_batch_size):
-                _, _, logits = head(raw, final)        # validation runs un-sharded on every rank: local batch mean
+                _, _, logits = head(raw, final, fold_gap=flags.fold_gap)        # validation runs un-sharded on every rank: local batch mean
                 pred = logits.argmax(dim=1)
                 correct += int((pred == y).sum())
                 cm += confusion_matrix(y.cpu(), pred.cpu(), num_classes)

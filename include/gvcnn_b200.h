@@ -309,6 +309,22 @@ int gvcnn_pool_fuse_gap_bwd(const void *dS_gap, const int32_t *bins, int64_t bin
                             const uint8_t *tie_mask, void *dF, int32_t *status,
                             int B, int V, int HW, int C, int G, int pool,
                             int g_layout, int dtype, void *stream);
+/* The same two with caller-supplied group weights (weights / weight_stride_b as in
+ * gvcnn_pool_fuse_fwd; paper mode: the mean score of the group's views, empty_fill = 0).
+ * Null weights = gvcnn_pool_fuse_gap_fwd / _bwd.  The per-position fused value is
+ * gvcnn_pool_fuse_fwd's with the same weights, bit for bit (before the rounding to
+ * `dtype`).  Supported as above, with G <= 64 when weights are given. */
+int gvcnn_pool_fuse_gap_weighted_fwd(const void *F, const int32_t *bins, int64_t bin_stride_b,
+                                     const float *weights, int64_t weight_stride_b,
+                                     void *S_gap, uint8_t *tie_mask, int32_t *status,
+                                     void *workspace, size_t workspace_bytes,
+                                     int B, int V, int HW, int C, int G, int pool, float empty_fill,
+                                     int f_layout, int dtype, void *stream);
+int gvcnn_pool_fuse_gap_weighted_bwd(const void *dS_gap, const int32_t *bins, int64_t bin_stride_b,
+                                     const float *weights, int64_t weight_stride_b,
+                                     const uint8_t *tie_mask, void *dF, int32_t *status,
+                                     int B, int V, int HW, int C, int G, int pool,
+                                     int g_layout, int dtype, void *stream);
 
 /* --- paper mode: score-derived, differentiable group weights ---------------
  * No counterpart in the reference (its weight is 1 + count and its score FC gets
@@ -337,6 +353,33 @@ size_t gvcnn_view_score_bwd_workspace_bytes(int V, int C);
 int gvcnn_view_score_bwd(const void *R, const float *dx, const float *W, float *dW, float *dbias,
                          void *dR, void *workspace, size_t workspace_bytes,
                          int B, int V, int C, int r_layout, int dtype, void *stream);
+
+/* Paper mode on spatial maps, the global average pools folded in (D = HW * C, channel-last):
+ *   gvcnn_pool_fuse_gap_bwd_weights: gvcnn_pool_fuse_bwd_weights for S_gap = mean over the
+ *     HW positions of S (gvcnn_pool_fuse_gap_weighted_fwd's output) and its gradient
+ *     dS_gap [B, C] (both in `dtype`, 16-byte aligned):
+ *       dweights[b, g] = (A_g / HW - <dS_gap_b, S_gap_b>) / sum_w,
+ *       A_g = sum_c dS_gap[b, c] * sum_p P_g[b, p, c]      (0 for an empty group)
+ *     - the unfolded formula for dS[b, p, c] = dS_gap[b, c] / HW, without dS or S.  Reads F
+ *     once; fixed reduction order (deterministic).  workspace from
+ *     gvcnn_pool_fuse_gap_bwd_weights_workspace_bytes.  Supported: 16-byte aligned rows,
+ *     V in {4, 6, 8, 12, 16, 20}, C a multiple of 1024 (f32) / 2048 (bf16), G <= 255;
+ *     otherwise GVCNN_E_UNSUPPORTED.
+ *   gvcnn_gap_score_bwd: gradient of the GlobalAveragePooling2D in front of the score FC
+ *     (gvcnn_gap_score_bin_fwd): dmaps[b, v, p, c] = dx[b, v] * W[v, c] / HW, written in `dtype`
+ *     and m_layout; dx float32 [B, V], W float32 [V, C] (16-byte aligned).  Needs 16-byte
+ *     aligned rows and C a multiple of 16 bytes' worth of elements (else GVCNN_E_UNSUPPORTED).
+ *     dW / dbias of the score FC come from gvcnn_view_score_bwd on the pooled R_out that
+ *     gvcnn_gap_score_bin_fwd writes (float32, BVD). */
+size_t gvcnn_pool_fuse_gap_bwd_weights_workspace_bytes(int B, int V, int HW, int C, int dtype);
+int gvcnn_pool_fuse_gap_bwd_weights(const void *F, const void *dS_gap, const void *S_gap,
+                                    const int32_t *bins, int64_t bin_stride_b,
+                                    const float *weights, int64_t weight_stride_b, float *dweights,
+                                    void *workspace, size_t workspace_bytes,
+                                    int B, int V, int HW, int C, int G, int pool,
+                                    int f_layout, int dtype, void *stream);
+int gvcnn_gap_score_bwd(const float *dx, const float *W, void *dmaps, int B, int V, int HW, int C,
+                        int m_layout, int dtype, void *stream);
 
 /* --- host-buffer path (end-to-end) ---------------------------------------
  * One call = what one `sess.partial_run` pair does for this path in
