@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 SO_PATH = os.path.join(_HERE, "libgvcnn_sm100.so")
 
-F32, BF16 = 0, 1
+F32, BF16, F16 = 0, 1, 2
 LAYOUT_BVD, LAYOUT_VBD, LAYOUT_PTRS = 0, 1, 2
 POOL_MAX, POOL_MEAN = 0, 1
 SCORE_REDUCE_SHAPE, SCORE_REDUCE_BATCH = 0, 1

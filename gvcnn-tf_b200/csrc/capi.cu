@@ -61,7 +61,7 @@ int check_dims(int B, int V, int64_t D, int G, int dtype)
     if (B < 0 || V <= 0 || D <= 0 || G <= 0) return GVCNN_E_BAD_ARG;
     if (V > GVCNN_MAX_VIEWS) return GVCNN_E_TOO_MANY_VIEWS;
     if (G > GVCNN_MAX_GROUPS) return GVCNN_E_TOO_MANY_GROUPS;
-    if (dtype != GVCNN_F32 && dtype != GVCNN_BF16) return GVCNN_E_BAD_DTYPE;
+    if (dtype != GVCNN_F32 && dtype != GVCNN_BF16 && dtype != GVCNN_F16) return GVCNN_E_BAD_DTYPE;
     return B == 0 ? kEmptyBatch : 0;
 }
 
@@ -111,7 +111,7 @@ const char *gvcnn_strerror(int code)
     switch (code) {
     case 0: return "ok";
     case GVCNN_E_BAD_ARG: return "bad argument (null pointer or non-positive dimension)";
-    case GVCNN_E_BAD_DTYPE: return "unsupported dtype (GVCNN_F32 or GVCNN_BF16)";
+    case GVCNN_E_BAD_DTYPE: return "unsupported dtype (GVCNN_F32, GVCNN_BF16 or GVCNN_F16)";
     case GVCNN_E_BAD_LAYOUT: return "unsupported layout (BVD, VBD or PTRS)";
     case GVCNN_E_TOO_MANY_VIEWS: return "too many views (GVCNN_MAX_VIEWS) or view slab exceeds shared memory";
     case GVCNN_E_TOO_MANY_GROUPS: return "too many groups (GVCNN_MAX_GROUPS)";

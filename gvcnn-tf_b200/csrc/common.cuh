@@ -2,6 +2,7 @@
 #pragma once
 
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -485,6 +486,45 @@ template <> struct Elem<__nv_bfloat16> {
     }
     __device__ static __forceinline__ float to_float(__nv_bfloat16 v) { return __bfloat162float(v); }
     __device__ static __forceinline__ __nv_bfloat16 from_float(float v) { return __float2bfloat16_rn(v); }
+};
+// float16: the same 16-byte vectors and instruction shapes as bfloat16, with the f16 forms of each instruction.  Every
+// float16 value (subnormals included) is exactly a float32, so the widening is exact; only pack / from_float round.
+template <> struct Elem<__half> {
+    static constexpr int kVec = 8;
+    // a[e] = RN(a[e] + float(r_e)): add.rn.f32.f16 (FHADD with a half-select on the f16 operand) widens exactly
+    // inside the add, the mirror of Elem<__nv_bfloat16>::add_to
+    __device__ static __forceinline__ void add_to(float (&a)[8], const uint4 &r)
+    {
+        const uint32_t w[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+            asm("{\n\t.reg .b16 lo, hi;\n\tmov.b32 {lo, hi}, %2;\n\tadd.rn.f32.f16 %0, lo, %0;\n\t"
+                "add.rn.f32.f16 %1, hi, %1;\n\t}"
+                : "+f"(a[2 * i]), "+f"(a[2 * i + 1])
+                : "r"(w[i]));
+    }
+    __device__ static __forceinline__ void unpack(const uint4 &r, float (&f)[8])
+    {
+        const uint32_t w[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            const float2 p = __half22float2(*reinterpret_cast<const __half2 *>(&w[i]));  // exact
+            f[2 * i] = p.x;
+            f[2 * i + 1] = p.y;
+        }
+    }
+    __device__ static __forceinline__ uint4 pack(const float (&f)[8])
+    {
+        uint32_t w[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            const __half2 p = __floats2half2_rn(f[2 * i], f[2 * i + 1]);  // one cvt.rn.f16x2.f32
+            w[i] = *reinterpret_cast<const uint32_t *>(&p);
+        }
+        return make_uint4(w[0], w[1], w[2], w[3]);
+    }
+    __device__ static __forceinline__ float to_float(__half v) { return __half2float(v); }
+    __device__ static __forceinline__ __half from_float(float v) { return __float2half_rn(v); }
 };
 
 // ---- score epilogue (shared by score.cu and score_ring.cu) --------------------------

@@ -174,8 +174,13 @@ int launch_gap_score(const ViewPtrs &mp, int64_t m_sb, const float *W, const flo
     if (dtype == GVCNN_F32)
         return launch_gap_score_t<float>(mp, m_sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW, C, G, fuse_bin,
                                          edge_ulps, clamp, st);
-    return launch_gap_score_t<__nv_bfloat16>(mp, m_sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW, C, G,
-                                             fuse_bin, edge_ulps, clamp, st);
+    if (dtype == GVCNN_BF16)
+        return launch_gap_score_t<__nv_bfloat16>(mp, m_sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW, C, G,
+                                                 fuse_bin, edge_ulps, clamp, st);
+    if (dtype == GVCNN_F16)
+        return launch_gap_score_t<__half>(mp, m_sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW, C, G,
+                                          fuse_bin, edge_ulps, clamp, st);
+    return GVCNN_E_BAD_DTYPE;
 }
 
 }  // namespace gvcnn

@@ -141,7 +141,7 @@ int gvcnn_grouping_fusion_host(gvcnn_host_pipeline *pipe, const void *R_host, co
     if (B < 0 || V <= 0 || D <= 0 || G <= 0) return GVCNN_E_BAD_ARG;
     if (V > GVCNN_MAX_VIEWS) return GVCNN_E_TOO_MANY_VIEWS;
     if (G > GVCNN_MAX_GROUPS) return GVCNN_E_TOO_MANY_GROUPS;
-    if (dtype != GVCNN_F32 && dtype != GVCNN_BF16) return GVCNN_E_BAD_DTYPE;
+    if (dtype != GVCNN_F32 && dtype != GVCNN_BF16 && dtype != GVCNN_F16) return GVCNN_E_BAD_DTYPE;
     if (score_reduce != GVCNN_SCORE_REDUCE_SHAPE && score_reduce != GVCNN_SCORE_REDUCE_BATCH) return GVCNN_E_BAD_MODE;
     const bool batch_mode = score_reduce == GVCNN_SCORE_REDUCE_BATCH;
     // an empty local batch is a no-op, except in batch mode with an exchange: the other ranks wait for this one

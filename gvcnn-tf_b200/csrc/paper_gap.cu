@@ -212,7 +212,9 @@ int launch_gap_bwd_weights(const ViewPtrs &fp, int64_t f_sb, const void *dS_gap,
     default: return -1000;                                                                                          \
     }
     if (dtype == GVCNN_F32) { GVCNN_GBW_CASE(float) }
-    GVCNN_GBW_CASE(__nv_bfloat16)
+    if (dtype == GVCNN_BF16) { GVCNN_GBW_CASE(__nv_bfloat16) }
+    if (dtype == GVCNN_F16) { GVCNN_GBW_CASE(__half) }
+    return GVCNN_E_BAD_DTYPE;
 #undef GVCNN_GBW_CASE
 }
 
@@ -258,8 +260,12 @@ int launch_gap_score_bwd(const float *dx, const float *W, const ViewPtrs &dp, in
     cudaError_t err;
     if (dtype == GVCNN_F32)
         err = launch_pdl(gap_score_bwd_kernel<float>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
-    else
+    else if (dtype == GVCNN_BF16)
         err = launch_pdl(gap_score_bwd_kernel<__nv_bfloat16>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
+    else if (dtype == GVCNN_F16)
+        err = launch_pdl(gap_score_bwd_kernel<__half>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
+    else
+        return GVCNN_E_BAD_DTYPE;
     return (int)err;
 }
 

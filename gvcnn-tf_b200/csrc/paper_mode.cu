@@ -215,8 +215,12 @@ int launch_group_weight_grad(const ViewPtrs &fp, int64_t f_sb, const void *dS, c
     } while (0)
     if (dtype == GVCNN_F32) {
         if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_GWG(float, GVCNN_POOL_MAX); else GVCNN_LAUNCH_GWG(float, GVCNN_POOL_MEAN);
-    } else {
+    } else if (dtype == GVCNN_BF16) {
         if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_GWG(__nv_bfloat16, GVCNN_POOL_MAX); else GVCNN_LAUNCH_GWG(__nv_bfloat16, GVCNN_POOL_MEAN);
+    } else if (dtype == GVCNN_F16) {
+        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_GWG(__half, GVCNN_POOL_MAX); else GVCNN_LAUNCH_GWG(__half, GVCNN_POOL_MEAN);
+    } else {
+        return GVCNN_E_BAD_DTYPE;
     }
 #undef GVCNN_LAUNCH_GWG
     return (int)cudaGetLastError();
@@ -246,7 +250,10 @@ int launch_view_score_bwd(const ViewPtrs &rp, int64_t r_sb, const float *dx, con
             view_score_bwd_partial_kernel<T_, false><<<grid, 256, 0, st>>>(rp, r_sb, dx, W, partial, pbias, drp, \
                                                                           dr_sb, want_dr, B, V, C, NS);        \
     } while (0)
-    if (dtype == GVCNN_F32) GVCNN_LAUNCH_VSB(float); else GVCNN_LAUNCH_VSB(__nv_bfloat16);
+    if (dtype == GVCNN_F32) GVCNN_LAUNCH_VSB(float);
+    else if (dtype == GVCNN_BF16) GVCNN_LAUNCH_VSB(__nv_bfloat16);
+    else if (dtype == GVCNN_F16) GVCNN_LAUNCH_VSB(__half);
+    else return GVCNN_E_BAD_DTYPE;
 #undef GVCNN_LAUNCH_VSB
     int rc = (int)cudaGetLastError();
     if (rc) return rc;

@@ -179,8 +179,13 @@ int launch_pool_fuse_bwd(const void *dS, const int32_t *bins, int64_t bin_sb, co
     if (dtype == GVCNN_F32)
         return launch_bwd_t<float>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool,
                                    aligned16 && D % 4 == 0, st);
-    return launch_bwd_t<__nv_bfloat16>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool,
-                                       aligned16 && D % 8 == 0, st);
+    if (dtype == GVCNN_BF16)
+        return launch_bwd_t<__nv_bfloat16>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool,
+                                           aligned16 && D % 8 == 0, st);
+    if (dtype == GVCNN_F16)
+        return launch_bwd_t<__half>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool,
+                                    aligned16 && D % 8 == 0, st);
+    return GVCNN_E_BAD_DTYPE;
 }
 
 }  // namespace gvcnn

@@ -161,9 +161,9 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
     const uint32_t fm = plan.first_mask;
 
     if constexpr (E == 8 && POOL == GVCNN_POOL_MAX) {
-        // bf16: tie bits of an element pair share a register (bits 0..15 / 16..31 = sorted views 0..15
-        // of the even / odd element; me2b covers views 16..31); the group's value is rounded to bf16 and
-        // packed once per group, each view then only masks the packed pairs.
+        // 16-bit types: tie bits of an element pair share a register (bits 0..15 / 16..31 = sorted views 0..15
+        // of the even / odd element; me2b covers views 16..31); the group's value is rounded to T (Elem<T>::pack)
+        // and packed once per group, each view then only masks the packed pairs.
         uint32_t me2[4], me2b[4];
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
@@ -307,7 +307,7 @@ static int launch_bwd_fast_t(const void *dS, const int32_t *bins, int64_t bin_sb
                              int pool, cudaStream_t st)
 {
     if (D < 256 * Elem<T>::kVec) {
-        // bf16 at D = 1024: one 128-thread tile per shape (see pool_fwd_ring.cu); anything shorter: generic kernel
+        // 16-bit types at D = 1024: one 128-thread tile per shape (see pool_fwd_ring.cu); anything shorter: generic kernel
         if constexpr (Elem<T>::kVec == 8) {
             if (D < 128 * Elem<T>::kVec) return -1000;
             switch (V) {
@@ -353,7 +353,9 @@ int launch_pool_fuse_gap_bwd(const void *dOut, const int32_t *bins, int64_t bin_
     default: return -1000;                                                                                    \
     }
     if (dtype == GVCNN_F32) { GVCNN_GAPB_CASE(float) }
-    GVCNN_GAPB_CASE(__nv_bfloat16)
+    if (dtype == GVCNN_BF16) { GVCNN_GAPB_CASE(__nv_bfloat16) }
+    if (dtype == GVCNN_F16) { GVCNN_GAPB_CASE(__half) }
+    return GVCNN_E_BAD_DTYPE;
 #undef GVCNN_GAPB_CASE
 }
 
@@ -367,7 +369,11 @@ int launch_pool_fuse_bwd_fast(const void *dS, const int32_t *bins, int64_t bin_s
         return launch_bwd_fast_t<float>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool, st);
     }
     if (D % 8) return -1000;
-    return launch_bwd_fast_t<__nv_bfloat16>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool, st);
+    if (dtype == GVCNN_BF16)
+        return launch_bwd_fast_t<__nv_bfloat16>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool, st);
+    if (dtype == GVCNN_F16)
+        return launch_bwd_fast_t<__half>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool, st);
+    return GVCNN_E_BAD_DTYPE;
 }
 
 }  // namespace gvcnn

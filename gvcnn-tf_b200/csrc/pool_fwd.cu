@@ -250,10 +250,11 @@ pool_fuse_fwd_chunked_kernel(const ViewPtrs fp, const int64_t f_sb, const int32_
     int k0 = 0;
     auto mark_members = [&](int from, int to) {  // tie bits of sorted positions [from, to) of this chunk vs m
         if constexpr (E == 8 && POOL == GVCNN_POOL_MAX) {
-            // bf16: the group max is a bf16 value, so members are compared PACKED (set.eq.bf16x2, IEEE: -0 == +0,
-            // NaN != NaN - the same answers as the float32 compare below) - 5 operations per element pair instead
-            // of 8+; the V = 80 tie mask cost as much as the whole pooling pass (bf16, D = 2048: 234 -> 414 us).
-            const uint4 mp = Elem<T>::pack(m);  // exact: m is a max of bf16 values
+            // 16-bit types: the group max is a value of type T, so members are compared PACKED (set.eq.bf16x2 /
+            // set.eq.f16x2, IEEE: -0 == +0, NaN != NaN - the same answers as the float32 compare below) - 5 operations
+            // per element pair instead of 8+; the V = 80 tie mask cost as much as the whole pooling pass (bf16,
+            // D = 2048: 234 -> 414 us).
+            const uint4 mp = Elem<T>::pack(m);  // exact: m is a max of values of type T
             const uint32_t m2[4] = {mp.x, mp.y, mp.z, mp.w};
 #pragma unroll 1
             for (int jj = from; jj < to; ++jj) {
@@ -261,7 +262,7 @@ pool_fuse_fwd_chunked_kernel(const ViewPtrs fp, const int64_t f_sb, const int32_
                 const uint32_t w[4] = {r.x, r.y, r.z, r.w};
 #pragma unroll
                 for (int i = 0; i < 4; ++i) {
-                    const uint32_t eq = bf16x2_eq_mask(w[i], m2[i]);         // 0xFFFF per equal half
+                    const uint32_t eq = Pair16<T>::eq_mask2(w[i], m2[i]);   // 0xFFFF per equal half
                     const uint32_t two = (eq & 1u) | ((eq >> 8) & 0x100u);   // element 2i -> bit 0, element 2i+1 -> bit 8
                     pw[i >> 1] |= two << (16 * (i & 1) + (jj & 7));
                 }
@@ -463,8 +464,13 @@ int launch_pool_fuse_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, 
     if (dtype == GVCNN_F32)
         return launch_fwd_t<float>(fp, f_sb, bins, bin_sb, S, Pout, mask, weights, w_sb, status, B, V, D, G, pool, fill,
                                    aligned16 && D % 4 == 0, variant, st);
-    return launch_fwd_t<__nv_bfloat16>(fp, f_sb, bins, bin_sb, S, Pout, mask, weights, w_sb, status, B, V, D, G, pool, fill,
-                                       aligned16 && D % 8 == 0, variant, st);
+    if (dtype == GVCNN_BF16)
+        return launch_fwd_t<__nv_bfloat16>(fp, f_sb, bins, bin_sb, S, Pout, mask, weights, w_sb, status, B, V, D, G, pool,
+                                           fill, aligned16 && D % 8 == 0, variant, st);
+    if (dtype == GVCNN_F16)
+        return launch_fwd_t<__half>(fp, f_sb, bins, bin_sb, S, Pout, mask, weights, w_sb, status, B, V, D, G, pool, fill,
+                                    aligned16 && D % 8 == 0, variant, st);
+    return GVCNN_E_BAD_DTYPE;
 }
 
 }  // namespace gvcnn

@@ -166,7 +166,11 @@ int launch_pool_fuse_fwd_direct(const ViewPtrs &fp, int64_t f_sb, const int32_t 
         return launch_direct_t<float>(fp, f_sb, bins, bin_sb, S, mask, status, B, V, D, G, pool, fill, forced, early, st);
     }
     if (D % 8) return -1000;
-    return launch_direct_t<__nv_bfloat16>(fp, f_sb, bins, bin_sb, S, mask, status, B, V, D, G, pool, fill, forced, early, st);
+    if (dtype == GVCNN_BF16)
+        return launch_direct_t<__nv_bfloat16>(fp, f_sb, bins, bin_sb, S, mask, status, B, V, D, G, pool, fill, forced, early, st);
+    if (dtype == GVCNN_F16)
+        return launch_direct_t<__half>(fp, f_sb, bins, bin_sb, S, mask, status, B, V, D, G, pool, fill, forced, early, st);
+    return GVCNN_E_BAD_DTYPE;
 }
 
 }  // namespace gvcnn

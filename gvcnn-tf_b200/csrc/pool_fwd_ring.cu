@@ -61,7 +61,7 @@ pool_fuse_fwd_ring_kernel(const ViewPtrs fp, const int64_t f_sb, const int32_t *
     constexpr int P = (V + 7) / 8;
     constexpr int kMaxStages = 8;
     constexpr int TD = NCONS * E;
-    constexpr bool kPackedMax = (E == 8) && (POOL == GVCNN_POOL_MAX);  // bf16 max pooling
+    constexpr bool kPackedMax = (E == 8) && (POOL == GVCNN_POOL_MAX);  // 16-bit (bf16 / f16) max pooling
     constexpr uint32_t kRowStride = (uint32_t)NCONS * 16u;   // bytes between sorted rows in a slot
     constexpr uint32_t kStageBytes = kRowStride * (uint32_t)V;
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -304,7 +304,7 @@ static int launch_ring_t(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, 
     // smoothly than two (V = 20: forward 111.7 -> 109.5 us, with tie mask 130.3 -> 126.1 us); for V <= 12 the
     // narrow tiles (four CTAs per SM) measured the same as the wide ones.
     if (D < 256 * Elem<T>::kVec) {
-        // descriptors shorter than one 256-column tile.  bf16 at D = 1024 (a point of the BASELINE sweep) is 128 columns
+        // descriptors shorter than one 256-column tile.  16-bit types at D = 1024 (a point of the BASELINE sweep) are 128 columns
         // of 16 bytes: 128-consumer CTAs, narrow slots, deeper ring.  Anything shorter: generic kernel.
 #ifndef GVCNN_NARROW_MINB
 #define GVCNN_NARROW_MINB 4  // CTAs per SM of the narrow (128-consumer) ring for V <= 12: with 12-24 KB tiles two CTAs
@@ -348,7 +348,11 @@ int launch_pool_fuse_fwd_ring(const ViewPtrs &fp, int64_t f_sb, const int32_t *b
         return launch_ring_t<float>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, V, D, G, pool, fill, st);
     }
     if (D % 8) return -1000;
-    return launch_ring_t<__nv_bfloat16>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, V, D, G, pool, fill, st);
+    if (dtype == GVCNN_BF16)
+        return launch_ring_t<__nv_bfloat16>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, V, D, G, pool, fill, st);
+    if (dtype == GVCNN_F16)
+        return launch_ring_t<__half>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, V, D, G, pool, fill, st);
+    return GVCNN_E_BAD_DTYPE;
 }
 
 }  // namespace gvcnn

@@ -291,7 +291,9 @@ int launch_pool_fuse_gap_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bi
     default: return -1000;                                                                                    \
     }
     if (dtype == GVCNN_F32) { GVCNN_GAP_CASE(float) }
-    GVCNN_GAP_CASE(__nv_bfloat16)
+    if (dtype == GVCNN_BF16) { GVCNN_GAP_CASE(__nv_bfloat16) }
+    if (dtype == GVCNN_F16) { GVCNN_GAP_CASE(__half) }
+    return GVCNN_E_BAD_DTYPE;
 #undef GVCNN_GAP_CASE
 }
 

@@ -1,4 +1,4 @@
-// Shared pieces of the persistent TMA-ring kernel (pool_fwd_ring.cu): plan, packed-bf16 helpers, and the
+// Shared pieces of the persistent TMA-ring kernel (pool_fwd_ring.cu): plan, packed 16-bit helpers, and the
 // per-thread tile consumer.
 #pragma once
 
@@ -36,6 +36,29 @@ __device__ __forceinline__ uint32_t bf16x2_eq_mask(uint32_t a, uint32_t b)
 {
     return __heq2_mask(*reinterpret_cast<const __nv_bfloat162 *>(&a), *reinterpret_cast<const __nv_bfloat162 *>(&b));
 }
+__device__ __forceinline__ uint32_t f16x2_max(uint32_t a, uint32_t b)
+{
+    const __half2 r = __hmax2(*reinterpret_cast<const __half2 *>(&a), *reinterpret_cast<const __half2 *>(&b));
+    return *reinterpret_cast<const uint32_t *>(&r);
+}
+// 0xFFFF in each half where the f16 values compare equal (IEEE: -0 == +0, NaN != NaN)
+__device__ __forceinline__ uint32_t f16x2_eq_mask(uint32_t a, uint32_t b)
+{
+    return __heq2_mask(*reinterpret_cast<const __half2 *>(&a), *reinterpret_cast<const __half2 *>(&b));
+}
+
+// Packed pairs of a 16-bit element type, in that type's arithmetic.  The walks choose the packed code by element
+// width (kVec == 8); the operations on the packed values go through this trait, so each 16-bit type gets its own
+// instruction and a bf16 max is never applied to f16 bits.
+template <typename T> struct Pair16;
+template <> struct Pair16<__nv_bfloat16> {
+    __device__ static __forceinline__ uint32_t max2(uint32_t a, uint32_t b) { return bf16x2_max(a, b); }
+    __device__ static __forceinline__ uint32_t eq_mask2(uint32_t a, uint32_t b) { return bf16x2_eq_mask(a, b); }
+};
+template <> struct Pair16<__half> {
+    __device__ static __forceinline__ uint32_t max2(uint32_t a, uint32_t b) { return f16x2_max(a, b); }
+    __device__ static __forceinline__ uint32_t eq_mask2(uint32_t a, uint32_t b) { return f16x2_eq_mask(a, b); }
+};
 
 __device__ __forceinline__ void mbar_arrive(uint64_t *bar)
 {
@@ -57,7 +80,7 @@ __device__ __forceinline__ void ring_consume_tile(const unsigned char *col, cons
     constexpr int NW = (E + 3) / 4;
     constexpr int P = (V + 7) / 8;
     constexpr uint32_t kRowStride = ROWSTRIDE;
-    constexpr bool kPackedMax = (E == 8) && (POOL == GVCNN_POOL_MAX);  // bf16 max pooling
+    constexpr bool kPackedMax = (E == 8) && (POOL == GVCNN_POOL_MAX);  // 16-bit (bf16 / f16) max pooling
 #ifndef GVCNN_MEAN_CHUNKED
 #define GVCNN_MEAN_CHUNKED 1  // A/B builds: 0 = fully unrolled mean walk for every V (round 1)
 #endif
@@ -68,7 +91,7 @@ __device__ __forceinline__ void ring_consume_tile(const unsigned char *col, cons
 #ifndef GVCNN_MEAN_CHUNKED_MINV
 #define GVCNN_MEAN_CHUNKED_MINV 4
 #endif
-    // bf16 only: float32 mean is closer to HBM-bound and measured no better on this walk (see GVCNN_MEAN_CHUNKED_F32)
+    // 16-bit types only: float32 mean is closer to HBM-bound and measured no better on this walk (see GVCNN_MEAN_CHUNKED_F32)
     constexpr bool kChunkedMean = GVCNN_MEAN_CHUNKED && (POOL == GVCNN_POOL_MEAN) && (V % 4 == 0) && V >= GVCNN_MEAN_CHUNKED_MINV && (E == 8 || (GVCNN_MEAN_CHUNKED_F32 && V >= 16));
     // the plan is the same for every thread: pass it through a warp reduction so the compiler keeps it
     // in uniform registers and the per-view branches below are uniform branches
@@ -102,10 +125,11 @@ __device__ __forceinline__ void ring_consume_tile(const unsigned char *col, cons
 #pragma unroll
     for (int e = 0; e < E; ++e) acc[e] = acc0;
     if (active && kPackedMax) {
-        // bf16 max pooling: the max of bf16 values is exact in bf16, so the running group max stays
-        // packed (2 elements per register, max.bf16x2) and is widened to float32 only when a group
+        // 16-bit max pooling: the max of bf16 (f16) values is exact in that type, so the running group max stays
+        // packed (2 elements per register, max.bf16x2 / max.f16x2) and is widened to float32 only when a group
         // closes.  Tie bits of an element pair share a register: bits 0..15 / 16..31 = sorted views
         // 0..15 of the even / odd element (a second register set covers views 16..31).
+        if constexpr (kPackedMax) {
         uint4 raw[V];
 #pragma unroll
         for (int k = 0; k < V; ++k) raw[k] = *reinterpret_cast<const uint4 *>(col + k * kRowStride);
@@ -125,7 +149,7 @@ __device__ __forceinline__ void ring_consume_tile(const unsigned char *col, cons
                         const uint32_t xw[4] = {raw[kl].x, raw[kl].y, raw[kl].z, raw[kl].w};
 #pragma unroll
                         for (int i = 0; i < 4; ++i) {
-                            const uint32_t eq = bf16x2_eq_mask(xw[i], m2[i]);
+                            const uint32_t eq = Pair16<T>::eq_mask2(xw[i], m2[i]);
                             if (kl < 16) me2[i] |= eq & (0x00010001u << (kl & 15));
                             else me2b[i] |= eq & (0x00010001u << (kl & 15));
                         }
@@ -152,8 +176,8 @@ __device__ __forceinline__ void ring_consume_tile(const unsigned char *col, cons
                 }
             } else {
                 const uint4 r = raw[k < V ? k : 0];
-                m2[0] = bf16x2_max(m2[0], r.x); m2[1] = bf16x2_max(m2[1], r.y);
-                m2[2] = bf16x2_max(m2[2], r.z); m2[3] = bf16x2_max(m2[3], r.w);
+                m2[0] = Pair16<T>::max2(m2[0], r.x); m2[1] = Pair16<T>::max2(m2[1], r.y);
+                m2[2] = Pair16<T>::max2(m2[2], r.z); m2[3] = Pair16<T>::max2(m2[3], r.w);
                 ++cnt;
             }
         }
@@ -170,7 +194,7 @@ __device__ __forceinline__ void ring_consume_tile(const unsigned char *col, cons
                     const uint32_t xw[4] = {raw[k].x, raw[k].y, raw[k].z, raw[k].w};
 #pragma unroll
                     for (int i = 0; i < 4; ++i) {
-                        const uint32_t eq = bf16x2_eq_mask(xw[i], cm[i]);
+                        const uint32_t eq = Pair16<T>::eq_mask2(xw[i], cm[i]);
                         if (k < 16) me2[i] |= eq & (0x00010001u << (k & 15));
                         else me2b[i] |= eq & (0x00010001u << (k & 15));
                     }
@@ -186,8 +210,9 @@ __device__ __forceinline__ void ring_consume_tile(const unsigned char *col, cons
                 *reinterpret_cast<uint2 *>(mask + ((int64_t)p * B) * D + out_off) = make_uint2(w0, w1);
             }
         }
+        }
     } else if (active && kChunkedMean) {
-        // bf16 mean pooling is bound by instruction issue and latency (two CTAs of four consumer warps per SM), not by
+        // 16-bit mean pooling is bound by instruction issue and latency (two CTAs of four consumer warps per SM), not by
         // HBM, so this walk is built for a short instruction stream:
         //  * the sorted rows are walked CH at a time - an outer loop that is NOT unrolled around a body that is; the
         //    fully unrolled walk below replicates the group-close code V + 1 times (113 KB of SASS at V = 20, consumers

@@ -444,8 +444,13 @@ int launch_view_score(const ViewPtrs &rp, int64_t r_sb, const float *W, const fl
                                           fuse_bin, edge_ulps, clamp, st);
     }
     const bool vec = aligned16 && (C % 8 == 0) && ((reinterpret_cast<uintptr_t>(W) & 15) == 0);
-    return launch_view_score_t<__nv_bfloat16>(rp, r_sb, W, bias, x, xabs, scores, bins, flags, status, B, V, C, G,
-                                              vec, fuse_bin, edge_ulps, clamp, st);
+    if (dtype == GVCNN_BF16)
+        return launch_view_score_t<__nv_bfloat16>(rp, r_sb, W, bias, x, xabs, scores, bins, flags, status, B, V, C, G,
+                                                  vec, fuse_bin, edge_ulps, clamp, st);
+    if (dtype == GVCNN_F16)
+        return launch_view_score_t<__half>(rp, r_sb, W, bias, x, xabs, scores, bins, flags, status, B, V, C, G, vec,
+                                           fuse_bin, edge_ulps, clamp, st);
+    return GVCNN_E_BAD_DTYPE;
 }
 
 int launch_batch_sum_x(const float *x, float *xsum, int B, int V, cudaStream_t st)

@@ -117,7 +117,9 @@ def _dtype_code(dt: torch.dtype) -> int:
         return C.F32
     if dt == torch.bfloat16:
         return C.BF16
-    raise TypeError("gvcnn_b200 supports float32 and bfloat16 descriptors, got %s" % dt)
+    if dt == torch.float16:
+        return C.F16
+    raise TypeError("gvcnn_b200 supports float32, bfloat16 and float16 descriptors, got %s" % dt)
 
 
 def _require_cuda(t: torch.Tensor, name: str):
@@ -309,7 +311,7 @@ def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulp
     """Per-view discrimination score and bin.
 
     R: raw view descriptors after GAP (nets/model.py:144), [B, V, C] ('bvd'),
-       [V, B, C] ('vbd') or a list of V [B, C] tensors; float32 or bfloat16.
+       [V, B, C] ('vbd') or a list of V [B, C] tensors; float32, bfloat16 or float16.
        Or the raw MAPS before the GAP ([B, V, h, w, C] / [V, B, h, w, C] / list of V [N, h, w, C], channel-last -
        end_points['resnet_v2_50/block3']): the GlobalAveragePooling2D of nets/model.py:144 then runs inside the
        score kernel (gvcnn_gap_score_bin_fwd) and the pooled [B, V, C] tensor is never written.

@@ -40,9 +40,12 @@ extern "C" {
 #define GVCNN_MAX_VIEWS 128      /* V: 6..80 in the reference's sweeps           */
 #define GVCNN_MAX_GROUPS 4096    /* num_group; the reference only ever uses 10   */
 
-/* dtype of R / F / S / dS / dF.  Arithmetic is always float32. */
+/* dtype of R / F / S / dS / dF.  Arithmetic is always float32.  The two 16-bit
+ * types (bf16, f16) have the same kernels, shapes and restrictions: inputs are
+ * widened exactly, the single rounding is at the output. */
 #define GVCNN_F32 0
 #define GVCNN_BF16 1
+#define GVCNN_F16 2
 
 /* layout of a per-view tensor X (R, F or dF)
  *   BVD : one array [B, V, D]     (north_star's shape-major layout)
@@ -113,7 +116,7 @@ int gvcnn_check_device(void);
  * nets/model.py:144-145 (V separate FC layers: W [V, C] float32, bias [V]).
  * x[b, v] = sum_c R[b, v, c] * W[v, c] + bias[v], one warp per (shape, view)
  * row, fixed summation order (see DESIGN.md "score kernel").
- * R: [B,V,C] / [V,B,C] / V pointers (r_layout), dtype f32 or bf16.
+ * R: [B,V,C] / [V,B,C] / V pointers (r_layout), dtype f32, bf16 or f16.
  * x: float32 [B, V].  xabs (nullable): float32 [B, V], sum_c |R W| + |bias| - the
  * input of the a-priori order-sensitivity report (GVCNN_FLAG_ORDER_EDGE), summed
  * over the batch with gvcnn_batch_sum_x and handed to gvcnn_score_bin. */
@@ -177,13 +180,13 @@ int gvcnn_score_bin_fwd(const void *R, const float *W, const float *bias,
  * reference: end_points['resnet_v2_50/block3'], [N, 10, 10, 1024] per view).
  *   R[b, v, c] = (sum over the HW positions, fixed order) / HW   (tf.reduce_mean)
  *   x[b, v]    = sum_c R[b, v, c] * W[v, c] + bias[v]             (float32 maps: == gvcnn_view_score_fwd on R, bit
- *                for bit; bf16 maps: the same fixed order with the bf16 kernels' lane-to-channel mapping)
+ *                for bit; 16-bit maps: the same fixed order with the 16-bit kernels' lane-to-channel mapping)
  * fuse_bin != 0: also scores / bins / flags [B, V] like gvcnn_score_bin_fwd (per-shape
  * mode; x may be null); fuse_bin == 0: only x (feed gvcnn_batch_sum_x / gvcnn_score_bin
  * for the literal batch mode; scores / bins may be null).  R_out (nullable): the
  * pooled raw descriptor, float32 [B, V, C].  The [B, V, C] tensor is otherwise never
  * written.  Supported: 16-byte aligned rows and C = 512 / 1024 (f32), 1024 / 2048
- * (bf16); anything else returns GVCNN_E_UNSUPPORTED (pool first, then
+ * (16-bit types); anything else returns GVCNN_E_UNSUPPORTED (pool first, then
  * gvcnn_score_bin_fwd). */
 int gvcnn_gap_score_bin_fwd(const void *maps, const float *W, const float *bias, float *R_out,
                             float *x, float *scores, int32_t *bins, int32_t *flags, int32_t *status,
@@ -294,7 +297,7 @@ int gvcnn_grouping_fusion_batch_fwd(const void *R, const float *W, const float *
  * exactly gvcnn_pool_fuse_fwd's; positions are added in order (split into a few
  * ascending chunks for parallelism, see gvcnn_pool_fuse_gap_workspace_bytes),
  * then divided by HW.  Supported: 16-byte aligned rows, V in {4, 6, 8, 12, 16, 20},
- * C a multiple of 1024 (f32) / 2048 (bf16), G <= 255, the reference's own
+ * C a multiple of 1024 (f32) / 2048 (16-bit types), G <= 255, the reference's own
  * weights; anything else returns GVCNN_E_UNSUPPORTED (use gvcnn_pool_fuse_fwd
  * and pool afterwards).  tie_mask as in gvcnn_pool_fuse_fwd ([ceil(V/8), B, D]).
  * gvcnn_pool_fuse_gap_bwd: dS_gap [B, C] -> dF (dS[b,p,c] = dS_gap[b,c] / HW is
@@ -363,7 +366,7 @@ int gvcnn_view_score_bwd(const void *R, const float *dx, const float *W, float *
  *     - the unfolded formula for dS[b, p, c] = dS_gap[b, c] / HW, without dS or S.  Reads F
  *     once; fixed reduction order (deterministic).  workspace from
  *     gvcnn_pool_fuse_gap_bwd_weights_workspace_bytes.  Supported: 16-byte aligned rows,
- *     V in {4, 6, 8, 12, 16, 20}, C a multiple of 1024 (f32) / 2048 (bf16), G <= 255;
+ *     V in {4, 6, 8, 12, 16, 20}, C a multiple of 1024 (f32) / 2048 (16-bit types), G <= 255;
  *     otherwise GVCNN_E_UNSUPPORTED.
  *   gvcnn_gap_score_bwd: gradient of the GlobalAveragePooling2D in front of the score FC
  *     (gvcnn_gap_score_bin_fwd): dmaps[b, v, p, c] = dx[b, v] * W[v, c] / HW, written in `dtype`
