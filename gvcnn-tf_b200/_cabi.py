@@ -52,6 +52,7 @@ SIGNATURES = {
                                  _i, _i, _i64, _i, _i, _f, _i, _i, _vp]),
     "gvcnn_pool_fuse_bwd": (_i, [_vp, _vp, _i64, _vp, _i64, _vp, _vp, _vp,
                                  _i, _i, _i64, _i, _i, _i, _i, _vp]),
+    "gvcnn_view_pooling_bwd": (_i, [_vp, _vp, _i64, _vp, _vp, _vp, _i, _i, _i64, _i, _i, _i, _i, _vp]),
     "gvcnn_grouping_fusion_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                                        _i, _i, _i, _i64, _i, _i, _f, _i, _i, _i, _i, _i, _vp]),
     "gvcnn_grouping_fusion_batch_fwd": (_i, [_vp] * 13 + [_i, _i, _i, _i64, _i, _i, _i, _f, _i, _i, _i, _i, _i, _i64,

@@ -346,6 +346,37 @@ int gvcnn_pool_fuse_bwd(const void *dS, const int32_t *bins, int64_t bin_stride_
                                 static_cast<cudaStream_t>(stream));
 }
 
+// backward of view_pooling alone: one gradient per group descriptor, dP [G, B, D]
+int gvcnn_view_pooling_bwd(const void *dP, const int32_t *bins, int64_t bin_stride_b, const uint8_t *tie_mask, void *dF,
+                           int32_t *status, int B, int V, int64_t D, int G, int pool, int g_layout, int dtype,
+                           void *stream)
+{
+    int rc = check_dims(B, V, D, G, dtype);
+    if (rc) return rc == kEmptyBatch ? 0 : rc;
+    if (!dP || !bins || bin_stride_b < 0) return GVCNN_E_BAD_ARG;
+    const int variant = GVCNN_POOL_VARIANT_OF(pool);
+    pool &= 0xff;
+    if ((pool != GVCNN_POOL_MAX && pool != GVCNN_POOL_MEAN) || variant > 4) return GVCNN_E_BAD_MODE;
+    if (pool == GVCNN_POOL_MAX && !tie_mask) return GVCNN_E_BAD_ARG;
+    const size_t es = elt_size(dtype);
+    if (!is_aligned(dP, es) || !is_aligned(bins, 4)) return GVCNN_E_MISALIGNED;
+    ViewPtrs gp;
+    int64_t sb;
+    bool al;
+    rc = make_view_ptrs(dF, g_layout, dtype, B, V, D, gp, sb, al);
+    if (rc) return rc;
+    al = al && is_aligned(dP, 16) && (D * es) % 16 == 0 && (!tie_mask || is_aligned(tie_mask, 8));
+    const bool forced_fast = variant == 3 || variant == 4;
+    if (al && (variant == 0 || forced_fast)) {
+        rc = launch_view_pooling_bwd_fast(dP, bins, bin_stride_b, tie_mask, gp, sb, status, B, V, D, G, pool, dtype,
+                                          static_cast<cudaStream_t>(stream));
+        if (rc != -1000) return rc;
+    }
+    if (forced_fast) return GVCNN_E_UNSUPPORTED;
+    return launch_view_pooling_bwd(dP, bins, bin_stride_b, tie_mask, gp, sb, status, B, V, D, G, pool, dtype, al,
+                                   static_cast<cudaStream_t>(stream));
+}
+
 // ---------------------------------------------------------------------------
 // whole forward in one call: score + bin, then pool + fuse, chained with programmatic dependent launch
 // ---------------------------------------------------------------------------

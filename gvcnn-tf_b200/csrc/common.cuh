@@ -654,5 +654,11 @@ int launch_pool_fuse_bwd(const void *dS, const int32_t *bins, int64_t bin_sb, co
                          const float *weights, int64_t w_sb,
                          const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
                          int pool, int dtype, bool aligned16, cudaStream_t st);
+int launch_view_pooling_bwd_fast(const void *dP, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
+                                 const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
+                                 int pool, int dtype, cudaStream_t st);
+int launch_view_pooling_bwd(const void *dP, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
+                            const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
+                            int pool, int dtype, bool aligned16, cudaStream_t st);
 
 }  // namespace gvcnn

@@ -17,6 +17,11 @@
 // writes the V matching 16-byte pieces of dF with streaming stores; its mask
 // bytes sit in a private shared-memory slot so they can be indexed by sorted
 // view position without spilling.
+//
+// GRP (gvcnn_view_pooling_bwd): the gradient of each group descriptor, dP [G, B, D], instead of dS - what
+// TF autodiff of nets/model.py:62-74 alone derives:
+//     max : dF_v = (1 / num_selected) * dP_g | 0      mean: dF_v = dP_g / n_g
+// Each group's row is read when the walk reaches the group; empty groups' rows are never read.
 #include "common.cuh"
 
 namespace gvcnn {
@@ -41,7 +46,7 @@ __device__ __forceinline__ uint32_t byte_msb_to_mask(uint32_t msb4, int e)
     return r;
 }
 
-template <typename T, bool VEC, int POOL>
+template <typename T, bool VEC, int POOL, bool GRP>
 __global__ void pool_fuse_bwd_kernel(const T *__restrict__ dS, const int32_t *__restrict__ bins,
                                      const int64_t bin_sb, const uint8_t *__restrict__ mask,
                                      const float *__restrict__ weights, const int64_t w_sb, const ViewPtrs gp,
@@ -69,7 +74,9 @@ __global__ void pool_fuse_bwd_kernel(const T *__restrict__ dS, const int32_t *__
 
     float t[E];
     if (active) {
-        if constexpr (VEC) {
+        if constexpr (GRP) {
+            // per group, in the walk below
+        } else if constexpr (VEC) {
             Elem<T>::unpack(ldg_stream_16(dS + off), t);
         } else {
             t[0] = Elem<T>::to_float(dS[off]);
@@ -85,18 +92,26 @@ __global__ void pool_fuse_bwd_kernel(const T *__restrict__ dS, const int32_t *__
     build_plan(plan, bins + (int64_t)b * bin_sb, V, G, status, weights ? weights + (int64_t)b * w_sb : nullptr);
     if (!active) return;
 
-    const float sumw = plan.sumw;
+    if constexpr (!GRP) {
+        const float sumw = plan.sumw;
 #pragma unroll
-    for (int e = 0; e < E; ++e) t[e] = __fdiv_rn(t[e], sumw);
+        for (int e = 0; e < E; ++e) t[e] = __fdiv_rn(t[e], sumw);
+    }
     const int64_t row_off = ((int64_t)b * g_sb + d0 + e0) * (int64_t)sizeof(T);
 
     int k = 0;
     while (k < V) {
         const int len = plan.glen[k];
-        const float w = plan.gw[k];
         float val[E];
+        if constexpr (GRP) {  // dP_g takes the place of g1
+            const int64_t goff = ((int64_t)plan.gbin[k] * B + b) * D + d0 + e0;
+            if constexpr (VEC) Elem<T>::unpack(ldg_stream_16(dS + goff), val);
+            else val[0] = Elem<T>::to_float(dS[goff]);
+        } else {
+            const float w = plan.gw[k];
 #pragma unroll
-        for (int e = 0; e < E; ++e) val[e] = __fmul_rn(t[e], w);
+            for (int e = 0; e < E; ++e) val[e] = __fmul_rn(t[e], w);
+        }
         if constexpr (POOL == GVCNN_POOL_MAX) {
             // pass 1: how many views of the group attain the max, per element (byte-parallel counters)
             uint32_t cnt[NW];
@@ -146,7 +161,7 @@ __global__ void pool_fuse_bwd_kernel(const T *__restrict__ dS, const int32_t *__
 template <typename T>
 static int launch_bwd_t(const void *dS, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
                         const float *weights, int64_t w_sb, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
-                        int pool, bool vec, cudaStream_t st)
+                        int pool, bool vec, cudaStream_t st, bool grp = false)
 {
     const int E = vec ? Elem<T>::kVec : 1;
     int nt = 256;
@@ -158,16 +173,22 @@ static int launch_bwd_t(const void *dS, const int32_t *bins, int64_t bin_sb, con
     const int64_t tiles = (D + td - 1) / td;
     if ((int64_t)B * tiles > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
     const unsigned grid = (unsigned)(B * tiles);
-#define GVCNN_LAUNCH_BWD(VEC_, POOL_)                                                                       \
-    pool_fuse_bwd_kernel<T, VEC_, POOL_><<<grid, nt, smem, st>>>(static_cast<const T *>(dS), bins, bin_sb, \
-                                                                 mask, weights, w_sb, gp, g_sb, status, B, \
-                                                                 V, D, G,                                  \
-                                                                 (int)tiles)
-    if (vec) {
-        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_BWD(true, GVCNN_POOL_MAX); else GVCNN_LAUNCH_BWD(true, GVCNN_POOL_MEAN);
+#define GVCNN_LAUNCH_BWD(VEC_, POOL_, GRP_)                                                                  \
+    pool_fuse_bwd_kernel<T, VEC_, POOL_, GRP_><<<grid, nt, smem, st>>>(static_cast<const T *>(dS), bins, bin_sb, \
+                                                                       mask, weights, w_sb, gp, g_sb, status, B, \
+                                                                       V, D, G,                                  \
+                                                                       (int)tiles)
+#define GVCNN_LAUNCH_BWD_P(VEC_, GRP_)                                                                         \
+    do {                                                                                                       \
+        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_BWD(VEC_, GVCNN_POOL_MAX, GRP_);                              \
+        else GVCNN_LAUNCH_BWD(VEC_, GVCNN_POOL_MEAN, GRP_);                                                    \
+    } while (0)
+    if (grp) {
+        if (vec) GVCNN_LAUNCH_BWD_P(true, true); else GVCNN_LAUNCH_BWD_P(false, true);
     } else {
-        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_BWD(false, GVCNN_POOL_MAX); else GVCNN_LAUNCH_BWD(false, GVCNN_POOL_MEAN);
+        if (vec) GVCNN_LAUNCH_BWD_P(true, false); else GVCNN_LAUNCH_BWD_P(false, false);
     }
+#undef GVCNN_LAUNCH_BWD_P
 #undef GVCNN_LAUNCH_BWD
     return (int)cudaGetLastError();
 }
@@ -185,6 +206,23 @@ int launch_pool_fuse_bwd(const void *dS, const int32_t *bins, int64_t bin_sb, co
     if (dtype == GVCNN_F16)
         return launch_bwd_t<__half>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool,
                                     aligned16 && D % 8 == 0, st);
+    return GVCNN_E_BAD_DTYPE;
+}
+
+// gvcnn_view_pooling_bwd, generic path: any V, unaligned or short rows, the scalar layout
+int launch_view_pooling_bwd(const void *dP, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
+                            const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
+                            int pool, int dtype, bool aligned16, cudaStream_t st)
+{
+    if (dtype == GVCNN_F32)
+        return launch_bwd_t<float>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool,
+                                   aligned16 && D % 4 == 0, st, true);
+    if (dtype == GVCNN_BF16)
+        return launch_bwd_t<__nv_bfloat16>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool,
+                                           aligned16 && D % 8 == 0, st, true);
+    if (dtype == GVCNN_F16)
+        return launch_bwd_t<__half>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool,
+                                    aligned16 && D % 8 == 0, st, true);
     return GVCNN_E_BAD_DTYPE;
 }
 

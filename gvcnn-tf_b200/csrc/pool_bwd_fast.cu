@@ -10,7 +10,21 @@
 // reciprocal from a shared table, two multiplies) is shared by the group's members; per view only a bit
 // test + select per element and one 128-bit streaming store remain.  Used when rows are 16-byte
 // aligned, V is one of the instantiated view counts and the reference's own group weights are wanted.
+//
+// GRP (gvcnn_view_pooling_bwd): the gradient arrives per group, dP [G, B, D] (the layout of the forward's
+// group_desc), instead of as one dS: at a group start the thread loads its 16 bytes of that group's dP row
+// and skips the fusion's scaling; max: dF_v = (1 / num_selected) * dP_g | 0, mean: dF_v = dP_g / n_g.  Empty
+// groups' rows are never read.
+#include <type_traits>
+
 #include "common.cuh"
+
+// GRP, max pooling (the walks with a compile-time k): 1 = issue the loads of all the shape's group rows right after
+// the barrier, before the first store; 0 = load each row at its group start.  A/B builds only (-D); the mean walk is a
+// rolled loop and always loads at the group start.
+#ifndef GVCNN_VP_BWD_PRELOAD
+#define GVCNN_VP_BWD_PRELOAD 0
+#endif
 
 namespace gvcnn {
 
@@ -20,6 +34,10 @@ struct __align__(16) BwdPlan {
     float gw[32];                   // caller-supplied weights only: weight of the group of sorted view k
     float sumw;                     // caller-supplied weights only: sum of all G weights (left to right)
     uint32_t first_mask;            // bit k: sorted view k starts a group
+};
+// GRP kernels only (a separate type, so the existing kernels' shared-memory layout stays as it was)
+struct __align__(16) BwdPlanGrp : BwdPlan {
+    unsigned long long grow[32];    // at a group start k: byte address of the group's dP row at this tile's d0
 };
 
 // prmt.b32, generic mode: a selector nibble with bit 3 set replicates the top bit of the selected byte over the
@@ -33,7 +51,7 @@ __device__ __forceinline__ uint32_t prmt_sign(const uint32_t a, const uint32_t s
 
 // GAP: dS is the gradient of the global average pool that follows the fusion, [B, C] (D = HW * C,
 // channel-last): dS[b, p, c] = dOut[b, c] / HW (tf.reduce_mean's gradient), never materialised.
-template <typename T, int POOL, int V, int NT, bool GAP, bool WTS, int UPC>
+template <typename T, int POOL, int V, int NT, bool GAP, bool WTS, int UPC, bool GRP>
 __global__ void __launch_bounds__(NT)
 pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ bins, const int64_t bin_sb,
                           const uint8_t *__restrict__ mask, const float *__restrict__ weights, const int64_t w_sb,
@@ -46,9 +64,11 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
     constexpr int P = (V + 7) / 8;
     constexpr int TD = NT * E;
     static_assert(UPC * 32 <= NT, "one planning warp per unit");
+    static_assert(!GRP || (!GAP && !WTS), "per-group gradients take no GAP and no weights");
+    using PlanT = std::conditional_t<GRP, BwdPlanGrp, BwdPlan>;
     // A CTA handles UPC consecutive (shape, tile) units: their loads are all in flight before the one barrier, and
     // warp i plans unit i, so the per-CTA costs (launch slot, barrier, reciprocal table) are paid once per UPC tiles.
-    __shared__ BwdPlan plans[UPC];
+    __shared__ PlanT plans[UPC];
     __shared__ float rcp_tab[V + 1];  // rcp_tab[n] = 1 / n, IEEE division
 
     const int u0 = blockIdx.x * UPC;
@@ -69,7 +89,9 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
         const int64_t off = (int64_t)b * D + d0 + e0;
         raws[i] = make_uint4(0u, 0u, 0u, 0u);
         if (actives[i]) {
-            if constexpr (GAP) raws[i] = *reinterpret_cast<const uint4 *>(dS + (int64_t)b * C + (int)((d0 + e0) % C));
+            if constexpr (GRP) {
+                // dP rows are known only once the plan is: loaded at each group start below
+            } else if constexpr (GAP) raws[i] = *reinterpret_cast<const uint4 *>(dS + (int64_t)b * C + (int)((d0 + e0) % C));
             else raws[i] = ldg_stream_16(dS + off);
             if constexpr (POOL == GVCNN_POOL_MAX) {
 #pragma unroll
@@ -90,7 +112,7 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
 
     // ---- plans: warp i ranks the views of unit i by (bin, view)
     if ((int)(threadIdx.x >> 5) < UPC && u0 + (int)(threadIdx.x >> 5) < num_units) {
-        BwdPlan &plan = plans[threadIdx.x >> 5];
+        PlanT &plan = plans[threadIdx.x >> 5];
         const int un = u0 + (int)(threadIdx.x >> 5);
         const int b = un / tiles_per_shape;
         const int tile = un - b * tiles_per_shape;
@@ -123,6 +145,9 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
             plan.seg[k] = (n >= 32 ? 0xffffffffu : ((1u << n) - 1u)) << start;
             plan.rowptr[k] = (unsigned long long)(gp.p[lane] + ((int64_t)b * g_sb + d0) * (int64_t)sizeof(T));
             if constexpr (WTS) plan.gw[k] = __ldg(weights + (int64_t)b * w_sb + bin);
+            if constexpr (GRP)
+                if (same_before == 0)
+                    plan.grow[k] = (unsigned long long)(dS + ((int64_t)bin * B + b) * D + d0);
         }
         if (lane == 0) {
             plan.first_mask = fm;
@@ -139,7 +164,7 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
 #pragma unroll
     for (int ui = 0; ui < UPC; ++ui) {
     if (!actives[ui]) continue;
-    const BwdPlan &plan = plans[ui];
+    const PlanT &plan = plans[ui];
     const uint4 raw = raws[ui];
     uint32_t (&pwd)[P][NW] = pwds[ui];
     constexpr bool wts = WTS;  // caller-supplied group weights: compiled out of the default instantiation
@@ -151,12 +176,28 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
 #pragma unroll
         for (int e = 0; e < E; ++e) t[e] = __fdiv_rn(t[e], (float)HW);  // gradient of the mean over positions
     }
-    if constexpr (wts) {  // g0 = dS / sum_w
+    if constexpr (GRP) {
+        // t is loaded per group below
+    } else if constexpr (wts) {  // g0 = dS / sum_w
 #pragma unroll
         for (int e = 0; e < E; ++e) t[e] = __fdiv_rn(t[e], sumw);
     } else {
         div_vec_by_rcp(t, sumw, rcp_sumw);  // one range test for the vector, IEEE fall-back out of line
     }
+    // g1 of the group starting at sorted position k, element e: g0 * w_g; GRP: dP_g itself, loaded by group_start(k)
+    constexpr bool preload = GRP && GVCNN_VP_BWD_PRELOAD && POOL == GVCNN_POOL_MAX;
+    uint4 graw[preload ? V : 1];
+    if constexpr (preload) {
+#pragma unroll
+        for (int k = 0; k < V; ++k)
+            if (k == 0 || ((plan.first_mask >> k) & 1u))
+                graw[k] = ldg_stream_16(reinterpret_cast<const char *>(plan.grow[k]) + thread_off);
+    }
+    auto group_start = [&](const int k) {
+        if constexpr (preload) Elem<T>::unpack(graw[k], t);
+        else if constexpr (GRP) Elem<T>::unpack(ldg_stream_16(reinterpret_cast<const char *>(plan.grow[k]) + thread_off), t);
+    };
+    auto g1 = [&](const int e, const float w) { return GRP ? t[e] : __fmul_rn(t[e], w); };
 
     const uint32_t fm = plan.first_mask;
 
@@ -175,20 +216,21 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
 #pragma unroll
         for (int k = 0; k < V; ++k) {
             if (k == 0 || ((fm >> k) & 1u)) {  // uniform: a group starts here
+                group_start(k);
                 const uint32_t seg = plan.seg[k];
                 const int n = __popc(seg);
                 const float w = wts ? plan.gw[k] : (float)(1 + n);
                 float val[E];
                 if (n == 1) {  // uniform: a group of one view - num_selected is 1 wherever the value is kept
 #pragma unroll
-                    for (int e = 0; e < E; ++e) val[e] = __fmul_rn(t[e], w);  // (1 / 1) * g1 = g1 exactly
+                    for (int e = 0; e < E; ++e) val[e] = g1(e, w);  // (1 / 1) * g1 = g1 exactly
                 } else {
 #pragma unroll
                     for (int e = 0; e < E; ++e) {
                         const uint32_t half = (e & 1) ? 0xffff0000u : 0x0000ffffu;
                         const uint32_t lo = (seg & 0xffffu) * 0x00010001u, hi = (seg >> 16) * 0x00010001u;
                         const int nsel = __popc(me2[e >> 1] & lo & half) + (V > 16 ? __popc(me2b[e >> 1] & hi & half) : 0);
-                        val[e] = __fmul_rn(rcp_tab[nsel], __fmul_rn(t[e], w));
+                        val[e] = __fmul_rn(rcp_tab[nsel], g1(e, w));
                     }
                 }
                 const uint4 pk = Elem<T>::pack(val);
@@ -214,12 +256,13 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
 #pragma unroll 1
         for (int k = 0; k < V; ++k) {
             if ((fm >> k) & 1u) {  // uniform: a group starts here (bit 0 is always set)
+                group_start(k);
                 const int n = __popc(plan.seg[k]);
                 const float w = wts ? plan.gw[k] : (float)(1 + n);
                 const float rn = rcp_tab[n];
                 float val[E];
 #pragma unroll
-                for (int e = 0; e < E; ++e) val[e] = __fmul_rn(t[e], w);
+                for (int e = 0; e < E; ++e) val[e] = g1(e, w);
                 if ((n & (n - 1)) == 0) {  // uniform branch
 #pragma unroll
                     for (int e = 0; e < E; ++e) val[e] = __fmul_rn(val[e], rn);
@@ -244,13 +287,14 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
 #pragma unroll
         for (int k = 0; k < V; ++k) {
             if (k == 0 || ((fm >> k) & 1u)) {  // uniform: a group starts here
+                group_start(k);
                 const uint32_t seg = plan.seg[k];
                 const int n = __popc(seg);
                 const float w = wts ? plan.gw[k] : (float)(1 + n);
 #pragma unroll
                 for (int e = 0; e < E; ++e) {
                     const int nsel = __popc(me[e] & seg);
-                    val[e] = __fmul_rn(rcp_tab[nsel], __fmul_rn(t[e], w));  // (1 / num_selected) * g1; nsel == 0 only for NaN
+                    val[e] = __fmul_rn(rcp_tab[nsel], g1(e, w));  // (1 / num_selected) * g1; nsel == 0 only for NaN
                 }
             }
             float o[E];
@@ -266,7 +310,7 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
 template <typename T, int V, int NT = 256>
 static int launch_bwd_fast_v(const void *dS, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
                              const float *weights, int64_t w_sb, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int64_t D, int G, int pool,
-                             cudaStream_t st, int gapC = 0, int gapHW = 0)
+                             cudaStream_t st, int gapC = 0, int gapHW = 0, bool grp = false)
 {
     constexpr int E = Elem<T>::kVec;
     const int64_t td = (int64_t)NT * E;
@@ -278,22 +322,24 @@ static int launch_bwd_fast_v(const void *dS, const int32_t *bins, int64_t bin_sb
     constexpr int upc = 1;
     const unsigned grid = (unsigned)((units + upc - 1) / upc);
     cudaError_t err;
-#define GVCNN_LAUNCH_BF(POOL_, GAP_, WTS_, UPC_)                                                              \
-    err = launch_pdl(pool_fuse_bwd_fast_kernel<T, POOL_, V, NT, GAP_, WTS_, UPC_>, dim3(grid), dim3(NT), 0, st, \
+#define GVCNN_LAUNCH_BF(POOL_, GAP_, WTS_, UPC_, GRP_)                                                        \
+    err = launch_pdl(pool_fuse_bwd_fast_kernel<T, POOL_, V, NT, GAP_, WTS_, UPC_, GRP_>, dim3(grid), dim3(NT), 0, st, \
                      static_cast<const T *>(dS), bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G,   \
                      (int)tiles, gapC, gapHW, units)
-#define GVCNN_LAUNCH_BF_P(GAP_, WTS_)                                                                         \
+#define GVCNN_LAUNCH_BF_P(GAP_, WTS_, GRP_)                                                                   \
     do {                                                                                                      \
-        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_BF(GVCNN_POOL_MAX, GAP_, WTS_, upc);                         \
-        else GVCNN_LAUNCH_BF(GVCNN_POOL_MEAN, GAP_, WTS_, upc);                                               \
+        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_BF(GVCNN_POOL_MAX, GAP_, WTS_, upc, GRP_);                   \
+        else GVCNN_LAUNCH_BF(GVCNN_POOL_MEAN, GAP_, WTS_, upc, GRP_);                                         \
     } while (0)
-    if (gapC > 0) {
-        if (weights) GVCNN_LAUNCH_BF_P(true, true);  // paper mode: caller-supplied weights
-        else GVCNN_LAUNCH_BF_P(true, false);
+    if (grp) {  // per-group gradients dP [G, B, D] (gvcnn_view_pooling_bwd)
+        GVCNN_LAUNCH_BF_P(false, false, true);
+    } else if (gapC > 0) {
+        if (weights) GVCNN_LAUNCH_BF_P(true, true, false);  // paper mode: caller-supplied weights
+        else GVCNN_LAUNCH_BF_P(true, false, false);
     } else if (weights) {
-        GVCNN_LAUNCH_BF_P(false, true);
+        GVCNN_LAUNCH_BF_P(false, true, false);
     } else {
-        GVCNN_LAUNCH_BF_P(false, false);
+        GVCNN_LAUNCH_BF_P(false, false, false);
     }
 #undef GVCNN_LAUNCH_BF_P
 #undef GVCNN_LAUNCH_BF
@@ -304,31 +350,31 @@ static int launch_bwd_fast_v(const void *dS, const int32_t *bins, int64_t bin_sb
 template <typename T>
 static int launch_bwd_fast_t(const void *dS, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
                              const float *weights, int64_t w_sb, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
-                             int pool, cudaStream_t st)
+                             int pool, cudaStream_t st, bool grp = false)
 {
     if (D < 256 * Elem<T>::kVec) {
         // 16-bit types at D = 1024: one 128-thread tile per shape (see pool_fwd_ring.cu); anything shorter: generic kernel
         if constexpr (Elem<T>::kVec == 8) {
             if (D < 128 * Elem<T>::kVec) return -1000;
             switch (V) {
-            case 4: return launch_bwd_fast_v<T, 4, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st);
-            case 6: return launch_bwd_fast_v<T, 6, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st);
-            case 8: return launch_bwd_fast_v<T, 8, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st);
-            case 12: return launch_bwd_fast_v<T, 12, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st);
-            case 16: return launch_bwd_fast_v<T, 16, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st);
-            case 20: return launch_bwd_fast_v<T, 20, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st);
+            case 4: return launch_bwd_fast_v<T, 4, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
+            case 6: return launch_bwd_fast_v<T, 6, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
+            case 8: return launch_bwd_fast_v<T, 8, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
+            case 12: return launch_bwd_fast_v<T, 12, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
+            case 16: return launch_bwd_fast_v<T, 16, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
+            case 20: return launch_bwd_fast_v<T, 20, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
             default: return -1000;
             }
         }
         return -1000;
     }
     switch (V) {
-    case 4: return launch_bwd_fast_v<T, 4>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st);
-    case 6: return launch_bwd_fast_v<T, 6>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st);
-    case 8: return launch_bwd_fast_v<T, 8>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st);
-    case 12: return launch_bwd_fast_v<T, 12>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st);
-    case 16: return launch_bwd_fast_v<T, 16>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st);
-    case 20: return launch_bwd_fast_v<T, 20>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st);
+    case 4: return launch_bwd_fast_v<T, 4>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
+    case 6: return launch_bwd_fast_v<T, 6>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
+    case 8: return launch_bwd_fast_v<T, 8>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
+    case 12: return launch_bwd_fast_v<T, 12>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
+    case 16: return launch_bwd_fast_v<T, 16>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
+    case 20: return launch_bwd_fast_v<T, 20>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
     default: return -1000;
     }
 }
@@ -373,6 +419,25 @@ int launch_pool_fuse_bwd_fast(const void *dS, const int32_t *bins, int64_t bin_s
         return launch_bwd_fast_t<__nv_bfloat16>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool, st);
     if (dtype == GVCNN_F16)
         return launch_bwd_fast_t<__half>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool, st);
+    return GVCNN_E_BAD_DTYPE;
+}
+
+// gvcnn_view_pooling_bwd, fast path: dP [G, B, D] -> dF.  Same applicability as launch_pool_fuse_bwd_fast;
+// returns -1000 when it does not apply
+int launch_view_pooling_bwd_fast(const void *dP, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
+                                 const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
+                                 int pool, int dtype, cudaStream_t st)
+{
+    if (dtype == GVCNN_F32) {
+        if (D % 4) return -1000;
+        return launch_bwd_fast_t<float>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool, st, true);
+    }
+    if (D % 8) return -1000;
+    if (dtype == GVCNN_BF16)
+        return launch_bwd_fast_t<__nv_bfloat16>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool, st,
+                                                true);
+    if (dtype == GVCNN_F16)
+        return launch_bwd_fast_t<__half>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool, st, true);
     return GVCNN_E_BAD_DTYPE;
 }
 

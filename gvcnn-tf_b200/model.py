@@ -808,6 +808,33 @@ def pool_fuse_gap(final_view_descriptors, bins, num_group, pool="max", empty_fil
     return S.reshape(S.shape[0], -1, Cch).mean(dim=1)
 
 
+class _ViewPoolingFn(torch.autograd.Function):
+    """The G group descriptors P [G, B, D] (nets/model.py:62-74); backward = TF autodiff of those lines from one
+    gradient per group, dP [G, B, D] (gvcnn_view_pooling_bwd): max routes dP_g to the views attaining the group max
+    (ties share), mean gives every member dP_g / n_g, the empty groups' dummy gets nothing."""
+
+    @staticmethod
+    def forward(ctx, bins, G, pool, empty_fill, variant, f_lay, *f_t):
+        fv = _Views.of(f_t, f_lay, "F")
+        out = _pool_fuse_fwd(fv, bins, G, pool, empty_fill, None, want_mask=any(t.requires_grad for t in f_t),
+                             want_groups=True, want_status=False)
+        ctx.fv, ctx.G, ctx.pool, ctx.variant, ctx.bin_stride = fv, G, pool, variant, out.bin_stride
+        ctx.save_for_backward(out.bins, out.mask)
+        return out.P
+
+    @staticmethod
+    def backward(ctx, dP):
+        bins, mask = ctx.saved_tensors
+        dP = dP.contiguous()
+        out, gv = ctx.fv.empty_like()
+        with _on(dP.device):
+            C.check(C.lib().gvcnn_view_pooling_bwd(_ptr(dP), _ptr(bins), ctx.bin_stride, _ptr(mask), gv.arg, None,
+                                                   gv.B, gv.V, gv.D, ctx.G, _pool_code(ctx.pool, ctx.variant),
+                                                   gv.layout, _dtype_code(gv.dtype), _stream()),
+                    "gvcnn_view_pooling_bwd")
+        return (None,) * 6 + (tuple(out) if isinstance(out, list) else (out,))
+
+
 class GroupDescriptors(dict):
     """What ``view_pooling`` returns: behaves like the reference's
     ``{group index: pooled descriptor}`` dict (nets/model.py:61,72), but lazy -
@@ -815,23 +842,40 @@ class GroupDescriptors(dict):
     if somebody indexes or iterates the dict.  ``group_fusion`` recognises an
     UNEDITED object of this type and runs the single-pass fused kernel on the
     original views; once an entry has been assigned or removed it is an
-    ordinary dict of tensors and is fused as such."""
+    ordinary dict of tensors and is fused as such.
 
-    def __init__(self, views, layout, bins, num_group, pool, empty_fill):
+    Like the reference's graph tensors, the entries are differentiable w.r.t.
+    the view descriptors: when gradients were enabled at the ``view_pooling``
+    call and a view requires grad, any use of an entry (an edited dict passed to
+    ``group_fusion``, a custom fusion, a loss on one group) carries its gradient
+    back to the views.  The dict materialises under the grad mode of that call,
+    so one built under ``torch.no_grad()`` stays gradient-free when indexed later."""
+
+    def __init__(self, views, layout, bins, num_group, pool, empty_fill, variant=0):
         super().__init__()
         self._views, self._layout = views, layout
         self._bins, self._G, self._pool, self._fill = bins, num_group, pool, empty_fill
+        self._grad = torch.is_grad_enabled()
+        self._variant = variant
         self._done = False
         self._edited = False
 
     def _materialise(self):
         if self._done:
             return
-        fv = _Views.of(self._views, self._layout, "F")
-        P = _pool_fuse_fwd(fv, self._bins, self._G, self._pool, self._fill, None, want_mask=False, want_groups=True,
-                           want_status=False).P
-        for g in range(self._G):
-            dict.__setitem__(self, g, P[g].reshape(fv.view_shape))
+        with torch.set_grad_enabled(self._grad):     # the grad mode of the view_pooling call, not of this one
+            if self._grad and any(t.requires_grad for t in self._views):
+                P = _ViewPoolingFn.apply(self._bins, self._G, self._pool, self._fill, self._variant, self._layout,
+                                         *self._views)
+                shape = self._views[0].shape if self._layout == "list" else \
+                    (P.shape[1],) + tuple(self._views[0].shape[2:])
+            else:
+                fv = _Views.of(self._views, self._layout, "F")
+                P = _pool_fuse_fwd(fv, self._bins, self._G, self._pool, self._fill, None, want_mask=False,
+                                   want_groups=True, want_status=False).P
+                shape = fv.view_shape
+            for g in range(self._G):
+                dict.__setitem__(self, g, P[g].reshape(shape))
         self._done = True
 
     def __getitem__(self, k):
@@ -888,7 +932,7 @@ class GroupDescriptors(dict):
         dict.update(self, *a, **kw)
 
 
-def view_pooling(final_view_descriptors, group_scheme, pool="max", empty_fill=1.0, layout=None):
+def view_pooling(final_view_descriptors, group_scheme, pool="max", empty_fill=1.0, layout=None, _variant=0):
     """Intra-group view pooling.  Mirrors nets/model.py:44-74.
 
     final_view_descriptors: list of V CUDA tensors [N, h, w, C] (as in the
@@ -896,14 +940,19 @@ def view_pooling(final_view_descriptors, group_scheme, pool="max", empty_fill=1.
     [num_group, num_view] (one scheme for the batch, as in the reference) or
     [B, num_group, num_view].  pool='max', empty_fill=1.0 is the shipped
     model.py behaviour (:63,:72); pool='mean', empty_fill=0.0 is unit_test.py's.
-    Returns a GroupDescriptors dict {g: pooled descriptor}.
+    Returns a GroupDescriptors dict {g: pooled descriptor}.  Its entries are
+    differentiable w.r.t. the view descriptors (the gradient of each entry
+    reaches the views as TF autodiff of :62-74 routes it: max to the views
+    attaining the group max, ties sharing; mean to every member, / n_g), unless
+    gradients are disabled at this call.  _variant (tests / A-B runs only): the
+    backward kernel, as in pool_fuse.
     """
     views, lay = _view_args(final_view_descriptors, layout)
     if len(views) == 0:
         raise ValueError("final_view_descriptors: empty view list")
     _require_cuda(views[0], "final_view_descriptors")
     bins, G = _scheme_to_bins(_small_to_device(group_scheme, views[0].device, torch.int32, "group_scheme"))
-    return GroupDescriptors(views, lay, bins, G, pool, empty_fill)
+    return GroupDescriptors(views, lay, bins, G, pool, empty_fill, _variant)
 
 
 def _fuse_plain_dict(group_descriptors, group_weight):

@@ -257,6 +257,28 @@ int gvcnn_pool_fuse_bwd(const void *dS, const int32_t *bins, int64_t bin_stride_
                         int B, int V, int64_t D, int G, int pool,
                         int g_layout, int dtype, void *stream);
 
+/* Backward of view_pooling alone (TF autodiff of nets/model.py:62-74): the
+ * gradient of each group descriptor, dP, instead of the one of the fused S - for
+ * callers that use gvcnn_pool_fuse_fwd's group_desc directly (an edited dict, a
+ * custom fusion, a loss on one group).  For view v in group g = bin(b, v):
+ *   dF_v = (1/num_selected | 0) * dP_g      max  (ties share; the tie mask's count;
+ *                                                  the 0 is +0, as in gvcnn_pool_fuse_bwd)
+ *   dF_v = dP_g / n_g                       mean
+ * dP: [G, B, D] in `dtype`, the layout of gvcnn_pool_fuse_fwd's group_desc.  The
+ * rows of empty groups are not read (their dummy gets no gradient).  Every view is
+ * in exactly one group, so every row of dF is written once.  bins / bin_stride_b /
+ * status as in gvcnn_pool_fuse_fwd; dF in g_layout (PTRS: host array of V device
+ * pointers).  tie_mask is required for GVCNN_POOL_MAX and must be the one written
+ * by the gvcnn_pool_fuse_fwd call that wrote group_desc.  Arithmetic in float32;
+ * 16-bit dP is widened exactly and dF rounded once.  Bits 8..11 of `pool` select
+ * the kernel: 0 = auto, 1 or 2 = the generic kernel, 3 or 4 = the V-specialised
+ * one (16-byte aligned rows and V in {4, 6, 8, 12, 16, 20}, else
+ * GVCNN_E_UNSUPPORTED). */
+int gvcnn_view_pooling_bwd(const void *dP, const int32_t *bins, int64_t bin_stride_b,
+                           const uint8_t *tie_mask, void *dF, int32_t *status,
+                           int B, int V, int64_t D, int G, int pool,
+                           int g_layout, int dtype, void *stream);
+
 /* --- the whole forward in one call ----------------------------------------
  * gvcnn_score_bin_fwd + gvcnn_pool_fuse_fwd (per-shape scores, the reference's
  * own weights): what one train.py step does between the backbone and the
