@@ -42,6 +42,7 @@ SIGNATURES = {
     "gvcnn_batch_sum_x": (_i, [_vp, _vp, _i, _i, _vp]),
     "gvcnn_score_bin": (_i, [_vp, _f, _vp, _vp, _vp, _vp, _vp, _i64, _i, _i, _i, _i, _vp, _i, _vp]),
     "gvcnn_batch_mean_bin": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i64, _vp, _vp, _vp]),
+    "gvcnn_score_bin_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i64, _vp, _vp, _vp]),
     "gvcnn_score_bin_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "gvcnn_gap_score_bin_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "gvcnn_bins_from_scores": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _i, _i, _i, _vp]),

@@ -190,6 +190,40 @@ int gvcnn_batch_mean_bin(const float *x, float *xsum, float *x_mean, float *scor
                             clamp, global_count, exchange, exchange_user, static_cast<cudaStream_t>(stream));
 }
 
+// backward of the score tail of gvcnn_score_bin / gvcnn_batch_mean_bin in TF's op order (score.cu): chain kernel,
+// [exchange of dx_mean], broadcast kernel ('batch'); the chain kernel alone ('shape')
+int gvcnn_score_bin_bwd(const float *dscores, const float *x, const float *scores, float *dx_mean, float *dx, int B,
+                        int V, int score_reduce, int64_t global_count, gvcnn_exchange_fn exchange, void *exchange_user,
+                        void *stream)
+{
+    if (B < 0 || V <= 0) return GVCNN_E_BAD_ARG;
+    if (V > GVCNN_MAX_VIEWS) return GVCNN_E_TOO_MANY_VIEWS;
+    if (score_reduce != GVCNN_SCORE_REDUCE_SHAPE && score_reduce != GVCNN_SCORE_REDUCE_BATCH) return GVCNN_E_BAD_MODE;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (score_reduce == GVCNN_SCORE_REDUCE_SHAPE) {
+        if (dx_mean || exchange) return GVCNN_E_BAD_ARG;
+        if (B == 0) return 0;
+        if (!dscores || !x || !scores || !dx) return GVCNN_E_BAD_ARG;
+        if (!is_aligned(dscores, 4) || !is_aligned(x, 4) || !is_aligned(scores, 4) || !is_aligned(dx, 4))
+            return GVCNN_E_MISALIGNED;
+        return launch_score_bin_bwd(dscores, x, scores, dx, (int64_t)B * V, st);
+    }
+    if (!dscores || !x || !scores || !dx_mean || (B > 0 && !dx)) return GVCNN_E_BAD_ARG;
+    if (global_count < B || global_count <= 0) return GVCNN_E_BAD_ARG;
+    if (B == 0 && !exchange) return GVCNN_E_BAD_ARG;  // as gvcnn_batch_mean_bin: a mean over nothing
+    if (!is_aligned(dscores, 4) || !is_aligned(x, 4) || !is_aligned(scores, 4) || !is_aligned(dx_mean, 4) ||
+        !is_aligned(dx, 4))
+        return GVCNN_E_MISALIGNED;
+    int rc = launch_score_bin_bwd(dscores, x, scores, dx_mean, V, st);
+    if (rc) return rc;
+    if (exchange) {  // the adjoint of the forward's all-reduce of the column sums: every rank gets the global dx_mean
+        rc = exchange(exchange_user, dx_mean, V, st);
+        if (rc) return rc;
+    }
+    if (B == 0) return 0;
+    return launch_batch_mean_bwd(dx_mean, dx, B, V, (float)global_count, st);
+}
+
 int gvcnn_bins_from_scores(const float *scores, int32_t *bins, int32_t *flags, int32_t *status, int64_t n,
                            int G, int multiplier, int edge_ulps, int clamp, void *stream)
 {

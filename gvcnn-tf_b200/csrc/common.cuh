@@ -609,6 +609,9 @@ int launch_batch_sum_x(const float *x, float *xsum, int B, int V, cudaStream_t s
 int launch_score_bin(const float *x, float denom, float *x_mean, float *scores, int32_t *bins, int32_t *flags,
                      int32_t *status, int64_t n, int G, int multiplier, int edge_ulps, int clamp, bool x_is_score,
                      const float *xabs, int bound_terms, cudaStream_t st);
+int launch_score_bin_bwd(const float *dscores, const float *x, const float *scores, float *out, int64_t n,
+                         cudaStream_t st);
+int launch_batch_mean_bwd(const float *dx_mean, float *dx, int B, int V, float N, cudaStream_t st);
 int launch_bins_to_scheme(const int32_t *bins, int32_t *scheme, int rows, int V, int G, cudaStream_t st);
 int launch_scheme_to_bins(const int32_t *scheme, int32_t *bins, int32_t *status, int rows, int V, int G,
                           cudaStream_t st);

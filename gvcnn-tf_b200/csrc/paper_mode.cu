@@ -96,6 +96,8 @@ __global__ void __launch_bounds__(256) group_weight_grad_kernel(const ViewPtrs f
 }
 
 // dx[row, v] = dw[row, bin_v] / n_{bin_v} * sign(x) / (1 + |x|)^2     (s = |x| / (1 + |x|))
+// The closed form on purpose: the paper-mode weights have no reference graph to follow (SURVEY D6, 8f n2).  The
+// reference's own scores do, and score_bin_bwd_kernel (score.cu) follows TF's op chain sigmoid -> log -> abs instead.
 __global__ void __launch_bounds__(256) score_weight_bwd_kernel(const float *__restrict__ dweights,
                                                               const int32_t *__restrict__ bins,
                                                               const float *__restrict__ x, float *__restrict__ dx,

@@ -286,6 +286,52 @@ __global__ void __launch_bounds__(256) score_bin_kernel(const float *__restrict_
     publish(flags, flag_out ? flag_out + i : nullptr, status);
 }
 
+// ---- backward of the score tail (gvcnn_score_bin_bwd) ----------------------------------------------------------
+// dL/dx from dL/ds for s = sigmoid(log|x|) (nets/model.py:147), as TF 1.x autodiff evaluates it, one float32 rounding
+// per op; s is this library's forward value |x| / (1 + |x|):
+//   t  = (g * s) * (1 - s)   SigmoidGrad.  Eigen's scalar_sigmoid_gradient_op multiplies left to right; its packet path
+//                            may form g * (s * (1 - s)).  The scalar order is the op's element definition, and the one
+//                            Eigen takes for every element outside whole packets (V = 6, 33, ...), so it is the one
+//                            restated here; tests hold the other within tolerance.
+//   r  = 1 / |x|             _LogGrad's math_ops.reciprocal, rounded on its own
+//   u  = t * r               _LogGrad
+//   dx = u * sign(x)         _AbsGrad; x = 0 gives u = t * inf or 0 * inf, and NaN * 0 or inf * 0 = NaN, as in TF
+// Paper mode's score_weight_bwd_kernel (paper_mode.cu) differentiates the same function in closed form,
+// sign(x) / (1 + |x|)^2: the paper-mode weights have no reference graph whose op order could be followed, this has one.
+__device__ __forceinline__ float score_tail_grad(const float g, const float x, const float s)
+{
+    const float t = __fmul_rn(__fmul_rn(g, s), __fsub_rn(1.0f, s));
+    const float r = __frcp_rn(fabsf(x));
+    const float u = __fmul_rn(t, r);
+    const float sg = x > 0.0f ? 1.0f : (x < 0.0f ? -1.0f : 0.0f);
+    return __fmul_rn(u, sg);
+}
+
+// out[i] = score_tail_grad(g[i], x[i], s[i]) for n values: dx [B, V] in 'shape' mode, the batch mean's dx_mean [V] in
+// 'batch' mode
+__global__ void __launch_bounds__(256) score_bin_bwd_kernel(const float *__restrict__ g, const float *__restrict__ x,
+                                                            const float *__restrict__ s, float *__restrict__ out,
+                                                            const int64_t n)
+{
+    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    pdl_wait();
+    pdl_launch_dependents();
+    if (i >= n) return;
+    out[i] = score_tail_grad(g[i], x[i], s[i]);
+}
+
+// _MeanGrad of tf.reduce_mean over the batch (nets/model.py:146): dx[b, v] = dx_mean[v] / float(N), N the global batch
+// size the forward divided by.  A kernel of its own so that a cross-rank exchange of dx_mean can run between the two.
+__global__ void __launch_bounds__(256) batch_mean_bwd_kernel(const float *__restrict__ dx_mean, float *__restrict__ dx,
+                                                             const int64_t total, const int V, const float N)
+{
+    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    pdl_wait();
+    pdl_launch_dependents();
+    if (i >= total) return;
+    dx[i] = __fdiv_rn(dx_mean[i % V], N);
+}
+
 // The literal batch mode's tail in ONE launch (nets/model.py:146-147, :23 on a batch that may be sharded over GPUs).
 // One CTA per view - nothing in this stage couples the views, so the CTAs never talk to each other:
 //   xsum[v] = sum_b x[b, v]          batch_sum_x_kernel's code and order (thread t adds b = t, t + 256, ...; warp
@@ -467,6 +513,24 @@ int launch_score_bin(const float *x, float denom, float *x_mean, float *scores, 
     const unsigned grid = (unsigned)((n + 255) / 256);
     const cudaError_t err = launch_pdl(score_bin_kernel, dim3(grid), dim3(256), 0, st, x, denom, x_mean, scores, bins,
                                        flags, status, n, G, multiplier, edge_ulps, clamp, x_is_score, xabs, bound_terms);
+    if (err != cudaSuccess) return (int)err;
+    return (int)cudaGetLastError();
+}
+
+int launch_score_bin_bwd(const float *dscores, const float *x, const float *scores, float *out, int64_t n,
+                         cudaStream_t st)
+{
+    const unsigned grid = (unsigned)((n + 255) / 256);
+    const cudaError_t err = launch_pdl(score_bin_bwd_kernel, dim3(grid), dim3(256), 0, st, dscores, x, scores, out, n);
+    if (err != cudaSuccess) return (int)err;
+    return (int)cudaGetLastError();
+}
+
+int launch_batch_mean_bwd(const float *dx_mean, float *dx, int B, int V, float N, cudaStream_t st)
+{
+    const int64_t total = (int64_t)B * V;
+    const unsigned grid = (unsigned)((total + 255) / 256);
+    const cudaError_t err = launch_pdl(batch_mean_bwd_kernel, dim3(grid), dim3(256), 0, st, dx_mean, dx, total, V, N);
     if (err != cudaSuccess) return (int)err;
     return (int)cudaGetLastError();
 }

@@ -329,6 +329,13 @@ def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulp
     status: optional persistent int32[4] device tensor the counters are ADDED to (check it every N steps
        with raise_for_status instead of synchronising every step); with check=False and no status given
        nothing is recorded.
+
+    ``scores`` is differentiable, as the reference's graph tensor is: when gradients are enabled and W, b or R
+    requires grad, a loss on the scores reaches W, b and R (or the block3 maps) in TF 1.x's op order
+    (gvcnn_score_bin_bwd, then gvcnn_view_score_bwd / gvcnn_gap_score_bwd).  x, bins and flags are not.  In 'batch'
+    mode with a ``process_group`` or an ``exchange`` that backward is collective like the forward: the gradient of
+    the batch mean is all-reduced over the ranks, so when a score gradient flows on one rank it must flow on every
+    rank, one with an empty shard included.
     """
     _check_score_fc(W, b)
     Wc, bc = W.contiguous(), b.contiguous()
@@ -337,11 +344,117 @@ def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulp
     if tuple(Wc.shape) != (rv.V, Craw) or tuple(bc.shape) != (rv.V,):
         raise ValueError("W must be [V, C] = %s and b [V], got %s and %s"
                          % ((rv.V, Craw), tuple(Wc.shape), tuple(bc.shape)))
+    if status is None and check:
+        status = _new_status(rv.device)
+
+    def run(want_r_out):
+        return _score_bin_fwd(rv, HW, Craw, Wc, bc, num_group, score_reduce, edge_ulps, clamp, status, process_group,
+                              multiplier, exchange, global_count, want_r_out)
+    if torch.is_grad_enabled() and (Wc.requires_grad or bc.requires_grad or any(t.requires_grad for t in rv.keep)):
+        x, scores, bins, flags = _ScoreFn.apply(run, Wc, bc, *rv.keep)
+    else:
+        x, scores, bins, flags = run(False)[:4]
+    res = ScoreResult(x, scores, bins, flags, status, num_group)
+    if check:
+        res.check()
+    return res
+
+
+class _ScoreGrad:
+    """What the score backward needs of its forward, besides W, x and the scores: the raw views (pointers, layout,
+    dtype, B) and their positions per view HW (> 1: block3 maps), the mode, and in 'batch' mode the N the forward
+    divided by and the exchange it used (a (fn, user) pair or a torch.distributed process group)."""
+    __slots__ = ("rv", "HW", "batch", "global_count", "exchange", "process_group")
+
+    def __init__(self, rv, HW, batch, global_count=0, exchange=None, process_group=None):
+        self.rv, self.HW, self.batch = rv, HW, batch
+        self.global_count, self.exchange, self.process_group = global_count, exchange, process_group
+
+
+def _score_bwd(dscores, W, x, scores, R_out, sg: _ScoreGrad, need_wb: bool, need_r: bool):
+    """The score part of a backward (shared by _ScoreFn and _PoolFuseFn): dscores -> dx (gvcnn_score_bin_bwd, with
+    the adjoint exchange in 'batch' mode), then dW, db and dR from dx (gvcnn_view_score_bwd; on block3 maps dW and db
+    from the pooled float32 R_out of the forward, and dmaps from gvcnn_gap_score_bwd).  Returns (dW, db, dR) with dR
+    a tuple in the layout of the raw views (one tensor per view for a list), or None where not asked for."""
+    L = C.lib()
+    rv, HW = sg.rv, sg.HW
+    B, V, Craw = rv.B, rv.V, rv.D // HW
+    dev = dscores.device
+    ds = dscores.to(torch.float32).contiguous()
+    dx = torch.empty((B, V), dtype=torch.float32, device=dev)
+    dW = db = dR = None
+    with _on(dev):
+        if sg.batch:
+            dx_mean = torch.empty(V, dtype=torch.float32, device=dev)
+            ex, keep = sg.exchange, None
+            if ex is None and sg.process_group is not None:
+                cb, keep = make_exchange(sg.process_group)
+                ex = (cb, None)
+            ex_ptr, _, ex_user = _exchange_forms(ex)
+            C.check(L.gvcnn_score_bin_bwd(_ptr(ds), _ptr(x), _ptr(scores), _ptr(dx_mean), _ptr(dx), B, V,
+                                          C.SCORE_REDUCE_BATCH, int(sg.global_count), ex_ptr, ex_user, _stream()),
+                    "gvcnn_score_bin_bwd")
+            del keep
+        else:
+            C.check(L.gvcnn_score_bin_bwd(_ptr(ds), _ptr(x), _ptr(scores), None, _ptr(dx), B, V, C.SCORE_REDUCE_SHAPE,
+                                          0, None, None, _stream()), "gvcnn_score_bin_bwd")
+        dR_out, dR_views = rv.empty_like() if need_r else (None, None)
+        if need_wb or (need_r and HW == 1):
+            if B == 0:                                  # a parameter gradient over an empty shard: zeros
+                dW, db = torch.zeros_like(W), torch.zeros(V, dtype=torch.float32, device=dev)
+            else:
+                ws_bytes = L.gvcnn_view_score_bwd_workspace_bytes(V, Craw)
+                scratch = torch.empty(W.numel() + V + (ws_bytes + 3) // 4, dtype=torch.float32, device=dev)
+                dW, db, ws = scratch[:W.numel()].view_as(W), scratch[W.numel():W.numel() + V], scratch[W.numel() + V:]
+                if HW > 1:
+                    C.check(L.gvcnn_view_score_bwd(_ptr(R_out), _ptr(dx), _ptr(W), _ptr(dW), _ptr(db), None, _ptr(ws),
+                                                   ws_bytes, B, V, Craw, C.LAYOUT_BVD, C.F32, _stream()),
+                            "gvcnn_view_score_bwd")
+                else:
+                    C.check(L.gvcnn_view_score_bwd(rv.arg, _ptr(dx), _ptr(W), _ptr(dW), _ptr(db),
+                                                   dR_views.arg if need_r else None, _ptr(ws), ws_bytes, B, V, Craw,
+                                                   rv.layout, _dtype_code(rv.dtype), _stream()),
+                            "gvcnn_view_score_bwd")
+        if need_r and HW > 1 and B > 0:
+            C.check(L.gvcnn_gap_score_bwd(_ptr(dx), _ptr(W), dR_views.arg, B, V, HW, Craw, rv.layout,
+                                          _dtype_code(rv.dtype), _stream()), "gvcnn_gap_score_bwd")
+    if need_r:
+        dR = tuple(dR_out) if isinstance(dR_out, list) else (dR_out,)
+    return (dW, db, dR) if need_wb else (None, None, dR)
+
+
+class _ScoreFn(torch.autograd.Function):
+    """score_bin with a gradient: (x, scores, bins, flags) from `run(want_r_out)`, only `scores` differentiable;
+    backward = _score_bwd.  No score gradient (a loss that does not use the scores) launches nothing."""
+
+    @staticmethod
+    def forward(ctx, run, W, b, *r_t):
+        ctx.set_materialize_grads(False)
+        x, scores, bins, flags, R_out, sg = run(W.requires_grad or b.requires_grad)
+        ctx.sg, ctx.n_r = sg, len(r_t)
+        ctx.save_for_backward(W, x, scores, R_out)
+        ctx.mark_non_differentiable(x, bins, flags)
+        return x, scores, bins, flags
+
+    @staticmethod
+    def backward(ctx, _dx, dscores, _dbins, _dflags):
+        ni = ctx.needs_input_grad
+        need_wb, need_r = ni[1] or ni[2], any(ni[3:])
+        if dscores is None or not (need_wb or need_r):
+            return (None,) * (3 + ctx.n_r)
+        W, x, scores, R_out = ctx.saved_tensors
+        dW, db, dR = _score_bwd(dscores, W, x, scores, R_out, ctx.sg, need_wb, need_r)
+        return (None, dW if ni[1] else None, db if ni[2] else None) + (dR if need_r else (None,) * ctx.n_r)
+
+
+def _score_bin_fwd(rv, HW, Craw, Wc, bc, num_group, score_reduce, edge_ulps, clamp, status, process_group, multiplier,
+                   exchange, global_count, want_r_out):
+    """score_bin's launches: (x, scores, bins, flags, R_out, _ScoreGrad).  want_r_out (block3 maps only): also
+    write the pooled float32 R [B, V, C] that dW and db of the score FC are computed from."""
     dev = rv.device
     L = C.lib()
-    if status is None and check:
-        status = _new_status(dev)
     dt = _dtype_code(rv.dtype)
+    R_out = torch.empty((rv.B, rv.V, Craw), dtype=torch.float32, device=dev) if (want_r_out and HW > 1) else None
     with _on(dev):
         if score_reduce == "shape":
             if multiplier not in (None, num_group):
@@ -349,22 +462,24 @@ def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulp
             buf = torch.empty((4, rv.B, rv.V), dtype=torch.int32, device=dev)      # x, scores, bins, flags: one allocation
             x, scores, bins, flags = buf[0].view(torch.float32), buf[1].view(torch.float32), buf[2], buf[3]
             if HW > 1:      # raw maps: GlobalAveragePooling2D folded into the score kernel (nets/model.py:144-145)
-                C.check(L.gvcnn_gap_score_bin_fwd(rv.arg, _ptr(Wc), _ptr(bc), None, _ptr(x), _ptr(scores), _ptr(bins),
-                                                  _ptr(flags), _ptr(status), rv.B, rv.V, HW, Craw, num_group, rv.layout,
-                                                  dt, 1, edge_ulps, int(clamp), _stream()), "gvcnn_gap_score_bin_fwd")
+                C.check(L.gvcnn_gap_score_bin_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(R_out), _ptr(x), _ptr(scores),
+                                                  _ptr(bins), _ptr(flags), _ptr(status), rv.B, rv.V, HW, Craw,
+                                                  num_group, rv.layout, dt, 1, edge_ulps, int(clamp), _stream()),
+                        "gvcnn_gap_score_bin_fwd")
             else:
                 C.check(L.gvcnn_score_bin_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(x), _ptr(scores), _ptr(bins),
                                               _ptr(flags), _ptr(status), rv.B, rv.V, rv.D, num_group,
                                               rv.layout, dt, edge_ulps, int(clamp), _stream()),
                         "gvcnn_score_bin_fwd")
+            return x, scores, bins, flags, R_out, _ScoreGrad(rv, HW, False)
         elif score_reduce == "batch":
             # x and (pooled-descriptor input only) A = sum |R W| + |b| per (shape, view); column sums of both in one
             # [2, V] buffer, so ONE exchange carries them across the ranks; A feeds the a-priori order-sensitivity flag
             want_bound = HW == 1 and edge_ulps > 0                   # view_scores() asks for scores only
             xb = torch.empty((2 if want_bound else 1, max(rv.B, 1), rv.V), dtype=torch.float32, device=dev)
             if HW > 1:
-                C.check(L.gvcnn_gap_score_bin_fwd(rv.arg, _ptr(Wc), _ptr(bc), None, _ptr(xb[0]), None, None, None, None,
-                                                  rv.B, rv.V, HW, Craw, 1, rv.layout, dt, 0, 0, 0, _stream()),
+                C.check(L.gvcnn_gap_score_bin_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(R_out), _ptr(xb[0]), None, None, None,
+                                                  None, rv.B, rv.V, HW, Craw, 1, rv.layout, dt, 0, 0, 0, _stream()),
                         "gvcnn_gap_score_bin_fwd")
             else:
                 C.check(L.gvcnn_view_score_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(xb[0]), _ptr(xb[1]) if want_bound else None,
@@ -382,10 +497,7 @@ def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulp
                 C.check(L.gvcnn_batch_mean_bin(_ptr(xb[0]), _ptr(sums[0]), _ptr(x), _ptr(scores), _ptr(bins), _ptr(flags),
                                                _ptr(status), rv.B, rv.V, num_group, int(multiplier or 0), edge_ulps,
                                                int(clamp), denom, ex_ptr, ex_user, _stream()), "gvcnn_batch_mean_bin")
-                res = ScoreResult(x, scores, bins, flags, status, num_group)
-                if check:
-                    res.check()
-                return res
+                return x, scores, bins, flags, R_out, _ScoreGrad(rv, HW, True, denom, exchange)
             nsum = 2 if want_bound else 1                            # rows of `sums` in use: sum x (and sum A)
             if rv.B > 0:
                 for j in range(nsum):
@@ -408,18 +520,16 @@ def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulp
                                       _ptr(flags), _ptr(status), rv.V, num_group, int(multiplier or 0), edge_ulps,
                                       int(clamp), _ptr(sums[1]) if want_bound else None, Craw + 2 + denom, _stream()),
                     "gvcnn_score_bin")
-        else:
-            raise ValueError("score_reduce must be 'shape' or 'batch'")
-    res = ScoreResult(x, scores, bins, flags, status, num_group)
-    if check:
-        res.check()
-    return res
+            return x, scores, bins, flags, R_out, _ScoreGrad(rv, HW, True, denom, exchange,
+                                                             None if exchange is not None else process_group)
+        raise ValueError("score_reduce must be 'shape' or 'batch'")
 
 
 def view_scores(raw_view_descriptors, W, b, score_reduce="batch", layout=None, process_group=None):
     """view_discrimination_scores as nets/model.py:144-148 produces them:
     sigmoid(log|mean_n(Dense(1)(raw))|) - [1, V] for the literal 'batch' mode,
-    [B, V] for 'shape'."""
+    [B, V] for 'shape'.  Differentiable w.r.t. W, b and the raw descriptors, as the reference's graph tensor is
+    (TF 1.x's op order; see score_bin)."""
     return score_bin(raw_view_descriptors, W, b, 1, score_reduce=score_reduce, layout=layout,
                      edge_ulps=0, clamp=True, check=False, process_group=process_group).scores
 
@@ -663,37 +773,61 @@ def _pool_fuse_bwd(dS: torch.Tensor, fv_like: _Views, bins, bin_stride, weights,
 
 
 class _PoolFuseFn(torch.autograd.Function):
-    """S from `launch(fv, want_mask)` -> (_Pooled, extra outputs): pooling + fusion, on its own or after score + bin
-    in the same call into the library; backward = TF autodiff of nets/model.py:62-100 (dF only: no gradient reaches
-    scores / weights, train.py:127-128, utils/train_utils.py:203-206).  The extra outputs are non-differentiable."""
+    """S from `launch(fv, want_mask)` -> (_Pooled, extra outputs, _ScoreGrad or None): pooling + fusion, on its own
+    or after score + bin in the same call into the library; backward = TF autodiff of nets/model.py:62-100 for dF (no
+    gradient reaches the group weights, train.py:127-128, utils/train_utils.py:203-206).  The extra outputs are
+    non-differentiable, except the scores (x, scores, bins, flags) when the launch returns a _ScoreGrad: then the
+    inputs after the n_f views of F are W, b and the raw views R, and a score gradient reaches them (_score_bwd)."""
 
     @staticmethod
-    def forward(ctx, launch, G, pool, variant, f_lay, *f_t):
+    def forward(ctx, launch, G, pool, variant, f_lay, n_f, *tensors):
+        ctx.set_materialize_grads(False)
+        f_t = tensors[:n_f]
         fv = _Views.of(f_t, f_lay, "F")
-        out, extras = launch(fv, True)
+        out, extras, sg = launch(fv, any(t.requires_grad for t in f_t))     # the tie mask only if dF can be asked for
         ctx.fv, ctx.G, ctx.pool, ctx.variant = fv, G, pool, variant
         ctx.bin_stride, ctx.w_stride = out.bin_stride, out.w_stride
-        ctx.save_for_backward(out.bins, out.weights, out.mask)
-        ctx.mark_non_differentiable(*[t for t in extras if t is not None])
+        ctx.n_f, ctx.n_in, ctx.sg = n_f, len(tensors), sg
+        if sg is None:
+            ctx.save_for_backward(out.bins, out.weights, out.mask)
+            ctx.mark_non_differentiable(*[t for t in extras if t is not None])
+        else:
+            x, scores, bins, flags = extras
+            ctx.save_for_backward(out.bins, out.weights, out.mask, tensors[n_f], x, scores)
+            ctx.mark_non_differentiable(x, bins, flags)
         return (out.S.reshape(fv.view_shape),) + extras
 
     @staticmethod
-    def backward(ctx, dS, *_unused):
-        bins, weights, mask = ctx.saved_tensors
-        fv = ctx.fv
-        # bins may hold the raw out-of-range value (clamp=False); the backward kernel clamps like the forward did
-        out = _pool_fuse_bwd(dS.reshape(fv.B, fv.D), fv, bins, ctx.bin_stride, weights, ctx.w_stride, mask,
-                             ctx.G, ctx.pool, ctx.variant)
-        return (None,) * 5 + (tuple(out) if isinstance(out, list) else (out,))
+    def backward(ctx, dS, *douts):
+        saved = ctx.saved_tensors
+        bins, weights, mask = saved[:3]
+        fv, n_f, ni = ctx.fv, ctx.n_f, ctx.needs_input_grad
+        grads = [None] * ctx.n_in
+        if dS is not None and any(ni[6:6 + n_f]):
+            # bins may hold the raw out-of-range value (clamp=False); the backward kernel clamps like the forward did
+            out = _pool_fuse_bwd(dS.reshape(fv.B, fv.D), fv, bins, ctx.bin_stride, weights, ctx.w_stride, mask,
+                                 ctx.G, ctx.pool, ctx.variant)
+            grads[:n_f] = out if isinstance(out, list) else [out]
+        if ctx.sg is not None and douts[1] is not None:
+            need_wb, need_r = ni[6 + n_f] or ni[7 + n_f], any(ni[8 + n_f:])
+            if need_wb or need_r:
+                W, x, scores = saved[3:]
+                dW, db, dR = _score_bwd(douts[1], W, x, scores, None, ctx.sg, need_wb, need_r)
+                grads[n_f] = dW if ni[6 + n_f] else None
+                grads[n_f + 1] = db if ni[7 + n_f] else None
+                if need_r:
+                    grads[n_f + 2:] = dR
+        return (None,) * 6 + tuple(grads)
 
 
-def _run_launch(launch, f_t, f_lay, G, pool, variant):
-    """(S in the shape of one view,) + the launch's extra outputs.  Through autograd only when a gradient can be asked for;
-    otherwise straight into the library (saves the autograd.Function bookkeeping on the inference path)."""
-    if torch.is_grad_enabled() and any(t.requires_grad for t in f_t):
-        return _PoolFuseFn.apply(launch, G, pool, variant, f_lay, *f_t)
+def _run_launch(launch, f_t, f_lay, G, pool, variant, score_in=()):
+    """(S in the shape of one view,) + the launch's extra outputs.  Through autograd only when a gradient can be asked for
+    (a view of F, or one of `score_in` = (W, b, *R) of a launch that scores, requires grad); otherwise straight into the
+    library (saves the autograd.Function bookkeeping on the inference path)."""
+    if torch.is_grad_enabled() and (any(t.requires_grad for t in f_t) or any(t.requires_grad for t in score_in)):
+        return _PoolFuseFn.apply(launch, G, pool, variant, f_lay, len(f_t), *f_t, *score_in)
     fv = _Views.of(f_t, f_lay, "F")
-    out, extras = launch(fv, False)
+    out, extras, _ = launch(fv, False)
     return (out.S.reshape(fv.view_shape),) + extras
 
 
@@ -701,7 +835,7 @@ def _run_pool_fuse(f_t, f_lay, bins, weights, G, pool, empty_fill, want_status, 
     """Pooling + fusion from a bin map: (S, status)."""
     def launch(fv, want_mask):
         out = _pool_fuse_fwd(fv, bins, G, pool, empty_fill, weights, want_mask, False, want_status, variant)
-        return out, (out.status,)
+        return out, (out.status,), None
     return _run_launch(launch, f_t, f_lay, G, pool, variant)
 
 
@@ -1084,7 +1218,13 @@ def grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_grou
     check=True turns out-of-range / NaN scores into the reference's IndexError / ValueError right away (one
     16-byte device->host read per call, i.e. a synchronisation); the default records nothing.  For a training
     loop pass a persistent ``status`` tensor (int32[4], zeros) - the counters accumulate into it without any
-    synchronisation - and call ``raise_for_status(status, num_group)`` every N steps."""
+    synchronisation - and call ``raise_for_status(status, num_group)`` every N steps.
+
+    ``ScoreResult.scores`` is differentiable w.r.t. W, b and the raw descriptors (or block3 maps) when gradients are
+    enabled and one of them requires grad, as in score_bin; the shape descriptor stays differentiable w.r.t. the
+    final view descriptors.  A loss that does not use the scores leaves W and b without a gradient (``.grad`` None)
+    and launches nothing for them.  In 'batch' mode with a ``process_group`` or ``exchange`` the score backward is
+    collective (see score_bin): it must run on every rank, an empty shard included."""
     if status is None and check:
         dev0 = W.device if isinstance(W, torch.Tensor) else None
         status = _new_status(dev0)
@@ -1123,11 +1263,20 @@ def grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_grou
             raise ValueError("score_reduce='batch' over an empty (global) batch")
         literal = (multiplier, global_count, ex_ptr, ex_user)
     rv = _Views.of(r_t, r_lay, "R")
+    Wc, bc = W.contiguous(), b.contiguous()
+    score_in, sg = (), None
+    if torch.is_grad_enabled() and (Wc.requires_grad or bc.requires_grad or any(t.requires_grad for t in rv.keep)):
+        score_in = (Wc, bc) + tuple(rv.keep)
+        if literal is None:
+            sg = _ScoreGrad(rv, 1, False)
+        else:   # the backward's exchange: the forward's callback, or the process group's (made again when needed)
+            sg = _ScoreGrad(rv, 1, True, literal[1], exchange if keep is None else None, process_group)
 
     def launch(fv, want_mask):
-        return _grouping_fusion_fwd(rv, fv, want_mask, W, b, num_group, pool, empty_fill, edge_ulps, clamp, status,
-                                    _variant, literal)
-    S, x, scores, bins, flags = _run_launch(launch, f_t, f_lay, num_group, pool, _variant)
+        out, extras = _grouping_fusion_fwd(rv, fv, want_mask, Wc, bc, num_group, pool, empty_fill, edge_ulps, clamp,
+                                           status, _variant, literal)
+        return out, extras, sg
+    S, x, scores, bins, flags = _run_launch(launch, f_t, f_lay, num_group, pool, _variant, score_in)
     del keep
     sr = ScoreResult(x, scores, bins, flags, status, num_group)
     if check:
@@ -1322,7 +1471,8 @@ def grouping_fusion_paper(raw_view_descriptors, W, b, final_view_descriptors, nu
                           status=None, fold_gap=False):
     """Paper-mode grouping + fusion: group weight = mean discrimination score of the group's views, empty
     groups vanish; differentiable w.r.t. the view descriptors AND the score FC (W, b, optionally the raw
-    descriptors).  Returns (shape_descriptor, scores, bins, weights).  Per-shape scores/bins.
+    descriptors).  Returns (shape_descriptor, scores, bins, weights).  Per-shape scores/bins.  The scores (like bins
+    and weights) are non-differentiable outputs: the score FC trains through the group weights here.
     raw_view_descriptors may be the pooled [.., C_raw] descriptors or the block3 maps themselves ([.., h, w, C_raw],
     told apart by the trailing dimension as in score_bin): the GlobalAveragePooling2D in front of the score FC then
     runs inside the score kernel, forward and backward.
@@ -1386,11 +1536,15 @@ class GVCNNHead(torch.nn.Module):
         (view_discrimination_scores, shape_descriptor, logits) like
         nets/model.py:166.  fold_gap=True folds the GlobalAveragePooling2D of nets/model.py:163 into the
         pooling kernels, in both weight modes (paper mode: grouping_fusion_paper(fold_gap=True)): the fused
-        map is never written and the second return value is the pooled [N, C] descriptor."""
+        map is never written and the second return value is the pooled [N, C] descriptor.
+        weight_mode 'count': the scores are differentiable w.r.t. the score FC (and the raw descriptors), as the
+        reference's graph tensor is; a loss on them trains score_kernel / score_bias, a classifier-only loss leaves
+        their .grad None.  weight_mode 'score': the scores are a non-differentiable output; the FC trains through the
+        group weights (grouping_fusion_paper)."""
         if fold_gap and self.weight_mode == "count":
-            sr = score_bin(raw_view_descriptors, self.score_kernel.detach(), self.score_bias.detach(),
-                           self.num_group, score_reduce=self.score_reduce, process_group=process_group, check=check,
-                           status=status, global_count=global_count)
+            sr = score_bin(raw_view_descriptors, self.score_kernel, self.score_bias, self.num_group,
+                           score_reduce=self.score_reduce, process_group=process_group, check=check, status=status,
+                           global_count=global_count)
             net = pool_fuse_gap(final_view_descriptors, sr.bins, self.num_group, pool=self.pool,
                                 empty_fill=self.empty_fill)
             return sr.scores, net, self.classifier(net.to(self.classifier.weight.dtype))
@@ -1399,11 +1553,10 @@ class GVCNNHead(torch.nn.Module):
                                                     final_view_descriptors, self.num_group, pool=self.pool,
                                                     status=status, fold_gap=fold_gap)
         else:
-            S, sr = grouping_fusion(raw_view_descriptors, self.score_kernel.detach(), self.score_bias.detach(),
-                                    final_view_descriptors, self.num_group, pool=self.pool,
-                                    empty_fill=self.empty_fill, score_reduce=self.score_reduce,
-                                    process_group=process_group, check=check, status=status,
-                                    global_count=global_count)
+            S, sr = grouping_fusion(raw_view_descriptors, self.score_kernel, self.score_bias, final_view_descriptors,
+                                    self.num_group, pool=self.pool, empty_fill=self.empty_fill,
+                                    score_reduce=self.score_reduce, process_group=process_group, check=check,
+                                    status=status, global_count=global_count)
             scores = sr.scores
         net = _spatial_mean(S)
         logits = self.classifier(net.to(self.classifier.weight.dtype))
@@ -1417,8 +1570,7 @@ def gvcnn_head(raw_view_descriptors, final_view_descriptors, head: GVCNNHead, gr
     pools and fuses with them; without, it computes them on the device."""
     if group_scheme is None:
         return head(raw_view_descriptors, final_view_descriptors)
-    scores = view_scores(raw_view_descriptors, head.score_kernel.detach(), head.score_bias.detach(),
-                         score_reduce=head.score_reduce)
+    scores = view_scores(raw_view_descriptors, head.score_kernel, head.score_bias, score_reduce=head.score_reduce)
     desc = view_pooling(final_view_descriptors, group_scheme, pool=head.pool, empty_fill=head.empty_fill)
     w = group_weight if group_weight is not None else globals()["group_weight"](group_scheme)
     S = group_fusion(desc, w)

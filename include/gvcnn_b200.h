@@ -147,7 +147,8 @@ int gvcnn_batch_sum_x(const float *x, float *xsum, int B, int V, void *stream);
  * sum), lets another evaluation order put the score in a different bin.
  * flags (nullable) gets GVCNN_FLAG_* per element; status counts them.
  * clamp != 0 stores min(bin, G-1) instead of the out-of-range value (the
- * flag / status are still raised). */
+ * flag / status are still raised).
+ * Gradient of the scores: gvcnn_score_bin_bwd (per-shape, denom = 1). */
 int gvcnn_score_bin(const float *x, float denom, float *x_mean, float *scores, int32_t *bins,
                     int32_t *flags, int32_t *status, int64_t n, int G, int multiplier,
                     int edge_ulps, int clamp, const float *xabs, int bound_terms, void *stream);
@@ -159,12 +160,34 @@ int gvcnn_score_bin(const float *x, float denom, float *x_mean, float *scores, i
  * x [B, V] (gvcnn_view_score_fwd's output); xsum [V] (the global sums on return);
  * x_mean / scores / flags (nullable), bins: ONE [V] row.  global_count, exchange:
  * as in gvcnn_grouping_fusion_batch_fwd, which is gvcnn_view_score_fwd + this +
- * gvcnn_pool_fuse_fwd. */
+ * gvcnn_pool_fuse_fwd.  Gradient of the scores: gvcnn_score_bin_bwd (batch mode). */
 typedef int (*gvcnn_exchange_fn)(void *user, float *xsum_dev, int n, void *stream);
 int gvcnn_batch_mean_bin(const float *x, float *xsum, float *x_mean, float *scores, int32_t *bins,
                          int32_t *flags, int32_t *status, int B, int V, int G, int multiplier,
                          int edge_ulps, int clamp, int64_t global_count,
                          gvcnn_exchange_fn exchange, void *exchange_user, void *stream);
+
+/* Backward of the score tail above, TF 1.x autodiff of nets/model.py:146-147 with one
+ * float32 rounding per op.  g = dscores, s = scores (this library's forward value),
+ * x = the value the score was taken of:
+ *   t = (g * s) * (1 - s)    SigmoidGrad (left to right)
+ *   u = t * (1 / |x|)        _LogGrad, the reciprocal rounded on its own
+ *   dx = u * sign(x)         _AbsGrad; x = 0 gives NaN, as in TF
+ * score_reduce = GVCNN_SCORE_REDUCE_SHAPE: dscores, x, scores and dx are float32
+ *   [B, V] (x from gvcnn_score_bin_fwd / gvcnn_view_score_fwd); dx_mean and exchange
+ *   must be null; B == 0 returns 0.
+ * score_reduce = GVCNN_SCORE_REDUCE_BATCH: dscores, x (= x_mean) and scores are [V];
+ *   dx_mean [V] receives the gradient of the batch mean, after the exchange when one
+ *   is given (the adjoint of the forward's all-reduce: a sum over the ranks, through
+ *   the callback, in stream order); dx [B, V] receives dx_mean[v] / (float)global_count
+ *   (_MeanGrad), global_count the N of the forward.  The exchange is collective: when
+ *   one rank calls this, every rank must, a rank with B == 0 included (dx may then be
+ *   null).  B == 0 without an exchange is GVCNN_E_BAD_ARG, as in gvcnn_batch_mean_bin.
+ * The Dense(1) part then comes from gvcnn_view_score_bwd (dW, dbias, dR from dx) and,
+ * for block3 maps, gvcnn_gap_score_bwd (dmaps). */
+int gvcnn_score_bin_bwd(const float *dscores, const float *x, const float *scores, float *dx_mean,
+                        float *dx, int B, int V, int score_reduce, int64_t global_count,
+                        gvcnn_exchange_fn exchange, void *exchange_user, void *stream);
 
 /* gvcnn_view_score_fwd + gvcnn_score_bin(denom = 1) in ONE kernel: the
  * per-shape path (SURVEY.md D5 'shape').  Replaces the device->host->device
