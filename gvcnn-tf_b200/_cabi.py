@@ -14,6 +14,7 @@ SO_PATH = os.path.join(_HERE, "libgvcnn_sm100.so")
 
 F32, BF16, F16 = 0, 1, 2
 LAYOUT_BVD, LAYOUT_VBD, LAYOUT_PTRS = 0, 1, 2
+LAYOUT_CHANNELS_FIRST = 0x10  # ORed into the layout of channel-major [C, HW] maps (GVCNN_LAYOUT_CHANNELS_FIRST)
 POOL_MAX, POOL_MEAN = 0, 1
 SCORE_REDUCE_SHAPE, SCORE_REDUCE_BATCH = 0, 1
 ABI_VERSION = 2

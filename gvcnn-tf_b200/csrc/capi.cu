@@ -67,6 +67,15 @@ int check_dims(int B, int V, int64_t D, int G, int dtype)
 
 bool is_aligned(const void *p, size_t a) { return reinterpret_cast<uintptr_t>(p) % a == 0; }
 
+// Takes GVCNN_LAYOUT_CHANNELS_FIRST off a layout argument of the entry points that accept it; make_view_ptrs then sees
+// the base layout (every other entry point hands it the flag, which it rejects with GVCNN_E_BAD_LAYOUT).
+bool take_channels_first(int &layout)
+{
+    const bool cf = (layout & GVCNN_LAYOUT_CHANNELS_FIRST) != 0;
+    layout &= ~GVCNN_LAYOUT_CHANNELS_FIRST;
+    return cf;
+}
+
 }  // namespace
 
 namespace gvcnn {
@@ -276,6 +285,7 @@ int gvcnn_gap_score_bin_fwd(const void *maps, const float *W, const float *bias,
                             int m_layout, int dtype, int fuse_bin, int edge_ulps, int clamp, void *stream)
 {
     if (HW <= 0 || C <= 0) return GVCNN_E_BAD_ARG;
+    const bool cf = take_channels_first(m_layout);
     const int64_t D = (int64_t)HW * C;
     int rc = check_dims(B, V, D, G, dtype);
     if (rc) return rc == kEmptyBatch ? 0 : rc;
@@ -289,7 +299,7 @@ int gvcnn_gap_score_bin_fwd(const void *maps, const float *W, const float *bias,
     if (rc) return rc;
     if (!al) return GVCNN_E_UNSUPPORTED;
     rc = launch_gap_score(mp, sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW, C, G, dtype, fuse_bin != 0,
-                          edge_ulps, clamp, static_cast<cudaStream_t>(stream));
+                          edge_ulps, clamp, cf, static_cast<cudaStream_t>(stream));
     return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
 }
 
@@ -488,10 +498,11 @@ static int pool_fuse_gap_fwd_impl(const void *F, const int32_t *bins, int64_t bi
                                   float empty_fill, int f_layout, int dtype, void *stream)
 {
     if (HW <= 0 || C <= 0) return GVCNN_E_BAD_ARG;
+    const bool cf = take_channels_first(f_layout);
     const int64_t D = (int64_t)HW * C;
     int rc = check_dims(B, V, D, G, dtype);
     if (rc) return rc == kEmptyBatch ? 0 : rc;
-    if (!bins || !S_gap || !workspace || bin_stride_b < 0) return GVCNN_E_BAD_ARG;
+    if (!bins || !S_gap || (!cf && !workspace) || bin_stride_b < 0) return GVCNN_E_BAD_ARG;
     if (pool != GVCNN_POOL_MAX && pool != GVCNN_POOL_MEAN) return GVCNN_E_BAD_MODE;
     if (weights && (!is_aligned(weights, 4) || weight_stride_b < 0)) return GVCNN_E_BAD_ARG;
     ViewPtrs fp;
@@ -499,6 +510,13 @@ static int pool_fuse_gap_fwd_impl(const void *F, const int32_t *bins, int64_t bi
     bool al;
     rc = make_view_ptrs(F, f_layout, dtype, B, V, D, fp, sb, al);
     if (rc) return rc;
+    if (cf) {  // no workspace: no position split
+        if (weights || !al || V > 32 || (tie_mask && !is_aligned(tie_mask, 8)) || !is_aligned(S_gap, elt_size(dtype)))
+            return GVCNN_E_UNSUPPORTED;
+        rc = launch_pool_fuse_gap_cf_fwd(fp, sb, bins, bin_stride_b, S_gap, tie_mask, status, B, V, HW, C, G, pool,
+                                         empty_fill, dtype, static_cast<cudaStream_t>(stream));
+        return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
+    }
     const size_t need = gap_workspace_bytes(B, C, HW, dtype);
     if (!al || need == 0 || V > 32 || (tie_mask && !is_aligned(tie_mask, 8)) || !is_aligned(workspace, 16))
         return GVCNN_E_UNSUPPORTED;
@@ -531,6 +549,7 @@ static int pool_fuse_gap_bwd_impl(const void *dS_gap, const int32_t *bins, int64
                                   int V, int HW, int C, int G, int pool, int g_layout, int dtype, void *stream)
 {
     if (HW <= 0 || C <= 0) return GVCNN_E_BAD_ARG;
+    const bool cf = take_channels_first(g_layout);
     const int64_t D = (int64_t)HW * C;
     int rc = check_dims(B, V, D, G, dtype);
     if (rc) return rc == kEmptyBatch ? 0 : rc;
@@ -543,9 +562,12 @@ static int pool_fuse_gap_bwd_impl(const void *dS_gap, const int32_t *bins, int64
     bool al;
     rc = make_view_ptrs(dF, g_layout, dtype, B, V, D, gp, sb, al);
     if (rc) return rc;
-    if (!al || !is_aligned(dS_gap, 16) || (tie_mask && !is_aligned(tie_mask, 8))) return GVCNN_E_UNSUPPORTED;
+    if (cf && weights) return GVCNN_E_UNSUPPORTED;
+    // channels-first reads dS_gap element by element (a 16-byte vector of dF can straddle two channels)
+    if (!al || !is_aligned(dS_gap, cf ? elt_size(dtype) : 16) || (tie_mask && !is_aligned(tie_mask, 8)))
+        return GVCNN_E_UNSUPPORTED;
     rc = launch_pool_fuse_gap_bwd(dS_gap, bins, bin_stride_b, weights, weight_stride_b, tie_mask, gp, sb, status, B, V,
-                                  HW, C, G, pool, dtype, static_cast<cudaStream_t>(stream));
+                                  HW, C, G, pool, dtype, cf, static_cast<cudaStream_t>(stream));
     return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
 }
 
@@ -652,6 +674,7 @@ int gvcnn_pool_fuse_gap_bwd_weights(const void *F, const void *dS_gap, const voi
     if (!dS_gap || !S_gap || !bins || !weights || !dweights || !workspace || bin_stride_b < 0 || weight_stride_b < 0)
         return GVCNN_E_BAD_ARG;
     if (pool != GVCNN_POOL_MAX && pool != GVCNN_POOL_MEAN) return GVCNN_E_BAD_MODE;
+    if (f_layout & GVCNN_LAYOUT_CHANNELS_FIRST) return GVCNN_E_UNSUPPORTED;  // channel-last maps only
     ViewPtrs fp;
     int64_t sb;
     bool al;
@@ -673,6 +696,7 @@ int gvcnn_gap_score_bwd(const float *dx, const float *W, void *dmaps, int B, int
                         int dtype, void *stream)
 {
     if (HW <= 0 || C <= 0) return GVCNN_E_BAD_ARG;
+    const bool cf = take_channels_first(m_layout);
     const int64_t D = (int64_t)HW * C;
     int rc = check_dims(B, V, D, 1, dtype);
     if (rc) return rc == kEmptyBatch ? 0 : rc;
@@ -684,7 +708,7 @@ int gvcnn_gap_score_bwd(const float *dx, const float *W, void *dmaps, int B, int
     if (rc) return rc;
     if (!is_aligned(dx, 4) || !is_aligned(W, 16)) return GVCNN_E_MISALIGNED;
     if (!al) return GVCNN_E_UNSUPPORTED;
-    rc = launch_gap_score_bwd(dx, W, dp, sb, B, V, HW, C, dtype, static_cast<cudaStream_t>(stream));
+    rc = launch_gap_score_bwd(dx, W, dp, sb, B, V, HW, C, dtype, cf, static_cast<cudaStream_t>(stream));
     return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
 }
 

@@ -604,7 +604,7 @@ int launch_view_score(const ViewPtrs &rp, int64_t r_sb, const float *W, const fl
                       cudaStream_t st);
 int launch_gap_score(const ViewPtrs &mp, int64_t m_sb, const float *W, const float *bias, float *R_out, float *x,
                      float *scores, int32_t *bins, int32_t *flags, int32_t *status, int B, int V, int HW, int C, int G,
-                     int dtype, bool fuse_bin, int edge_ulps, int clamp, cudaStream_t st);
+                     int dtype, bool fuse_bin, int edge_ulps, int clamp, bool cf, cudaStream_t st);
 int launch_batch_sum_x(const float *x, float *xsum, int B, int V, cudaStream_t st);
 int launch_score_bin(const float *x, float denom, float *x_mean, float *scores, int32_t *bins, int32_t *flags,
                      int32_t *status, int64_t n, int G, int multiplier, int edge_ulps, int clamp, bool x_is_score,
@@ -642,14 +642,17 @@ int launch_pool_fuse_gap_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bi
                              cudaStream_t st);
 int launch_pool_fuse_gap_bwd(const void *dOut, const int32_t *bins, int64_t bin_sb, const float *weights, int64_t w_sb,
                              const uint8_t *mask, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V,
-                             int HW, int C, int G, int pool, int dtype, cudaStream_t st);
+                             int HW, int C, int G, int pool, int dtype, bool cf, cudaStream_t st);
+int launch_pool_fuse_gap_cf_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb, void *out,
+                                uint8_t *mask, int32_t *status, int B, int V, int HW, int C, int G, int pool, float fill,
+                                int dtype, cudaStream_t st);
 void gap_split(int B, int CB, int HW, int &nsplit, int &pps);
 size_t gap_bwd_weights_workspace_bytes(int B, int V, int HW, int C, int dtype);
 int launch_gap_bwd_weights(const ViewPtrs &fp, int64_t f_sb, const void *dS_gap, const void *S_gap,
                            const int32_t *bins, int64_t bin_sb, const float *weights, int64_t w_sb, float *dweights,
                            float *partial, int B, int V, int HW, int C, int G, int pool, int dtype, cudaStream_t st);
 int launch_gap_score_bwd(const float *dx, const float *W, const ViewPtrs &dp, int64_t d_sb, int B, int V, int HW, int C,
-                         int dtype, cudaStream_t st);
+                         int dtype, bool cf, cudaStream_t st);
 int launch_pool_fuse_bwd_fast(const void *dS, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
                               const float *weights, int64_t w_sb, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
                               int pool, int dtype, cudaStream_t st);

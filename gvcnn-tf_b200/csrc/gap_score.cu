@@ -22,6 +22,68 @@ namespace gvcnn {
 
 constexpr int kGapWarps = 8;
 
+// Warp 0's part of a GAP-score kernel, from the 8 slice sums of every channel in part[s][c]: R, x, score, bin, flags.
+template <typename T, int NB, bool FUSE_BIN>
+__device__ __forceinline__ void gap_score_finish(const float (*part)[NB * 32 * Elem<T>::kVec], const int lane, const int b,
+                                                 const int v, const float *__restrict__ W,
+                                                 const float *__restrict__ bias, float *__restrict__ R_out,
+                                                 float *__restrict__ x_out, float *__restrict__ scores,
+                                                 int32_t *__restrict__ bins, int32_t *__restrict__ flag_out,
+                                                 int32_t *status, const int V, const int HW, const int G,
+                                                 const int edge_ulps, const int clamp)
+{
+    constexpr int E = Elem<T>::kVec;
+    constexpr int C = NB * 32 * E;
+
+    const float hw = (float)HW;
+    const float *__restrict__ w = W + (int64_t)v * C + lane * E;
+    float a = 0.0f;
+#pragma unroll
+    for (int u = 0; u < NB; ++u) {
+        float m[E];
+#pragma unroll
+        for (int e = 0; e < E; e += 4) {
+            float4 s4 = *reinterpret_cast<const float4 *>(&part[0][(u * 32 + lane) * E + e]);
+#pragma unroll
+            for (int s = 1; s < kGapWarps; ++s) {  // slices in ascending order; empty slices hold exact zeros
+                const float4 t = *reinterpret_cast<const float4 *>(&part[s][(u * 32 + lane) * E + e]);
+                s4.x = __fadd_rn(s4.x, t.x); s4.y = __fadd_rn(s4.y, t.y);
+                s4.z = __fadd_rn(s4.z, t.z); s4.w = __fadd_rn(s4.w, t.w);
+            }
+            m[e] = __fdiv_rn(s4.x, hw); m[e + 1] = __fdiv_rn(s4.y, hw);
+            m[e + 2] = __fdiv_rn(s4.z, hw); m[e + 3] = __fdiv_rn(s4.w, hw);
+        }
+        if (R_out) {
+            float *ro = R_out + ((int64_t)b * V + v) * C + (u * 32 + lane) * E;
+#pragma unroll
+            for (int e = 0; e < E; e += 4) *reinterpret_cast<float4 *>(ro + e) = make_float4(m[e], m[e + 1], m[e + 2], m[e + 3]);
+        }
+#pragma unroll
+        for (int e = 0; e < E; e += 4) {
+            const float4 wv = __ldg(reinterpret_cast<const float4 *>(w + u * 32 * E + e));
+            a = fmaf(m[e + 0], wv.x, a);
+            a = fmaf(m[e + 1], wv.y, a);
+            a = fmaf(m[e + 2], wv.z, a);
+            a = fmaf(m[e + 3], wv.w, a);
+        }
+    }
+#pragma unroll
+    for (int off = 16; off >= 1; off >>= 1) a = __fadd_rn(a, __shfl_xor_sync(0xffffffffu, a, off));
+    if (lane == 0) {
+        const int64_t row = (int64_t)b * V + v;
+        const float x = __fadd_rn(a, __ldg(bias + v));
+        if (x_out) x_out[row] = x;
+        if constexpr (FUSE_BIN) {
+            float s;
+            int bin;
+            const int flags = score_and_bin(x, 1.0f, G, edge_ulps, clamp, s, bin);
+            scores[row] = s;
+            bins[row] = bin;
+            publish(flags, flag_out ? flag_out + row : nullptr, status);
+        }
+    }
+}
+
 template <typename T, int NB, bool FUSE_BIN>  // NB = 16-byte chunks per lane per position = C / (32 * E)
 __global__ void __launch_bounds__(kGapWarps * 32, 2)
 gap_score_kernel(const ViewPtrs mp, const int64_t m_sb, const float *__restrict__ W, const float *__restrict__ bias,
@@ -86,73 +148,192 @@ gap_score_kernel(const ViewPtrs mp, const int64_t m_sb, const float *__restrict_
                 make_float4(acc[u][e], acc[u][e + 1], acc[u][e + 2], acc[u][e + 3]);
     __syncthreads();
     if (warp != 0) return;
+    gap_score_finish<T, NB, FUSE_BIN>(part, lane, b, v, W, bias, R_out, x_out, scores, bins, flag_out, status, V, HW, G,
+                                      edge_ulps, clamp);
+}
 
-    const float hw = (float)HW;
-    const float *__restrict__ w = W + (int64_t)v * C + lane * E;
-    float a = 0.0f;
+// Channels-first maps (GVCNN_LAYOUT_CHANNELS_FIRST): an item is C rows of HW positions, C * HW contiguous elements.  The
+// item streams in chunks of kGapCfRows whole channels (contiguous, 16-byte aligned at both ends), 16-byte vectors
+// prefetched in registers one chunk ahead, and is widened (exactly) into float32 rows in shared memory whose stride HW | 1
+// is odd, so 32 lanes walking 32 rows position by position hit 32 different banks.  Warp s then sums slice s of every
+// staged row - the channel-last kernel's slices, each sequentially from 0.0f - into part[s][c]: the very partial sums
+// the channel-last kernel leaves there for the transposed maps, so its finishing code gives the same R, x, score, bin
+// and flags bit for bit.
+constexpr int kGapCfRows = 64;  // channels staged per step: two rows per lane
+constexpr int kGapCfRegs = 16;  // 16-byte vectors per thread per step: HW <= 256 (float32) / 512 (16-bit types); larger
+                                // maps take gap_score_cf_blocked_kernel
+constexpr int kGapCfBlk = 128;  // larger maps (gap_score_cf_blocked_kernel): positions staged per step
+
+template <typename T, int NB, bool FUSE_BIN>
+__global__ void __launch_bounds__(kGapWarps * 32, 2)
+gap_score_cf_kernel(const ViewPtrs mp, const int64_t m_sb, const float *__restrict__ W, const float *__restrict__ bias,
+                    float *__restrict__ R_out, float *__restrict__ x_out, float *__restrict__ scores,
+                    int32_t *__restrict__ bins, int32_t *__restrict__ flag_out, int32_t *status, const int B,
+                    const int V, const int HW, const int G, const int edge_ulps, const int clamp)
+{
+    constexpr int E = Elem<T>::kVec;
+    constexpr int C = NB * 32 * E;
+    constexpr int NT = kGapWarps * 32;
+    extern __shared__ __align__(16) float part_raw[];  // [kGapWarps][C] partial channel sums, then [kGapCfRows][HW | 1]
+    float (*part)[C] = reinterpret_cast<float (*)[C]>(part_raw);
+    float *const rows = part_raw + kGapWarps * C;
+
+    const int lane = threadIdx.x & 31;
+    const int warp = threadIdx.x >> 5;
+    const int item = blockIdx.x;
+    const int b = item / V;
+    const int v = item - b * V;
+    const int q = HW / kGapWarps, r = HW % kGapWarps;
+    const int p0 = warp * q + min(warp, r);
+    const int np = q + (warp < r ? 1 : 0);
+    const int ld = HW | 1;
+    const int nvec = kGapCfRows * HW / E;  // exact: kGapCfRows * sizeof(T) is a multiple of 16
+
+    pdl_wait();
+    pdl_launch_dependents();
+    const T *__restrict__ src = reinterpret_cast<const T *>(mp.p[v]) + (int64_t)b * m_sb;
+    uint4 buf[kGapCfRegs];
+    auto load = [&](const int ch) {
+        const uint4 *s4 = reinterpret_cast<const uint4 *>(src + (int64_t)ch * kGapCfRows * HW);
 #pragma unroll
-    for (int u = 0; u < NB; ++u) {
-        float m[E];
+        for (int i = 0; i < kGapCfRegs; ++i)
+            if ((int)threadIdx.x + i * NT < nvec) buf[i] = ldg_stream_16(s4 + threadIdx.x + i * NT);
+    };
+    load(0);
+#pragma unroll 1
+    for (int ch = 0; ch < C / kGapCfRows; ++ch) {
 #pragma unroll
-        for (int e = 0; e < E; e += 4) {
-            float4 s4 = *reinterpret_cast<const float4 *>(&part[0][(u * 32 + lane) * E + e]);
+        for (int i = 0; i < kGapCfRegs; ++i) {
+            const int j = (int)threadIdx.x + i * NT;
+            if (j < nvec) {
+                float f[E];
+                Elem<T>::unpack(buf[i], f);
+                int row = j * E / HW, p = j * E - row * HW;
 #pragma unroll
-            for (int s = 1; s < kGapWarps; ++s) {  // slices in ascending order; empty slices hold exact zeros
-                const float4 t = *reinterpret_cast<const float4 *>(&part[s][(u * 32 + lane) * E + e]);
-                s4.x = __fadd_rn(s4.x, t.x); s4.y = __fadd_rn(s4.y, t.y);
-                s4.z = __fadd_rn(s4.z, t.z); s4.w = __fadd_rn(s4.w, t.w);
+                for (int e = 0; e < E; ++e) {
+                    rows[row * ld + p] = f[e];
+                    if (++p == HW) { p = 0; ++row; }
+                }
             }
-            m[e] = __fdiv_rn(s4.x, hw); m[e + 1] = __fdiv_rn(s4.y, hw);
-            m[e + 2] = __fdiv_rn(s4.z, hw); m[e + 3] = __fdiv_rn(s4.w, hw);
         }
-        if (R_out) {
-            float *ro = R_out + ((int64_t)b * V + v) * C + (u * 32 + lane) * E;
-#pragma unroll
-            for (int e = 0; e < E; e += 4) *reinterpret_cast<float4 *>(ro + e) = make_float4(m[e], m[e + 1], m[e + 2], m[e + 3]);
+        __syncthreads();
+        if (ch + 1 < C / kGapCfRows) load(ch + 1);
+        const float *r0 = rows + lane * ld + p0;
+        const float *r1 = r0 + 32 * ld;
+        float a0 = 0.0f, a1 = 0.0f;
+        for (int j = 0; j < np; ++j) {
+            a0 = __fadd_rn(a0, r0[j]);
+            a1 = __fadd_rn(a1, r1[j]);
         }
-#pragma unroll
-        for (int e = 0; e < E; e += 4) {
-            const float4 wv = __ldg(reinterpret_cast<const float4 *>(w + u * 32 * E + e));
-            a = fmaf(m[e + 0], wv.x, a);
-            a = fmaf(m[e + 1], wv.y, a);
-            a = fmaf(m[e + 2], wv.z, a);
-            a = fmaf(m[e + 3], wv.w, a);
-        }
+        part[warp][ch * kGapCfRows + lane] = a0;
+        part[warp][ch * kGapCfRows + 32 + lane] = a1;
+        __syncthreads();
     }
+    if (warp != 0) return;
+    gap_score_finish<T, NB, FUSE_BIN>(part, lane, b, v, W, bias, R_out, x_out, scores, bins, flag_out, status, V, HW, G,
+                                      edge_ulps, clamp);
+}
+
+// Channels-first maps whose 64-channel chunk does not fit the register prefetch (HW > 256 float32 / 512 16-bit): the
+// chunk is staged in blocks of kGapCfBlk positions (element loads: a block's rows are not contiguous), and each warp
+// carries its slice sums across the blocks.  A slice is a contiguous range of positions, so every slice is still summed
+// in position order from 0.0f and part[s][c] - hence R, x, score, bin and flags - is the channel-last kernel's.
+template <typename T, int NB, bool FUSE_BIN>
+__global__ void __launch_bounds__(kGapWarps * 32, 2)
+gap_score_cf_blocked_kernel(const ViewPtrs mp, const int64_t m_sb, const float *__restrict__ W,
+                            const float *__restrict__ bias, float *__restrict__ R_out, float *__restrict__ x_out,
+                            float *__restrict__ scores, int32_t *__restrict__ bins, int32_t *__restrict__ flag_out,
+                            int32_t *status, const int B, const int V, const int HW, const int G, const int edge_ulps,
+                            const int clamp)
+{
+    constexpr int E = Elem<T>::kVec;
+    constexpr int C = NB * 32 * E;
+    constexpr int NT = kGapWarps * 32;
+    constexpr int ld = kGapCfBlk + 1;  // odd: conflict-free row walks
+    constexpr int kBatch = 8;          // element loads in flight per thread
+    extern __shared__ __align__(16) float part_raw[];  // [kGapWarps][C] partial channel sums, then [kGapCfRows][ld]
+    float (*part)[C] = reinterpret_cast<float (*)[C]>(part_raw);
+    float *const rows = part_raw + kGapWarps * C;
+
+    const int lane = threadIdx.x & 31;
+    const int warp = threadIdx.x >> 5;
+    const int item = blockIdx.x;
+    const int b = item / V;
+    const int v = item - b * V;
+    const int q = HW / kGapWarps, r = HW % kGapWarps;
+    const int p0 = warp * q + min(warp, r);
+    const int p1 = p0 + q + (warp < r ? 1 : 0);
+
+    pdl_wait();
+    pdl_launch_dependents();
+    const T *__restrict__ src = reinterpret_cast<const T *>(mp.p[v]) + (int64_t)b * m_sb;
+#pragma unroll 1
+    for (int ch = 0; ch < C / kGapCfRows; ++ch) {
+        const T *__restrict__ csrc = src + (int64_t)ch * kGapCfRows * HW;
+        float a0 = 0.0f, a1 = 0.0f;
+#pragma unroll 1
+        for (int q0 = 0; q0 < HW; q0 += kGapCfBlk) {
+            const int nb = min(kGapCfBlk, HW - q0);
+            const int n = kGapCfRows * nb;
+#pragma unroll 1
+            for (int j0 = threadIdx.x; j0 < n; j0 += kBatch * NT) {
+                float f[kBatch];
+                int at[kBatch];
 #pragma unroll
-    for (int off = 16; off >= 1; off >>= 1) a = __fadd_rn(a, __shfl_xor_sync(0xffffffffu, a, off));
-    if (lane == 0) {
-        const int64_t row = (int64_t)b * V + v;
-        const float x = __fadd_rn(a, __ldg(bias + v));
-        if (x_out) x_out[row] = x;
-        if constexpr (FUSE_BIN) {
-            float s;
-            int bin;
-            const int flags = score_and_bin(x, 1.0f, G, edge_ulps, clamp, s, bin);
-            scores[row] = s;
-            bins[row] = bin;
-            publish(flags, flag_out ? flag_out + row : nullptr, status);
+                for (int u = 0; u < kBatch; ++u) {
+                    const int j = j0 + u * NT;
+                    const int row = j / nb, p = j - row * nb;
+                    at[u] = j < n ? row * ld + p : -1;
+                    if (j < n) f[u] = Elem<T>::to_float(csrc[(int64_t)row * HW + q0 + p]);
+                }
+#pragma unroll
+                for (int u = 0; u < kBatch; ++u)
+                    if (at[u] >= 0) rows[at[u]] = f[u];
+            }
+            __syncthreads();
+            const int lo = max(p0, q0), hi = min(p1, q0 + nb);
+            const float *r0 = rows + lane * ld - q0;
+            const float *r1 = r0 + 32 * ld;
+            for (int p = lo; p < hi; ++p) {
+                a0 = __fadd_rn(a0, r0[p]);
+                a1 = __fadd_rn(a1, r1[p]);
+            }
+            __syncthreads();
         }
+        part[warp][ch * kGapCfRows + lane] = a0;
+        part[warp][ch * kGapCfRows + 32 + lane] = a1;
     }
+    __syncthreads();
+    if (warp != 0) return;
+    gap_score_finish<T, NB, FUSE_BIN>(part, lane, b, v, W, bias, R_out, x_out, scores, bins, flag_out, status, V, HW, G,
+                                      edge_ulps, clamp);
 }
 
 template <typename T>
 static int launch_gap_score_t(const ViewPtrs &mp, int64_t m_sb, const float *W, const float *bias, float *R_out, float *x,
                               float *scores, int32_t *bins, int32_t *flags, int32_t *status, int B, int V, int HW, int C,
-                              int G, bool fuse_bin, int edge_ulps, int clamp, cudaStream_t st)
+                              int G, bool fuse_bin, int edge_ulps, int clamp, bool cf, cudaStream_t st)
 {
     constexpr int E = Elem<T>::kVec;
     const int64_t items = (int64_t)B * V;
     if (items > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
+    const bool blocked = cf && (int64_t)kGapCfRows * HW > (int64_t)kGapCfRegs * kGapWarps * 32 * E;
     const dim3 grid((unsigned)items), block(kGapWarps * 32);
+    const size_t cf_rows = !cf ? 0 : (size_t)kGapCfRows * (blocked ? kGapCfBlk + 1 : (HW | 1)) * sizeof(float);
     cudaError_t err = cudaSuccess;
+#define GVCNN_LAUNCH_GAP_SCORE_K(KERN_, NB_, FUSE_, EXTRA_)                                                      \
+    do {                                                                                                          \
+        const size_t smem = (size_t)kGapWarps * NB_ * 32 * E * sizeof(float) + EXTRA_;                            \
+        err = ensure_dyn_smem<KERN_<T, NB_, FUSE_>>((int)smem);                                                   \
+        if (err == cudaSuccess)                                                                                   \
+            err = launch_pdl(KERN_<T, NB_, FUSE_>, grid, block, smem, st, mp, m_sb, W, bias, R_out, x, scores,    \
+                             bins, flags, status, B, V, HW, G, edge_ulps, clamp);                                 \
+    } while (0)
 #define GVCNN_LAUNCH_GAP_SCORE(NB_, FUSE_)                                                                        \
     do {                                                                                                          \
-        const size_t smem = (size_t)kGapWarps * NB_ * 32 * E * sizeof(float);                                     \
-        err = ensure_dyn_smem<gap_score_kernel<T, NB_, FUSE_>>((int)smem);                                        \
-        if (err == cudaSuccess)                                                                                   \
-            err = launch_pdl(gap_score_kernel<T, NB_, FUSE_>, grid, block, smem, st, mp, m_sb, W, bias, R_out, x, \
-                             scores, bins, flags, status, B, V, HW, G, edge_ulps, clamp);                         \
+        if (blocked) GVCNN_LAUNCH_GAP_SCORE_K(gap_score_cf_blocked_kernel, NB_, FUSE_, cf_rows);                  \
+        else if (cf) GVCNN_LAUNCH_GAP_SCORE_K(gap_score_cf_kernel, NB_, FUSE_, cf_rows);                          \
+        else GVCNN_LAUNCH_GAP_SCORE_K(gap_score_kernel, NB_, FUSE_, 0);                                           \
     } while (0)
     if (C == 8 * 32 * E) {
         if (fuse_bin) GVCNN_LAUNCH_GAP_SCORE(8, true); else GVCNN_LAUNCH_GAP_SCORE(8, false);
@@ -162,24 +343,25 @@ static int launch_gap_score_t(const ViewPtrs &mp, int64_t m_sb, const float *W, 
         return -1000;
     }
 #undef GVCNN_LAUNCH_GAP_SCORE
+#undef GVCNN_LAUNCH_GAP_SCORE_K
     if (err != cudaSuccess) return (int)err;
     return (int)cudaGetLastError();
 }
 
-// returns -1000 when the channel count is not one of the instantiated ones
+// cf: channels-first maps.  Returns -1000 when the channel count is not one of the instantiated ones
 int launch_gap_score(const ViewPtrs &mp, int64_t m_sb, const float *W, const float *bias, float *R_out, float *x,
                      float *scores, int32_t *bins, int32_t *flags, int32_t *status, int B, int V, int HW, int C, int G,
-                     int dtype, bool fuse_bin, int edge_ulps, int clamp, cudaStream_t st)
+                     int dtype, bool fuse_bin, int edge_ulps, int clamp, bool cf, cudaStream_t st)
 {
     if (dtype == GVCNN_F32)
         return launch_gap_score_t<float>(mp, m_sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW, C, G, fuse_bin,
-                                         edge_ulps, clamp, st);
+                                         edge_ulps, clamp, cf, st);
     if (dtype == GVCNN_BF16)
         return launch_gap_score_t<__nv_bfloat16>(mp, m_sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW, C, G,
-                                                 fuse_bin, edge_ulps, clamp, st);
+                                                 fuse_bin, edge_ulps, clamp, cf, st);
     if (dtype == GVCNN_F16)
         return launch_gap_score_t<__half>(mp, m_sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW, C, G,
-                                          fuse_bin, edge_ulps, clamp, st);
+                                          fuse_bin, edge_ulps, clamp, cf, st);
     return GVCNN_E_BAD_DTYPE;
 }
 

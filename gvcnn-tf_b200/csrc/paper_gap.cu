@@ -248,16 +248,64 @@ gap_score_bwd_kernel(const float *__restrict__ dx, const float *__restrict__ W, 
     for (int p = 0; p < HW; ++p) stg_stream_16(dst + (int64_t)p * C, packed);
 }
 
-// returns -1000 when C is not a multiple of the 16-byte vector
+// Channels-first dmaps[b, v, c, p]: the item's C * HW elements are contiguous, channel-major, written in 16-byte vectors
+// (a vector may straddle two channels).  A thread computes RN(RN(dx[b, v] * W[v, c]) / HW) when its walk reaches a new
+// channel - once per vector for HW >= E - so there is no table of C values and no bound on C.  grid = B * V.
+template <typename T>
+__global__ void __launch_bounds__(256)
+gap_score_bwd_cf_kernel(const float *__restrict__ dx, const float *__restrict__ W, const ViewPtrs dp, const int64_t d_sb,
+                        const int V, const int HW, const int C)
+{
+    constexpr int E = Elem<T>::kVec;
+    const int item = blockIdx.x;
+    const int b = item / V, v = item - b * V;
+    pdl_wait();
+    pdl_launch_dependents();
+    const float g = dx[item];
+    const float hw = (float)HW;
+    const float *__restrict__ w = W + (int64_t)v * C;
+    T *dst = reinterpret_cast<T *>(dp.p[v]) + (int64_t)b * d_sb;
+    const int64_t nvec = (int64_t)C * HW / E;
+    for (int64_t i = threadIdx.x; i < nvec; i += 256) {
+        const int64_t j = i * E;
+        int c = (int)(j / HW), p = (int)(j - (int64_t)c * HW);
+        float val = __fdiv_rn(__fmul_rn(g, __ldg(w + c)), hw);
+        float o[E];
+#pragma unroll
+        for (int e = 0; e < E; ++e) {
+            o[e] = val;
+            if (++p == HW && e + 1 < E) {
+                p = 0;
+                val = __fdiv_rn(__fmul_rn(g, __ldg(w + ++c)), hw);
+            }
+        }
+        stg_stream_16(dst + j, Elem<T>::pack(o));
+    }
+}
+
+// cf: channels-first dmaps.  Returns -1000 when C (channel-last) or C * HW (channels-first) is not a multiple of the
+// 16-byte vector
 int launch_gap_score_bwd(const float *dx, const float *W, const ViewPtrs &dp, int64_t d_sb, int B, int V, int HW, int C,
-                         int dtype, cudaStream_t st)
+                         int dtype, bool cf, cudaStream_t st)
 {
     const int E = dtype == GVCNN_F32 ? 4 : 8;
-    if (C % E) return -1000;
+    if (cf ? ((int64_t)C * HW) % E != 0 : C % E != 0) return -1000;
     const int64_t items = (int64_t)B * V;
     if (items > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
-    const dim3 grid((unsigned)items, (unsigned)((C / E + 255) / 256));
     cudaError_t err;
+    if (cf) {
+        const dim3 grid((unsigned)items);
+        if (dtype == GVCNN_F32)
+            err = launch_pdl(gap_score_bwd_cf_kernel<float>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
+        else if (dtype == GVCNN_BF16)
+            err = launch_pdl(gap_score_bwd_cf_kernel<__nv_bfloat16>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
+        else if (dtype == GVCNN_F16)
+            err = launch_pdl(gap_score_bwd_cf_kernel<__half>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
+        else
+            return GVCNN_E_BAD_DTYPE;
+        return (int)err;
+    }
+    const dim3 grid((unsigned)items, (unsigned)((C / E + 255) / 256));
     if (dtype == GVCNN_F32)
         err = launch_pdl(gap_score_bwd_kernel<float>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
     else if (dtype == GVCNN_BF16)

@@ -49,9 +49,32 @@ __device__ __forceinline__ uint32_t prmt_sign(const uint32_t a, const uint32_t s
     return d;
 }
 
+// 16-byte vector of dOut values for descriptor elements d .. d + E - 1 of channels-first maps (D = C * HW): element d
+// belongs to channel d / HW, so a vector can straddle two channels.  Bit-identical to the channel-last vector of the
+// same channels.
+template <typename T>
+__device__ __forceinline__ uint4 gather_channels_first(const T *__restrict__ row, const int64_t d, const int HW)
+{
+    constexpr int E = Elem<T>::kVec;
+    int c = (int)(d / HW), p = (int)(d - (int64_t)c * HW);
+    uint32_t w[4];
+#pragma unroll
+    for (int e = 0; e < E; ++e) {
+        uint32_t x;
+        if constexpr (sizeof(T) == 4) x = __ldg(reinterpret_cast<const uint32_t *>(row) + c);
+        else x = __ldg(reinterpret_cast<const unsigned short *>(row) + c);
+        if constexpr (sizeof(T) == 4) w[e] = x;
+        else if (e & 1) w[e >> 1] |= x << 16;
+        else w[e >> 1] = x;
+        if (++p == HW) { p = 0; ++c; }
+    }
+    return make_uint4(w[0], w[1], w[2], w[3]);
+}
+
 // GAP: dS is the gradient of the global average pool that follows the fusion, [B, C] (D = HW * C,
 // channel-last): dS[b, p, c] = dOut[b, c] / HW (tf.reduce_mean's gradient), never materialised.
-template <typename T, int POOL, int V, int NT, bool GAP, bool WTS, int UPC, bool GRP>
+// CF (with GAP): channels-first maps, dS[b, c, p] = dOut[b, c] / HW.
+template <typename T, int POOL, int V, int NT, bool GAP, bool WTS, int UPC, bool GRP, bool CF>
 __global__ void __launch_bounds__(NT)
 pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ bins, const int64_t bin_sb,
                           const uint8_t *__restrict__ mask, const float *__restrict__ weights, const int64_t w_sb,
@@ -65,6 +88,7 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
     constexpr int TD = NT * E;
     static_assert(UPC * 32 <= NT, "one planning warp per unit");
     static_assert(!GRP || (!GAP && !WTS), "per-group gradients take no GAP and no weights");
+    static_assert(!CF || (GAP && !WTS), "channels-first: the GAP-folded backward with the reference's weights only");
     using PlanT = std::conditional_t<GRP, BwdPlanGrp, BwdPlan>;
     // A CTA handles UPC consecutive (shape, tile) units: their loads are all in flight before the one barrier, and
     // warp i plans unit i, so the per-CTA costs (launch slot, barrier, reciprocal table) are paid once per UPC tiles.
@@ -91,7 +115,8 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
         if (actives[i]) {
             if constexpr (GRP) {
                 // dP rows are known only once the plan is: loaded at each group start below
-            } else if constexpr (GAP) raws[i] = *reinterpret_cast<const uint4 *>(dS + (int64_t)b * C + (int)((d0 + e0) % C));
+            } else if constexpr (CF) raws[i] = gather_channels_first(dS + (int64_t)b * C, d0 + e0, HW);
+            else if constexpr (GAP) raws[i] = *reinterpret_cast<const uint4 *>(dS + (int64_t)b * C + (int)((d0 + e0) % C));
             else raws[i] = ldg_stream_16(dS + off);
             if constexpr (POOL == GVCNN_POOL_MAX) {
 #pragma unroll
@@ -310,7 +335,7 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
 template <typename T, int V, int NT = 256>
 static int launch_bwd_fast_v(const void *dS, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
                              const float *weights, int64_t w_sb, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int64_t D, int G, int pool,
-                             cudaStream_t st, int gapC = 0, int gapHW = 0, bool grp = false)
+                             cudaStream_t st, int gapC = 0, int gapHW = 0, bool grp = false, bool cf = false)
 {
     constexpr int E = Elem<T>::kVec;
     const int64_t td = (int64_t)NT * E;
@@ -322,24 +347,27 @@ static int launch_bwd_fast_v(const void *dS, const int32_t *bins, int64_t bin_sb
     constexpr int upc = 1;
     const unsigned grid = (unsigned)((units + upc - 1) / upc);
     cudaError_t err;
-#define GVCNN_LAUNCH_BF(POOL_, GAP_, WTS_, UPC_, GRP_)                                                        \
-    err = launch_pdl(pool_fuse_bwd_fast_kernel<T, POOL_, V, NT, GAP_, WTS_, UPC_, GRP_>, dim3(grid), dim3(NT), 0, st, \
+#define GVCNN_LAUNCH_BF(POOL_, GAP_, WTS_, UPC_, GRP_, CF_)                                                   \
+    err = launch_pdl(pool_fuse_bwd_fast_kernel<T, POOL_, V, NT, GAP_, WTS_, UPC_, GRP_, CF_>, dim3(grid), dim3(NT), 0, st, \
                      static_cast<const T *>(dS), bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G,   \
                      (int)tiles, gapC, gapHW, units)
-#define GVCNN_LAUNCH_BF_P(GAP_, WTS_, GRP_)                                                                   \
+#define GVCNN_LAUNCH_BF_P(GAP_, WTS_, GRP_, CF_)                                                              \
     do {                                                                                                      \
-        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_BF(GVCNN_POOL_MAX, GAP_, WTS_, upc, GRP_);                   \
-        else GVCNN_LAUNCH_BF(GVCNN_POOL_MEAN, GAP_, WTS_, upc, GRP_);                                         \
+        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_BF(GVCNN_POOL_MAX, GAP_, WTS_, upc, GRP_, CF_);              \
+        else GVCNN_LAUNCH_BF(GVCNN_POOL_MEAN, GAP_, WTS_, upc, GRP_, CF_);                                    \
     } while (0)
     if (grp) {  // per-group gradients dP [G, B, D] (gvcnn_view_pooling_bwd)
-        GVCNN_LAUNCH_BF_P(false, false, true);
+        GVCNN_LAUNCH_BF_P(false, false, true, false);
+    } else if (gapC > 0 && cf) {
+        if (weights) return -1000;
+        GVCNN_LAUNCH_BF_P(true, false, false, true);
     } else if (gapC > 0) {
-        if (weights) GVCNN_LAUNCH_BF_P(true, true, false);  // paper mode: caller-supplied weights
-        else GVCNN_LAUNCH_BF_P(true, false, false);
+        if (weights) GVCNN_LAUNCH_BF_P(true, true, false, false);  // paper mode: caller-supplied weights
+        else GVCNN_LAUNCH_BF_P(true, false, false, false);
     } else if (weights) {
-        GVCNN_LAUNCH_BF_P(false, true, false);
+        GVCNN_LAUNCH_BF_P(false, true, false, false);
     } else {
-        GVCNN_LAUNCH_BF_P(false, false, false);
+        GVCNN_LAUNCH_BF_P(false, false, false, false);
     }
 #undef GVCNN_LAUNCH_BF_P
 #undef GVCNN_LAUNCH_BF
@@ -380,22 +408,23 @@ static int launch_bwd_fast_t(const void *dS, const int32_t *bins, int64_t bin_sb
 }
 
 // GAP-folded backward: dOut [B, C] -> dF; same applicability as the forward GAP kernel plus the fast-kernel V set.
-// weights (nullable): caller-supplied group weights, as in the forward
+// weights (nullable): caller-supplied group weights, as in the forward.  cf: channels-first maps (16-byte aligned rows,
+// any C; the reference's weights only)
 int launch_pool_fuse_gap_bwd(const void *dOut, const int32_t *bins, int64_t bin_sb, const float *weights, int64_t w_sb,
                              const uint8_t *mask, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V,
-                             int HW, int C, int G, int pool, int dtype, cudaStream_t st)
+                             int HW, int C, int G, int pool, int dtype, bool cf, cudaStream_t st)
 {
     const int64_t D = (int64_t)HW * C;
     const int td = 256 * (dtype == GVCNN_F32 ? 4 : 8);
-    if (C % td != 0) return -1000;
+    if (cf ? (weights != nullptr || D % (dtype == GVCNN_F32 ? 4 : 8) != 0) : C % td != 0) return -1000;
 #define GVCNN_GAPB_CASE(T_)                                                                                   \
     switch (V) {                                                                                              \
-    case 4: return launch_bwd_fast_v<T_, 4>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW);   \
-    case 6: return launch_bwd_fast_v<T_, 6>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW);   \
-    case 8: return launch_bwd_fast_v<T_, 8>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW);   \
-    case 12: return launch_bwd_fast_v<T_, 12>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW); \
-    case 16: return launch_bwd_fast_v<T_, 16>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW); \
-    case 20: return launch_bwd_fast_v<T_, 20>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW); \
+    case 4: return launch_bwd_fast_v<T_, 4>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW, false, cf);   \
+    case 6: return launch_bwd_fast_v<T_, 6>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW, false, cf);   \
+    case 8: return launch_bwd_fast_v<T_, 8>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW, false, cf);   \
+    case 12: return launch_bwd_fast_v<T_, 12>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW, false, cf); \
+    case 16: return launch_bwd_fast_v<T_, 16>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW, false, cf); \
+    case 20: return launch_bwd_fast_v<T_, 20>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW, false, cf); \
     default: return -1000;                                                                                    \
     }
     if (dtype == GVCNN_F32) { GVCNN_GAPB_CASE(float) }

@@ -9,6 +9,8 @@
 // writes one float32 partial row; gap_finish_kernel adds the splits in ascending order and divides by h*w.
 // Saves the write of S ([N, h*w*C], 1/(V+1) of the forward traffic) and, with gvcnn_pool_fuse_gap_bwd, the
 // read of dS in the backward.  Max pooling does not commute with the GAP, so the pooling itself is unchanged.
+#include <algorithm>
+
 #include "ring_common.cuh"
 
 namespace gvcnn {
@@ -184,6 +186,142 @@ __global__ void __launch_bounds__(256) gap_finish_kernel(const float *__restrict
     out[i] = Elem<T>::from_float(__fdiv_rn(sum, hw));
 }
 
+// Channels-first maps (GVCNN_LAYOUT_CHANNELS_FIRST): D = C * HW with the HW positions of a channel contiguous.  A work
+// unit is (shape b, block cb of K whole channels): for every view ONE contiguous run of K * HW elements, 16-byte aligned
+// at both ends (the launcher chooses K so), streamed through the same ring in tiles of NCONS * E elements (the last one
+// shorter) with the same producer plan and ring_consume_tile - S at every position is pool_fwd_ring.cu's, and the tie
+// planes are written at the channels-first index of D.  The consumers park S (float32) in one shared row per channel,
+// stride HW | 1 (odd: the summing threads below hit different banks); after the run, thread c < K adds its channel's HW
+// values in position order from 0.0f, divides once by HW and rounds once to T.  No position split: B * C / K units
+// fill the machine at the batch sizes of training, and no partial rows or finishing kernel are needed.
+template <typename T, int POOL, bool MASK, int V, int NCONS, int MINB>
+__global__ void __launch_bounds__(NCONS + kRingProducerThreads, MINB)
+pool_fuse_gap_cf_fwd_kernel(const ViewPtrs fp, const int64_t f_sb, const int32_t *__restrict__ bins,
+                            const int64_t bin_sb, T *__restrict__ out, uint8_t *__restrict__ mask, int32_t *status,
+                            const int B, const int C, const int HW, const int G, const float fill, const int K,
+                            const int num_units, const int stages)
+{
+    constexpr int E = Elem<T>::kVec;
+    constexpr int kMaxStages = 8;
+    constexpr int TD = NCONS * E;
+    constexpr uint32_t kRowStride = (uint32_t)NCONS * 16u;
+    constexpr uint32_t kStageBytes = kRowStride * (uint32_t)V;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    __shared__ RingPlan plans[kMaxStages];
+    __shared__ int32_t sorted_bin[32];
+    __shared__ __align__(8) uint64_t full_bar[kMaxStages];
+    __shared__ __align__(8) uint64_t empty_bar[kMaxStages];
+    float *const srow = reinterpret_cast<float *>(smem_raw + (size_t)stages * kStageBytes);  // [K][HW | 1]
+
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < stages; ++s) {
+            mbar_init(&full_bar[s], 1);
+            mbar_init(&empty_bar[s], (uint32_t)(NCONS >> 5));
+        }
+        mbar_fence_init();
+    }
+    __syncthreads();
+    pdl_wait();
+    pdl_launch_dependents();
+
+    const int64_t D = (int64_t)HW * C;
+    const int L = K * HW;  // elements of one view in a unit
+    const int CB = C / K;
+    const int ntiles = (L + TD - 1) / TD;
+    int s = 0;
+    uint32_t ph = 0;
+
+    if ((int)threadIdx.x >= NCONS) {
+        // ------------------------------------------------------------------ producer warp
+        const int lane = threadIdx.x & 31;
+        for (int u = blockIdx.x; u < num_units; u += gridDim.x) {
+            const int cb = u % CB;
+            const int b = u / CB;
+            int bin = 0x7fffffff;
+            if (lane < V) {
+                bin = __ldg(bins + (int64_t)b * bin_sb + lane);
+                if (bin < 0 || bin >= G) {
+                    if (status && cb == 0) atomicAdd(status + GVCNN_STATUS_BIN_RANGE, 1);
+                    bin = bin < 0 ? 0 : G - 1;
+                }
+            }
+            int below = 0, same_before = 0;
+#pragma unroll
+            for (int q = 0; q < V; ++q) {
+                const int bu = __shfl_sync(0xffffffffu, bin, q);
+                below += (bu < bin);
+                same_before += (bu == bin) & (q < lane);
+            }
+            const int k = below + same_before;
+            const bool first = lane < V && same_before == 0;
+            const uint32_t fm = __reduce_or_sync(0xffffffffu, first ? (1u << k) : 0u);
+            __syncwarp();
+            if (lane < V) sorted_bin[k] = bin;
+            __syncwarp();
+            const int prev = (lane < V && k > 0) ? sorted_bin[k - 1] : -1;
+            const int last_bin = sorted_bin[V - 1];
+            for (int t = 0; t < ntiles; ++t) {
+                const uint32_t bytes = (uint32_t)min(TD, L - t * TD) * (uint32_t)sizeof(T);
+                const int64_t d0 = (int64_t)cb * L + (int64_t)t * TD;
+                if (lane == 0) mbar_wait(&empty_bar[s], ph ^ 1u);
+                __syncwarp();
+                if (lane < V) plans[s].skip[k] = (uint8_t)(first ? bin - prev - 1 : 0);
+                if (lane == 0) {
+                    plans[s].first_mask = fm;
+                    plans[s].tail_skip = (uint32_t)(G - 1 - last_bin);
+                }
+                __syncwarp();
+                if (lane == 0) mbar_expect_tx(&full_bar[s], bytes * (uint32_t)V);
+                __syncwarp();
+                if (lane < V)
+                    bulk_g2s(smem_raw + (size_t)s * kStageBytes + (size_t)k * kRowStride,
+                             fp.p[lane] + ((int64_t)b * f_sb + d0) * (int64_t)sizeof(T), bytes, &full_bar[s]);
+                if (++s == stages) { s = 0; ph ^= 1u; }
+            }
+        }
+        return;
+    }
+
+    // ---------------------------------------------------------------------- consumer warps
+    const int e0 = threadIdx.x * E;
+    const int ld = HW | 1;
+    const float sumw = (float)(G + V);
+    const float rcp_sumw = __frcp_rn(sumw);
+    for (int u = blockIdx.x; u < num_units; u += gridDim.x) {
+        const int cb = u % CB;
+        const int b = u / CB;
+        for (int t = 0; t < ntiles; ++t) {
+            const int j0 = t * TD + e0;  // element of the run
+            const bool active = j0 < L;
+            const unsigned char *col = smem_raw + (size_t)s * kStageBytes + (size_t)threadIdx.x * 16;
+            mbar_wait(&full_bar[s], ph);
+            float acc[E];
+            ring_consume_tile<T, POOL, MASK, V, kRowStride>(col, plans[s], fill, active, mask, B, D,
+                                                            (int64_t)b * D + (int64_t)cb * L + j0, acc);
+            __syncwarp();
+            if ((threadIdx.x & 31) == 0) mbar_arrive(&empty_bar[s]);
+            div_vec_by_rcp(acc, sumw, rcp_sumw);  // S at these positions (pool_fwd_ring.cu's division)
+            if (active) {
+                int c = j0 / HW, p = j0 - c * HW;
+#pragma unroll
+                for (int e = 0; e < E; ++e) {
+                    srow[c * ld + p] = acc[e];
+                    if (++p == HW) { p = 0; ++c; }
+                }
+            }
+            if (++s == stages) { s = 0; ph ^= 1u; }
+        }
+        asm volatile("bar.sync 1, %0;" ::"r"(NCONS) : "memory");  // the consumers only: the run's S is parked
+        if ((int)threadIdx.x < K) {
+            const float *row = srow + threadIdx.x * ld;
+            float sum = 0.0f;
+            for (int p = 0; p < HW; ++p) sum = __fadd_rn(sum, row[p]);
+            out[(int64_t)b * C + (int64_t)cb * K + threadIdx.x] = Elem<T>::from_float(__fdiv_rn(sum, (float)HW));
+        }
+        asm volatile("bar.sync 1, %0;" ::"r"(NCONS) : "memory");  // rows read before the next unit parks its S
+    }
+}
+
 static int gap_sm_count()
 {
     static int cached = 0;
@@ -295,6 +433,79 @@ int launch_pool_fuse_gap_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bi
     if (dtype == GVCNN_F16) { GVCNN_GAP_CASE(__half) }
     return GVCNN_E_BAD_DTYPE;
 #undef GVCNN_GAP_CASE
+}
+
+// Channels-first: K whole channels per unit - K divides C, the runs of K * HW elements start and end 16-byte aligned,
+// one summing thread per channel, and the K parked rows fit next to at least two ring stages.  The largest such K.
+template <typename T, int V, int MINB>
+static int launch_gap_cf_v(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb, void *out,
+                           uint8_t *mask, int32_t *status, int B, int HW, int C, int G, int pool, float fill,
+                           cudaStream_t st)
+{
+    constexpr int NCONS = 256;
+    constexpr size_t stage_bytes = (size_t)V * NCONS * 16;
+    const size_t budget = (size_t)(226 * 1024) / MINB - 3 * 1024;  // static shared memory per CTA: ~1.3 KB
+    if (budget < 2 * stage_bytes) return -1000;
+    const size_t row_cap = std::min<size_t>(budget - 2 * stage_bytes, 32 * 1024);
+    const int ld = HW | 1;
+    int K = 0;
+    for (int k = std::min(C, NCONS); k >= 1 && K == 0; --k)
+        if (C % k == 0 && ((int64_t)k * HW * (int64_t)sizeof(T)) % 16 == 0 && (size_t)k * ld * sizeof(float) <= row_cap)
+            K = k;
+    if (K == 0) return -1000;
+    const size_t row_bytes = ((size_t)K * ld * sizeof(float) + 15) & ~(size_t)15;
+    int stages = (int)((budget - row_bytes) / stage_bytes);
+    if (stages > 8) stages = 8;
+    const int64_t units = (int64_t)B * (C / K);
+    if (units > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
+    const size_t smem = stage_bytes * stages + row_bytes;
+    const int64_t max_grid = (int64_t)gap_sm_count() * MINB;
+    const int grid = (int)(units < max_grid ? units : max_grid);
+    const bool want_mask = (mask != nullptr) && pool == GVCNN_POOL_MAX;
+    cudaError_t err = cudaSuccess;
+#define GVCNN_LAUNCH_GAP_CF(POOL_, MASK_)                                                                     \
+    do {                                                                                                      \
+        auto kern = pool_fuse_gap_cf_fwd_kernel<T, POOL_, MASK_, V, NCONS, MINB>;                             \
+        err = ensure_dyn_smem<pool_fuse_gap_cf_fwd_kernel<T, POOL_, MASK_, V, NCONS, MINB>>((int)smem);       \
+        if (err == cudaSuccess)                                                                               \
+            err = launch_pdl(kern, dim3(grid), dim3(NCONS + kRingProducerThreads), smem, st, fp, f_sb, bins,  \
+                             bin_sb, static_cast<T *>(out), mask, status, B, C, HW, G, fill, K, (int)units,   \
+                             stages);                                                                         \
+    } while (0)
+    if (pool == GVCNN_POOL_MAX) {
+        if (want_mask) GVCNN_LAUNCH_GAP_CF(GVCNN_POOL_MAX, true); else GVCNN_LAUNCH_GAP_CF(GVCNN_POOL_MAX, false);
+    } else {
+        GVCNN_LAUNCH_GAP_CF(GVCNN_POOL_MEAN, false);
+    }
+#undef GVCNN_LAUNCH_GAP_CF
+    if (err != cudaSuccess) return (int)err;
+    return (int)cudaGetLastError();
+}
+
+// channels-first maps, the reference's own weights; returns -1000 when the shapes are not supported (V not
+// instantiated, G > 255, or no channel block whose runs align)
+int launch_pool_fuse_gap_cf_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb, void *out,
+                                uint8_t *mask, int32_t *status, int B, int V, int HW, int C, int G, int pool, float fill,
+                                int dtype, cudaStream_t st)
+{
+    if (G > 255) return -1000;
+    // V = 12 with the tie planes needs more than the 96 registers two CTAs per SM leave (it spilled): one CTA per SM, which
+    // still holds four ring stages
+#define GVCNN_GAP_CF_CASE(T_)                                                                                 \
+    switch (V) {                                                                                              \
+    case 4: return launch_gap_cf_v<T_, 4, 2>(fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st);   \
+    case 6: return launch_gap_cf_v<T_, 6, 2>(fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st);   \
+    case 8: return launch_gap_cf_v<T_, 8, 2>(fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st);   \
+    case 12: return launch_gap_cf_v<T_, 12, 1>(fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st); \
+    case 16: return launch_gap_cf_v<T_, 16, 1>(fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st); \
+    case 20: return launch_gap_cf_v<T_, 20, 1>(fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st); \
+    default: return -1000;                                                                                    \
+    }
+    if (dtype == GVCNN_F32) { GVCNN_GAP_CF_CASE(float) }
+    if (dtype == GVCNN_BF16) { GVCNN_GAP_CF_CASE(__nv_bfloat16) }
+    if (dtype == GVCNN_F16) { GVCNN_GAP_CF_CASE(__half) }
+    return GVCNN_E_BAD_DTYPE;
+#undef GVCNN_GAP_CF_CASE
 }
 
 }  // namespace gvcnn

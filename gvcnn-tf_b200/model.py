@@ -135,6 +135,7 @@ class _Views:
 
     def __init__(self, x, layout: Optional[str], name: str):
         self.keep = []
+        self.cf = False                                       # channels-first maps: see map_layout
         if isinstance(x, (list, tuple)):                      # the reference's Python list of views
             if len(x) == 0:
                 raise ValueError("%s: empty view list" % name)
@@ -192,10 +193,18 @@ class _Views:
         """From what _view_args returns."""
         return cls(tensors if lay == "list" else tensors[0], lay, name)
 
+    @property
+    def map_layout(self):
+        """Layout code for the entry points that read spatial maps: with GVCNN_LAYOUT_CHANNELS_FIRST when the maps are
+        channel-major ([C, h, w] per shape and view)."""
+        return self.layout | (C.LAYOUT_CHANNELS_FIRST if self.cf else 0)
+
     def empty_like(self):
         """Fresh storage of the same layout (for dF)."""
         out = [torch.empty_like(t) for t in self.keep] if self.kind == "list" else torch.empty_like(self.tensor)
-        return out, _Views(out, self.kind, "dF")
+        gv = _Views(out, self.kind, "dF")
+        gv.cf = self.cf
+        return out, gv
 
 
 def _view_args(x, layout):
@@ -204,6 +213,51 @@ def _view_args(x, layout):
     if isinstance(x, (list, tuple)):
         return tuple(x), "list"
     return (x,), (layout or "bvd")
+
+
+_DATA_FORMATS = ("channels_last", "channels_first")
+
+
+def _check_data_format(data_format):
+    if data_format not in _DATA_FORMATS:
+        raise ValueError("data_format must be 'channels_last' or 'channels_first', got %r" % (data_format,))
+
+
+def _nhwc(t):
+    """A channels-first map tensor [..., C, h, w] as its [..., h, w, C] permutation when that is contiguous (e.g. an
+    [N, C, h, w] tensor in torch.channels_last memory format), else None."""
+    p = t.movedim(-3, -1)
+    return p if p.is_contiguous() else None
+
+
+def _maps_in_memory_order(views, lay):
+    """Channels-first maps ([..., C, h, w]; `views`, `lay` from _view_args) as the kernels read them: (tensors, cf).
+    cf False: the [..., h, w, C] permutations of maps whose memory is channel-last (torch.channels_last), no copy -
+    the channel-last kernels.  cf True: contiguous [..., C, h, w] - the channels-first kernels; other strides are
+    copied once.  A list follows its first view's memory order; a view in another order is copied to that one."""
+    first = _nhwc(views[0])
+    if first is not None:
+        return (first,) + tuple(v.movedim(-3, -1).contiguous() for v in views[1:]), False
+    return tuple(v.contiguous() for v in views), True
+
+
+def _is_maps(views, lay):
+    """The view argument holds spatial maps: two axes after the channel axis."""
+    return views[0].dim() >= (4 if lay == "list" else 5)
+
+
+def _final_maps(final_view_descriptors, layout, data_format):
+    """Final view maps for the element-wise pooling + fusion: with data_format='channels_first', maps whose memory is
+    channel-last go in as their [..., h, w, C] permutation (no copy) and the second value is True (the fused map is
+    permuted back); anything else goes in unchanged."""
+    _check_data_format(data_format)
+    if data_format != "channels_first":
+        return final_view_descriptors, False
+    views, lay = _view_args(final_view_descriptors, layout)
+    if not (len(views) and isinstance(views[0], torch.Tensor) and _is_maps(views, lay)) or _nhwc(views[0]) is None:
+        return final_view_descriptors, False
+    views, _ = _maps_in_memory_order(views, lay)
+    return (list(views) if lay == "list" else views[0]), True
 
 
 def _tie_mask(fv, pool, want):
@@ -290,13 +344,30 @@ def _new_status(dev):
     return torch.zeros(C.STATUS_WORDS, dtype=torch.int32, device=dev)
 
 
-def _raw_views(R, layout, c_raw):
+def _raw_views(R, layout, c_raw, data_format="channels_last"):
     """The raw view descriptors in either form the reference has them in: already pooled ([N, C_raw] per view,
     after GlobalAveragePooling2D, nets/model.py:144) or the block3 maps themselves ([N, h, w, C_raw] per view,
-    channel-last) - told apart by the trailing shape against the Dense(1) kernel's C_raw.  Returns (_Views, HW)."""
+    channel-last; [N, C_raw, h, w] with data_format='channels_first') - told apart by the shape against the Dense(1)
+    kernel's C_raw.  Returns (_Views, HW)."""
+    _check_data_format(data_format)
+    cf = False
+    if data_format == "channels_first" and c_raw > 0:
+        views, lay = _view_args(R, layout)
+        if not isinstance(views[0], torch.Tensor):
+            raise TypeError("R must be a torch.Tensor or a list of them")
+        if _is_maps(views, lay):
+            if views[0].shape[-3] != c_raw:
+                raise ValueError("raw view maps: channel dimension %d (dim -3, data_format='channels_first') does not "
+                                 "match the score kernel's C_raw = %d" % (views[0].shape[-3], c_raw))
+            _require_cuda(views[0], "R")
+            views, cf = _maps_in_memory_order(views, lay)
+            R = list(views) if lay == "list" else views[0]
     rv = _Views(R, layout, "R")
+    rv.cf = cf
     HW = 1
-    if c_raw > 0 and rv.D != c_raw:
+    if cf:
+        HW = rv.D // c_raw
+    elif c_raw > 0 and rv.D != c_raw:
         last = rv.view_shape[-1]
         if last != c_raw or rv.D % c_raw:
             raise ValueError("raw view descriptors: trailing dimension %d does not match the score kernel's C_raw = %d"
@@ -307,7 +378,7 @@ def _raw_views(R, layout, c_raw):
 
 def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulps=4, clamp=False,
               check=True, process_group=None, multiplier=None, status=None, exchange=None,
-              global_count=None) -> ScoreResult:
+              global_count=None, data_format="channels_last") -> ScoreResult:
     """Per-view discrimination score and bin.
 
     R: raw view descriptors after GAP (nets/model.py:144), [B, V, C] ('bvd'),
@@ -315,6 +386,10 @@ def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulp
        Or the raw MAPS before the GAP ([B, V, h, w, C] / [V, B, h, w, C] / list of V [N, h, w, C], channel-last -
        end_points['resnet_v2_50/block3']): the GlobalAveragePooling2D of nets/model.py:144 then runs inside the
        score kernel (gvcnn_gap_score_bin_fwd) and the pooled [B, V, C] tensor is never written.
+    data_format: where the channel axis of the maps is, as in Keras's GlobalAveragePooling2D: 'channels_last'
+       ([..., h, w, C], the reference's) or 'channels_first' ([..., C, h, w], PyTorch's).  Channels-first maps are read
+       as they lie in memory: contiguous NCHW by the channels-first kernels, torch.channels_last (NHWC) memory by the
+       channel-last ones through a permuted view; neither is copied.  The bins do not depend on the memory format.
     W [V, C], b [V]: the V separate Dense(1) layers (nets/model.py:145), float32.
     score_reduce 'shape': one score per (shape, view), bins [B, V] - the
        reference at batch size 1 per shape.  'batch': the literal
@@ -337,9 +412,10 @@ def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulp
     the batch mean is all-reduced over the ranks, so when a score gradient flows on one rank it must flow on every
     rank, one with an empty shard included.
     """
+    _check_data_format(data_format)
     _check_score_fc(W, b)
     Wc, bc = W.contiguous(), b.contiguous()
-    rv, HW = _raw_views(R, layout, int(Wc.shape[-1]) if Wc.dim() == 2 else -1)
+    rv, HW = _raw_views(R, layout, int(Wc.shape[-1]) if Wc.dim() == 2 else -1, data_format)
     Craw = rv.D // HW
     if tuple(Wc.shape) != (rv.V, Craw) or tuple(bc.shape) != (rv.V,):
         raise ValueError("W must be [V, C] = %s and b [V], got %s and %s"
@@ -416,7 +492,7 @@ def _score_bwd(dscores, W, x, scores, R_out, sg: _ScoreGrad, need_wb: bool, need
                                                    rv.layout, _dtype_code(rv.dtype), _stream()),
                             "gvcnn_view_score_bwd")
         if need_r and HW > 1 and B > 0:
-            C.check(L.gvcnn_gap_score_bwd(_ptr(dx), _ptr(W), dR_views.arg, B, V, HW, Craw, rv.layout,
+            C.check(L.gvcnn_gap_score_bwd(_ptr(dx), _ptr(W), dR_views.arg, B, V, HW, Craw, rv.map_layout,
                                           _dtype_code(rv.dtype), _stream()), "gvcnn_gap_score_bwd")
     if need_r:
         dR = tuple(dR_out) if isinstance(dR_out, list) else (dR_out,)
@@ -464,7 +540,7 @@ def _score_bin_fwd(rv, HW, Craw, Wc, bc, num_group, score_reduce, edge_ulps, cla
             if HW > 1:      # raw maps: GlobalAveragePooling2D folded into the score kernel (nets/model.py:144-145)
                 C.check(L.gvcnn_gap_score_bin_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(R_out), _ptr(x), _ptr(scores),
                                                   _ptr(bins), _ptr(flags), _ptr(status), rv.B, rv.V, HW, Craw,
-                                                  num_group, rv.layout, dt, 1, edge_ulps, int(clamp), _stream()),
+                                                  num_group, rv.map_layout, dt, 1, edge_ulps, int(clamp), _stream()),
                         "gvcnn_gap_score_bin_fwd")
             else:
                 C.check(L.gvcnn_score_bin_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(x), _ptr(scores), _ptr(bins),
@@ -479,7 +555,7 @@ def _score_bin_fwd(rv, HW, Craw, Wc, bc, num_group, score_reduce, edge_ulps, cla
             xb = torch.empty((2 if want_bound else 1, max(rv.B, 1), rv.V), dtype=torch.float32, device=dev)
             if HW > 1:
                 C.check(L.gvcnn_gap_score_bin_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(R_out), _ptr(xb[0]), None, None, None,
-                                                  None, rv.B, rv.V, HW, Craw, 1, rv.layout, dt, 0, 0, 0, _stream()),
+                                                  None, rv.B, rv.V, HW, Craw, 1, rv.map_layout, dt, 0, 0, 0, _stream()),
                         "gvcnn_gap_score_bin_fwd")
             else:
                 C.check(L.gvcnn_view_score_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(xb[0]), _ptr(xb[1]) if want_bound else None,
@@ -525,13 +601,15 @@ def _score_bin_fwd(rv, HW, Craw, Wc, bc, num_group, score_reduce, edge_ulps, cla
         raise ValueError("score_reduce must be 'shape' or 'batch'")
 
 
-def view_scores(raw_view_descriptors, W, b, score_reduce="batch", layout=None, process_group=None):
+def view_scores(raw_view_descriptors, W, b, score_reduce="batch", layout=None, process_group=None,
+                data_format="channels_last"):
     """view_discrimination_scores as nets/model.py:144-148 produces them:
     sigmoid(log|mean_n(Dense(1)(raw))|) - [1, V] for the literal 'batch' mode,
     [B, V] for 'shape'.  Differentiable w.r.t. W, b and the raw descriptors, as the reference's graph tensor is
-    (TF 1.x's op order; see score_bin)."""
+    (TF 1.x's op order; see score_bin).  data_format: of block3 maps, as in score_bin."""
     return score_bin(raw_view_descriptors, W, b, 1, score_reduce=score_reduce, layout=layout,
-                     edge_ulps=0, clamp=True, check=False, process_group=process_group).scores
+                     edge_ulps=0, clamp=True, check=False, process_group=process_group,
+                     data_format=data_format).scores
 
 
 # --------------------------------------------------------------------------
@@ -863,9 +941,10 @@ class _PoolFuseGapFn(torch.autograd.Function):
     weights ([G] or [B, G]), None for the reference's 1 + n_g."""
 
     @staticmethod
-    def forward(ctx, bins, G, pool, empty_fill, layout, HW, Cch, weights, *views):
+    def forward(ctx, bins, G, pool, empty_fill, layout, HW, Cch, weights, cf, *views):
         L = C.lib()
         fv = _Views.of(views, layout, "F")
+        fv.cf = cf
         dev = fv.device
         dt = _dtype_code(fv.dtype)
         bins_c, bstride = _bin_rows(bins, fv)
@@ -873,19 +952,19 @@ class _PoolFuseGapFn(torch.autograd.Function):
         out = torch.empty((fv.B, Cch), dtype=fv.dtype, device=dev)
         mask = _tie_mask(fv, pool, any(v.requires_grad for v in views))
         status = _new_status(dev)
-        ws_bytes = L.gvcnn_pool_fuse_gap_workspace_bytes(fv.B, Cch, HW, dt)
-        ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
+        ws_bytes = 0 if cf else L.gvcnn_pool_fuse_gap_workspace_bytes(fv.B, Cch, HW, dt)   # channels-first: none
+        ws = None if cf else torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
         with _on(dev):
             if w_c is None:
                 C.check(L.gvcnn_pool_fuse_gap_fwd(fv.arg, _ptr(bins_c), bstride, _ptr(out), _ptr(mask), _ptr(status),
                                                   _ptr(ws), ws_bytes, fv.B, fv.V, HW, Cch, G, _POOL[pool],
-                                                  ctypes.c_float(empty_fill), fv.layout, dt, _stream()),
+                                                  ctypes.c_float(empty_fill), fv.map_layout, dt, _stream()),
                         "gvcnn_pool_fuse_gap_fwd")
             else:
                 C.check(L.gvcnn_pool_fuse_gap_weighted_fwd(fv.arg, _ptr(bins_c), bstride, _ptr(w_c), wstride, _ptr(out),
                                                            _ptr(mask), _ptr(status), _ptr(ws), ws_bytes, fv.B, fv.V, HW,
-                                                           Cch, G, _POOL[pool], ctypes.c_float(empty_fill), fv.layout,
-                                                           dt, _stream()),
+                                                           Cch, G, _POOL[pool], ctypes.c_float(empty_fill),
+                                                           fv.map_layout, dt, _stream()),
                         "gvcnn_pool_fuse_gap_weighted_fwd")
         ctx.fv, ctx.G, ctx.pool, ctx.HW, ctx.Cch, ctx.bstride, ctx.wstride = fv, G, pool, HW, Cch, bstride, wstride
         ctx.save_for_backward(bins_c, w_c, mask)
@@ -904,41 +983,57 @@ class _PoolFuseGapFn(torch.autograd.Function):
             if w_c is None:
                 C.check(L.gvcnn_pool_fuse_gap_bwd(_ptr(dOut), _ptr(bins_c), ctx.bstride, _ptr(mask), gv.arg,
                                                   _ptr(status), gv.B, gv.V, ctx.HW, ctx.Cch, ctx.G, _POOL[ctx.pool],
-                                                  gv.layout, _dtype_code(gv.dtype), _stream()),
+                                                  gv.map_layout, _dtype_code(gv.dtype), _stream()),
                         "gvcnn_pool_fuse_gap_bwd")
             else:
                 C.check(L.gvcnn_pool_fuse_gap_weighted_bwd(_ptr(dOut), _ptr(bins_c), ctx.bstride, _ptr(w_c), ctx.wstride,
                                                            _ptr(mask), gv.arg, _ptr(status), gv.B, gv.V, ctx.HW,
-                                                           ctx.Cch, ctx.G, _POOL[ctx.pool], gv.layout,
+                                                           ctx.Cch, ctx.G, _POOL[ctx.pool], gv.map_layout,
                                                            _dtype_code(gv.dtype), _stream()),
                         "gvcnn_pool_fuse_gap_weighted_bwd")
         grads = tuple(out) if isinstance(out, list) else (out,)
-        return (None,) * 8 + grads
+        return (None,) * 9 + grads
 
 
-def pool_fuse_gap(final_view_descriptors, bins, num_group, pool="max", empty_fill=1.0, layout=None, group_weight=None):
+def pool_fuse_gap(final_view_descriptors, bins, num_group, pool="max", empty_fill=1.0, layout=None, group_weight=None,
+                  data_format="channels_last"):
     """view_pooling + group_fusion + GlobalAveragePooling2D (nets/model.py:154-163) in one pass: the
     descriptors are channel-last maps ([N, h, w, C] per view, or [B, V, h, w, C] / [V, B, h, w, C]); returns
     the pooled shape descriptor [N, C].  The fused map is never written.  group_weight: caller-supplied group
     weights ([G] or [B, G] float32, e.g. paper mode's mean scores) instead of the reference's 1 + n_g.  Shapes
     the specialised kernel does not cover (see gvcnn_pool_fuse_gap_fwd) run pool_fuse and average afterwards -
-    same result up to the float32 rounding of the mean."""
+    same result up to the float32 rounding of the mean.
+    data_format='channels_first': the maps are [N, C, h, w] per view (or [B, V, C, h, w] / [V, B, C, h, w]), read
+    without a copy as they lie in memory (see score_bin); dF comes back in the maps' shape and memory format.  With
+    contiguous maps the mean adds each channel's positions in order, which may differ from the channel-last kernel's
+    split sum by float32 re-association; caller-supplied group weights take the fallback."""
+    _check_data_format(data_format)
     views, lay = _view_args(final_view_descriptors, layout)
+    cf = False
+    if data_format == "channels_first":
+        _require_cuda(views[0], "final_view_descriptors")
+        if not _is_maps(views, lay):
+            raise ValueError("pool_fuse_gap with data_format='channels_first' expects maps, e.g. [N, C, h, w] per view")
+        views, cf = _maps_in_memory_order(views, lay)
     shp = tuple(views[0].shape)
-    spatial = shp[1:-1] if lay == "list" else shp[2:-1]
     if len(shp) < 3:
         raise ValueError("pool_fuse_gap expects channel-last maps, e.g. [N, h, w, C] per view")
-    Cch = shp[-1]
+    if cf:
+        Cch, spatial = shp[-3], shp[-2:]
+    else:
+        Cch, spatial = shp[-1], (shp[1:-1] if lay == "list" else shp[2:-1])
     HW = int(math.prod(spatial)) if len(spatial) else 1
     _require_cuda(bins, "bins")
     try:
-        out, _ = _PoolFuseGapFn.apply(bins, num_group, pool, empty_fill, lay, HW, Cch, group_weight, *views)
+        out, _ = _PoolFuseGapFn.apply(bins, num_group, pool, empty_fill, lay, HW, Cch, group_weight, cf, *views)
         return out
     except C.GvcnnError as e:
         if e.code != C.E_UNSUPPORTED:
             raise
-    S = pool_fuse(final_view_descriptors, bins, num_group, pool=pool, empty_fill=empty_fill, layout=layout,
-                  group_weight=group_weight)
+    S = pool_fuse(list(views) if lay == "list" else views[0], bins, num_group, pool=pool, empty_fill=empty_fill,
+                  layout=None if lay == "list" else lay, group_weight=group_weight)
+    if cf:
+        return S.reshape(S.shape[0], Cch, -1).mean(dim=2)
     return S.reshape(S.shape[0], -1, Cch).mean(dim=1)
 
 
@@ -1190,13 +1285,16 @@ def _grouping_fusion_fwd(rv, fv, want_mask, W, b, G, pool, empty_fill, edge_ulps
     return _Pooled(S, mask, None, status, bins, bin_stride, None, 0), (x, scores, bins, flags)
 
 
-def _is_raw_maps(raw, W, layout):
-    """True when `raw` holds the un-pooled block3 maps ([..., h, w, C_raw]) rather than [..., C_raw] descriptors."""
+def _is_raw_maps(raw, W, layout, data_format="channels_last"):
+    """True when `raw` holds the un-pooled block3 maps ([..., h, w, C_raw], or [..., C_raw, h, w] with
+    data_format='channels_first') rather than [..., C_raw] descriptors."""
     if not (isinstance(W, torch.Tensor) and W.dim() == 2):
         return False
     t = raw[0] if isinstance(raw, (list, tuple)) and len(raw) else raw
     if not isinstance(t, torch.Tensor):
         return False
+    if data_format == "channels_first":     # maps by their rank; _raw_views checks C_raw at dim -3
+        return _is_maps(*_view_args(raw, layout))
     lead = 1 if isinstance(raw, (list, tuple)) else 2
     return t.dim() > lead + 1 and t.shape[-1] == W.shape[1]
 
@@ -1204,7 +1302,7 @@ def _is_raw_maps(raw, W, layout):
 def grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_group, pool="max",
                     empty_fill=1.0, score_reduce="shape", layout=None, clamp=False, check=False,
                     process_group=None, edge_ulps=4, status=None, multiplier=None, exchange=None,
-                    global_count=None, _variant=0):
+                    global_count=None, data_format="channels_last", _variant=0):
     """The whole hot path with no host hop (replaces the partial_run split of
     train.py:264-288), one call into the library in either mode: per shape, score + bin
     then pool + fuse, chained on the device; in the literal batch-mean mode, x -> column
@@ -1224,16 +1322,30 @@ def grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_grou
     enabled and one of them requires grad, as in score_bin; the shape descriptor stays differentiable w.r.t. the
     final view descriptors.  A loss that does not use the scores leaves W and b without a gradient (``.grad`` None)
     and launches nothing for them.  In 'batch' mode with a ``process_group`` or ``exchange`` the score backward is
-    collective (see score_bin): it must run on every rank, an empty shard included."""
+    collective (see score_bin): it must run on every rank, an empty shard included.
+
+    data_format='channels_first': block3 and final maps are [N, C, h, w] per view (PyTorch's order).  The scores read
+    the block3 maps without a copy (see score_bin); pooling + fusion is element-wise, so the final maps go in as they
+    lie in memory too, and the shape descriptor comes back in their shape and memory format."""
+    final_view_descriptors, f_perm = _final_maps(final_view_descriptors, layout, data_format)
+    S, sr = _grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_group, pool, empty_fill,
+                             score_reduce, layout, clamp, check, process_group, edge_ulps, status, multiplier, exchange,
+                             global_count, data_format, _variant)
+    return (S.movedim(-1, -3) if f_perm else S), sr
+
+
+def _grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_group, pool, empty_fill, score_reduce,
+                     layout, clamp, check, process_group, edge_ulps, status, multiplier, exchange, global_count,
+                     data_format, _variant):
     if status is None and check:
         dev0 = W.device if isinstance(W, torch.Tensor) else None
         status = _new_status(dev0)
-    if _is_raw_maps(raw_view_descriptors, W, layout):
+    if _is_raw_maps(raw_view_descriptors, W, layout, data_format):
         # block3 maps instead of pooled raw descriptors: the GAP of nets/model.py:144 runs inside the score kernel
         # (gvcnn_gap_score_bin_fwd); pooling + fusion follow on the stream, chained with programmatic dependent launch
         sr = score_bin(raw_view_descriptors, W, b, num_group, score_reduce=score_reduce, layout=layout,
                        edge_ulps=edge_ulps, clamp=clamp, check=check, process_group=process_group, status=status,
-                       multiplier=multiplier, exchange=exchange, global_count=global_count)
+                       multiplier=multiplier, exchange=exchange, global_count=global_count, data_format=data_format)
         S = pool_fuse(final_view_descriptors, sr.bins, num_group, pool=pool, empty_fill=empty_fill, layout=layout,
                       _variant=_variant)
         return S, sr
@@ -1302,10 +1414,11 @@ class _PaperModeFn(torch.autograd.Function):
     cover the shapes the fused map is returned instead (the caller's _spatial_mean then averages it)."""
 
     @staticmethod
-    def forward(ctx, W, b, G, pool, f_layout, r_layout, n_r, status, HW_r, fold, *tensors):
+    def forward(ctx, W, b, G, pool, f_layout, r_layout, n_r, status, HW_r, fold, r_cf, *tensors):
         L = C.lib()
         r_t, f_t = tensors[:n_r], tensors[n_r:]
         rv = _Views.of(r_t, r_layout, "R")
+        rv.cf = r_cf
         fv = _Views.of(f_t, f_layout, "F")
         dev = fv.device
         R_out = None
@@ -1322,7 +1435,7 @@ class _PaperModeFn(torch.autograd.Function):
             R_out = torch.empty((rv.B, rv.V, Craw), dtype=torch.float32, device=dev)
             with _on(dev):
                 rc = L.gvcnn_gap_score_bin_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(R_out), _ptr(x), _ptr(scores),
-                                               _ptr(bins), None, _ptr(status), rv.B, rv.V, HW_r, Craw, G, rv.layout,
+                                               _ptr(bins), None, _ptr(status), rv.B, rv.V, HW_r, Craw, G, rv.map_layout,
                                                _dtype_code(rv.dtype), 1, 1, 1, _stream())
             if rc == C.E_UNSUPPORTED:
                 raise _GapScoreUnsupported()
@@ -1391,13 +1504,14 @@ class _PaperModeFn(torch.autograd.Function):
                         "gvcnn_view_score_bwd")
                 if dR_views is not None:
                     C.check(L.gvcnn_gap_score_bwd(_ptr(dx), _ptr(W), dR_views.arg, rv.B, rv.V, ctx.HW_r, Cr,
-                                                  rv.layout, _dtype_code(rv.dtype), _stream()), "gvcnn_gap_score_bwd")
+                                                  rv.map_layout, _dtype_code(rv.dtype), _stream()),
+                            "gvcnn_gap_score_bwd")
         if dR_out is None:
             gr = (None,) * ctx.n_r
         else:
             gr = tuple(dR_out) if isinstance(dR_out, list) else (dR_out,)
         gf = tuple(dF) if isinstance(dF, list) else (dF,)
-        return (dW, dbias, None, None, None, None, None, None, None, None) + gr + gf
+        return (dW, dbias) + (None,) * 9 + gr + gf
 
 
 def _fold_geometry(fv):
@@ -1458,9 +1572,11 @@ def _paper_gap_bwd_weights(fv, dS_gap, S_gap, bins, bin_stride, weights, w_strid
             "gvcnn_pool_fuse_gap_bwd_weights")
 
 
-def _spatial_mean_views(t, lay):
-    """GlobalAveragePooling2D of block3 maps in a view argument (list of [N, h, w, C], or stacked): the pooled raw
-    descriptors, through torch so that autograd carries their gradient back to the maps."""
+def _spatial_mean_views(t, lay, cf=False):
+    """GlobalAveragePooling2D of block3 maps in a view argument (list of [N, h, w, C], or stacked; [.., C, h, w] with
+    cf): the pooled raw descriptors, through torch so that autograd carries their gradient back to the maps."""
+    if cf:
+        return [v.mean(dim=(-2, -1)) for v in t] if lay == "list" else t[0].mean(dim=(-2, -1))
     if lay == "list":
         return [v.reshape(v.shape[0], -1, v.shape[-1]).mean(dim=1) for v in t]
     x = t[0]
@@ -1468,7 +1584,7 @@ def _spatial_mean_views(t, lay):
 
 
 def grouping_fusion_paper(raw_view_descriptors, W, b, final_view_descriptors, num_group, pool="max", layout=None,
-                          status=None, fold_gap=False):
+                          status=None, fold_gap=False, data_format="channels_last"):
     """Paper-mode grouping + fusion: group weight = mean discrimination score of the group's views, empty
     groups vanish; differentiable w.r.t. the view descriptors AND the score FC (W, b, optionally the raw
     descriptors).  Returns (shape_descriptor, scores, bins, weights).  Per-shape scores/bins.  The scores (like bins
@@ -1478,32 +1594,47 @@ def grouping_fusion_paper(raw_view_descriptors, W, b, final_view_descriptors, nu
     runs inside the score kernel, forward and backward.
     fold_gap=True also folds the GlobalAveragePooling2D after the fusion (nets/model.py:163) into the pooling: the
     shape descriptor returned is the pooled [N, C] one and the fused map is never written.  Shapes the folded kernels
-    do not cover run the unfolded path and average the map afterwards."""
+    do not cover run the unfolded path and average the map afterwards.
+    data_format='channels_first': block3 and final maps are [N, C, h, w] per view, read without a copy as in
+    score_bin and grouping_fusion.  The post-fusion GAP is folded only for final maps in torch.channels_last memory;
+    contiguous NCHW final maps run the unfolded path and the mean."""
+    _check_data_format(data_format)
+    final_view_descriptors, f_perm = _final_maps(final_view_descriptors, layout, data_format)
     r_t, r_lay = _view_args(raw_view_descriptors, layout)
     f_t, f_lay = _view_args(final_view_descriptors, layout)
     _check_score_fc(W, b)
-    HW_r = 1
-    if _is_raw_maps(raw_view_descriptors, W, layout):
-        HW_r = _raw_views(raw_view_descriptors, layout, int(W.shape[1]))[1]
-    if HW_r == 1 and not fold_gap:
-        return _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, 1, False, *r_t, *f_t)
-    try:
-        S, scores, bins, w = _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, HW_r, fold_gap,
+    HW_r, r_cf = 1, False
+    if _is_raw_maps(raw_view_descriptors, W, layout, data_format):
+        rv, HW_r = _raw_views(raw_view_descriptors, layout, int(W.shape[1]), data_format)
+        r_t, r_cf = tuple(rv.keep), rv.cf
+    f_cf = data_format == "channels_first" and not f_perm
+    fold = fold_gap and not f_cf            # the weighted folded kernels read channel-last maps only
+    if HW_r == 1 and not fold:
+        S, scores, bins, w = _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, 1, False, False,
                                                 *r_t, *f_t)
-    except _GapScoreUnsupported:
-        # block3 maps the GAP-folded score kernel does not cover: pool them here, autograd carries dR to the maps
-        pooled = _spatial_mean_views(r_t, r_lay)
-        r_t = tuple(pooled) if r_lay == "list" else (pooled,)
-        S, scores, bins, w = _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, 1, fold_gap,
-                                                *r_t, *f_t)
-    return (_spatial_mean(S) if fold_gap else S), scores, bins, w
+    else:
+        try:
+            S, scores, bins, w = _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, HW_r, fold,
+                                                    r_cf, *r_t, *f_t)
+        except _GapScoreUnsupported:
+            # block3 maps the GAP-folded score kernel does not cover: pool them here, autograd carries dR to the maps
+            pooled = _spatial_mean_views(r_t, r_lay, r_cf)
+            r_t = tuple(pooled) if r_lay == "list" else (pooled,)
+            S, scores, bins, w = _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, 1, fold,
+                                                    False, *r_t, *f_t)
+    if fold_gap:
+        return _spatial_mean(S, "channels_first" if f_cf else "channels_last"), scores, bins, w
+    return (S.movedim(-1, -3) if f_perm else S), scores, bins, w
 
 
-def _spatial_mean(S):
-    """GlobalAveragePooling2D of the fused map [N, h, w, C] -> [N, C] (nets/model.py:163) for the un-folded path;
-    an empty batch (a rank whose shard is exhausted) stays empty."""
+def _spatial_mean(S, data_format="channels_last"):
+    """GlobalAveragePooling2D of the fused map [N, h, w, C] ([N, C, h, w] with data_format='channels_first', in either
+    memory format, without a copy) -> [N, C] (nets/model.py:163) for the un-folded path; an empty batch (a rank whose
+    shard is exhausted) stays empty."""
     if S.dim() <= 2:
         return S
+    if data_format == "channels_first":
+        return S.mean(dim=tuple(range(2, S.dim())))
     return S.reshape(S.shape[0], int(math.prod(S.shape[1:-1])), S.shape[-1]).mean(dim=1)
 
 
@@ -1514,8 +1645,13 @@ class GVCNNHead(torch.nn.Module):
     average pooling (nets/model.py:163-164)."""
 
     def __init__(self, num_views, raw_channels, final_channels, num_classes, num_group=10, pool="max",
-                 empty_fill=1.0, score_reduce="batch", weight_mode="count"):
+                 empty_fill=1.0, score_reduce="batch", weight_mode="count", data_format="channels_last"):
+        """data_format: 'channels_last' (the reference's [N, h, w, C] maps) or 'channels_first' (PyTorch's
+        [N, C, h, w], e.g. a torchvision backbone's layer3 / layer4 output, contiguous or in torch.channels_last
+        memory - read without a copy either way; gradients come back in the maps' shape and memory format)."""
         super().__init__()
+        _check_data_format(data_format)
+        self.data_format = data_format
         self.num_views, self.num_group = num_views, num_group
         self.pool, self.empty_fill, self.score_reduce = pool, empty_fill, score_reduce
         if weight_mode not in ("count", "score"):
@@ -1544,21 +1680,21 @@ class GVCNNHead(torch.nn.Module):
         if fold_gap and self.weight_mode == "count":
             sr = score_bin(raw_view_descriptors, self.score_kernel, self.score_bias, self.num_group,
                            score_reduce=self.score_reduce, process_group=process_group, check=check, status=status,
-                           global_count=global_count)
+                           global_count=global_count, data_format=self.data_format)
             net = pool_fuse_gap(final_view_descriptors, sr.bins, self.num_group, pool=self.pool,
-                                empty_fill=self.empty_fill)
+                                empty_fill=self.empty_fill, data_format=self.data_format)
             return sr.scores, net, self.classifier(net.to(self.classifier.weight.dtype))
         if self.weight_mode == "score":
             S, scores, _, _ = grouping_fusion_paper(raw_view_descriptors, self.score_kernel, self.score_bias,
                                                     final_view_descriptors, self.num_group, pool=self.pool,
-                                                    status=status, fold_gap=fold_gap)
+                                                    status=status, fold_gap=fold_gap, data_format=self.data_format)
         else:
             S, sr = grouping_fusion(raw_view_descriptors, self.score_kernel, self.score_bias, final_view_descriptors,
                                     self.num_group, pool=self.pool, empty_fill=self.empty_fill,
                                     score_reduce=self.score_reduce, process_group=process_group, check=check,
-                                    status=status, global_count=global_count)
+                                    status=status, global_count=global_count, data_format=self.data_format)
             scores = sr.scores
-        net = _spatial_mean(S)
+        net = _spatial_mean(S, self.data_format)
         logits = self.classifier(net.to(self.classifier.weight.dtype))
         return scores, S, logits
 
@@ -1570,9 +1706,10 @@ def gvcnn_head(raw_view_descriptors, final_view_descriptors, head: GVCNNHead, gr
     pools and fuses with them; without, it computes them on the device."""
     if group_scheme is None:
         return head(raw_view_descriptors, final_view_descriptors)
-    scores = view_scores(raw_view_descriptors, head.score_kernel, head.score_bias, score_reduce=head.score_reduce)
+    scores = view_scores(raw_view_descriptors, head.score_kernel, head.score_bias, score_reduce=head.score_reduce,
+                         data_format=head.data_format)
     desc = view_pooling(final_view_descriptors, group_scheme, pool=head.pool, empty_fill=head.empty_fill)
     w = group_weight if group_weight is not None else globals()["group_weight"](group_scheme)
     S = group_fusion(desc, w)
-    net = _spatial_mean(S)
+    net = _spatial_mean(S, head.data_format)
     return scores, S, head.classifier(net.to(head.classifier.weight.dtype))

@@ -57,6 +57,16 @@ extern "C" {
 #define GVCNN_LAYOUT_BVD 0
 #define GVCNN_LAYOUT_VBD 1
 #define GVCNN_LAYOUT_PTRS 2
+/* Flag bit ORed into the layout of per-view spatial MAPS (D = C * HW): the map of
+ * one (shape, view) is channel-major [C, HW] - PyTorch's contiguous NCHW - instead
+ * of the channel-last [HW, C].  Accepted by gvcnn_gap_score_bin_fwd (m_layout),
+ * gvcnn_gap_score_bwd (m_layout), gvcnn_pool_fuse_gap_fwd (f_layout) and
+ * gvcnn_pool_fuse_gap_bwd (g_layout); the weighted GAP-folded entry points and
+ * gvcnn_pool_fuse_gap_bwd_weights return GVCNN_E_UNSUPPORTED for it, every other
+ * entry point GVCNN_E_BAD_LAYOUT.  Pooling and fusion are element-wise over D, so
+ * gvcnn_pool_fuse_fwd / _bwd and gvcnn_view_pooling_bwd take NCHW-flattened maps
+ * with the plain layout. */
+#define GVCNN_LAYOUT_CHANNELS_FIRST 0x10
 
 #define GVCNN_POOL_MAX 0         /* tf.reduce_max, nets/model.py:72 (shipped)    */
 #define GVCNN_POOL_MEAN 1        /* tf.reduce_mean, unit_test.py:31              */
@@ -210,7 +220,11 @@ int gvcnn_score_bin_fwd(const void *R, const float *W, const float *bias,
  * pooled raw descriptor, float32 [B, V, C].  The [B, V, C] tensor is otherwise never
  * written.  Supported: 16-byte aligned rows and C = 512 / 1024 (f32), 1024 / 2048
  * (16-bit types); anything else returns GVCNN_E_UNSUPPORTED (pool first, then
- * gvcnn_score_bin_fwd). */
+ * gvcnn_score_bin_fwd).
+ * m_layout | GVCNN_LAYOUT_CHANNELS_FIRST: channels-first maps [B, V, C, HW] / [V, B, C, HW]
+ * / V pointers to [B, C, HW]; R, x, scores, bins and flags are bit-identical to the
+ * channel-last call on the transposed maps.  Supported: the same C values, 16-byte
+ * aligned map rows, any HW. */
 int gvcnn_gap_score_bin_fwd(const void *maps, const float *W, const float *bias, float *R_out,
                             float *x, float *scores, int32_t *bins, int32_t *flags, int32_t *status,
                             int B, int V, int HW, int C, int G, int m_layout, int dtype,
@@ -346,7 +360,15 @@ int gvcnn_grouping_fusion_batch_fwd(const void *R, const float *W, const float *
  * weights; anything else returns GVCNN_E_UNSUPPORTED (use gvcnn_pool_fuse_fwd
  * and pool afterwards).  tie_mask as in gvcnn_pool_fuse_fwd ([ceil(V/8), B, D]).
  * gvcnn_pool_fuse_gap_bwd: dS_gap [B, C] -> dF (dS[b,p,c] = dS_gap[b,c] / HW is
- * never materialised). */
+ * never materialised).
+ * f_layout / g_layout | GVCNN_LAYOUT_CHANNELS_FIRST: channels-first maps, D = C * HW in
+ * [C, HW] order (the tie mask indexes D in that order too).  Forward: no workspace
+ * (workspace may be null; gvcnn_pool_fuse_gap_workspace_bytes is for channel-last
+ * maps); each channel's positions are added in order from 0.0f, then divided by HW -
+ * it may differ from the channel-last sum by float32 re-association.  Supported:
+ * 16-byte aligned rows, V in {4, 6, 8, 12, 16, 20}, G <= 255, any C for which some
+ * block of K channels (K | C, K <= 256) has K * HW elements a multiple of 16 bytes.
+ * Backward: bit-identical to the channel-last dF, transposed (16-byte aligned dF rows). */
 size_t gvcnn_pool_fuse_gap_workspace_bytes(int B, int C, int HW, int dtype);
 int gvcnn_pool_fuse_gap_fwd(const void *F, const int32_t *bins, int64_t bin_stride_b,
                             void *S_gap, uint8_t *tie_mask, int32_t *status,
@@ -359,6 +381,7 @@ int gvcnn_pool_fuse_gap_bwd(const void *dS_gap, const int32_t *bins, int64_t bin
                             int g_layout, int dtype, void *stream);
 /* The same two with caller-supplied group weights (weights / weight_stride_b as in
  * gvcnn_pool_fuse_fwd; paper mode: the mean score of the group's views, empty_fill = 0).
+ * Channel-last maps only: GVCNN_LAYOUT_CHANNELS_FIRST gives GVCNN_E_UNSUPPORTED.
  * Null weights = gvcnn_pool_fuse_gap_fwd / _bwd.  The per-position fused value is
  * gvcnn_pool_fuse_fwd's with the same weights, bit for bit (before the rounding to
  * `dtype`).  Supported as above, with G <= 64 when weights are given. */
@@ -412,11 +435,13 @@ int gvcnn_view_score_bwd(const void *R, const float *dx, const float *W, float *
  *     once; fixed reduction order (deterministic).  workspace from
  *     gvcnn_pool_fuse_gap_bwd_weights_workspace_bytes.  Supported: 16-byte aligned rows,
  *     V in {4, 6, 8, 12, 16, 20}, C a multiple of 1024 (f32) / 2048 (16-bit types), G <= 255;
- *     otherwise GVCNN_E_UNSUPPORTED.
+ *     otherwise (GVCNN_LAYOUT_CHANNELS_FIRST included) GVCNN_E_UNSUPPORTED.
  *   gvcnn_gap_score_bwd: gradient of the GlobalAveragePooling2D in front of the score FC
  *     (gvcnn_gap_score_bin_fwd): dmaps[b, v, p, c] = dx[b, v] * W[v, c] / HW, written in `dtype`
  *     and m_layout; dx float32 [B, V], W float32 [V, C] (16-byte aligned).  Needs 16-byte
  *     aligned rows and C a multiple of 16 bytes' worth of elements (else GVCNN_E_UNSUPPORTED).
+ *     m_layout | GVCNN_LAYOUT_CHANNELS_FIRST: dmaps[b, v, c, p], channel-major; needs C * HW
+ *     a multiple of 16 bytes' worth of elements instead.
  *     dW / dbias of the score FC come from gvcnn_view_score_bwd on the pooled R_out that
  *     gvcnn_gap_score_bin_fwd writes (float32, BVD). */
 size_t gvcnn_pool_fuse_gap_bwd_weights_workspace_bytes(int B, int V, int HW, int C, int dtype);
