@@ -199,6 +199,13 @@ class _Views:
         channel-major ([C, h, w] per shape and view)."""
         return self.layout | (C.LAYOUT_CHANNELS_FIRST if self.cf else 0)
 
+    @property
+    def map_geometry(self):
+        """(HW, C) of spatial maps: positions and channels per view, the channel axis last ([.., h, w, C]) or, with
+        cf, third from last ([.., C, h, w])."""
+        c = int(self.view_shape[-3] if self.cf else self.view_shape[-1])
+        return self.D // c, c
+
     def empty_like(self):
         """Fresh storage of the same layout (for dF)."""
         out = [torch.empty_like(t) for t in self.keep] if self.kind == "list" else torch.empty_like(self.tensor)
@@ -283,16 +290,36 @@ def _check_score_fc(W, b):
         raise TypeError("W and b must be float32")
 
 
-def _exchange_forms(exchange):
-    """A gvcnn_exchange_fn given as (fn, user) - fn a ctypes function (P2PComm.exchange, an EXCHANGE_FN callback)
-    or its address as an int or c_void_p (P2PComm.exchange_c) - as (address, callable, user): the address for the
-    C entry points, the callable for score_bin's staged path.  None (no exchange) gives three Nones."""
+def _exchange_args(exchange, process_group):
+    """The exchange of a 'batch'-mode call as (address, callable, user, keep-alive): a gvcnn_exchange_fn given as
+    (fn, user) - fn a ctypes function (P2PComm.exchange, an EXCHANGE_FN callback) or its address as an int or
+    c_void_p (P2PComm.exchange_c) - or else, with a ``process_group``, make_exchange's callback (keep the fourth value
+    referenced while it can be called).  The address is for the C entry points, the callable for score_bin's staged
+    path.  Neither given: four Nones."""
+    keep = None
     if exchange is None:
-        return None, None, None
+        if process_group is None:
+            return None, None, None, None
+        cb, keep = make_exchange(process_group)
+        exchange = (cb, None)
     fn, user = exchange
     if isinstance(fn, (int, ctypes.c_void_p)):
-        return fn, C.EXCHANGE_FN(fn if isinstance(fn, int) else fn.value), user
-    return ctypes.cast(fn, ctypes.c_void_p), fn, user
+        return fn, C.EXCHANGE_FN(fn if isinstance(fn, int) else fn.value), user, keep
+    return ctypes.cast(fn, ctypes.c_void_p), fn, user, keep
+
+
+def _batch_count(B, global_count, process_group, dev):
+    """The N that score_reduce='batch' divides the column sums by: ``global_count`` if given, else the local B, summed
+    over the ranks of ``process_group`` when there is one.  An empty (global) batch raises."""
+    n = B if global_count is None else int(global_count)
+    if global_count is None and process_group is not None:
+        import torch.distributed as dist
+        cnt = torch.tensor([B], dtype=torch.int64, device=dev)
+        dist.all_reduce(cnt, group=process_group)
+        n = int(cnt.item())
+    if n <= 0:
+        raise ValueError("score_reduce='batch' over an empty (global) batch")
+    return n
 
 
 def raise_for_status(status: torch.Tensor, num_group: int):
@@ -364,16 +391,27 @@ def _raw_views(R, layout, c_raw, data_format="channels_last"):
             R = list(views) if lay == "list" else views[0]
     rv = _Views(R, layout, "R")
     rv.cf = cf
-    HW = 1
-    if cf:
-        HW = rv.D // c_raw
-    elif c_raw > 0 and rv.D != c_raw:
+    if not cf:
+        if c_raw <= 0 or rv.D == c_raw:
+            return rv, 1
         last = rv.view_shape[-1]
         if last != c_raw or rv.D % c_raw:
             raise ValueError("raw view descriptors: trailing dimension %d does not match the score kernel's C_raw = %d"
                              % (last, c_raw))
-        HW = rv.D // c_raw
-    return rv, HW
+    return rv, rv.map_geometry[0]
+
+
+def _score_args(R, W, b, layout, data_format):
+    """The score FC's inputs checked against each other before anything is launched: (rv, HW, C_raw, W, b) with
+    (rv, HW) from _raw_views, W [V, C_raw] and b [V] float32 and contiguous."""
+    _check_score_fc(W, b)
+    Wc, bc = W.contiguous(), b.contiguous()
+    rv, HW = _raw_views(R, layout, int(Wc.shape[-1]) if Wc.dim() == 2 else -1, data_format)
+    Craw = rv.D // HW
+    if tuple(Wc.shape) != (rv.V, Craw) or tuple(bc.shape) != (rv.V,):
+        raise ValueError("W must be [V, C] = %s and b [V], got %s and %s"
+                         % ((rv.V, Craw), tuple(Wc.shape), tuple(bc.shape)))
+    return rv, HW, Craw, Wc, bc
 
 
 def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulps=4, clamp=False,
@@ -412,17 +450,16 @@ def score_bin(R, W, b, num_group, *, score_reduce="shape", layout=None, edge_ulp
     the batch mean is all-reduced over the ranks, so when a score gradient flows on one rank it must flow on every
     rank, one with an empty shard included.
     """
-    _check_data_format(data_format)
-    _check_score_fc(W, b)
-    Wc, bc = W.contiguous(), b.contiguous()
-    rv, HW = _raw_views(R, layout, int(Wc.shape[-1]) if Wc.dim() == 2 else -1, data_format)
-    Craw = rv.D // HW
-    if tuple(Wc.shape) != (rv.V, Craw) or tuple(bc.shape) != (rv.V,):
-        raise ValueError("W must be [V, C] = %s and b [V], got %s and %s"
-                         % ((rv.V, Craw), tuple(Wc.shape), tuple(bc.shape)))
+    rv, HW, Craw, Wc, bc = _score_args(R, W, b, layout, data_format)
     if status is None and check:
         status = _new_status(rv.device)
+    return _score_bin(rv, HW, Craw, Wc, bc, num_group, score_reduce, edge_ulps, clamp, check, status, process_group,
+                      multiplier, exchange, global_count)
 
+
+def _score_bin(rv, HW, Craw, Wc, bc, num_group, score_reduce, edge_ulps, clamp, check, status, process_group,
+               multiplier, exchange, global_count):
+    """score_bin on the arguments _score_args checked."""
     def run(want_r_out):
         return _score_bin_fwd(rv, HW, Craw, Wc, bc, num_group, score_reduce, edge_ulps, clamp, status, process_group,
                               multiplier, exchange, global_count, want_r_out)
@@ -449,24 +486,16 @@ class _ScoreGrad:
 
 def _score_bwd(dscores, W, x, scores, R_out, sg: _ScoreGrad, need_wb: bool, need_r: bool):
     """The score part of a backward (shared by _ScoreFn and _PoolFuseFn): dscores -> dx (gvcnn_score_bin_bwd, with
-    the adjoint exchange in 'batch' mode), then dW, db and dR from dx (gvcnn_view_score_bwd; on block3 maps dW and db
-    from the pooled float32 R_out of the forward, and dmaps from gvcnn_gap_score_bwd).  Returns (dW, db, dR) with dR
-    a tuple in the layout of the raw views (one tensor per view for a list), or None where not asked for."""
+    the adjoint exchange in 'batch' mode), then _score_fc_bwd."""
     L = C.lib()
-    rv, HW = sg.rv, sg.HW
-    B, V, Craw = rv.B, rv.V, rv.D // HW
+    B, V = sg.rv.B, sg.rv.V
     dev = dscores.device
     ds = dscores.to(torch.float32).contiguous()
     dx = torch.empty((B, V), dtype=torch.float32, device=dev)
-    dW = db = dR = None
     with _on(dev):
         if sg.batch:
             dx_mean = torch.empty(V, dtype=torch.float32, device=dev)
-            ex, keep = sg.exchange, None
-            if ex is None and sg.process_group is not None:
-                cb, keep = make_exchange(sg.process_group)
-                ex = (cb, None)
-            ex_ptr, _, ex_user = _exchange_forms(ex)
+            ex_ptr, _, ex_user, keep = _exchange_args(sg.exchange, sg.process_group)
             C.check(L.gvcnn_score_bin_bwd(_ptr(ds), _ptr(x), _ptr(scores), _ptr(dx_mean), _ptr(dx), B, V,
                                           C.SCORE_REDUCE_BATCH, int(sg.global_count), ex_ptr, ex_user, _stream()),
                     "gvcnn_score_bin_bwd")
@@ -474,6 +503,18 @@ def _score_bwd(dscores, W, x, scores, R_out, sg: _ScoreGrad, need_wb: bool, need
         else:
             C.check(L.gvcnn_score_bin_bwd(_ptr(ds), _ptr(x), _ptr(scores), None, _ptr(dx), B, V, C.SCORE_REDUCE_SHAPE,
                                           0, None, None, _stream()), "gvcnn_score_bin_bwd")
+    return _score_fc_bwd(dx, W, R_out, sg.rv, sg.HW, need_wb, need_r)
+
+
+def _score_fc_bwd(dx, W, R_out, rv, HW, need_wb: bool, need_r: bool):
+    """dx -> dW, db and dR through the score FC (gvcnn_view_score_bwd; on block3 maps (HW > 1) dW and db from the
+    pooled float32 R_out of the forward, and dmaps from gvcnn_gap_score_bwd).  Returns (dW, db, dR) with dR a tuple in
+    the layout of the raw views (one tensor per view for a list), or None where not asked for."""
+    L = C.lib()
+    B, V, Craw = rv.B, rv.V, rv.D // HW
+    dev = dx.device
+    dW = db = dR = None
+    with _on(dev):
         dR_out, dR_views = rv.empty_like() if need_r else (None, None)
         if need_wb or (need_r and HW == 1):
             if B == 0:                                  # a parameter gradient over an empty shard: zeros
@@ -523,6 +564,12 @@ class _ScoreFn(torch.autograd.Function):
         return (None, dW if ni[1] else None, db if ni[2] else None) + (dR if need_r else (None,) * ctx.n_r)
 
 
+def _score_outputs(rows, V, dev):
+    """x, scores (float32), bins and flags (int32), [rows, V] each, in one allocation."""
+    buf = torch.empty((4, rows, V), dtype=torch.int32, device=dev)
+    return buf[0].view(torch.float32), buf[1].view(torch.float32), buf[2], buf[3]
+
+
 def _score_bin_fwd(rv, HW, Craw, Wc, bc, num_group, score_reduce, edge_ulps, clamp, status, process_group, multiplier,
                    exchange, global_count, want_r_out):
     """score_bin's launches: (x, scores, bins, flags, R_out, _ScoreGrad).  want_r_out (block3 maps only): also
@@ -535,8 +582,7 @@ def _score_bin_fwd(rv, HW, Craw, Wc, bc, num_group, score_reduce, edge_ulps, cla
         if score_reduce == "shape":
             if multiplier not in (None, num_group):
                 raise ValueError("multiplier is only selectable with score_reduce='batch' or through group_scheme")
-            buf = torch.empty((4, rv.B, rv.V), dtype=torch.int32, device=dev)      # x, scores, bins, flags: one allocation
-            x, scores, bins, flags = buf[0].view(torch.float32), buf[1].view(torch.float32), buf[2], buf[3]
+            x, scores, bins, flags = _score_outputs(rv.B, rv.V, dev)
             if HW > 1:      # raw maps: GlobalAveragePooling2D folded into the score kernel (nets/model.py:144-145)
                 C.check(L.gvcnn_gap_score_bin_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(R_out), _ptr(x), _ptr(scores),
                                                   _ptr(bins), _ptr(flags), _ptr(status), rv.B, rv.V, HW, Craw,
@@ -561,43 +607,32 @@ def _score_bin_fwd(rv, HW, Craw, Wc, bc, num_group, score_reduce, edge_ulps, cla
                 C.check(L.gvcnn_view_score_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(xb[0]), _ptr(xb[1]) if want_bound else None,
                                                rv.B, rv.V, rv.D, rv.layout, dt, _stream()), "gvcnn_view_score_fwd")
             sums = torch.empty((2, rv.V), dtype=torch.float32, device=dev)
-            buf = torch.empty((4, 1, rv.V), dtype=torch.int32, device=dev)
-            x, scores = buf[0].view(torch.float32), buf[1].view(torch.float32)
-            bins, flags = buf[2], buf[3]
-            ex_ptr, ex_fn, ex_user = _exchange_forms(exchange)
+            x, scores, bins, flags = _score_outputs(1, rv.V, dev)
+            ex_ptr, ex_fn, ex_user, _ = _exchange_args(exchange, None)
             if not want_bound and process_group is None:
                 # no order-sensitivity report asked for: column sums + [exchange] + mean / score / bin in ONE call
-                denom = rv.B if global_count is None else int(global_count)
-                if denom <= 0:
-                    raise ValueError("score_reduce='batch' over an empty (global) batch")
+                denom = _batch_count(rv.B, global_count, None, dev)
                 C.check(L.gvcnn_batch_mean_bin(_ptr(xb[0]), _ptr(sums[0]), _ptr(x), _ptr(scores), _ptr(bins), _ptr(flags),
                                                _ptr(status), rv.B, rv.V, num_group, int(multiplier or 0), edge_ulps,
                                                int(clamp), denom, ex_ptr, ex_user, _stream()), "gvcnn_batch_mean_bin")
-                return x, scores, bins, flags, R_out, _ScoreGrad(rv, HW, True, denom, exchange)
+                return x, scores, bins, flags, R_out, _ScoreGrad(rv, HW, True, denom, exchange, process_group)
             nsum = 2 if want_bound else 1                            # rows of `sums` in use: sum x (and sum A)
             if rv.B > 0:
                 for j in range(nsum):
                     C.check(L.gvcnn_batch_sum_x(_ptr(xb[j]), _ptr(sums[j]), rv.B, rv.V, _stream()), "gvcnn_batch_sum_x")
             else:
                 sums.zero_()
-            denom = rv.B if global_count is None else int(global_count)
             if exchange is not None:                                 # a gvcnn_exchange_fn (e.g. parallel.P2PComm)
                 C.check(ex_fn(ex_user, _ptr(sums), nsum * rv.V, _stream()), "exchange")
             elif process_group is not None:
                 import torch.distributed as dist
                 dist.all_reduce(sums[:nsum], group=process_group)
-                if global_count is None:
-                    cnt = torch.tensor([rv.B], dtype=torch.int64, device=dev)
-                    dist.all_reduce(cnt, group=process_group)
-                    denom = int(cnt.item())
-            if denom <= 0:
-                raise ValueError("score_reduce='batch' over an empty (global) batch")
+            denom = _batch_count(rv.B, global_count, None if exchange is not None else process_group, dev)
             C.check(L.gvcnn_score_bin(_ptr(sums[0]), ctypes.c_float(float(denom)), _ptr(x), _ptr(scores), _ptr(bins),
                                       _ptr(flags), _ptr(status), rv.V, num_group, int(multiplier or 0), edge_ulps,
                                       int(clamp), _ptr(sums[1]) if want_bound else None, Craw + 2 + denom, _stream()),
                     "gvcnn_score_bin")
-            return x, scores, bins, flags, R_out, _ScoreGrad(rv, HW, True, denom, exchange,
-                                                             None if exchange is not None else process_group)
+            return x, scores, bins, flags, R_out, _ScoreGrad(rv, HW, True, denom, exchange, process_group)
         raise ValueError("score_reduce must be 'shape' or 'batch'")
 
 
@@ -935,64 +970,60 @@ def pool_fuse(final_view_descriptors, bins, num_group, pool="max", empty_fill=1.
     return S
 
 
+def _pool_fuse_gap_fwd(fv: _Views, bins, weights, G, pool, empty_fill, want_mask, status) -> _Pooled:
+    """Pooling + fusion + GlobalAveragePooling2D of the maps in `fv` (gvcnn_pool_fuse_gap_weighted_fwd; weights None:
+    the reference's 1 + n_g): S_gap [B, C] in `S`.  GvcnnError E_UNSUPPORTED where the kernels do not cover the
+    shapes, raised before anything is launched."""
+    L = C.lib()
+    HW, Cch = fv.map_geometry
+    dt = _dtype_code(fv.dtype)
+    bins_c, bstride = _bin_rows(bins, fv)
+    w_c, wstride = _weight_rows(weights, G, fv)
+    S_gap = torch.empty((fv.B, Cch), dtype=fv.dtype, device=fv.device)
+    mask = _tie_mask(fv, pool, want_mask)
+    ws_bytes = 0 if fv.cf else L.gvcnn_pool_fuse_gap_workspace_bytes(fv.B, Cch, HW, dt)   # channels-first: none
+    ws = None if fv.cf else torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=fv.device)
+    with _on(fv.device):
+        C.check(L.gvcnn_pool_fuse_gap_weighted_fwd(fv.arg, _ptr(bins_c), bstride, _ptr(w_c), wstride, _ptr(S_gap),
+                                                   _ptr(mask), _ptr(status), _ptr(ws), ws_bytes, fv.B, fv.V, HW, Cch, G,
+                                                   _POOL[pool], ctypes.c_float(empty_fill), fv.map_layout, dt,
+                                                   _stream()),
+                "gvcnn_pool_fuse_gap_weighted_fwd")
+    return _Pooled(S_gap, mask, None, status, bins_c, bstride, w_c, wstride)
+
+
+def _pool_fuse_gap_bwd(dS_gap, fv_like: _Views, bins, bin_stride, weights, w_stride, mask, G, pool):
+    """dF from the [B, C] gradient of S_gap (gvcnn_pool_fuse_gap_weighted_bwd), in the layout of `fv_like`."""
+    HW, Cch = fv_like.map_geometry
+    dS_gap = dS_gap.contiguous()
+    out, gv = fv_like.empty_like()
+    with _on(dS_gap.device):
+        C.check(C.lib().gvcnn_pool_fuse_gap_weighted_bwd(_ptr(dS_gap), _ptr(bins), bin_stride, _ptr(weights), w_stride,
+                                                         _ptr(mask), gv.arg, None, gv.B, gv.V, HW, Cch, G, _POOL[pool],
+                                                         gv.map_layout, _dtype_code(gv.dtype), _stream()),
+                "gvcnn_pool_fuse_gap_weighted_bwd")
+    return out
+
+
 class _PoolFuseGapFn(torch.autograd.Function):
     """Pooling + fusion + the global average pooling that follows it (nets/model.py:154-163) without ever
     writing the fused map: [B, C] out; backward takes the [B, C] gradient.  `weights`: caller-supplied group
-    weights ([G] or [B, G]), None for the reference's 1 + n_g."""
+    weights ([G] or [B, G]), None for the reference's 1 + n_g.  `fv`: the maps, which are also the inputs after
+    `weights`."""
 
     @staticmethod
-    def forward(ctx, bins, G, pool, empty_fill, layout, HW, Cch, weights, cf, *views):
-        L = C.lib()
-        fv = _Views.of(views, layout, "F")
-        fv.cf = cf
-        dev = fv.device
-        dt = _dtype_code(fv.dtype)
-        bins_c, bstride = _bin_rows(bins, fv)
-        w_c, wstride = _weight_rows(weights, G, fv)
-        out = torch.empty((fv.B, Cch), dtype=fv.dtype, device=dev)
-        mask = _tie_mask(fv, pool, any(v.requires_grad for v in views))
-        status = _new_status(dev)
-        ws_bytes = 0 if cf else L.gvcnn_pool_fuse_gap_workspace_bytes(fv.B, Cch, HW, dt)   # channels-first: none
-        ws = None if cf else torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
-        with _on(dev):
-            if w_c is None:
-                C.check(L.gvcnn_pool_fuse_gap_fwd(fv.arg, _ptr(bins_c), bstride, _ptr(out), _ptr(mask), _ptr(status),
-                                                  _ptr(ws), ws_bytes, fv.B, fv.V, HW, Cch, G, _POOL[pool],
-                                                  ctypes.c_float(empty_fill), fv.map_layout, dt, _stream()),
-                        "gvcnn_pool_fuse_gap_fwd")
-            else:
-                C.check(L.gvcnn_pool_fuse_gap_weighted_fwd(fv.arg, _ptr(bins_c), bstride, _ptr(w_c), wstride, _ptr(out),
-                                                           _ptr(mask), _ptr(status), _ptr(ws), ws_bytes, fv.B, fv.V, HW,
-                                                           Cch, G, _POOL[pool], ctypes.c_float(empty_fill),
-                                                           fv.map_layout, dt, _stream()),
-                        "gvcnn_pool_fuse_gap_weighted_fwd")
-        ctx.fv, ctx.G, ctx.pool, ctx.HW, ctx.Cch, ctx.bstride, ctx.wstride = fv, G, pool, HW, Cch, bstride, wstride
-        ctx.save_for_backward(bins_c, w_c, mask)
-        ctx.mark_non_differentiable(status)
-        return out, status
+    def forward(ctx, fv, bins, G, pool, empty_fill, weights, *views):
+        out = _pool_fuse_gap_fwd(fv, bins, weights, G, pool, empty_fill, any(v.requires_grad for v in views),
+                                 _new_status(fv.device))
+        ctx.fv, ctx.G, ctx.pool, ctx.bstride, ctx.wstride = fv, G, pool, out.bin_stride, out.w_stride
+        ctx.save_for_backward(out.bins, out.weights, out.mask)
+        return out.S
 
     @staticmethod
-    def backward(ctx, dOut, _dstatus):
+    def backward(ctx, dOut):
         bins_c, w_c, mask = ctx.saved_tensors
-        fv = ctx.fv
-        dOut = dOut.contiguous()
-        out, gv = fv.empty_like()
-        status = _new_status(dOut.device)
-        L = C.lib()
-        with _on(dOut.device):
-            if w_c is None:
-                C.check(L.gvcnn_pool_fuse_gap_bwd(_ptr(dOut), _ptr(bins_c), ctx.bstride, _ptr(mask), gv.arg,
-                                                  _ptr(status), gv.B, gv.V, ctx.HW, ctx.Cch, ctx.G, _POOL[ctx.pool],
-                                                  gv.map_layout, _dtype_code(gv.dtype), _stream()),
-                        "gvcnn_pool_fuse_gap_bwd")
-            else:
-                C.check(L.gvcnn_pool_fuse_gap_weighted_bwd(_ptr(dOut), _ptr(bins_c), ctx.bstride, _ptr(w_c), ctx.wstride,
-                                                           _ptr(mask), gv.arg, _ptr(status), gv.B, gv.V, ctx.HW,
-                                                           ctx.Cch, ctx.G, _POOL[ctx.pool], gv.map_layout,
-                                                           _dtype_code(gv.dtype), _stream()),
-                        "gvcnn_pool_fuse_gap_weighted_bwd")
-        grads = tuple(out) if isinstance(out, list) else (out,)
-        return (None,) * 9 + grads
+        out = _pool_fuse_gap_bwd(dOut, ctx.fv, bins_c, ctx.bstride, w_c, ctx.wstride, mask, ctx.G, ctx.pool)
+        return (None,) * 6 + (tuple(out) if isinstance(out, list) else (out,))
 
 
 def pool_fuse_gap(final_view_descriptors, bins, num_group, pool="max", empty_fill=1.0, layout=None, group_weight=None,
@@ -1015,21 +1046,17 @@ def pool_fuse_gap(final_view_descriptors, bins, num_group, pool="max", empty_fil
         if not _is_maps(views, lay):
             raise ValueError("pool_fuse_gap with data_format='channels_first' expects maps, e.g. [N, C, h, w] per view")
         views, cf = _maps_in_memory_order(views, lay)
-    shp = tuple(views[0].shape)
-    if len(shp) < 3:
+    if len(views[0].shape) < 3:
         raise ValueError("pool_fuse_gap expects channel-last maps, e.g. [N, h, w, C] per view")
-    if cf:
-        Cch, spatial = shp[-3], shp[-2:]
-    else:
-        Cch, spatial = shp[-1], (shp[1:-1] if lay == "list" else shp[2:-1])
-    HW = int(math.prod(spatial)) if len(spatial) else 1
     _require_cuda(bins, "bins")
+    fv = _Views.of(views, lay, "F")
+    fv.cf = cf
     try:
-        out, _ = _PoolFuseGapFn.apply(bins, num_group, pool, empty_fill, lay, HW, Cch, group_weight, cf, *views)
-        return out
+        return _PoolFuseGapFn.apply(fv, bins, num_group, pool, empty_fill, group_weight, *views)
     except C.GvcnnError as e:
         if e.code != C.E_UNSUPPORTED:
             raise
+    Cch = fv.map_geometry[1]
     S = pool_fuse(list(views) if lay == "list" else views[0], bins, num_group, pool=pool, empty_fill=empty_fill,
                   layout=None if lay == "list" else lay, group_weight=group_weight)
     if cf:
@@ -1256,8 +1283,7 @@ def _grouping_fusion_fwd(rv, fv, want_mask, W, b, G, pool, empty_fill, edge_ulps
     dev = fv.device
     Wc, bc = W.contiguous(), b.contiguous()
     if literal is None:
-        buf = torch.empty((4, fv.B, fv.V), dtype=torch.int32, device=dev)      # x, scores, bins, flags: one allocation
-        x, scores, bins, flags = buf[0].view(torch.float32), buf[1].view(torch.float32), buf[2], buf[3]
+        x, scores, bins, flags = _score_outputs(fv.B, fv.V, dev)
     else:
         xb = torch.empty((max(fv.B, 1), fv.V), dtype=torch.float32, device=dev)
         buf = torch.empty((5, 1, fv.V), dtype=torch.int32, device=dev)           # xsum, x_mean, scores, bins, flags
@@ -1283,20 +1309,6 @@ def _grouping_fusion_fwd(rv, fv, want_mask, W, b, G, pool, empty_fill, edge_ulps
                     "gvcnn_grouping_fusion_batch_fwd")
     bin_stride = fv.V if (literal is None and fv.B > 1) else 0
     return _Pooled(S, mask, None, status, bins, bin_stride, None, 0), (x, scores, bins, flags)
-
-
-def _is_raw_maps(raw, W, layout, data_format="channels_last"):
-    """True when `raw` holds the un-pooled block3 maps ([..., h, w, C_raw], or [..., C_raw, h, w] with
-    data_format='channels_first') rather than [..., C_raw] descriptors."""
-    if not (isinstance(W, torch.Tensor) and W.dim() == 2):
-        return False
-    t = raw[0] if isinstance(raw, (list, tuple)) and len(raw) else raw
-    if not isinstance(t, torch.Tensor):
-        return False
-    if data_format == "channels_first":     # maps by their rank; _raw_views checks C_raw at dim -3
-        return _is_maps(*_view_args(raw, layout))
-    lead = 1 if isinstance(raw, (list, tuple)) else 2
-    return t.dim() > lead + 1 and t.shape[-1] == W.shape[1]
 
 
 def grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_group, pool="max",
@@ -1337,15 +1349,14 @@ def grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_grou
 def _grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_group, pool, empty_fill, score_reduce,
                      layout, clamp, check, process_group, edge_ulps, status, multiplier, exchange, global_count,
                      data_format, _variant):
+    rv, HW, Craw, Wc, bc = _score_args(raw_view_descriptors, W, b, layout, data_format)
     if status is None and check:
-        dev0 = W.device if isinstance(W, torch.Tensor) else None
-        status = _new_status(dev0)
-    if _is_raw_maps(raw_view_descriptors, W, layout, data_format):
+        status = _new_status(rv.device)
+    if HW > 1:
         # block3 maps instead of pooled raw descriptors: the GAP of nets/model.py:144 runs inside the score kernel
         # (gvcnn_gap_score_bin_fwd); pooling + fusion follow on the stream, chained with programmatic dependent launch
-        sr = score_bin(raw_view_descriptors, W, b, num_group, score_reduce=score_reduce, layout=layout,
-                       edge_ulps=edge_ulps, clamp=clamp, check=check, process_group=process_group, status=status,
-                       multiplier=multiplier, exchange=exchange, global_count=global_count, data_format=data_format)
+        sr = _score_bin(rv, HW, Craw, Wc, bc, num_group, score_reduce, edge_ulps, clamp, check, status, process_group,
+                        multiplier, exchange, global_count)
         S = pool_fuse(final_view_descriptors, sr.bins, num_group, pool=pool, empty_fill=empty_fill, layout=layout,
                       _variant=_variant)
         return S, sr
@@ -1354,35 +1365,17 @@ def _grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_gro
             raise ValueError("multiplier is only selectable with score_reduce='batch' or through group_scheme")
     elif score_reduce != "batch":
         raise ValueError("score_reduce must be 'shape' or 'batch'")
-    r_t, r_lay = _view_args(raw_view_descriptors, layout)
     f_t, f_lay = _view_args(final_view_descriptors, layout)
-    _check_score_fc(W, b)
     literal, keep = None, None
     if score_reduce == "batch":
-        B_local = r_t[0].shape[0] if r_lay in ("list", "bvd") else r_t[0].shape[1]
-        if exchange is None and process_group is not None:
-            cb, keep = make_exchange(process_group)
-            exchange = (cb, None)
-        ex_ptr, _, ex_user = _exchange_forms(exchange)
-        if global_count is None:
-            global_count = B_local
-            if process_group is not None:
-                import torch.distributed as dist
-                cnt = torch.tensor([B_local], dtype=torch.int64, device=W.device)
-                dist.all_reduce(cnt, group=process_group)
-                global_count = int(cnt.item())
-        if global_count <= 0:
-            raise ValueError("score_reduce='batch' over an empty (global) batch")
+        ex_ptr, _, ex_user, keep = _exchange_args(exchange, process_group)
+        global_count = _batch_count(rv.B, global_count, process_group, rv.device)
         literal = (multiplier, global_count, ex_ptr, ex_user)
-    rv = _Views.of(r_t, r_lay, "R")
-    Wc, bc = W.contiguous(), b.contiguous()
     score_in, sg = (), None
     if torch.is_grad_enabled() and (Wc.requires_grad or bc.requires_grad or any(t.requires_grad for t in rv.keep)):
         score_in = (Wc, bc) + tuple(rv.keep)
-        if literal is None:
-            sg = _ScoreGrad(rv, 1, False)
-        else:   # the backward's exchange: the forward's callback, or the process group's (made again when needed)
-            sg = _ScoreGrad(rv, 1, True, literal[1], exchange if keep is None else None, process_group)
+        # the backward's exchange: the forward's callback, or the process group's (made again when needed)
+        sg = _ScoreGrad(rv, 1, literal is not None, global_count, exchange, process_group)
 
     def launch(fv, want_mask):
         out, extras = _grouping_fusion_fwd(rv, fv, want_mask, Wc, bc, num_group, pool, empty_fill, edge_ulps, clamp,
@@ -1399,64 +1392,46 @@ def _grouping_fusion(raw_view_descriptors, W, b, final_view_descriptors, num_gro
 # --------------------------------------------------------------------------
 # paper mode: score-derived, differentiable group weights (SURVEY.md 8f n2)
 # --------------------------------------------------------------------------
-class _GapScoreUnsupported(Exception):
-    """gvcnn_gap_score_bin_fwd does not cover these block3 maps (raised before anything was launched)."""
-
-
 class _PaperModeFn(torch.autograd.Function):
     """S = sum_g w_g P_g / sum_g w_g with w_g = mean score of the group's views (0 for an empty group).
     Unlike the reference (weights fed through placeholders, train.py:127-128), the gradient reaches the
     V Dense(1) score layers: dL/dW, dL/db (and dL/dR if the raw descriptors require grad) besides dL/dF.
     No reference counterpart - checked against float64 autograd of the same formulas.
-    maps: R holds the block3 maps (HW_r > 1 positions); their GlobalAveragePooling2D runs inside the score kernel,
-    which also writes the pooled float32 R the score FC's gradient needs.  fold: the GlobalAveragePooling2D after
-    the fusion is folded into the pooling (S_gap [B, C] out, the [B, C] gradient in); where the folded kernels do not
-    cover the shapes the fused map is returned instead (the caller's _spatial_mean then averages it)."""
+    rv, HW: the raw views as _score_args returns them, which are also the inputs after `fold`; HW > 1: block3 maps,
+    whose GlobalAveragePooling2D runs inside the score kernel, which also writes the pooled float32 R the score FC's
+    gradient needs.  fold: the GlobalAveragePooling2D after the fusion is folded into the pooling (S_gap [B, C] out,
+    the [B, C] gradient in); where the folded kernels do not cover the shapes the fused map is returned instead (the
+    caller's _spatial_mean then averages it)."""
 
     @staticmethod
-    def forward(ctx, W, b, G, pool, f_layout, r_layout, n_r, status, HW_r, fold, r_cf, *tensors):
+    def forward(ctx, W, b, rv, HW, G, pool, f_layout, status, fold, *tensors):
         L = C.lib()
-        r_t, f_t = tensors[:n_r], tensors[n_r:]
-        rv = _Views.of(r_t, r_layout, "R")
-        rv.cf = r_cf
-        fv = _Views.of(f_t, f_layout, "F")
+        n_r = len(rv.keep)
+        fv = _Views.of(tensors[n_r:], f_layout, "F")
         dev = fv.device
-        R_out = None
         # no synchronisation in the training step: out-of-range / NaN scores are clamped for pooling and counted
         # into the caller's persistent `status` tensor (checked every N steps), as in grouping_fusion
-        if HW_r > 1:
-            Craw = rv.D // HW_r
-            Wc, bc = W.contiguous(), b.contiguous()
-            if tuple(Wc.shape) != (rv.V, Craw) or tuple(bc.shape) != (rv.V,):
-                raise ValueError("W must be [V, C] = %s and b [V], got %s and %s"
-                                 % ((rv.V, Craw), tuple(Wc.shape), tuple(bc.shape)))
-            buf = torch.empty((3, rv.B, rv.V), dtype=torch.int32, device=dev)     # x, scores, bins: one allocation
-            x, scores, bins = buf[0].view(torch.float32), buf[1].view(torch.float32), buf[2]
-            R_out = torch.empty((rv.B, rv.V, Craw), dtype=torch.float32, device=dev)
-            with _on(dev):
-                rc = L.gvcnn_gap_score_bin_fwd(rv.arg, _ptr(Wc), _ptr(bc), _ptr(R_out), _ptr(x), _ptr(scores),
-                                               _ptr(bins), None, _ptr(status), rv.B, rv.V, HW_r, Craw, G, rv.map_layout,
-                                               _dtype_code(rv.dtype), 1, 1, 1, _stream())
-            if rc == C.E_UNSUPPORTED:
-                raise _GapScoreUnsupported()
-            C.check(rc, "gvcnn_gap_score_bin_fwd")
-        else:
-            sr = score_bin(r_t if r_layout == "list" else r_t[0], W, b, G, score_reduce="shape", layout=r_layout,
-                           edge_ulps=1, clamp=True, check=False, status=status)
-            x, scores, bins = sr.x, sr.scores, sr.bins
+        x, scores, bins, _, R_out, _ = _score_bin_fwd(rv, HW, rv.D // HW, W, b, G, "shape", 1, True, status, None, None,
+                                                      None, None, HW > 1)
         weights = torch.empty((rv.B, G), dtype=torch.float32, device=dev)
         with _on(dev):
             C.check(L.gvcnn_group_weight_from_scores(_ptr(scores), _ptr(bins), _ptr(weights), rv.B, rv.V, G,
                                                      _stream()), "gvcnn_group_weight_from_scores")
-        out = _paper_gap_fwd(fv, bins, weights, G, pool) if fold else None
+        out = None
+        if fold and len(fv.view_shape) >= 3:
+            try:
+                out = _pool_fuse_gap_fwd(fv, bins, weights, G, pool, 0.0, True, None)
+            except C.GvcnnError as e:
+                if e.code != C.E_UNSUPPORTED:
+                    raise
         ctx.fold = out is not None
         if out is None:
             out = _pool_fuse_fwd(fv, bins, G, pool, 0.0, weights, want_mask=True, want_groups=False, want_status=False)
-        ctx.rv, ctx.fv, ctx.G, ctx.pool, ctx.HW_r = rv, fv, G, pool, HW_r
+        ctx.rv, ctx.fv, ctx.G, ctx.pool, ctx.HW = rv, fv, G, pool, HW
         ctx.bstride, ctx.wstride = out.bin_stride, out.w_stride
-        ctx.need_dr = any(t.requires_grad for t in r_t)
+        ctx.need_dr = any(t.requires_grad for t in rv.keep)
         ctx.n_r = n_r
-        ctx.save_for_backward(W.contiguous(), x, out.bins, out.weights, out.S, out.mask, R_out)
+        ctx.save_for_backward(W, x, out.bins, out.weights, out.S, out.mask, R_out)
         ctx.mark_non_differentiable(scores, bins, weights)
         S = out.S if ctx.fold else out.S.reshape(fv.view_shape)
         return S, scores, bins, weights
@@ -1465,23 +1440,15 @@ class _PaperModeFn(torch.autograd.Function):
     def backward(ctx, dS, _ds, _db, _dw):
         L = C.lib()
         W, x, bins_c, w_c, S, mask, R_out = ctx.saved_tensors
-        rv, fv, G, pool = ctx.rv, ctx.fv, ctx.G, ctx.pool
+        fv, G, pool = ctx.fv, ctx.G, ctx.pool
         dS2 = dS.contiguous() if ctx.fold else dS.reshape(fv.B, fv.D).contiguous()
         dev = dS2.device
-        Cr = rv.D // ctx.HW_r
         if ctx.fold:
-            dF = _paper_gap_bwd_f(dS2, fv, bins_c, ctx.bstride, w_c, ctx.wstride, mask, G, pool)
+            dF = _pool_fuse_gap_bwd(dS2, fv, bins_c, ctx.bstride, w_c, ctx.wstride, mask, G, pool)
         else:
             dF = _pool_fuse_bwd(dS2, fv, bins_c, ctx.bstride, w_c, ctx.wstride, mask, G, pool)
-        ws_bytes = L.gvcnn_view_score_bwd_workspace_bytes(rv.V, Cr)
-        n_dw, n_dx, n_W = fv.B * G, fv.B * fv.V, W.numel()
-        scratch = torch.empty(n_dw + n_dx + n_W + rv.V + (ws_bytes + 3) // 4, dtype=torch.float32, device=dev)  # one allocation
-        dweights = scratch[:n_dw].view(fv.B, G)
-        dx = scratch[n_dw:n_dw + n_dx].view(fv.B, fv.V)
-        dW = scratch[n_dw + n_dx:n_dw + n_dx + n_W].view_as(W)
-        dbias = scratch[n_dw + n_dx + n_W:n_dw + n_dx + n_W + rv.V]
-        ws = scratch[n_dw + n_dx + n_W + rv.V:]
-        dR_out, dR_views = (rv.empty_like() if ctx.need_dr else (None, None))
+        scratch = torch.empty(fv.B * (G + fv.V), dtype=torch.float32, device=dev)      # one allocation
+        dweights, dx = scratch[:fv.B * G].view(fv.B, G), scratch[fv.B * G:].view(fv.B, fv.V)
         with _on(dev):
             if ctx.fold:
                 _paper_gap_bwd_weights(fv, dS2, S, bins_c, ctx.bstride, w_c, ctx.wstride, dweights, G, pool)
@@ -1492,76 +1459,15 @@ class _PaperModeFn(torch.autograd.Function):
                         "gvcnn_pool_fuse_bwd_weights")
             C.check(L.gvcnn_score_weight_bwd(_ptr(dweights), _ptr(bins_c), _ptr(x), _ptr(dx), fv.B, fv.V, G, _stream()),
                     "gvcnn_score_weight_bwd")
-            if R_out is None:
-                C.check(L.gvcnn_view_score_bwd(rv.arg, _ptr(dx), _ptr(W), _ptr(dW), _ptr(dbias),
-                                               dR_views.arg if dR_views is not None else None, _ptr(ws), ws_bytes,
-                                               rv.B, rv.V, rv.D, rv.layout, _dtype_code(rv.dtype), _stream()),
-                        "gvcnn_view_score_bwd")
-            else:
-                # block3 maps: dW, db from the pooled R the score kernel wrote; dmaps = dx W / HW, only if asked for
-                C.check(L.gvcnn_view_score_bwd(_ptr(R_out), _ptr(dx), _ptr(W), _ptr(dW), _ptr(dbias), None, _ptr(ws),
-                                               ws_bytes, rv.B, rv.V, Cr, C.LAYOUT_BVD, C.F32, _stream()),
-                        "gvcnn_view_score_bwd")
-                if dR_views is not None:
-                    C.check(L.gvcnn_gap_score_bwd(_ptr(dx), _ptr(W), dR_views.arg, rv.B, rv.V, ctx.HW_r, Cr,
-                                                  rv.map_layout, _dtype_code(rv.dtype), _stream()),
-                            "gvcnn_gap_score_bwd")
-        if dR_out is None:
-            gr = (None,) * ctx.n_r
-        else:
-            gr = tuple(dR_out) if isinstance(dR_out, list) else (dR_out,)
+        dW, dbias, dR = _score_fc_bwd(dx, W, R_out, ctx.rv, ctx.HW, True, ctx.need_dr)
+        gr = dR if dR is not None else (None,) * ctx.n_r
         gf = tuple(dF) if isinstance(dF, list) else (dF,)
-        return (dW, dbias) + (None,) * 9 + gr + gf
-
-
-def _fold_geometry(fv):
-    """(HW, C) of channel-last per-view maps, or None when the views have no spatial axes."""
-    if len(fv.view_shape) < 3:
-        return None
-    Cch = int(fv.view_shape[-1])
-    return fv.D // Cch, Cch
-
-
-def _paper_gap_fwd(fv, bins, weights, G, pool):
-    """Paper-mode pooling + fusion + GlobalAveragePooling2D in one pass (S_gap [B, C] in `S`), or None when
-    gvcnn_pool_fuse_gap_weighted_fwd does not cover the shapes."""
-    geo = _fold_geometry(fv)
-    if geo is None:
-        return None
-    HW, Cch = geo
-    L = C.lib()
-    dt = _dtype_code(fv.dtype)
-    bins_c, bstride = _bin_rows(bins, fv)
-    w_c, wstride = _weight_rows(weights, G, fv)
-    S_gap = torch.empty((fv.B, Cch), dtype=fv.dtype, device=fv.device)
-    mask = _tie_mask(fv, pool, True)
-    ws_bytes = L.gvcnn_pool_fuse_gap_workspace_bytes(fv.B, Cch, HW, dt)
-    ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=fv.device)
-    with _on(fv.device):
-        rc = L.gvcnn_pool_fuse_gap_weighted_fwd(fv.arg, _ptr(bins_c), bstride, _ptr(w_c), wstride, _ptr(S_gap),
-                                                _ptr(mask), None, _ptr(ws), ws_bytes, fv.B, fv.V, HW, Cch, G,
-                                                _POOL[pool], ctypes.c_float(0.0), fv.layout, dt, _stream())
-    if rc == C.E_UNSUPPORTED:
-        return None
-    C.check(rc, "gvcnn_pool_fuse_gap_weighted_fwd")
-    return _Pooled(S_gap, mask, None, None, bins_c, bstride, w_c, wstride)
-
-
-def _paper_gap_bwd_f(dS_gap, fv, bins, bin_stride, weights, w_stride, mask, G, pool):
-    """dF from the [B, C] gradient of S_gap (gvcnn_pool_fuse_gap_weighted_bwd)."""
-    HW, Cch = _fold_geometry(fv)
-    out, gv = fv.empty_like()
-    with _on(dS_gap.device):
-        C.check(C.lib().gvcnn_pool_fuse_gap_weighted_bwd(_ptr(dS_gap), _ptr(bins), bin_stride, _ptr(weights), w_stride,
-                                                         _ptr(mask), gv.arg, None, gv.B, gv.V, HW, Cch, G, _POOL[pool],
-                                                         gv.layout, _dtype_code(gv.dtype), _stream()),
-                "gvcnn_pool_fuse_gap_weighted_bwd")
-    return out
+        return (dW, dbias) + (None,) * 7 + gr + gf
 
 
 def _paper_gap_bwd_weights(fv, dS_gap, S_gap, bins, bin_stride, weights, w_stride, dweights, G, pool):
     """dL/dw_g from the [B, C] gradient of S_gap (gvcnn_pool_fuse_gap_bwd_weights), into `dweights` [B, G]."""
-    HW, Cch = _fold_geometry(fv)
+    HW, Cch = fv.map_geometry
     L = C.lib()
     dt = _dtype_code(fv.dtype)
     ws_bytes = L.gvcnn_pool_fuse_gap_bwd_weights_workspace_bytes(fv.B, fv.V, HW, Cch, dt)
@@ -1598,30 +1504,19 @@ def grouping_fusion_paper(raw_view_descriptors, W, b, final_view_descriptors, nu
     data_format='channels_first': block3 and final maps are [N, C, h, w] per view, read without a copy as in
     score_bin and grouping_fusion.  The post-fusion GAP is folded only for final maps in torch.channels_last memory;
     contiguous NCHW final maps run the unfolded path and the mean."""
-    _check_data_format(data_format)
     final_view_descriptors, f_perm = _final_maps(final_view_descriptors, layout, data_format)
-    r_t, r_lay = _view_args(raw_view_descriptors, layout)
+    rv, HW, _, Wc, bc = _score_args(raw_view_descriptors, W, b, layout, data_format)
     f_t, f_lay = _view_args(final_view_descriptors, layout)
-    _check_score_fc(W, b)
-    HW_r, r_cf = 1, False
-    if _is_raw_maps(raw_view_descriptors, W, layout, data_format):
-        rv, HW_r = _raw_views(raw_view_descriptors, layout, int(W.shape[1]), data_format)
-        r_t, r_cf = tuple(rv.keep), rv.cf
     f_cf = data_format == "channels_first" and not f_perm
     fold = fold_gap and not f_cf            # the weighted folded kernels read channel-last maps only
-    if HW_r == 1 and not fold:
-        S, scores, bins, w = _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, 1, False, False,
-                                                *r_t, *f_t)
-    else:
-        try:
-            S, scores, bins, w = _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, HW_r, fold,
-                                                    r_cf, *r_t, *f_t)
-        except _GapScoreUnsupported:
-            # block3 maps the GAP-folded score kernel does not cover: pool them here, autograd carries dR to the maps
-            pooled = _spatial_mean_views(r_t, r_lay, r_cf)
-            r_t = tuple(pooled) if r_lay == "list" else (pooled,)
-            S, scores, bins, w = _PaperModeFn.apply(W, b, num_group, pool, f_lay, r_lay, len(r_t), status, 1, fold,
-                                                    False, *r_t, *f_t)
+    try:
+        S, scores, bins, w = _PaperModeFn.apply(Wc, bc, rv, HW, num_group, pool, f_lay, status, fold, *rv.keep, *f_t)
+    except C.GvcnnError as e:
+        if e.code != C.E_UNSUPPORTED or HW == 1:
+            raise
+        # block3 maps the GAP-folded score kernel does not cover: pool them here, autograd carries dR to the maps
+        rv = _Views(_spatial_mean_views(rv.keep, rv.kind, rv.cf), rv.kind, "R")
+        S, scores, bins, w = _PaperModeFn.apply(Wc, bc, rv, 1, num_group, pool, f_lay, status, fold, *rv.keep, *f_t)
     if fold_gap:
         return _spatial_mean(S, "channels_first" if f_cf else "channels_last"), scores, bins, w
     return (S.movedim(-1, -3) if f_perm else S), scores, bins, w

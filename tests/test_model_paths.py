@@ -102,3 +102,16 @@ def test_score_bin_batch_exchange_in_both_forms(model, form, edge_ulps):
     assert len(calls) == 1
     assert torch.equal(got.bins, want.bins) and torch.equal(got.scores, want.scores)
     assert len(np.unique(got.bins.cpu().numpy())) > 2
+
+
+@pytest.mark.parametrize("score_reduce", ["shape", "batch"])
+def test_grouping_fusion_rejects_score_fc_shape_mismatch(model, score_reduce):
+    """A W narrower than R's channels, a b shorter than V, and channel-last maps whose trailing dimension is not C_raw
+    raise ValueError before anything is launched, as in score_bin (the score kernel would read past W or b)."""
+    B, V, Cr, D, G = 8, 12, 256, 64, 8
+    R, W, b, F, _ = _inputs(5, B, V, Cr, D)
+    Rd, Wd, bd, Fd = (torch.tensor(a, device="cuda") for a in (R, W, b, F))
+    maps = torch.randn((B, V, 2, 2, Cr // 2), device="cuda")          # h * w * C' = 2 C_raw: not descriptors either
+    for args in ((Rd, Wd[:, :Cr // 2], bd), (Rd, Wd, bd[:V - 1]), (maps, Wd, bd)):
+        with pytest.raises(ValueError):
+            model.grouping_fusion(*args, Fd, G, score_reduce=score_reduce)
