@@ -13,8 +13,6 @@ using namespace gvcnn;
 
 namespace {
 
-size_t elt_size(int dtype) { return dtype == GVCNN_F32 ? 4 : 2; }
-
 // Fills vp and the shape stride (elements) for tensor X of logical shape
 // [B, V, D]; reports whether every row start is 16-byte aligned.
 int make_view_ptrs(const void *X, int layout, int dtype, int B, int V, int64_t D, ViewPtrs &vp, int64_t &sb,
@@ -65,7 +63,13 @@ int check_dims(int B, int V, int64_t D, int G, int dtype)
     return B == 0 ? kEmptyBatch : 0;
 }
 
-bool is_aligned(const void *p, size_t a) { return reinterpret_cast<uintptr_t>(p) % a == 0; }
+// The pooling entry points' pool argument: the pool mode in the low byte, a kernel variant above it.  Splits it in place.
+int take_pool_variant(int &pool, int &variant)
+{
+    variant = GVCNN_POOL_VARIANT_OF(pool);
+    pool &= 0xff;
+    return (pool != GVCNN_POOL_MAX && pool != GVCNN_POOL_MEAN) || variant > 4 ? GVCNN_E_BAD_MODE : 0;
+}
 
 // Takes GVCNN_LAYOUT_CHANNELS_FIRST off a layout argument of the entry points that accept it; make_view_ptrs then sees
 // the base layout (every other entry point hands it the flag, which it rejects with GVCNN_E_BAD_LAYOUT).
@@ -90,11 +94,11 @@ int batch_score_tail(const float *x, float *xsum, float *x_mean, float *scores, 
     const CommPeers *peers = nullptr;
     int crank = 0, cworld = 1;
     const bool own_comm = exchange == &gvcnn_comm_allreduce_f32 && comm_device_view(exchange_user, &peers, &crank, &cworld);
-    int rc = -1000;
+    int rc = kNotApplicable;
     if (!exchange || own_comm)
         rc = launch_batch_mean_bin_fused(x, xsum, x_mean, scores, bins, flags, status, B, V, G, multiplier, edge_ulps,
                                          clamp, (float)global_count, own_comm ? peers : nullptr, crank, cworld, st);
-    if (rc != -1000) return rc;
+    if (rc != kNotApplicable) return rc;
     if (B == 0 || !x) {
         const cudaError_t e = cudaMemsetAsync(xsum, 0, (size_t)V * sizeof(float), st);
         if (e != cudaSuccess) return (int)e;
@@ -300,7 +304,7 @@ int gvcnn_gap_score_bin_fwd(const void *maps, const float *W, const float *bias,
     if (!al) return GVCNN_E_UNSUPPORTED;
     rc = launch_gap_score(mp, sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW, C, G, dtype, fuse_bin != 0,
                           edge_ulps, clamp, cf, static_cast<cudaStream_t>(stream));
-    return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
+    return rc == kNotApplicable ? GVCNN_E_UNSUPPORTED : rc;
 }
 
 // f_ready: the caller launched the kernel(s) directly in front of this one on the stream itself and they do not write
@@ -315,9 +319,9 @@ static int pool_fuse_fwd_impl(const void *F, const int32_t *bins, int64_t bin_st
     int rc = check_dims(B, V, D, G, dtype);
     if (rc) return rc == kEmptyBatch ? 0 : rc;
     if (!bins || !S || bin_stride_b < 0) return GVCNN_E_BAD_ARG;
-    const int variant = GVCNN_POOL_VARIANT_OF(pool);
-    pool &= 0xff;
-    if ((pool != GVCNN_POOL_MAX && pool != GVCNN_POOL_MEAN) || variant > 4) return GVCNN_E_BAD_MODE;
+    int variant;
+    rc = take_pool_variant(pool, variant);
+    if (rc) return rc;
     const size_t es = elt_size(dtype);
     if (!is_aligned(S, es) || !is_aligned(bins, 4)) return GVCNN_E_MISALIGNED;
     ViewPtrs fp;
@@ -333,7 +337,7 @@ static int pool_fuse_fwd_impl(const void *F, const int32_t *bins, int64_t bin_st
         if (!al || group_desc || weights) return GVCNN_E_UNSUPPORTED;
         rc = launch_pool_fuse_fwd_direct(fp, sb, bins, bin_stride_b, S, tie_mask, status, B, V, D, G, pool, empty_fill, dtype, true,
                                          f_ready, static_cast<cudaStream_t>(stream));
-        return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
+        return rc == kNotApplicable ? GVCNN_E_UNSUPPORTED : rc;
     }
     if (al && !group_desc && (variant == 0 || variant == 3)) {
         // fast path: persistent warp-specialised TMA ring (pool_fwd_ring.cu), with the reference's own weights or
@@ -342,11 +346,11 @@ static int pool_fuse_fwd_impl(const void *F, const int32_t *bins, int64_t bin_st
         if (direct && !weights && variant == 0) {  // few views: one tile per CTA, no ring (pool_fwd_direct.cu)
             rc = launch_pool_fuse_fwd_direct(fp, sb, bins, bin_stride_b, S, tie_mask, status, B, V, D, G, pool, empty_fill, dtype,
                                              false, f_ready, static_cast<cudaStream_t>(stream));
-            if (rc != -1000) return rc;
+            if (rc != kNotApplicable) return rc;
         }
         rc = launch_pool_fuse_fwd_ring(fp, sb, bins, bin_stride_b, weights, weight_stride_b, S, tie_mask, status, B, V, D, G, pool,
                                        empty_fill, dtype, static_cast<cudaStream_t>(stream));
-        if (rc != -1000) return rc;
+        if (rc != kNotApplicable) return rc;
     }
     return launch_pool_fuse_fwd(fp, sb, bins, bin_stride_b, S, group_desc, tie_mask, weights, weight_stride_b, status, B, V, D, G, pool, empty_fill,
                                 dtype, al, variant, static_cast<cudaStream_t>(stream));
@@ -367,9 +371,9 @@ int gvcnn_pool_fuse_bwd(const void *dS, const int32_t *bins, int64_t bin_stride_
     int rc = check_dims(B, V, D, G, dtype);
     if (rc) return rc == kEmptyBatch ? 0 : rc;
     if (!dS || !bins || bin_stride_b < 0) return GVCNN_E_BAD_ARG;
-    const int variant = GVCNN_POOL_VARIANT_OF(pool);
-    pool &= 0xff;
-    if ((pool != GVCNN_POOL_MAX && pool != GVCNN_POOL_MEAN) || variant > 4) return GVCNN_E_BAD_MODE;
+    int variant;
+    rc = take_pool_variant(pool, variant);
+    if (rc) return rc;
     if (pool == GVCNN_POOL_MAX && !tie_mask) return GVCNN_E_BAD_ARG;
     const size_t es = elt_size(dtype);
     if (!is_aligned(dS, es) || !is_aligned(bins, 4)) return GVCNN_E_MISALIGNED;
@@ -384,7 +388,7 @@ int gvcnn_pool_fuse_bwd(const void *dS, const int32_t *bins, int64_t bin_stride_
         // fast path: V-templated kernel (pool_bwd_fast.cu)
         rc = launch_pool_fuse_bwd_fast(dS, bins, bin_stride_b, tie_mask, weights, weight_stride_b, gp, sb, status, B, V, D, G, pool, dtype,
                                        static_cast<cudaStream_t>(stream));
-        if (rc != -1000) return rc;
+        if (rc != kNotApplicable) return rc;
     }
     return launch_pool_fuse_bwd(dS, bins, bin_stride_b, tie_mask, weights, weight_stride_b, gp, sb, status, B, V, D, G, pool, dtype, al,
                                 static_cast<cudaStream_t>(stream));
@@ -398,9 +402,9 @@ int gvcnn_view_pooling_bwd(const void *dP, const int32_t *bins, int64_t bin_stri
     int rc = check_dims(B, V, D, G, dtype);
     if (rc) return rc == kEmptyBatch ? 0 : rc;
     if (!dP || !bins || bin_stride_b < 0) return GVCNN_E_BAD_ARG;
-    const int variant = GVCNN_POOL_VARIANT_OF(pool);
-    pool &= 0xff;
-    if ((pool != GVCNN_POOL_MAX && pool != GVCNN_POOL_MEAN) || variant > 4) return GVCNN_E_BAD_MODE;
+    int variant;
+    rc = take_pool_variant(pool, variant);
+    if (rc) return rc;
     if (pool == GVCNN_POOL_MAX && !tie_mask) return GVCNN_E_BAD_ARG;
     const size_t es = elt_size(dtype);
     if (!is_aligned(dP, es) || !is_aligned(bins, 4)) return GVCNN_E_MISALIGNED;
@@ -414,7 +418,7 @@ int gvcnn_view_pooling_bwd(const void *dP, const int32_t *bins, int64_t bin_stri
     if (al && (variant == 0 || forced_fast)) {
         rc = launch_view_pooling_bwd_fast(dP, bins, bin_stride_b, tie_mask, gp, sb, status, B, V, D, G, pool, dtype,
                                           static_cast<cudaStream_t>(stream));
-        if (rc != -1000) return rc;
+        if (rc != kNotApplicable) return rc;
     }
     if (forced_fast) return GVCNN_E_UNSUPPORTED;
     return launch_view_pooling_bwd(dP, bins, bin_stride_b, tie_mask, gp, sb, status, B, V, D, G, pool, dtype, al,
@@ -515,7 +519,7 @@ static int pool_fuse_gap_fwd_impl(const void *F, const int32_t *bins, int64_t bi
             return GVCNN_E_UNSUPPORTED;
         rc = launch_pool_fuse_gap_cf_fwd(fp, sb, bins, bin_stride_b, S_gap, tie_mask, status, B, V, HW, C, G, pool,
                                          empty_fill, dtype, static_cast<cudaStream_t>(stream));
-        return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
+        return rc == kNotApplicable ? GVCNN_E_UNSUPPORTED : rc;
     }
     const size_t need = gap_workspace_bytes(B, C, HW, dtype);
     if (!al || need == 0 || V > 32 || (tie_mask && !is_aligned(tie_mask, 8)) || !is_aligned(workspace, 16))
@@ -524,7 +528,7 @@ static int pool_fuse_gap_fwd_impl(const void *F, const int32_t *bins, int64_t bi
     rc = launch_pool_fuse_gap_fwd(fp, sb, bins, bin_stride_b, weights, weight_stride_b, S_gap, tie_mask, status,
                                   static_cast<float *>(workspace), B, V, HW, C, G, pool, empty_fill, dtype,
                                   static_cast<cudaStream_t>(stream));
-    return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
+    return rc == kNotApplicable ? GVCNN_E_UNSUPPORTED : rc;
 }
 
 int gvcnn_pool_fuse_gap_fwd(const void *F, const int32_t *bins, int64_t bin_stride_b, void *S_gap, uint8_t *tie_mask,
@@ -568,7 +572,7 @@ static int pool_fuse_gap_bwd_impl(const void *dS_gap, const int32_t *bins, int64
         return GVCNN_E_UNSUPPORTED;
     rc = launch_pool_fuse_gap_bwd(dS_gap, bins, bin_stride_b, weights, weight_stride_b, tie_mask, gp, sb, status, B, V,
                                   HW, C, G, pool, dtype, cf, static_cast<cudaStream_t>(stream));
-    return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
+    return rc == kNotApplicable ? GVCNN_E_UNSUPPORTED : rc;
 }
 
 int gvcnn_pool_fuse_gap_bwd(const void *dS_gap, const int32_t *bins, int64_t bin_stride_b, const uint8_t *tie_mask,
@@ -654,7 +658,6 @@ int gvcnn_view_score_bwd(const void *R, const float *dx, const float *W, float *
 // ---------------------------------------------------------------------------
 // paper mode on spatial maps: the GAP-folded weight gradient and the gradient of the score FC's GAP (paper_gap.cu)
 // ---------------------------------------------------------------------------
-static bool gap_view_count(int V) { return V == 4 || V == 6 || V == 8 || V == 12 || V == 16 || V == 20; }
 
 size_t gvcnn_pool_fuse_gap_bwd_weights_workspace_bytes(int B, int V, int HW, int C, int dtype)
 {
@@ -681,7 +684,7 @@ int gvcnn_pool_fuse_gap_bwd_weights(const void *F, const void *dS_gap, const voi
     rc = make_view_ptrs(F, f_layout, dtype, B, V, D, fp, sb, al);
     if (rc) return rc;
     const size_t need = gap_bwd_weights_workspace_bytes(B, V, HW, C, dtype);
-    if (!al || need == 0 || !gap_view_count(V) || G > 255) return GVCNN_E_UNSUPPORTED;
+    if (!al || need == 0 || !kFastViews.has(V) || G > 255) return GVCNN_E_UNSUPPORTED;
     if (!is_aligned(dS_gap, 16) || !is_aligned(S_gap, 16) || !is_aligned(bins, 4) || !is_aligned(weights, 4) ||
         !is_aligned(dweights, 4) || !is_aligned(workspace, 16))
         return GVCNN_E_MISALIGNED;
@@ -689,7 +692,7 @@ int gvcnn_pool_fuse_gap_bwd_weights(const void *F, const void *dS_gap, const voi
     rc = launch_gap_bwd_weights(fp, sb, dS_gap, S_gap, bins, bin_stride_b, weights, weight_stride_b, dweights,
                                 static_cast<float *>(workspace), B, V, HW, C, G, pool, dtype,
                                 static_cast<cudaStream_t>(stream));
-    return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
+    return rc == kNotApplicable ? GVCNN_E_UNSUPPORTED : rc;
 }
 
 int gvcnn_gap_score_bwd(const float *dx, const float *W, void *dmaps, int B, int V, int HW, int C, int m_layout,
@@ -709,7 +712,7 @@ int gvcnn_gap_score_bwd(const float *dx, const float *W, void *dmaps, int B, int
     if (!is_aligned(dx, 4) || !is_aligned(W, 16)) return GVCNN_E_MISALIGNED;
     if (!al) return GVCNN_E_UNSUPPORTED;
     rc = launch_gap_score_bwd(dx, W, dp, sb, B, V, HW, C, dtype, cf, static_cast<cudaStream_t>(stream));
-    return rc == -1000 ? GVCNN_E_UNSUPPORTED : rc;
+    return rc == kNotApplicable ? GVCNN_E_UNSUPPORTED : rc;
 }
 
 }  // extern "C"

@@ -8,6 +8,7 @@
 
 #include <atomic>
 #include <cstdlib>
+#include <type_traits>
 
 #include "gvcnn_b200.h"
 
@@ -262,11 +263,86 @@ inline int resident_ctas(int threads, size_t dyn_smem = 0)
     return n;
 }
 
+// SMs of the current device, asked once per process; 148 (a B200), not cached, when the query fails.
+inline int sm_count()
+{
+    static std::atomic<int> cached{0};
+    int n = cached.load(std::memory_order_relaxed);
+    if (n > 0) return n;
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess ||
+        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) {
+        cudaGetLastError();
+        return 148;
+    }
+    cached.store(n, std::memory_order_relaxed);
+    return n;
+}
+
 // A/B tuning knobs are environment variables read ONCE per process (first use), never per launch.
 inline int env_int_once(const char *name, int dflt)
 {
     const char *v = getenv(name);
     return v ? atoi(v) : dflt;
+}
+
+inline size_t elt_size(int dtype) { return dtype == GVCNN_F32 ? 4 : 2; }
+inline bool is_aligned(const void *p, size_t a) { return reinterpret_cast<uintptr_t>(p) % a == 0; }
+
+// ---- launcher dispatch --------------------------------------------------------
+// A launcher picks its kernel's template arguments with these, innermost last, and launches once.  Each helper calls
+// f with the compile-time value matching its run-time argument, so only the combinations a launcher names are built.
+
+// Launcher result: these shapes are not covered by the kernel; the caller falls back to another kernel or reports
+// GVCNN_E_UNSUPPORTED.  Never returned through the ABI.
+constexpr int kNotApplicable = -1000;
+
+template <class T> struct Tag { using type = T; };
+
+// f(Tag<float>{}) / f(Tag<__nv_bfloat16>{}) / f(Tag<__half>{}) for GVCNN_F32 / GVCNN_BF16 / GVCNN_F16
+template <class F>
+int with_dtype(int dtype, F &&f)
+{
+    switch (dtype) {
+    case GVCNN_F32: return f(Tag<float>{});
+    case GVCNN_BF16: return f(Tag<__nv_bfloat16>{});
+    case GVCNN_F16: return f(Tag<__half>{});
+    default: return GVCNN_E_BAD_DTYPE;
+    }
+}
+
+// A set of view counts a kernel is instantiated for.
+template <int... Vs>
+struct ViewCounts {
+    static constexpr bool has(int V) { return ((V == Vs) || ...); }
+};
+// The view counts of the fast kernels (ring and GAP forward, fast backward, GAP weight gradient): the reference's
+// configurations (train.py:96 default 6; BASELINE sweep 6 / 12 / 20) plus the other common multi-view rigs.
+constexpr ViewCounts<4, 6, 8, 12, 16, 20> kFastViews{};
+
+// f(std::integral_constant<int, V>{}) when V is in the set, else kNotApplicable
+template <int... Vs, class F>
+int with_views(ViewCounts<Vs...>, int V, F &&f)
+{
+    int rc = kNotApplicable;
+    (void)((V == Vs && (rc = f(std::integral_constant<int, Vs>{}), true)) || ...);
+    return rc;
+}
+
+template <class F>
+int with_flag(bool b, F &&f)
+{
+    return b ? f(std::true_type{}) : f(std::false_type{});
+}
+
+// f(pool, mask) with compile-time pool mode and tie-mask flag: the tie planes exist for max pooling only, so the
+// combinations are (MAX, mask), (MAX, no mask) and (MEAN, no mask).
+template <class F>
+int with_pool(int pool, bool want_mask, F &&f)
+{
+    using Max = std::integral_constant<int, GVCNN_POOL_MAX>;
+    if (pool != GVCNN_POOL_MAX) return f(std::integral_constant<int, GVCNN_POOL_MEAN>{}, std::false_type{});
+    return want_mask ? f(Max{}, std::true_type{}) : f(Max{}, std::false_type{});
 }
 
 // ---- exact division with a precomputed reciprocal -----------------------------

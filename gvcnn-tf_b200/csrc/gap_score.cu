@@ -309,6 +309,10 @@ gap_score_cf_blocked_kernel(const ViewPtrs mp, const int64_t m_sb, const float *
                                       edge_ulps, clamp);
 }
 
+// a kernel as a type, to pass one of several kernels to a generic lambda that needs it at compile time
+template <auto K>
+using KernelC = std::integral_constant<decltype(K), K>;
+
 template <typename T>
 static int launch_gap_score_t(const ViewPtrs &mp, int64_t m_sb, const float *W, const float *bias, float *R_out, float *x,
                               float *scores, int32_t *bins, int32_t *flags, int32_t *status, int B, int V, int HW, int C,
@@ -320,49 +324,37 @@ static int launch_gap_score_t(const ViewPtrs &mp, int64_t m_sb, const float *W, 
     const bool blocked = cf && (int64_t)kGapCfRows * HW > (int64_t)kGapCfRegs * kGapWarps * 32 * E;
     const dim3 grid((unsigned)items), block(kGapWarps * 32);
     const size_t cf_rows = !cf ? 0 : (size_t)kGapCfRows * (blocked ? kGapCfBlk + 1 : (HW | 1)) * sizeof(float);
-    cudaError_t err = cudaSuccess;
-#define GVCNN_LAUNCH_GAP_SCORE_K(KERN_, NB_, FUSE_, EXTRA_)                                                      \
-    do {                                                                                                          \
-        const size_t smem = (size_t)kGapWarps * NB_ * 32 * E * sizeof(float) + EXTRA_;                            \
-        err = ensure_dyn_smem<KERN_<T, NB_, FUSE_>>((int)smem);                                                   \
-        if (err == cudaSuccess)                                                                                   \
-            err = launch_pdl(KERN_<T, NB_, FUSE_>, grid, block, smem, st, mp, m_sb, W, bias, R_out, x, scores,    \
-                             bins, flags, status, B, V, HW, G, edge_ulps, clamp);                                 \
-    } while (0)
-#define GVCNN_LAUNCH_GAP_SCORE(NB_, FUSE_)                                                                        \
-    do {                                                                                                          \
-        if (blocked) GVCNN_LAUNCH_GAP_SCORE_K(gap_score_cf_blocked_kernel, NB_, FUSE_, cf_rows);                  \
-        else if (cf) GVCNN_LAUNCH_GAP_SCORE_K(gap_score_cf_kernel, NB_, FUSE_, cf_rows);                          \
-        else GVCNN_LAUNCH_GAP_SCORE_K(gap_score_kernel, NB_, FUSE_, 0);                                           \
-    } while (0)
-    if (C == 8 * 32 * E) {
-        if (fuse_bin) GVCNN_LAUNCH_GAP_SCORE(8, true); else GVCNN_LAUNCH_GAP_SCORE(8, false);
-    } else if (C == 4 * 32 * E) {
-        if (fuse_bin) GVCNN_LAUNCH_GAP_SCORE(4, true); else GVCNN_LAUNCH_GAP_SCORE(4, false);
-    } else {
-        return -1000;
-    }
-#undef GVCNN_LAUNCH_GAP_SCORE
-#undef GVCNN_LAUNCH_GAP_SCORE_K
-    if (err != cudaSuccess) return (int)err;
-    return (int)cudaGetLastError();
+    if (C != 8 * 32 * E && C != 4 * 32 * E) return kNotApplicable;
+    // the three kernels share one parameter list: kern_c names the one these maps take
+    auto launch = [&](auto kern_c, size_t smem) {
+        constexpr auto kern = decltype(kern_c)::value;
+        cudaError_t e = ensure_dyn_smem<kern>((int)smem);
+        if (e == cudaSuccess)
+            e = launch_pdl(kern, grid, block, smem, st, mp, m_sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW,
+                           G, edge_ulps, clamp);
+        return (int)e;
+    };
+    const int rc = with_flag(C == 8 * 32 * E, [&](auto nb8) {
+        return with_flag(fuse_bin, [&](auto fuse) {
+            constexpr int NB = nb8 ? 8 : 4;
+            const size_t smem = (size_t)kGapWarps * NB * 32 * E * sizeof(float) + cf_rows;
+            if (blocked) return launch(KernelC<gap_score_cf_blocked_kernel<T, NB, fuse>>{}, smem);
+            if (cf) return launch(KernelC<gap_score_cf_kernel<T, NB, fuse>>{}, smem);
+            return launch(KernelC<gap_score_kernel<T, NB, fuse>>{}, smem);
+        });
+    });
+    return rc ? rc : (int)cudaGetLastError();
 }
 
-// cf: channels-first maps.  Returns -1000 when the channel count is not one of the instantiated ones
+// cf: channels-first maps.  Returns kNotApplicable when the channel count is not one of the instantiated ones
 int launch_gap_score(const ViewPtrs &mp, int64_t m_sb, const float *W, const float *bias, float *R_out, float *x,
                      float *scores, int32_t *bins, int32_t *flags, int32_t *status, int B, int V, int HW, int C, int G,
                      int dtype, bool fuse_bin, int edge_ulps, int clamp, bool cf, cudaStream_t st)
 {
-    if (dtype == GVCNN_F32)
-        return launch_gap_score_t<float>(mp, m_sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW, C, G, fuse_bin,
-                                         edge_ulps, clamp, cf, st);
-    if (dtype == GVCNN_BF16)
-        return launch_gap_score_t<__nv_bfloat16>(mp, m_sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW, C, G,
-                                                 fuse_bin, edge_ulps, clamp, cf, st);
-    if (dtype == GVCNN_F16)
-        return launch_gap_score_t<__half>(mp, m_sb, W, bias, R_out, x, scores, bins, flags, status, B, V, HW, C, G,
-                                          fuse_bin, edge_ulps, clamp, cf, st);
-    return GVCNN_E_BAD_DTYPE;
+    return with_dtype(dtype, [&](auto tag) {
+        return launch_gap_score_t<typename decltype(tag)::type>(mp, m_sb, W, bias, R_out, x, scores, bins, flags, status,
+                                                                B, V, HW, C, G, fuse_bin, edge_ulps, clamp, cf, st);
+    });
 }
 
 }  // namespace gvcnn

@@ -23,9 +23,7 @@ namespace {
 constexpr int kHostBufs = 3;
 constexpr int kMaxInStreams = 2;
 
-size_t elt_size(int dtype) { return dtype == GVCNN_F32 ? 4 : 2; }
 size_t align_up(size_t x) { return (x + 255) & ~size_t(255); }
-bool is_aligned(const void *p, size_t a) { return reinterpret_cast<uintptr_t>(p) % a == 0; }
 
 struct ChunkLayout {
     size_t R, F, S, scores, bins, dS, mask, dF, total;

@@ -181,41 +181,29 @@ static int launch_gbw_v(const ViewPtrs &fp, int64_t f_sb, const void *dS_gap, co
     const int64_t units = (int64_t)B * CB * nsplit;
     if (units > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
     const T *ds = static_cast<const T *>(dS_gap);
-    cudaError_t err;
-    if (pool == GVCNN_POOL_MAX)
-        err = launch_pdl(gap_bwd_weights_kernel<T, GVCNN_POOL_MAX, V>, dim3((unsigned)units), dim3(kPgThreads), 0, st,
-                         fp, f_sb, ds, bins, bin_sb, partial, C, HW, G, CB, nsplit, pps);
-    else
-        err = launch_pdl(gap_bwd_weights_kernel<T, GVCNN_POOL_MEAN, V>, dim3((unsigned)units), dim3(kPgThreads), 0, st,
-                         fp, f_sb, ds, bins, bin_sb, partial, C, HW, G, CB, nsplit, pps);
-    if (err != cudaSuccess) return (int)err;
-    err = launch_pdl(gap_bwd_weights_finish_kernel<T>, dim3((unsigned)B), dim3(256), 0, st, (const float *)partial, ds,
+    const int rc = with_pool(pool, false, [&](auto pool_c, auto) {
+        return (int)launch_pdl(gap_bwd_weights_kernel<T, pool_c, V>, dim3((unsigned)units), dim3(kPgThreads), 0, st, fp,
+                               f_sb, ds, bins, bin_sb, partial, C, HW, G, CB, nsplit, pps);
+    });
+    if (rc) return rc;
+    const cudaError_t err = launch_pdl(gap_bwd_weights_finish_kernel<T>, dim3((unsigned)B), dim3(256), 0, st, (const float *)partial, ds,
                      static_cast<const T *>(S_gap), bins, bin_sb, weights, w_sb, dweights, V, C, HW, G, nsplit, CB, pool);
     return (int)err;
 }
 
-// returns -1000 when the shapes are not supported (V not instantiated, C not a multiple of the tile, G > 255)
+// returns kNotApplicable when the shapes are not supported (V not instantiated, C not a multiple of the tile, G > 255)
 int launch_gap_bwd_weights(const ViewPtrs &fp, int64_t f_sb, const void *dS_gap, const void *S_gap,
                            const int32_t *bins, int64_t bin_sb, const float *weights, int64_t w_sb, float *dweights,
                            float *partial, int B, int V, int HW, int C, int G, int pool, int dtype, cudaStream_t st)
 {
     const int CB = pg_channel_blocks(C, dtype);
-    if (CB == 0 || G > 255) return -1000;
-#define GVCNN_GBW_CASE(T_)                                                                                          \
-    switch (V) {                                                                                                    \
-    case 4: return launch_gbw_v<T_, 4>(fp, f_sb, dS_gap, S_gap, bins, bin_sb, weights, w_sb, dweights, partial, B, HW, C, G, pool, CB, st);   \
-    case 6: return launch_gbw_v<T_, 6>(fp, f_sb, dS_gap, S_gap, bins, bin_sb, weights, w_sb, dweights, partial, B, HW, C, G, pool, CB, st);   \
-    case 8: return launch_gbw_v<T_, 8>(fp, f_sb, dS_gap, S_gap, bins, bin_sb, weights, w_sb, dweights, partial, B, HW, C, G, pool, CB, st);   \
-    case 12: return launch_gbw_v<T_, 12>(fp, f_sb, dS_gap, S_gap, bins, bin_sb, weights, w_sb, dweights, partial, B, HW, C, G, pool, CB, st); \
-    case 16: return launch_gbw_v<T_, 16>(fp, f_sb, dS_gap, S_gap, bins, bin_sb, weights, w_sb, dweights, partial, B, HW, C, G, pool, CB, st); \
-    case 20: return launch_gbw_v<T_, 20>(fp, f_sb, dS_gap, S_gap, bins, bin_sb, weights, w_sb, dweights, partial, B, HW, C, G, pool, CB, st); \
-    default: return -1000;                                                                                          \
-    }
-    if (dtype == GVCNN_F32) { GVCNN_GBW_CASE(float) }
-    if (dtype == GVCNN_BF16) { GVCNN_GBW_CASE(__nv_bfloat16) }
-    if (dtype == GVCNN_F16) { GVCNN_GBW_CASE(__half) }
-    return GVCNN_E_BAD_DTYPE;
-#undef GVCNN_GBW_CASE
+    if (CB == 0 || G > 255) return kNotApplicable;
+    return with_dtype(dtype, [&](auto tag) {
+        return with_views(kFastViews, V, [&](auto v) {
+            return launch_gbw_v<typename decltype(tag)::type, v>(fp, f_sb, dS_gap, S_gap, bins, bin_sb, weights, w_sb,
+                                                                 dweights, partial, B, HW, C, G, pool, CB, st);
+        });
+    });
 }
 
 // dmaps[b, v, p, c] = RN(RN(dx[b, v] * W[v, c]) / HW): a thread computes its E channels once and stores them at every
@@ -283,38 +271,23 @@ gap_score_bwd_cf_kernel(const float *__restrict__ dx, const float *__restrict__ 
     }
 }
 
-// cf: channels-first dmaps.  Returns -1000 when C (channel-last) or C * HW (channels-first) is not a multiple of the
+// cf: channels-first dmaps.  Returns kNotApplicable when C (channel-last) or C * HW (channels-first) is not a multiple of the
 // 16-byte vector
 int launch_gap_score_bwd(const float *dx, const float *W, const ViewPtrs &dp, int64_t d_sb, int B, int V, int HW, int C,
                          int dtype, bool cf, cudaStream_t st)
 {
     const int E = dtype == GVCNN_F32 ? 4 : 8;
-    if (cf ? ((int64_t)C * HW) % E != 0 : C % E != 0) return -1000;
+    if (cf ? ((int64_t)C * HW) % E != 0 : C % E != 0) return kNotApplicable;
     const int64_t items = (int64_t)B * V;
     if (items > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
-    cudaError_t err;
-    if (cf) {
-        const dim3 grid((unsigned)items);
-        if (dtype == GVCNN_F32)
-            err = launch_pdl(gap_score_bwd_cf_kernel<float>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
-        else if (dtype == GVCNN_BF16)
-            err = launch_pdl(gap_score_bwd_cf_kernel<__nv_bfloat16>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
-        else if (dtype == GVCNN_F16)
-            err = launch_pdl(gap_score_bwd_cf_kernel<__half>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
-        else
-            return GVCNN_E_BAD_DTYPE;
-        return (int)err;
-    }
-    const dim3 grid((unsigned)items, (unsigned)((C / E + 255) / 256));
-    if (dtype == GVCNN_F32)
-        err = launch_pdl(gap_score_bwd_kernel<float>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
-    else if (dtype == GVCNN_BF16)
-        err = launch_pdl(gap_score_bwd_kernel<__nv_bfloat16>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
-    else if (dtype == GVCNN_F16)
-        err = launch_pdl(gap_score_bwd_kernel<__half>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
-    else
-        return GVCNN_E_BAD_DTYPE;
-    return (int)err;
+    return with_dtype(dtype, [&](auto tag) {
+        using T = typename decltype(tag)::type;
+        if (cf)
+            return (int)launch_pdl(gap_score_bwd_cf_kernel<T>, dim3((unsigned)items), dim3(256), 0, st, dx, W, dp, d_sb, V,
+                                   HW, C);
+        const dim3 grid((unsigned)items, (unsigned)((C / E + 255) / 256));
+        return (int)launch_pdl(gap_score_bwd_kernel<T>, grid, dim3(256), 0, st, dx, W, dp, d_sb, V, HW, C);
+    });
 }
 
 }  // namespace gvcnn

@@ -204,28 +204,18 @@ int launch_group_weight_grad(const ViewPtrs &fp, int64_t f_sb, const void *dS, c
                              int64_t bin_sb, const float *weights, int64_t w_sb, float *dweights, int B, int V,
                              int64_t D, int G, int pool, int dtype, bool aligned16, cudaStream_t st)
 {
-#define GVCNN_LAUNCH_GWG(T_, POOL_)                                                                              \
-    do {                                                                                                         \
-        if (aligned16 && D % Elem<T_>::kVec == 0)                                                                \
-            group_weight_grad_kernel<T_, POOL_, true><<<B, 256, 0, st>>>(                                        \
-                fp, f_sb, static_cast<const T_ *>(dS), static_cast<const T_ *>(S), bins, bin_sb, weights, w_sb,  \
-                dweights, V, D, G);                                                                              \
-        else                                                                                                     \
-            group_weight_grad_kernel<T_, POOL_, false><<<B, 256, 0, st>>>(                                       \
-                fp, f_sb, static_cast<const T_ *>(dS), static_cast<const T_ *>(S), bins, bin_sb, weights, w_sb,  \
-                dweights, V, D, G);                                                                              \
-    } while (0)
-    if (dtype == GVCNN_F32) {
-        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_GWG(float, GVCNN_POOL_MAX); else GVCNN_LAUNCH_GWG(float, GVCNN_POOL_MEAN);
-    } else if (dtype == GVCNN_BF16) {
-        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_GWG(__nv_bfloat16, GVCNN_POOL_MAX); else GVCNN_LAUNCH_GWG(__nv_bfloat16, GVCNN_POOL_MEAN);
-    } else if (dtype == GVCNN_F16) {
-        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_GWG(__half, GVCNN_POOL_MAX); else GVCNN_LAUNCH_GWG(__half, GVCNN_POOL_MEAN);
-    } else {
-        return GVCNN_E_BAD_DTYPE;
-    }
-#undef GVCNN_LAUNCH_GWG
-    return (int)cudaGetLastError();
+    const int rc = with_dtype(dtype, [&](auto tag) {
+        using T = typename decltype(tag)::type;
+        return with_pool(pool, false, [&](auto pool_c, auto) {
+            return with_flag(aligned16 && D % Elem<T>::kVec == 0, [&](auto vec_c) {
+                group_weight_grad_kernel<T, pool_c, vec_c><<<B, 256, 0, st>>>(
+                    fp, f_sb, static_cast<const T *>(dS), static_cast<const T *>(S), bins, bin_sb, weights, w_sb, dweights,
+                    V, D, G);
+                return 0;
+            });
+        });
+    });
+    return rc ? rc : (int)cudaGetLastError();
 }
 
 int launch_score_weight_bwd(const float *dweights, const int32_t *bins, const float *x, float *dx, int rows, int V,
@@ -243,21 +233,15 @@ int launch_view_score_bwd(const ViewPtrs &rp, int64_t r_sb, const float *dx, con
     float *partial = workspace;
     float *pbias = workspace + (size_t)NS * V * C;
     const dim3 grid(V, NS);
-#define GVCNN_LAUNCH_VSB(T_)                                                                                   \
-    do {                                                                                                       \
-        if (aligned16 && C % Elem<T_>::kVec == 0)                                                              \
-            view_score_bwd_partial_kernel<T_, true><<<grid, 256, 0, st>>>(rp, r_sb, dx, W, partial, pbias, drp, \
-                                                                         dr_sb, want_dr, B, V, C, NS);         \
-        else                                                                                                   \
-            view_score_bwd_partial_kernel<T_, false><<<grid, 256, 0, st>>>(rp, r_sb, dx, W, partial, pbias, drp, \
-                                                                          dr_sb, want_dr, B, V, C, NS);        \
-    } while (0)
-    if (dtype == GVCNN_F32) GVCNN_LAUNCH_VSB(float);
-    else if (dtype == GVCNN_BF16) GVCNN_LAUNCH_VSB(__nv_bfloat16);
-    else if (dtype == GVCNN_F16) GVCNN_LAUNCH_VSB(__half);
-    else return GVCNN_E_BAD_DTYPE;
-#undef GVCNN_LAUNCH_VSB
-    int rc = (int)cudaGetLastError();
+    int rc = with_dtype(dtype, [&](auto tag) {
+        using T = typename decltype(tag)::type;
+        return with_flag(aligned16 && C % Elem<T>::kVec == 0, [&](auto vec_c) {
+            view_score_bwd_partial_kernel<T, vec_c><<<grid, 256, 0, st>>>(rp, r_sb, dx, W, partial, pbias, drp, dr_sb,
+                                                                          want_dr, B, V, C, NS);
+            return 0;
+        });
+    });
+    if (!rc) rc = (int)cudaGetLastError();
     if (rc) return rc;
     const int64_t n = (int64_t)V * C;
     view_score_bwd_final_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(partial, pbias, dW, dbias, V, C, NS);

@@ -173,23 +173,15 @@ static int launch_bwd_t(const void *dS, const int32_t *bins, int64_t bin_sb, con
     const int64_t tiles = (D + td - 1) / td;
     if ((int64_t)B * tiles > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
     const unsigned grid = (unsigned)(B * tiles);
-#define GVCNN_LAUNCH_BWD(VEC_, POOL_, GRP_)                                                                  \
-    pool_fuse_bwd_kernel<T, VEC_, POOL_, GRP_><<<grid, nt, smem, st>>>(static_cast<const T *>(dS), bins, bin_sb, \
-                                                                       mask, weights, w_sb, gp, g_sb, status, B, \
-                                                                       V, D, G,                                  \
-                                                                       (int)tiles)
-#define GVCNN_LAUNCH_BWD_P(VEC_, GRP_)                                                                         \
-    do {                                                                                                       \
-        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_BWD(VEC_, GVCNN_POOL_MAX, GRP_);                              \
-        else GVCNN_LAUNCH_BWD(VEC_, GVCNN_POOL_MEAN, GRP_);                                                    \
-    } while (0)
-    if (grp) {
-        if (vec) GVCNN_LAUNCH_BWD_P(true, true); else GVCNN_LAUNCH_BWD_P(false, true);
-    } else {
-        if (vec) GVCNN_LAUNCH_BWD_P(true, false); else GVCNN_LAUNCH_BWD_P(false, false);
-    }
-#undef GVCNN_LAUNCH_BWD_P
-#undef GVCNN_LAUNCH_BWD
+    with_pool(pool, false, [&](auto pool_c, auto) {
+        return with_flag(vec, [&](auto vec_c) {
+            return with_flag(grp, [&](auto grp_c) {
+                pool_fuse_bwd_kernel<T, vec_c, pool_c, grp_c><<<grid, nt, smem, st>>>(
+                    static_cast<const T *>(dS), bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, (int)tiles);
+                return 0;
+            });
+        });
+    });
     return (int)cudaGetLastError();
 }
 
@@ -197,16 +189,11 @@ int launch_pool_fuse_bwd(const void *dS, const int32_t *bins, int64_t bin_sb, co
                          const float *weights, int64_t w_sb, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
                          int pool, int dtype, bool aligned16, cudaStream_t st)
 {
-    if (dtype == GVCNN_F32)
-        return launch_bwd_t<float>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool,
-                                   aligned16 && D % 4 == 0, st);
-    if (dtype == GVCNN_BF16)
-        return launch_bwd_t<__nv_bfloat16>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool,
-                                           aligned16 && D % 8 == 0, st);
-    if (dtype == GVCNN_F16)
-        return launch_bwd_t<__half>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool,
-                                    aligned16 && D % 8 == 0, st);
-    return GVCNN_E_BAD_DTYPE;
+    return with_dtype(dtype, [&](auto tag) {
+        using T = typename decltype(tag)::type;
+        return launch_bwd_t<T>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool,
+                               aligned16 && D % Elem<T>::kVec == 0, st);
+    });
 }
 
 // gvcnn_view_pooling_bwd, generic path: any V, unaligned or short rows, the scalar layout
@@ -214,16 +201,11 @@ int launch_view_pooling_bwd(const void *dP, const int32_t *bins, int64_t bin_sb,
                             const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
                             int pool, int dtype, bool aligned16, cudaStream_t st)
 {
-    if (dtype == GVCNN_F32)
-        return launch_bwd_t<float>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool,
-                                   aligned16 && D % 4 == 0, st, true);
-    if (dtype == GVCNN_BF16)
-        return launch_bwd_t<__nv_bfloat16>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool,
-                                           aligned16 && D % 8 == 0, st, true);
-    if (dtype == GVCNN_F16)
-        return launch_bwd_t<__half>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool,
-                                    aligned16 && D % 8 == 0, st, true);
-    return GVCNN_E_BAD_DTYPE;
+    return with_dtype(dtype, [&](auto tag) {
+        using T = typename decltype(tag)::type;
+        return launch_bwd_t<T>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool,
+                               aligned16 && D % Elem<T>::kVec == 0, st, true);
+    });
 }
 
 }  // namespace gvcnn

@@ -332,10 +332,10 @@ pool_fuse_bwd_fast_kernel(const T *__restrict__ dS, const int32_t *__restrict__ 
     }  // units
 }
 
-template <typename T, int V, int NT = 256>
+template <typename T, int V, int NT, bool GAP, bool WTS, bool GRP, bool CF>
 static int launch_bwd_fast_v(const void *dS, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
                              const float *weights, int64_t w_sb, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int64_t D, int G, int pool,
-                             cudaStream_t st, int gapC = 0, int gapHW = 0, bool grp = false, bool cf = false)
+                             cudaStream_t st, int gapC = 0, int gapHW = 0)
 {
     constexpr int E = Elem<T>::kVec;
     const int64_t td = (int64_t)NT * E;
@@ -346,65 +346,40 @@ static int launch_bwd_fast_v(const void *dS, const int32_t *bins, int64_t bin_sb
     // configs[1], 10.3 vs 12.8 us at 512 shapes (profiles/r03_bwd_units_per_cta_ab.jsonl) - so only UPC = 1 is built
     constexpr int upc = 1;
     const unsigned grid = (unsigned)((units + upc - 1) / upc);
-    cudaError_t err;
-#define GVCNN_LAUNCH_BF(POOL_, GAP_, WTS_, UPC_, GRP_, CF_)                                                   \
-    err = launch_pdl(pool_fuse_bwd_fast_kernel<T, POOL_, V, NT, GAP_, WTS_, UPC_, GRP_, CF_>, dim3(grid), dim3(NT), 0, st, \
-                     static_cast<const T *>(dS), bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G,   \
-                     (int)tiles, gapC, gapHW, units)
-#define GVCNN_LAUNCH_BF_P(GAP_, WTS_, GRP_, CF_)                                                              \
-    do {                                                                                                      \
-        if (pool == GVCNN_POOL_MAX) GVCNN_LAUNCH_BF(GVCNN_POOL_MAX, GAP_, WTS_, upc, GRP_, CF_);              \
-        else GVCNN_LAUNCH_BF(GVCNN_POOL_MEAN, GAP_, WTS_, upc, GRP_, CF_);                                    \
-    } while (0)
-    if (grp) {  // per-group gradients dP [G, B, D] (gvcnn_view_pooling_bwd)
-        GVCNN_LAUNCH_BF_P(false, false, true, false);
-    } else if (gapC > 0 && cf) {
-        if (weights) return -1000;
-        GVCNN_LAUNCH_BF_P(true, false, false, true);
-    } else if (gapC > 0) {
-        if (weights) GVCNN_LAUNCH_BF_P(true, true, false, false);  // paper mode: caller-supplied weights
-        else GVCNN_LAUNCH_BF_P(true, false, false, false);
-    } else if (weights) {
-        GVCNN_LAUNCH_BF_P(false, true, false, false);
-    } else {
-        GVCNN_LAUNCH_BF_P(false, false, false, false);
-    }
-#undef GVCNN_LAUNCH_BF_P
-#undef GVCNN_LAUNCH_BF
-    if (err != cudaSuccess) return (int)err;
-    return (int)cudaGetLastError();
+    const int rc = with_pool(pool, false, [&](auto pool_c, auto) {
+        return (int)launch_pdl(pool_fuse_bwd_fast_kernel<T, pool_c, V, NT, GAP, WTS, upc, GRP, CF>, dim3(grid), dim3(NT), 0,
+                               st, static_cast<const T *>(dS), bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D,
+                               G, (int)tiles, gapC, gapHW, units);
+    });
+    return rc ? rc : (int)cudaGetLastError();
 }
 
+// grp: per-group gradients dP [G, B, D] (gvcnn_view_pooling_bwd), no weights
 template <typename T>
 static int launch_bwd_fast_t(const void *dS, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
                              const float *weights, int64_t w_sb, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
-                             int pool, cudaStream_t st, bool grp = false)
+                             int pool, cudaStream_t st, bool grp)
 {
-    if (D < 256 * Elem<T>::kVec) {
+    constexpr int E = Elem<T>::kVec;
+    if (D % E) return kNotApplicable;
+    return with_flag(D >= 256 * E, [&](auto wide) {
         // 16-bit types at D = 1024: one 128-thread tile per shape (see pool_fwd_ring.cu); anything shorter: generic kernel
-        if constexpr (Elem<T>::kVec == 8) {
-            if (D < 128 * Elem<T>::kVec) return -1000;
-            switch (V) {
-            case 4: return launch_bwd_fast_v<T, 4, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
-            case 6: return launch_bwd_fast_v<T, 6, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
-            case 8: return launch_bwd_fast_v<T, 8, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
-            case 12: return launch_bwd_fast_v<T, 12, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
-            case 16: return launch_bwd_fast_v<T, 16, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
-            case 20: return launch_bwd_fast_v<T, 20, 128>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
-            default: return -1000;
-            }
+        if constexpr (!wide && E != 8) {
+            return kNotApplicable;
+        } else {
+            if (!wide && D < 128 * E) return kNotApplicable;
+            constexpr int NT = wide ? 256 : 128;
+            return with_views(kFastViews, V, [&](auto v) {
+                if (grp)
+                    return launch_bwd_fast_v<T, v, NT, false, false, true, false>(dS, bins, bin_sb, mask, weights, w_sb, gp,
+                                                                                g_sb, status, B, D, G, pool, st);
+                return with_flag(weights != nullptr, [&](auto wts) {
+                    return launch_bwd_fast_v<T, v, NT, false, wts, false, false>(dS, bins, bin_sb, mask, weights, w_sb, gp,
+                                                                               g_sb, status, B, D, G, pool, st);
+                });
+            });
         }
-        return -1000;
-    }
-    switch (V) {
-    case 4: return launch_bwd_fast_v<T, 4>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
-    case 6: return launch_bwd_fast_v<T, 6>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
-    case 8: return launch_bwd_fast_v<T, 8>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
-    case 12: return launch_bwd_fast_v<T, 12>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
-    case 16: return launch_bwd_fast_v<T, 16>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
-    case 20: return launch_bwd_fast_v<T, 20>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, 0, 0, grp);
-    default: return -1000;
-    }
+    });
 }
 
 // GAP-folded backward: dOut [B, C] -> dF; same applicability as the forward GAP kernel plus the fast-kernel V set.
@@ -416,58 +391,42 @@ int launch_pool_fuse_gap_bwd(const void *dOut, const int32_t *bins, int64_t bin_
 {
     const int64_t D = (int64_t)HW * C;
     const int td = 256 * (dtype == GVCNN_F32 ? 4 : 8);
-    if (cf ? (weights != nullptr || D % (dtype == GVCNN_F32 ? 4 : 8) != 0) : C % td != 0) return -1000;
-#define GVCNN_GAPB_CASE(T_)                                                                                   \
-    switch (V) {                                                                                              \
-    case 4: return launch_bwd_fast_v<T_, 4>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW, false, cf);   \
-    case 6: return launch_bwd_fast_v<T_, 6>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW, false, cf);   \
-    case 8: return launch_bwd_fast_v<T_, 8>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW, false, cf);   \
-    case 12: return launch_bwd_fast_v<T_, 12>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW, false, cf); \
-    case 16: return launch_bwd_fast_v<T_, 16>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW, false, cf); \
-    case 20: return launch_bwd_fast_v<T_, 20>(dOut, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, D, G, pool, st, C, HW, false, cf); \
-    default: return -1000;                                                                                    \
-    }
-    if (dtype == GVCNN_F32) { GVCNN_GAPB_CASE(float) }
-    if (dtype == GVCNN_BF16) { GVCNN_GAPB_CASE(__nv_bfloat16) }
-    if (dtype == GVCNN_F16) { GVCNN_GAPB_CASE(__half) }
-    return GVCNN_E_BAD_DTYPE;
-#undef GVCNN_GAPB_CASE
+    if (cf ? (weights != nullptr || D % (dtype == GVCNN_F32 ? 4 : 8) != 0) : C % td != 0) return kNotApplicable;
+    return with_dtype(dtype, [&](auto tag) {
+        using T = typename decltype(tag)::type;
+        return with_views(kFastViews, V, [&](auto v) {
+            if (cf)
+                return launch_bwd_fast_v<T, v, 256, true, false, false, true>(dOut, bins, bin_sb, mask, weights, w_sb, gp,
+                                                                            g_sb, status, B, D, G, pool, st, C, HW);
+            return with_flag(weights != nullptr, [&](auto wts) {  // paper mode: caller-supplied weights
+                return launch_bwd_fast_v<T, v, 256, true, wts, false, false>(dOut, bins, bin_sb, mask, weights, w_sb, gp,
+                                                                           g_sb, status, B, D, G, pool, st, C, HW);
+            });
+        });
+    });
 }
 
-// returns -1000 when this fast path does not apply
+// returns kNotApplicable when this fast path does not apply
 int launch_pool_fuse_bwd_fast(const void *dS, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
                               const float *weights, int64_t w_sb, const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
                               int pool, int dtype, cudaStream_t st)
 {
-    if (dtype == GVCNN_F32) {
-        if (D % 4) return -1000;
-        return launch_bwd_fast_t<float>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool, st);
-    }
-    if (D % 8) return -1000;
-    if (dtype == GVCNN_BF16)
-        return launch_bwd_fast_t<__nv_bfloat16>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool, st);
-    if (dtype == GVCNN_F16)
-        return launch_bwd_fast_t<__half>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B, V, D, G, pool, st);
-    return GVCNN_E_BAD_DTYPE;
+    return with_dtype(dtype, [&](auto tag) {
+        return launch_bwd_fast_t<typename decltype(tag)::type>(dS, bins, bin_sb, mask, weights, w_sb, gp, g_sb, status, B,
+                                                               V, D, G, pool, st, false);
+    });
 }
 
 // gvcnn_view_pooling_bwd, fast path: dP [G, B, D] -> dF.  Same applicability as launch_pool_fuse_bwd_fast;
-// returns -1000 when it does not apply
+// returns kNotApplicable when it does not apply
 int launch_view_pooling_bwd_fast(const void *dP, const int32_t *bins, int64_t bin_sb, const uint8_t *mask,
                                  const ViewPtrs &gp, int64_t g_sb, int32_t *status, int B, int V, int64_t D, int G,
                                  int pool, int dtype, cudaStream_t st)
 {
-    if (dtype == GVCNN_F32) {
-        if (D % 4) return -1000;
-        return launch_bwd_fast_t<float>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool, st, true);
-    }
-    if (D % 8) return -1000;
-    if (dtype == GVCNN_BF16)
-        return launch_bwd_fast_t<__nv_bfloat16>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool, st,
-                                                true);
-    if (dtype == GVCNN_F16)
-        return launch_bwd_fast_t<__half>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B, V, D, G, pool, st, true);
-    return GVCNN_E_BAD_DTYPE;
+    return with_dtype(dtype, [&](auto tag) {
+        return launch_bwd_fast_t<typename decltype(tag)::type>(dP, bins, bin_sb, mask, nullptr, 0, gp, g_sb, status, B,
+                                                               V, D, G, pool, st, true);
+    });
 }
 
 }  // namespace gvcnn

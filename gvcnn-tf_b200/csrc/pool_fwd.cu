@@ -393,30 +393,18 @@ static int launch_fwd_t(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, i
         const int64_t tilesv = (D + tdv - 1) / tdv;
         if ((int64_t)B * tilesv > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
         const size_t smemv = (size_t)2 * kChunkViews * ntv * 16;  // 64 KB (32 KB): 3 (6) CTAs per SM
-        const bool wm = (mask != nullptr) && pool == GVCNN_POOL_MAX;
-        cudaError_t e2 = cudaSuccess;
-#define GVCNN_LAUNCH_CHUNKED_NT(POOL_, MASK_, NT_)                                                             \
-    do {                                                                                                       \
-        auto kern = pool_fuse_fwd_chunked_kernel<T, POOL_, MASK_, NT_>;                                        \
-        e2 = ensure_dyn_smem<pool_fuse_fwd_chunked_kernel<T, POOL_, MASK_, NT_>>((int)smemv);                  \
-        if (e2 == cudaSuccess)                                                                                 \
-            kern<<<(unsigned)(B * tilesv), NT_, smemv, st>>>(fp, f_sb, bins, bin_sb, static_cast<T *>(S),       \
-                                                            static_cast<T *>(Pout), mask, weights, w_sb, status, \
-                                                            B, V, D, G, fill, (int)tilesv);                    \
-    } while (0)
-#define GVCNN_LAUNCH_CHUNKED(POOL_, MASK_)                                                                     \
-    do {                                                                                                       \
-        if (ntv == 256) GVCNN_LAUNCH_CHUNKED_NT(POOL_, MASK_, 256); else GVCNN_LAUNCH_CHUNKED_NT(POOL_, MASK_, 128); \
-    } while (0)
-        if (pool == GVCNN_POOL_MAX) {
-            if (wm) GVCNN_LAUNCH_CHUNKED(GVCNN_POOL_MAX, true); else GVCNN_LAUNCH_CHUNKED(GVCNN_POOL_MAX, false);
-        } else {
-            GVCNN_LAUNCH_CHUNKED(GVCNN_POOL_MEAN, false);
-        }
-#undef GVCNN_LAUNCH_CHUNKED
-#undef GVCNN_LAUNCH_CHUNKED_NT
-        if (e2 != cudaSuccess) return (int)e2;
-        return (int)cudaGetLastError();
+        const int rc = with_pool(pool, mask != nullptr, [&](auto pool_c, auto mask_c) {
+            return with_flag(ntv == 256, [&](auto wide) {
+                constexpr auto kern = pool_fuse_fwd_chunked_kernel<T, pool_c, mask_c, wide ? 256 : 128>;
+                const cudaError_t e = ensure_dyn_smem<kern>((int)smemv);
+                if (e == cudaSuccess)
+                    kern<<<(unsigned)(B * tilesv), ntv, smemv, st>>>(fp, f_sb, bins, bin_sb, static_cast<T *>(S),
+                                                                    static_cast<T *>(Pout), mask, weights, w_sb, status,
+                                                                    B, V, D, G, fill, (int)tilesv);
+                return (int)e;
+            });
+        });
+        return rc ? rc : (int)cudaGetLastError();
     }
     const int E = vec ? Elem<T>::kVec : 1;
     const int nt = pick_threads(V, D, E, sizeof(T), 56 * 1024);
@@ -425,52 +413,36 @@ static int launch_fwd_t(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, i
     const int64_t td = (int64_t)nt * E;
     const int64_t tiles = (D + td - 1) / td;
     if ((int64_t)B * tiles > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
-    const bool bulk = vec && variant != 2;
-    const bool want_mask = (mask != nullptr) && pool == GVCNN_POOL_MAX;
-    cudaError_t err = cudaSuccess;
-#define GVCNN_LAUNCH_FWD(VEC_, POOL_, MASK_, BULK_)                                                        \
-    do {                                                                                                   \
-        auto kern = pool_fuse_fwd_kernel<T, VEC_, POOL_, MASK_, BULK_>;                                    \
-        if (smem + 8192 > 48 * 1024)                                                                            \
-            err = ensure_dyn_smem<pool_fuse_fwd_kernel<T, VEC_, POOL_, MASK_, BULK_>>((int)smem);         \
-        if (err == cudaSuccess)                                                                            \
-            kern<<<(unsigned)(B * tiles), nt, smem, st>>>(fp, f_sb, bins, bin_sb, static_cast<T *>(S),      \
-                                                          static_cast<T *>(Pout), mask, weights, w_sb,     \
-                                                          status, B, V, D, G, fill, (int)tiles);           \
-    } while (0)
-    if (vec) {
-        if (pool == GVCNN_POOL_MAX) {
-            if (want_mask) { if (bulk) GVCNN_LAUNCH_FWD(true, GVCNN_POOL_MAX, true, true); else GVCNN_LAUNCH_FWD(true, GVCNN_POOL_MAX, true, false); }
-            else           { if (bulk) GVCNN_LAUNCH_FWD(true, GVCNN_POOL_MAX, false, true); else GVCNN_LAUNCH_FWD(true, GVCNN_POOL_MAX, false, false); }
-        } else {
-            if (bulk) GVCNN_LAUNCH_FWD(true, GVCNN_POOL_MEAN, false, true); else GVCNN_LAUNCH_FWD(true, GVCNN_POOL_MEAN, false, false);
-        }
-    } else {
-        if (pool == GVCNN_POOL_MAX) {
-            if (want_mask) GVCNN_LAUNCH_FWD(false, GVCNN_POOL_MAX, true, false); else GVCNN_LAUNCH_FWD(false, GVCNN_POOL_MAX, false, false);
-        } else {
-            GVCNN_LAUNCH_FWD(false, GVCNN_POOL_MEAN, false, false);
-        }
-    }
-#undef GVCNN_LAUNCH_FWD
-    if (err != cudaSuccess) return (int)err;
-    return (int)cudaGetLastError();
+    const int rc = with_pool(pool, mask != nullptr, [&](auto pool_c, auto mask_c) {
+        auto launch = [&](auto vec_c, auto bulk_c) {
+            constexpr auto kern = pool_fuse_fwd_kernel<T, vec_c, pool_c, mask_c, bulk_c>;
+            cudaError_t e = cudaSuccess;
+            if (smem + 8192 > 48 * 1024) e = ensure_dyn_smem<kern>((int)smem);
+            if (e == cudaSuccess)
+                kern<<<(unsigned)(B * tiles), nt, smem, st>>>(fp, f_sb, bins, bin_sb, static_cast<T *>(S),
+                                                              static_cast<T *>(Pout), mask, weights, w_sb, status, B, V,
+                                                              D, G, fill, (int)tiles);
+            return (int)e;
+        };
+        return with_flag(vec, [&](auto vec_c) {
+            if constexpr (vec_c)  // bulk = vec && variant != 2
+                return with_flag(variant != 2, [&](auto bulk_c) { return launch(vec_c, bulk_c); });
+            else
+                return launch(vec_c, std::false_type{});
+        });
+    });
+    return rc ? rc : (int)cudaGetLastError();
 }
 
 int launch_pool_fuse_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb, void *S,
                          void *Pout, uint8_t *mask, const float *weights, int64_t w_sb, int32_t *status, int B, int V, int64_t D, int G, int pool, float fill,
                          int dtype, bool aligned16, int variant, cudaStream_t st)
 {
-    if (dtype == GVCNN_F32)
-        return launch_fwd_t<float>(fp, f_sb, bins, bin_sb, S, Pout, mask, weights, w_sb, status, B, V, D, G, pool, fill,
-                                   aligned16 && D % 4 == 0, variant, st);
-    if (dtype == GVCNN_BF16)
-        return launch_fwd_t<__nv_bfloat16>(fp, f_sb, bins, bin_sb, S, Pout, mask, weights, w_sb, status, B, V, D, G, pool,
-                                           fill, aligned16 && D % 8 == 0, variant, st);
-    if (dtype == GVCNN_F16)
-        return launch_fwd_t<__half>(fp, f_sb, bins, bin_sb, S, Pout, mask, weights, w_sb, status, B, V, D, G, pool, fill,
-                                    aligned16 && D % 8 == 0, variant, st);
-    return GVCNN_E_BAD_DTYPE;
+    return with_dtype(dtype, [&](auto tag) {
+        using T = typename decltype(tag)::type;
+        return launch_fwd_t<T>(fp, f_sb, bins, bin_sb, S, Pout, mask, weights, w_sb, status, B, V, D, G, pool, fill,
+                               aligned16 && D % Elem<T>::kVec == 0, variant, st);
+    });
 }
 
 }  // namespace gvcnn

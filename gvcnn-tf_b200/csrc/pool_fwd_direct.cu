@@ -95,82 +95,45 @@ pool_fuse_fwd_direct_kernel(const ViewPtrs fp, const int64_t f_sb, const int32_t
     }
 }
 
-template <typename T, int V, int NT>
-static int launch_direct_v(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb, void *S, uint8_t *mask,
-                           int32_t *status, int B, int64_t D, int G, int pool, float fill, bool early, cudaStream_t st)
-{
-    constexpr int E = Elem<T>::kVec;
-    const int64_t td = (int64_t)NT * E;
-    const int64_t tps = (D + td - 1) / td;
-    if ((int64_t)B * tps > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
-    const unsigned grid = (unsigned)(B * tps);
-    const size_t smem = (size_t)V * NT * 16;
-    const bool want_mask = (mask != nullptr) && pool == GVCNN_POOL_MAX;
-    cudaError_t err = cudaSuccess;
-#define GVCNN_LAUNCH_DIRECT_E(POOL_, MASK_, EARLY_)                                                          \
-    do {                                                                                                     \
-        err = ensure_dyn_smem<pool_fuse_fwd_direct_kernel<T, POOL_, MASK_, V, NT, EARLY_>>((int)smem);       \
-        if (err == cudaSuccess)                                                                              \
-            err = launch_pdl(pool_fuse_fwd_direct_kernel<T, POOL_, MASK_, V, NT, EARLY_>, dim3(grid), dim3(NT), smem, st, \
-                             fp, f_sb, bins, bin_sb, static_cast<T *>(S), mask, status, B, D, G, fill, (int)tps); \
-    } while (0)
-#define GVCNN_LAUNCH_DIRECT(POOL_, MASK_)                                                                    \
-    do {                                                                                                     \
-        if (early) GVCNN_LAUNCH_DIRECT_E(POOL_, MASK_, true); else GVCNN_LAUNCH_DIRECT_E(POOL_, MASK_, false); \
-    } while (0)
-    if (pool == GVCNN_POOL_MAX) {
-        if (want_mask) GVCNN_LAUNCH_DIRECT(GVCNN_POOL_MAX, true); else GVCNN_LAUNCH_DIRECT(GVCNN_POOL_MAX, false);
-    } else {
-        GVCNN_LAUNCH_DIRECT(GVCNN_POOL_MEAN, false);
-    }
-#undef GVCNN_LAUNCH_DIRECT
-#undef GVCNN_LAUNCH_DIRECT_E
-    if (err != cudaSuccess) return (int)err;
-    return (int)cudaGetLastError();
-}
-
-template <typename T>
-static int launch_direct_t(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb, void *S, uint8_t *mask,
-                           int32_t *status, int B, int V, int64_t D, int G, int pool, float fill, bool forced, bool early, cudaStream_t st)
-{
-    // 128-thread tiles when the descriptor is one of them long (bf16, D = 1024), 256-thread tiles otherwise
-    const bool narrow = D <= 128 * Elem<T>::kVec;
-    // Measured against the ring in the graph-replayed steps (profiles/r03_fwd_direct_ab.jsonl): ahead at V = 4, 6, 8
-    // everywhere (float32 V = 6, D = 2048: forward step 61.3 -> 54.7 us, training 102.0 -> 97.0) except bf16 with the
-    // tie planes on 256-thread tiles at V < 8 (V = 6: training 58.1 -> 59.1 us, V = 4: 47.1 -> 48.8), which stay on
-    // the ring; at V = 12 the ring wins clearly (69.5 vs 92.2 us), so larger V are not built.
-    if (!forced && mask != nullptr && pool == GVCNN_POOL_MAX && Elem<T>::kVec == 8 && !narrow && V < 8) return -1000;
-#define GVCNN_DIRECT_CASE(V_)                                                                                          \
-    case V_:                                                                                                           \
-        return narrow ? launch_direct_v<T, V_, 128>(fp, f_sb, bins, bin_sb, S, mask, status, B, D, G, pool, fill, early, st)  \
-                      : launch_direct_v<T, V_, 256>(fp, f_sb, bins, bin_sb, S, mask, status, B, D, G, pool, fill, early, st);
-    switch (V) {
-        GVCNN_DIRECT_CASE(4)
-        GVCNN_DIRECT_CASE(6)
-        GVCNN_DIRECT_CASE(8)
-    default: return -1000;
-    }
-#undef GVCNN_DIRECT_CASE
-}
-
-// returns -1000 when this path does not apply (caller weights, V not in {4, 6, 8}, rows not 16-byte multiples)
+// returns kNotApplicable when this path does not apply (V not in {4, 6, 8}, rows not 16-byte multiples)
 int launch_pool_fuse_fwd_direct(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb, void *S,
                                 uint8_t *mask, int32_t *status, int B, int V, int64_t D, int G, int pool, float fill,
                                 int dtype, bool forced, bool f_ready, cudaStream_t st)
 {
     static const int env_early = env_int_once("GVCNN_DIRECT_EARLY", 1);  // A/B knob
     const bool early = f_ready && env_early != 0;
-    if (G > 255) return -1000;
-    if (dtype == GVCNN_F32) {
-        if (D % 4) return -1000;
-        return launch_direct_t<float>(fp, f_sb, bins, bin_sb, S, mask, status, B, V, D, G, pool, fill, forced, early, st);
-    }
-    if (D % 8) return -1000;
-    if (dtype == GVCNN_BF16)
-        return launch_direct_t<__nv_bfloat16>(fp, f_sb, bins, bin_sb, S, mask, status, B, V, D, G, pool, fill, forced, early, st);
-    if (dtype == GVCNN_F16)
-        return launch_direct_t<__half>(fp, f_sb, bins, bin_sb, S, mask, status, B, V, D, G, pool, fill, forced, early, st);
-    return GVCNN_E_BAD_DTYPE;
+    if (G > 255) return kNotApplicable;
+    return with_dtype(dtype, [&](auto tag) {
+        using T = typename decltype(tag)::type;
+        constexpr int E = Elem<T>::kVec;
+        if (D % E) return kNotApplicable;
+        // 128-thread tiles when the descriptor is one of them long (bf16, D = 1024), 256-thread tiles otherwise
+        const bool narrow = D <= 128 * E;
+        // Measured against the ring in the graph-replayed steps (profiles/r03_fwd_direct_ab.jsonl): ahead at V = 4, 6, 8
+        // everywhere (float32 V = 6, D = 2048: forward step 61.3 -> 54.7 us, training 102.0 -> 97.0) except bf16 with the
+        // tie planes on 256-thread tiles at V < 8 (V = 6: training 58.1 -> 59.1 us, V = 4: 47.1 -> 48.8), which stay on
+        // the ring; at V = 12 the ring wins clearly (69.5 vs 92.2 us), so larger V are not built.
+        if (!forced && mask != nullptr && pool == GVCNN_POOL_MAX && E == 8 && !narrow && V < 8) return kNotApplicable;
+        const int rc = with_views(ViewCounts<4, 6, 8>{}, V, [&](auto v) {
+            const int nt = narrow ? 128 : 256;
+            const int64_t tps = (D + (int64_t)nt * E - 1) / ((int64_t)nt * E);
+            if ((int64_t)B * tps > 0x7fffffffLL) return (int)GVCNN_E_BAD_ARG;
+            const size_t smem = (size_t)v * nt * 16;
+            return with_flag(narrow, [&](auto narrow_c) {
+                return with_pool(pool, mask != nullptr, [&](auto pool_c, auto mask_c) {
+                    return with_flag(early, [&](auto early_c) {
+                        constexpr auto kern = pool_fuse_fwd_direct_kernel<T, pool_c, mask_c, v, narrow_c ? 128 : 256, early_c>;
+                        cudaError_t e = ensure_dyn_smem<kern>((int)smem);
+                        if (e == cudaSuccess)
+                            e = launch_pdl(kern, dim3((unsigned)(B * tps)), dim3(nt), smem, st, fp, f_sb, bins, bin_sb,
+                                           static_cast<T *>(S), mask, status, B, D, G, fill, (int)tps);
+                        return (int)e;
+                    });
+                });
+            });
+        });
+        return rc ? rc : (int)cudaGetLastError();
+    });
 }
 
 }  // namespace gvcnn

@@ -228,131 +228,78 @@ pool_fuse_fwd_ring_kernel(const ViewPtrs fp, const int64_t f_sb, const int32_t *
     if (threadIdx.x == 0) GVCNN_RING_MARK(2);
 }
 
-static int ring_sm_count()
-{
-    static int cached = 0;
-    if (cached == 0) {
-        int dev = 0, n = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess ||
-            cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) {
-            cudaGetLastError();
-            return 148;
-        }
-        cached = n;
-    }
-    return cached;
-}
-
 template <typename T, int V, int NCONS, int MINB>
 static int launch_ring_v(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb,
                          const float *weights, int64_t w_sb, void *S, uint8_t *mask, int32_t *status, int B, int64_t D, int G, int pool, float fill,
-                         cudaStream_t st)
+                         int env_stages, int l2_hint, cudaStream_t st)
 {
     constexpr int E = Elem<T>::kVec;
     constexpr size_t stage_bytes = (size_t)V * NCONS * 16;
     // shared memory an SM can give to MINB co-resident CTAs of this kernel (1 KB reserved + ~1.3 KB static each)
     int stages = (int)(((226 * 1024) / MINB - 3 * 1024) / stage_bytes);
     if (stages > 8) stages = 8;
-    static const int env_stages = env_int_once("GVCNN_RING_STAGES", 0);  // tuning knobs for A/B runs, read once
-    static const int env_l2hint = env_int_once("GVCNN_RING_L2HINT", 1);
     if (env_stages >= 2 && env_stages <= stages) stages = env_stages;
-    if (stages < 2) return -1000;
-    const int l2_hint = env_l2hint;
+    if (stages < 2) return kNotApplicable;
     const int64_t td = (int64_t)NCONS * E;
     const int64_t tps = (D + td - 1) / td;
     const int64_t tiles = (int64_t)B * tps;
     if (tiles > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
     const size_t smem = stage_bytes * stages;
-    const int64_t max_grid = (int64_t)ring_sm_count() * MINB;
+    const int64_t max_grid = (int64_t)sm_count() * MINB;
     const int grid = (int)(tiles < max_grid ? tiles : max_grid);
-    const bool want_mask = (mask != nullptr) && pool == GVCNN_POOL_MAX;
-    cudaError_t err = cudaSuccess;
-#define GVCNN_LAUNCH_RING(POOL_, MASK_, WTS_)                                                                \
-    do {                                                                                                     \
-        auto kern = pool_fuse_fwd_ring_kernel<T, POOL_, MASK_, WTS_, V, NCONS, MINB>;                        \
-        err = ensure_dyn_smem<pool_fuse_fwd_ring_kernel<T, POOL_, MASK_, WTS_, V, NCONS, MINB>>((int)smem);  \
-        if (err == cudaSuccess)                                                                              \
-            err = launch_pdl(kern, dim3(grid), dim3(NCONS + kRingProducerThreads), smem, st, fp, f_sb, bins,  \
-                             bin_sb, weights, w_sb, static_cast<T *>(S), mask, status, B, D, G, fill,        \
-                             (int)tps, (int)tiles, stages, l2_hint);                                         \
-    } while (0)
-    if (weights) {
-        if (pool == GVCNN_POOL_MAX) {
-            if (want_mask) GVCNN_LAUNCH_RING(GVCNN_POOL_MAX, true, true); else GVCNN_LAUNCH_RING(GVCNN_POOL_MAX, false, true);
-        } else {
-            GVCNN_LAUNCH_RING(GVCNN_POOL_MEAN, false, true);
-        }
-    } else if (pool == GVCNN_POOL_MAX) {
-        if (want_mask) GVCNN_LAUNCH_RING(GVCNN_POOL_MAX, true, false); else GVCNN_LAUNCH_RING(GVCNN_POOL_MAX, false, false);
-    } else {
-        GVCNN_LAUNCH_RING(GVCNN_POOL_MEAN, false, false);
-    }
-#undef GVCNN_LAUNCH_RING
-    if (err != cudaSuccess) return (int)err;
-    return (int)cudaGetLastError();
+    const int rc = with_pool(pool, mask != nullptr, [&](auto pool_c, auto mask_c) {
+        return with_flag(weights != nullptr, [&](auto wts_c) {
+            constexpr auto kern = pool_fuse_fwd_ring_kernel<T, pool_c, mask_c, wts_c, V, NCONS, MINB>;
+            cudaError_t e = ensure_dyn_smem<kern>((int)smem);
+            if (e == cudaSuccess)
+                e = launch_pdl(kern, dim3(grid), dim3(NCONS + kRingProducerThreads), smem, st, fp, f_sb, bins, bin_sb,
+                               weights, w_sb, static_cast<T *>(S), mask, status, B, D, G, fill, (int)tps, (int)tiles,
+                               stages, l2_hint);
+            return (int)e;
+        });
+    });
+    return rc ? rc : (int)cudaGetLastError();
 }
 
-template <typename T>
-static int launch_ring_t(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb,
-                         const float *weights, int64_t w_sb, void *S, uint8_t *mask, int32_t *status, int B, int V, int64_t D, int G, int pool, float fill,
-                         cudaStream_t st)
-{
-    // the view counts of the reference's configurations (train.py:96 default 6; BASELINE sweep 6/12/20)
-    // plus the other common multi-view rigs (4, 8, 16).  V <= 12: 256-column tiles, two CTAs per SM, 4 slots
-    // each.  V = 16 / 20: a 256-column slot is 64 / 80 KB and only two fit per SM, so tiles are 128 columns
-    // wide and two CTAs share the SM with two slots each - four independent slots drain and refill more
-    // smoothly than two (V = 20: forward 111.7 -> 109.5 us, with tie mask 130.3 -> 126.1 us); for V <= 12 the
-    // narrow tiles (four CTAs per SM) measured the same as the wide ones.
-    if (D < 256 * Elem<T>::kVec) {
-        // descriptors shorter than one 256-column tile.  16-bit types at D = 1024 (a point of the BASELINE sweep) are 128 columns
-        // of 16 bytes: 128-consumer CTAs, narrow slots, deeper ring.  Anything shorter: generic kernel.
 #ifndef GVCNN_NARROW_MINB
 #define GVCNN_NARROW_MINB 4  // CTAs per SM of the narrow (128-consumer) ring for V <= 12: with 12-24 KB tiles two CTAs
                              // (8 consumer warps, 2 producers per SM) left the SM idle between tiles; bf16 V = 6,
                              // D = 1024: 19.3 -> 14.2 us, V = 12 mean: 46.6 -> 30.2 us (A/B builds: -DGVCNN_NARROW_MINB=2)
 #endif
-        if constexpr (Elem<T>::kVec == 8) {
-            if (D < 128 * Elem<T>::kVec) return -1000;
-            switch (V) {
-            case 4: return launch_ring_v<T, 4, 128, GVCNN_NARROW_MINB>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D, G, pool, fill, st);
-            case 6: return launch_ring_v<T, 6, 128, GVCNN_NARROW_MINB>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D, G, pool, fill, st);
-            case 8: return launch_ring_v<T, 8, 128, GVCNN_NARROW_MINB>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D, G, pool, fill, st);
-            case 12: return launch_ring_v<T, 12, 128, GVCNN_NARROW_MINB>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D, G, pool, fill, st);
-            case 16: return launch_ring_v<T, 16, 128, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D, G, pool, fill, st);
-            case 20: return launch_ring_v<T, 20, 128, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D, G, pool, fill, st);
-            default: return -1000;
-            }
-        }
-        return -1000;
-    }
-    switch (V) {
-    case 4: return launch_ring_v<T, 4, 256, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D, G, pool, fill, st);
-    case 6: return launch_ring_v<T, 6, 256, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D, G, pool, fill, st);
-    case 8: return launch_ring_v<T, 8, 256, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D, G, pool, fill, st);  // GVCNN paper: 8 / 12 views
-    case 12: return launch_ring_v<T, 12, 256, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D, G, pool, fill, st);
-    case 16: return launch_ring_v<T, 16, 128, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D, G, pool, fill, st);
-    case 20: return launch_ring_v<T, 20, 128, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D, G, pool, fill, st);
-    default: return -1000;
-    }
-}
 
-// returns -1000 when this fast path does not apply
+// returns kNotApplicable when this fast path does not apply
 int launch_pool_fuse_fwd_ring(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb,
                               const float *weights, int64_t w_sb, void *S, uint8_t *mask, int32_t *status, int B, int V, int64_t D, int G, int pool,
                               float fill, int dtype, cudaStream_t st)
 {
-    if (V > 32 || G > 255) return -1000;
-    if (weights && fill != 0.0f && G > kRingMaxWtsGroups) return -1000;  // weight row per ring slot (RingWts)
-    if (dtype == GVCNN_F32) {
-        if (D % 4) return -1000;
-        return launch_ring_t<float>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, V, D, G, pool, fill, st);
-    }
-    if (D % 8) return -1000;
-    if (dtype == GVCNN_BF16)
-        return launch_ring_t<__nv_bfloat16>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, V, D, G, pool, fill, st);
-    if (dtype == GVCNN_F16)
-        return launch_ring_t<__half>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, V, D, G, pool, fill, st);
-    return GVCNN_E_BAD_DTYPE;
+    static const int env_stages = env_int_once("GVCNN_RING_STAGES", 0);  // tuning knobs for A/B runs, read once
+    static const int env_l2hint = env_int_once("GVCNN_RING_L2HINT", 1);
+    if (V > 32 || G > 255) return kNotApplicable;
+    if (weights && fill != 0.0f && G > kRingMaxWtsGroups) return kNotApplicable;  // weight row per ring slot (RingWts)
+    return with_dtype(dtype, [&](auto tag) {
+        using T = typename decltype(tag)::type;
+        constexpr int E = Elem<T>::kVec;
+        if (D % E) return kNotApplicable;
+        // V <= 12: 256-column tiles, two CTAs per SM, 4 slots each.  V = 16 / 20: a 256-column slot is 64 / 80 KB and
+        // only two fit per SM, so tiles are 128 columns wide and two CTAs share the SM with two slots each - four
+        // independent slots drain and refill more smoothly than two (V = 20: forward 111.7 -> 109.5 us, with tie mask
+        // 130.3 -> 126.1 us); for V <= 12 the narrow tiles (four CTAs per SM) measured the same as the wide ones.
+        return with_flag(D >= 256 * E, [&](auto wide) {
+            // Descriptors shorter than one 256-column tile.  16-bit types at D = 1024 (a point of the BASELINE sweep)
+            // are 128 columns of 16 bytes: 128-consumer CTAs, narrow slots, deeper ring.  Anything shorter: generic kernel.
+            if constexpr (!wide && E != 8) {
+                return kNotApplicable;
+            } else {
+                if (!wide && D < 128 * E) return kNotApplicable;
+                return with_views(kFastViews, V, [&](auto v) {
+                    constexpr int NCONS = wide && v <= 12 ? 256 : 128;
+                    constexpr int MINB = !wide && v <= 12 ? GVCNN_NARROW_MINB : 2;
+                    return launch_ring_v<T, v, NCONS, MINB>(fp, f_sb, bins, bin_sb, weights, w_sb, S, mask, status, B, D,
+                                                            G, pool, fill, env_stages, env_l2hint, st);
+                });
+            }
+        });
+    });
 }
 
 }  // namespace gvcnn

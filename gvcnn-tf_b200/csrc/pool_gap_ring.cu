@@ -322,26 +322,11 @@ pool_fuse_gap_cf_fwd_kernel(const ViewPtrs fp, const int64_t f_sb, const int32_t
     }
 }
 
-static int gap_sm_count()
-{
-    static int cached = 0;
-    if (cached == 0) {
-        int dev = 0, n = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess ||
-            cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) {
-            cudaGetLastError();
-            return 148;
-        }
-        cached = n;
-    }
-    return cached;
-}
-
 // how the positions are split: enough units to fill the machine twice, never more splits than positions
 void gap_split(int B, int CB, int HW, int &nsplit, int &pps)
 {
     const int64_t base = (int64_t)B * CB;
-    int64_t want = (4LL * gap_sm_count() + base - 1) / base;
+    int64_t want = (4LL * sm_count() + base - 1) / base;
     if (want < 1) want = 1;
     if (want > HW) want = HW;
     pps = (int)((HW + want - 1) / want);
@@ -357,43 +342,31 @@ static int launch_gap_v(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, i
     constexpr int E = Elem<T>::kVec;
     constexpr int TD = NCONS * E;
     constexpr size_t stage_bytes = (size_t)V * NCONS * 16;
-    if (C % TD != 0) return -1000;
+    if (C % TD != 0) return kNotApplicable;
     // static shared memory per CTA: ~1.3 KB, plus 2 KB of weight rows with caller-supplied weights
     int stages = (int)(((226 * 1024) / MINB - (weights ? 5 : 3) * 1024) / stage_bytes);
     if (stages > 8) stages = 8;
-    if (stages < 2) return -1000;
+    if (stages < 2) return kNotApplicable;
     const int CB = C / TD;
     int nsplit, pps;
     gap_split(B, CB, HW, nsplit, pps);
     const int64_t units = (int64_t)B * CB * nsplit;
     if (units > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
     const size_t smem = stage_bytes * stages;
-    const int64_t max_grid = (int64_t)gap_sm_count() * MINB;
+    const int64_t max_grid = (int64_t)sm_count() * MINB;
     const int grid = (int)(units < max_grid ? units : max_grid);
-    const bool want_mask = (mask != nullptr) && pool == GVCNN_POOL_MAX;
-    cudaError_t err = cudaSuccess;
-#define GVCNN_LAUNCH_GAP(POOL_, MASK_, WTS_)                                                                  \
-    do {                                                                                                      \
-        auto kern = pool_fuse_gap_fwd_kernel<T, POOL_, MASK_, V, NCONS, MINB, WTS_>;                          \
-        err = ensure_dyn_smem<pool_fuse_gap_fwd_kernel<T, POOL_, MASK_, V, NCONS, MINB, WTS_>>((int)smem);    \
-        if (err == cudaSuccess)                                                                               \
-            err = launch_pdl(kern, dim3(grid), dim3(NCONS + kRingProducerThreads), smem, st, fp, f_sb, bins,  \
-                             bin_sb, partial, mask, status, B, C, HW, G, fill, CB, nsplit, pps, (int)units,   \
-                             stages, weights, w_sb);                                                          \
-    } while (0)
-    if (weights) {
-        if (pool == GVCNN_POOL_MAX) {
-            if (want_mask) GVCNN_LAUNCH_GAP(GVCNN_POOL_MAX, true, true); else GVCNN_LAUNCH_GAP(GVCNN_POOL_MAX, false, true);
-        } else {
-            GVCNN_LAUNCH_GAP(GVCNN_POOL_MEAN, false, true);
-        }
-    } else if (pool == GVCNN_POOL_MAX) {
-        if (want_mask) GVCNN_LAUNCH_GAP(GVCNN_POOL_MAX, true, false); else GVCNN_LAUNCH_GAP(GVCNN_POOL_MAX, false, false);
-    } else {
-        GVCNN_LAUNCH_GAP(GVCNN_POOL_MEAN, false, false);
-    }
-#undef GVCNN_LAUNCH_GAP
-    if (err != cudaSuccess) return (int)err;
+    const int rc = with_pool(pool, mask != nullptr, [&](auto pool_c, auto mask_c) {
+        return with_flag(weights != nullptr, [&](auto wts_c) {
+            constexpr auto kern = pool_fuse_gap_fwd_kernel<T, pool_c, mask_c, V, NCONS, MINB, wts_c>;
+            cudaError_t e = ensure_dyn_smem<kern>((int)smem);
+            if (e == cudaSuccess)
+                e = launch_pdl(kern, dim3(grid), dim3(NCONS + kRingProducerThreads), smem, st, fp, f_sb, bins, bin_sb,
+                               partial, mask, status, B, C, HW, G, fill, CB, nsplit, pps, (int)units, stages, weights,
+                               w_sb);
+            return (int)e;
+        });
+    });
+    if (rc) return rc;
     const int64_t total = (int64_t)B * C;
     gap_finish_kernel<T><<<(unsigned)((total + 255) / 256), 256, 0, st>>>(partial, static_cast<T *>(out), total, C,
                                                                          nsplit, (float)HW);
@@ -409,30 +382,21 @@ size_t gap_workspace_bytes(int B, int C, int HW, int dtype)
     return (size_t)B * nsplit * C * sizeof(float);
 }
 
-// returns -1000 when the shapes are not supported (V not instantiated, C not a multiple of the tile, G > 255, or
+// returns kNotApplicable when the shapes are not supported (V not instantiated, C not a multiple of the tile, G > 255, or
 // caller-supplied weights and more groups than a slot's weight row holds)
 int launch_pool_fuse_gap_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb,
                              const float *weights, int64_t w_sb, void *out, uint8_t *mask, int32_t *status,
                              float *partial, int B, int V, int HW, int C, int G, int pool, float fill, int dtype,
                              cudaStream_t st)
 {
-    if (G > 255) return -1000;
-    if (weights && G > kRingMaxWtsGroups) return -1000;
-#define GVCNN_GAP_CASE(T_)                                                                                    \
-    switch (V) {                                                                                              \
-    case 4: return launch_gap_v<T_, 4, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
-    case 6: return launch_gap_v<T_, 6, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
-    case 8: return launch_gap_v<T_, 8, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
-    case 12: return launch_gap_v<T_, 12, 2>(fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
-    case 16: return launch_gap_v<T_, 16, 1>(fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
-    case 20: return launch_gap_v<T_, 20, 1>(fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st); \
-    default: return -1000;                                                                                    \
-    }
-    if (dtype == GVCNN_F32) { GVCNN_GAP_CASE(float) }
-    if (dtype == GVCNN_BF16) { GVCNN_GAP_CASE(__nv_bfloat16) }
-    if (dtype == GVCNN_F16) { GVCNN_GAP_CASE(__half) }
-    return GVCNN_E_BAD_DTYPE;
-#undef GVCNN_GAP_CASE
+    if (G > 255) return kNotApplicable;
+    if (weights && G > kRingMaxWtsGroups) return kNotApplicable;
+    return with_dtype(dtype, [&](auto tag) {
+        return with_views(kFastViews, V, [&](auto v) {
+            return launch_gap_v<typename decltype(tag)::type, v, v <= 12 ? 2 : 1>(
+                fp, f_sb, bins, bin_sb, weights, w_sb, out, mask, status, partial, B, HW, C, G, pool, fill, st);
+        });
+    });
 }
 
 // Channels-first: K whole channels per unit - K divides C, the runs of K * HW elements start and end 16-byte aligned,
@@ -445,67 +409,48 @@ static int launch_gap_cf_v(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins
     constexpr int NCONS = 256;
     constexpr size_t stage_bytes = (size_t)V * NCONS * 16;
     const size_t budget = (size_t)(226 * 1024) / MINB - 3 * 1024;  // static shared memory per CTA: ~1.3 KB
-    if (budget < 2 * stage_bytes) return -1000;
+    if (budget < 2 * stage_bytes) return kNotApplicable;
     const size_t row_cap = std::min<size_t>(budget - 2 * stage_bytes, 32 * 1024);
     const int ld = HW | 1;
     int K = 0;
     for (int k = std::min(C, NCONS); k >= 1 && K == 0; --k)
         if (C % k == 0 && ((int64_t)k * HW * (int64_t)sizeof(T)) % 16 == 0 && (size_t)k * ld * sizeof(float) <= row_cap)
             K = k;
-    if (K == 0) return -1000;
+    if (K == 0) return kNotApplicable;
     const size_t row_bytes = ((size_t)K * ld * sizeof(float) + 15) & ~(size_t)15;
     int stages = (int)((budget - row_bytes) / stage_bytes);
     if (stages > 8) stages = 8;
     const int64_t units = (int64_t)B * (C / K);
     if (units > 0x7fffffffLL) return GVCNN_E_BAD_ARG;
     const size_t smem = stage_bytes * stages + row_bytes;
-    const int64_t max_grid = (int64_t)gap_sm_count() * MINB;
+    const int64_t max_grid = (int64_t)sm_count() * MINB;
     const int grid = (int)(units < max_grid ? units : max_grid);
-    const bool want_mask = (mask != nullptr) && pool == GVCNN_POOL_MAX;
-    cudaError_t err = cudaSuccess;
-#define GVCNN_LAUNCH_GAP_CF(POOL_, MASK_)                                                                     \
-    do {                                                                                                      \
-        auto kern = pool_fuse_gap_cf_fwd_kernel<T, POOL_, MASK_, V, NCONS, MINB>;                             \
-        err = ensure_dyn_smem<pool_fuse_gap_cf_fwd_kernel<T, POOL_, MASK_, V, NCONS, MINB>>((int)smem);       \
-        if (err == cudaSuccess)                                                                               \
-            err = launch_pdl(kern, dim3(grid), dim3(NCONS + kRingProducerThreads), smem, st, fp, f_sb, bins,  \
-                             bin_sb, static_cast<T *>(out), mask, status, B, C, HW, G, fill, K, (int)units,   \
-                             stages);                                                                         \
-    } while (0)
-    if (pool == GVCNN_POOL_MAX) {
-        if (want_mask) GVCNN_LAUNCH_GAP_CF(GVCNN_POOL_MAX, true); else GVCNN_LAUNCH_GAP_CF(GVCNN_POOL_MAX, false);
-    } else {
-        GVCNN_LAUNCH_GAP_CF(GVCNN_POOL_MEAN, false);
-    }
-#undef GVCNN_LAUNCH_GAP_CF
-    if (err != cudaSuccess) return (int)err;
-    return (int)cudaGetLastError();
+    const int rc = with_pool(pool, mask != nullptr, [&](auto pool_c, auto mask_c) {
+        constexpr auto kern = pool_fuse_gap_cf_fwd_kernel<T, pool_c, mask_c, V, NCONS, MINB>;
+        cudaError_t e = ensure_dyn_smem<kern>((int)smem);
+        if (e == cudaSuccess)
+            e = launch_pdl(kern, dim3(grid), dim3(NCONS + kRingProducerThreads), smem, st, fp, f_sb, bins, bin_sb,
+                           static_cast<T *>(out), mask, status, B, C, HW, G, fill, K, (int)units, stages);
+        return (int)e;
+    });
+    return rc ? rc : (int)cudaGetLastError();
 }
 
-// channels-first maps, the reference's own weights; returns -1000 when the shapes are not supported (V not
+// channels-first maps, the reference's own weights; returns kNotApplicable when the shapes are not supported (V not
 // instantiated, G > 255, or no channel block whose runs align)
 int launch_pool_fuse_gap_cf_fwd(const ViewPtrs &fp, int64_t f_sb, const int32_t *bins, int64_t bin_sb, void *out,
                                 uint8_t *mask, int32_t *status, int B, int V, int HW, int C, int G, int pool, float fill,
                                 int dtype, cudaStream_t st)
 {
-    if (G > 255) return -1000;
+    if (G > 255) return kNotApplicable;
     // V = 12 with the tie planes needs more than the 96 registers two CTAs per SM leave (it spilled): one CTA per SM, which
     // still holds four ring stages
-#define GVCNN_GAP_CF_CASE(T_)                                                                                 \
-    switch (V) {                                                                                              \
-    case 4: return launch_gap_cf_v<T_, 4, 2>(fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st);   \
-    case 6: return launch_gap_cf_v<T_, 6, 2>(fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st);   \
-    case 8: return launch_gap_cf_v<T_, 8, 2>(fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st);   \
-    case 12: return launch_gap_cf_v<T_, 12, 1>(fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st); \
-    case 16: return launch_gap_cf_v<T_, 16, 1>(fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st); \
-    case 20: return launch_gap_cf_v<T_, 20, 1>(fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st); \
-    default: return -1000;                                                                                    \
-    }
-    if (dtype == GVCNN_F32) { GVCNN_GAP_CF_CASE(float) }
-    if (dtype == GVCNN_BF16) { GVCNN_GAP_CF_CASE(__nv_bfloat16) }
-    if (dtype == GVCNN_F16) { GVCNN_GAP_CF_CASE(__half) }
-    return GVCNN_E_BAD_DTYPE;
-#undef GVCNN_GAP_CF_CASE
+    return with_dtype(dtype, [&](auto tag) {
+        return with_views(kFastViews, V, [&](auto v) {
+            return launch_gap_cf_v<typename decltype(tag)::type, v, v <= 8 ? 2 : 1>(
+                fp, f_sb, bins, bin_sb, out, mask, status, B, HW, C, G, pool, fill, st);
+        });
+    });
 }
 
 }  // namespace gvcnn

@@ -394,7 +394,7 @@ int launch_batch_mean_bin_fused(const float *x, float *xsum, float *x_mean, floa
                                 int32_t *status, int B, int V, int G, int multiplier, int edge_ulps, int clamp,
                                 float denom, const CommPeers *peers, int rank, int world, cudaStream_t st)
 {
-    if (V > GVCNN_MAX_VIEWS) return -1000;
+    if (V > GVCNN_MAX_VIEWS) return kNotApplicable;
     cudaError_t err;
     if (peers && world > 1) {
         err = launch_pdl(batch_mean_bin_fused_kernel<true>, dim3(V), dim3(256), 0, st, x, xsum, x_mean, scores, bins,
@@ -408,75 +408,46 @@ int launch_batch_mean_bin_fused(const float *x, float *xsum, float *x_mean, floa
     return (int)cudaGetLastError();
 }
 
-static int score_sm_count()
-{
-    static int cached = 0;
-    if (cached == 0) {
-        int dev = 0, n = 0;
-        if (cudaGetDevice(&dev) != cudaSuccess ||
-            cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) {
-            cudaGetLastError();
-            return 148;
-        }
-        cached = n;
-    }
-    return cached;
-}
-
 template <typename T>
 static int launch_view_score_t(const ViewPtrs &rp, int64_t r_sb, const float *W, const float *bias, float *x,
                                float *xabs, float *scores, int32_t *bins, int32_t *flags, int32_t *status, int B, int V,
-                               int C, int G, bool vec, bool fuse_bin, int edge_ulps, int clamp,
+                               int C, int G, bool vec, bool fuse_bin, int edge_ulps, int clamp, int env_rpw,
                                cudaStream_t st)
 {
+    constexpr int E = Elem<T>::kVec;
     const int64_t rows = (int64_t)B * V;
     const bool bound = fuse_bin ? (flags != nullptr) : (xabs != nullptr);  // the order-sensitivity report is opt-in
-    cudaError_t err = cudaSuccess;
-    if (vec && (C == 8 * 32 * Elem<T>::kVec || C == 4 * 32 * Elem<T>::kVec)) {
+    const dim3 block(kScoreWarps * 32);
+    int rc;
+    if (vec && (C == 8 * 32 * E || C == 4 * 32 * E)) {
         // C_raw = 1024 (block3 of ResNet-v2-50, nets/resnet_v2.py:242) is the reference's only width
         // rows per warp: the smallest multiple of 4 for which all CTAs are resident at once (one wave; the CTAs per SM
         // come from the occupancy calculator for the instantiation).  B = 4096, V = 12, fp32 on 148 SMs: 3 CTAs of 8
         // warps per SM -> 16 rows per warp, 384 CTAs on 444 slots.
-        static const int env_rpw = env_int_once("GVCNN_SCORE_RPW", 0);  // A/B knob: 4 = one butterfly per warp (round 1)
-        const dim3 fblock(kScoreWarps * 32);
-#define GVCNN_LAUNCH_FAST(NB_, BOUND_)                                                                       \
-    do {                                                                                                     \
-        const int64_t warp_slots = (int64_t)score_sm_count() *                                               \
-            resident_ctas<view_score_fast_kernel<T, NB_, BOUND_>>(kScoreWarps * 32) * kScoreWarps;           \
-        int rpw = (int)(kFastRows * ((rows + kFastRows * warp_slots - 1) / (kFastRows * warp_slots)));       \
-        if (env_rpw >= kFastRows && env_rpw % kFastRows == 0) rpw = env_rpw;                                 \
-        const int64_t items = (int64_t)V * ((B + rpw - 1) / rpw);                                            \
-        const dim3 fgrid((unsigned)((items + kScoreWarps - 1) / kScoreWarps));                               \
-        err = launch_pdl(view_score_fast_kernel<T, NB_, BOUND_>, fgrid, fblock, 0, st, rp, r_sb, W, bias, x, \
-                         xabs, fuse_bin ? scores : nullptr, bins, flags, status, B, V, G, edge_ulps, clamp, items, rpw); \
-    } while (0)
-#define GVCNN_LAUNCH_FAST_B(NB_)                                                                             \
-    do {                                                                                                     \
-        if (bound) GVCNN_LAUNCH_FAST(NB_, true); else GVCNN_LAUNCH_FAST(NB_, false);                         \
-    } while (0)
-        if (C == 8 * 32 * Elem<T>::kVec) GVCNN_LAUNCH_FAST_B(8); else GVCNN_LAUNCH_FAST_B(4);
-#undef GVCNN_LAUNCH_FAST_B
-#undef GVCNN_LAUNCH_FAST
-        if (err != cudaSuccess) return (int)err;
-        return (int)cudaGetLastError();
-    }
-    const dim3 grid((unsigned)((rows + kScoreWarps - 1) / kScoreWarps)), block(kScoreWarps * 32);
-#define GVCNN_LAUNCH_SCORE(VEC_, FUSE_, BOUND_)                                                       \
-    err = launch_pdl(view_score_kernel<T, VEC_, FUSE_, BOUND_>, grid, block, 0, st, rp, r_sb, W, bias, x, xabs, scores, \
-                     bins, flags, status, B, V, C, G, edge_ulps, clamp)
-#define GVCNN_LAUNCH_SCORE_B(VEC_, FUSE_)                                                             \
-    do {                                                                                              \
-        if (bound) GVCNN_LAUNCH_SCORE(VEC_, FUSE_, true); else GVCNN_LAUNCH_SCORE(VEC_, FUSE_, false); \
-    } while (0)
-    if (vec) {
-        if (fuse_bin) GVCNN_LAUNCH_SCORE_B(true, true); else GVCNN_LAUNCH_SCORE_B(true, false);
+        rc = with_flag(C == 8 * 32 * E, [&](auto nb8) {
+            return with_flag(bound, [&](auto bound_c) {
+                constexpr auto kern = view_score_fast_kernel<T, nb8 ? 8 : 4, bound_c>;
+                const int64_t warp_slots = (int64_t)sm_count() * resident_ctas<kern>(kScoreWarps * 32) * kScoreWarps;
+                int rpw = (int)(kFastRows * ((rows + kFastRows * warp_slots - 1) / (kFastRows * warp_slots)));
+                if (env_rpw >= kFastRows && env_rpw % kFastRows == 0) rpw = env_rpw;
+                const int64_t items = (int64_t)V * ((B + rpw - 1) / rpw);
+                const dim3 grid((unsigned)((items + kScoreWarps - 1) / kScoreWarps));
+                return (int)launch_pdl(kern, grid, block, 0, st, rp, r_sb, W, bias, x, xabs, fuse_bin ? scores : nullptr,
+                                       bins, flags, status, B, V, G, edge_ulps, clamp, items, rpw);
+            });
+        });
     } else {
-        if (fuse_bin) GVCNN_LAUNCH_SCORE_B(false, true); else GVCNN_LAUNCH_SCORE_B(false, false);
+        const dim3 grid((unsigned)((rows + kScoreWarps - 1) / kScoreWarps));
+        rc = with_flag(vec, [&](auto vec_c) {
+            return with_flag(fuse_bin, [&](auto fuse_c) {
+                return with_flag(bound, [&](auto bound_c) {
+                    return (int)launch_pdl(view_score_kernel<T, vec_c, fuse_c, bound_c>, grid, block, 0, st, rp, r_sb, W,
+                                           bias, x, xabs, scores, bins, flags, status, B, V, C, G, edge_ulps, clamp);
+                });
+            });
+        });
     }
-#undef GVCNN_LAUNCH_SCORE_B
-#undef GVCNN_LAUNCH_SCORE
-    if (err != cudaSuccess) return (int)err;
-    return (int)cudaGetLastError();
+    return rc ? rc : (int)cudaGetLastError();
 }
 
 int launch_view_score(const ViewPtrs &rp, int64_t r_sb, const float *W, const float *bias, float *x, float *xabs,
@@ -484,19 +455,13 @@ int launch_view_score(const ViewPtrs &rp, int64_t r_sb, const float *W, const fl
                       int G, int dtype, bool aligned16, bool fuse_bin, int edge_ulps, int clamp,
                       cudaStream_t st)
 {
-    if (dtype == GVCNN_F32) {
-        const bool vec = aligned16 && (C % 4 == 0) && ((reinterpret_cast<uintptr_t>(W) & 15) == 0);
-        return launch_view_score_t<float>(rp, r_sb, W, bias, x, xabs, scores, bins, flags, status, B, V, C, G, vec,
-                                          fuse_bin, edge_ulps, clamp, st);
-    }
-    const bool vec = aligned16 && (C % 8 == 0) && ((reinterpret_cast<uintptr_t>(W) & 15) == 0);
-    if (dtype == GVCNN_BF16)
-        return launch_view_score_t<__nv_bfloat16>(rp, r_sb, W, bias, x, xabs, scores, bins, flags, status, B, V, C, G,
-                                                  vec, fuse_bin, edge_ulps, clamp, st);
-    if (dtype == GVCNN_F16)
-        return launch_view_score_t<__half>(rp, r_sb, W, bias, x, xabs, scores, bins, flags, status, B, V, C, G, vec,
-                                           fuse_bin, edge_ulps, clamp, st);
-    return GVCNN_E_BAD_DTYPE;
+    static const int env_rpw = env_int_once("GVCNN_SCORE_RPW", 0);  // A/B knob: 4 = one butterfly per warp (round 1)
+    return with_dtype(dtype, [&](auto tag) {
+        using T = typename decltype(tag)::type;
+        const bool vec = aligned16 && (C % Elem<T>::kVec == 0) && ((reinterpret_cast<uintptr_t>(W) & 15) == 0);
+        return launch_view_score_t<T>(rp, r_sb, W, bias, x, xabs, scores, bins, flags, status, B, V, C, G, vec, fuse_bin,
+                                      edge_ulps, clamp, env_rpw, st);
+    });
 }
 
 int launch_batch_sum_x(const float *x, float *xsum, int B, int V, cudaStream_t st)
